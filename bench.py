@@ -48,6 +48,16 @@ def make_blob(n_elems: int, seed: int):
     return a.reshape(-1)
 
 
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """Each value is a run of 32-byte compressed G1 points; written as DIR/<name>.npy, float32 of shape (points, 32), one
+    byte per element (exact in float32), so the outputs of two builds compare element for element."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, raw in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.frombuffer(raw, dtype=np.uint8).reshape(-1, 32).astype(np.float32))
+
+
 class ClockSampler(threading.Thread):
     """SM clocks and throttle reasons DURING the timed region.  NVML in-process (nvidia_ml_py: the library nvidia-smi itself
     reads) when importable, the nvidia-smi binary otherwise -- a forked nvidia-smi costs ~0.15 CPU-seconds per call on an 8-GPU
@@ -208,7 +218,14 @@ def main():
                     help="c2 (default, headline): 16 MiB blobs; c3: 1024 x 2^16-Fr blobs sharded by blob; "
                          "c4: 2^26-point MSM sharded by point range; c5: batch-verify RLC over 4096 pairs")
     ap.add_argument("--log-n", type=int, default=0, help="override the problem size of c3/c4/c5")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="c2: write the last timed step's commitments and proofs (every rank's, in rank order; arkworks compressed) "
+                         "and the config-4 leg's point (gnark compressed) to DIR as float32 .npy files, one byte per element")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config != "c2"):
+        ap.error("--dump-outputs is implemented for the c2 configuration of the b200 implementation")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -332,10 +349,10 @@ def main():
 
         for _ in range(2):
             step16()
-        ms16, _ = timed(step16, 6)
+        ms16, _ = timed(step16, args.steps)
         assert cm16.raw == out_dev[0][: 32 * 16] and pf16.raw == out_dev[1][: 32 * 16]
-        batch16 = {"value": world * 16 * 6 / (ms16 * 1e-3), "unit": "blobs/s", "blobs_per_step_per_gpu": 16, "steps": 6,
-                   "ms_per_step": ms16 / 6}
+        batch16 = {"value": world * 16 * args.steps / (ms16 * 1e-3), "unit": "blobs/s", "blobs_per_step_per_gpu": 16,
+                   "steps": args.steps, "ms_per_step": ms16 / args.steps}
 
     # one blob alone through the same call (latency, not throughput): commit -> transcript hash -> proof
     one_ptr = (C.c_void_p * 1)(host_blobs[0].data_ptr())
@@ -349,6 +366,10 @@ def main():
         lat.append((time.perf_counter() - t0) * 1e3)
     single_blob_ms = min(lat[1:])
     assert cm1.raw == out_dev[0][:32] and pf1.raw == out_dev[1][:32]
+    outs_dev = [out_dev]
+    if args.dump_outputs and world > 1:
+        outs_dev = [None] * world
+        dist.all_gather_object(outs_dev, out_dev)
 
     if rank != 0:
         # the other ranks go straight to the config-4 leg (rank 0 joins after its single-GPU roofline measurements)
@@ -499,9 +520,15 @@ def main():
                                    "which overlaps the commitment MSM; GPU work is ~4.5 ms of it"},
     }
     print(json.dumps(line))
+    if args.dump_outputs:
+        outputs = {"commitments": b"".join(o[0] for o in outs_dev), "proofs": b"".join(o[1] for o in outs_dev)}
+        if msm_leg:
+            outputs["msm_leg_point"] = bytes.fromhex(msm_leg["result_gnark_be"])
+        dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
     main()

@@ -130,3 +130,27 @@ def test_bench_payload_blob_distribution():
     a, b = bench.make_blob(64, 7), bench.make_blob(64, 7)
     assert a.shape == (64 * 32,) and (a == b).all() and (a.reshape(64, 32)[:, 0] == 0).all()
     assert (bench.make_blob(64, 8) != a).any()
+
+
+def test_bench_dump_outputs_round_trip(tmp_path):
+    """--dump-outputs: every 32-byte point becomes one float32 row of its bytes, read back exactly."""
+    import numpy as np
+
+    import bench
+
+    raw = bytes(range(256)) * 3
+    bench.dump_outputs(str(tmp_path / "out"), {"commitments": raw, "proofs": raw[:32]})
+    got = np.load(tmp_path / "out" / "commitments.npy")
+    assert got.dtype == np.float32 and got.shape == (24, 32)
+    assert got.astype(np.uint8).tobytes() == raw
+    assert np.load(tmp_path / "out" / "proofs.npy").shape == (1, 32)
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--dump-outputs", "d", "--config", "c3"], ["--dump-outputs", "d", "--impl", "reference"]])
+def test_bench_rejects_arguments_it_cannot_honour(argv, tmp_path):
+    import subprocess
+    import sys
+
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, cwd=tmp_path, capture_output=True, text=True)
+    assert r.returncode == 2 and "error" in r.stderr
+    assert not (tmp_path / "d").exists()
