@@ -74,6 +74,15 @@ def g1_from_abi(xy: bytes, inf: Optional[bytes] = None) -> List[Affine]:
     return out
 
 
+def _blobs_to_abi(blobs: Sequence["Blob"]):
+    """The (blob pointers, lengths) arguments of the blob-batch calls, and the buffers the pointers point into: the
+    caller keeps those alive for the length of the call."""
+    keep = [C.create_string_buffer(b.blob_data, max(1, len(b.blob_data))) for b in blobs]
+    ptrs = (C.c_void_p * len(blobs))(*[C.cast(k, C.c_void_p).value for k in keep])
+    lens = (C.c_size_t * len(blobs))(*[len(b.blob_data) for b in blobs])
+    return keep, ptrs, lens
+
+
 def _next_pow2(n: int) -> int:
     return 1 if n <= 1 else 1 << (n - 1).bit_length()
 
@@ -185,9 +194,7 @@ class Group:
     # -- the sharded calls --------------------------------------------------------------
     def commit_and_prove_blobs(self, blobs: Sequence["Blob"]) -> Tuple[List[bytes], List[bytes]]:
         count = len(blobs)
-        keep = [C.create_string_buffer(b.blob_data, max(1, len(b.blob_data))) for b in blobs]
-        ptrs = (C.c_void_p * count)(*[C.cast(k, C.c_void_p).value for k in keep])
-        lens = (C.c_size_t * count)(*[len(b.blob_data) for b in blobs])
+        keep, ptrs, lens = _blobs_to_abi(blobs)  # keep: the buffers ptrs points into
         cs = C.create_string_buffer(32 * count if count else 1)
         ps = C.create_string_buffer(32 * count if count else 1)
         self.check(lib.kzgb_group_commit_and_prove_blobs(self.h, ptrs, lens, count, cs, ps))
@@ -578,9 +585,7 @@ class KZG:
         arkworks-compressed commitment and proof bytes."""
         e = srs.engine
         count = len(blobs)
-        keep = [C.create_string_buffer(b.blob_data, max(1, len(b.blob_data))) for b in blobs]
-        ptrs = (C.c_void_p * count)(*[C.cast(k, C.c_void_p).value for k in keep])
-        lens = (C.c_size_t * count)(*[len(b.blob_data) for b in blobs])
+        keep, ptrs, lens = _blobs_to_abi(blobs)  # keep: the buffers ptrs points into
         cs = C.create_string_buffer(32 * count if count else 1)
         ps = C.create_string_buffer(32 * count if count else 1)
         e.check(lib.kzgb_commit_and_prove_blobs(e.h, ptrs, lens, count, cs, ps))
@@ -644,9 +649,7 @@ def verify_blob_kzg_proof_batch_rlc(
         raise KzgError("GenericError", "length's of the input are not the same")
     e = engine or default_engine()
     count = len(blobs)
-    keep = [C.create_string_buffer(b.blob_data, max(1, len(b.blob_data))) for b in blobs]
-    ptrs = (C.c_void_p * count)(*[C.cast(k, C.c_void_p).value for k in keep])
-    lens = (C.c_size_t * count)(*[len(b.blob_data) for b in blobs])
+    keep, ptrs, lens = _blobs_to_abi(blobs)  # keep: the buffers ptrs points into
     cxy, cinf = g1_to_abi(commitments)
     pxy, pinf = g1_to_abi(proofs)
     lhs = C.create_string_buffer(64)

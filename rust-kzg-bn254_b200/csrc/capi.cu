@@ -1,4 +1,5 @@
-// Host orchestration and the C ABI (include/kzg_bn254_b200.h).
+// Host orchestration and the C ABI (include/kzg_bn254_b200.h): the context, its tables, the MSM plumbing, every
+// single-call entry point, the measurement hooks and the option table.  The blob-batch pipelines are in batch.cu.
 //
 // One context = one GPU.  The context owns the HBM-resident SRS (monomial points plus the
 // fixed-base window tables), the omega_N twiddle table, and a small set of "lanes": a lane is a
@@ -8,7 +9,6 @@
 // several times the GPU time of the same blob, so it must overlap).
 #include <algorithm>
 #include <chrono>
-#include <condition_variable>
 #include <cstdio>
 #include <cstring>
 #include <ctime>
@@ -16,140 +16,31 @@
 #include <string>
 #include <thread>
 #include <vector>
-#include <sys/resource.h>
-#include <sys/syscall.h>
-#include <unistd.h>
 
 #include "../../include/kzg_bn254_b200.h"
 #include "../../include/kzg_bn254_b200_bench.h"
+#include "ctx.hpp"
 #include "kzgb_internal.hpp"
 #include "sha256.hpp"
+#include "transcript.hpp"
 
-namespace kzgb {
-std::atomic<uint64_t> g_launch_count{0};
-}
 using namespace kzgb;
 
-namespace {
+namespace kzgb {
 
-constexpr int MAX_LANES = 8;
-constexpr int MAX_SETS = 96;
+std::atomic<uint64_t> g_launch_count{0};
 
-struct DevBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
-        size_t want = (bytes + (1u << 20) - 1) & ~(size_t)((1u << 20) - 1);
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
-};
-
-struct Lane {
-    cudaStream_t st = nullptr;      // everything but the bucket accumulation (high priority when owned)
-    cudaStream_t st_acc = nullptr;  // bucket accumulation: low priority, so other lanes' short kernels
-                                    // slip in between its blocks instead of queueing behind the whole grid
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    bool own_stream = false;
-    DevBuf bytes, evals, work, ntt_scratch, eval_scratch, msm_ws, small, bases, bucket_total;
-    XYZZ* h_sets = nullptr;   // pinned
-    uint32_t* h_entries = nullptr;  // pinned: length of the sorted list of the MSM in flight (= its point additions)
-    Fr* h_fr = nullptr;       // pinned, 16 elements
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_done = nullptr, ev_block = nullptr;
-    bool ev_pending = false;
-    double acc_ms = 0;        // summed duration of bucket-accumulation kernels
-    uint64_t acc_launches = 0;
-    uint64_t acc_adds = 0;    // sorted-list entries those kernels consumed (every entry is one point addition or install)
-};
-
-}  // namespace
-
-struct kzgb_ctx {
-    int device = 0;
-    std::mutex mu;
-    std::string err;
-    Lane lanes[MAX_LANES];
-    int n_lanes = 0;
-    // SRS
-    Affine* srs = nullptr;
-    size_t srs_n = 0;
-    Affine* wtable = nullptr;   // fixed-base window table over SRS points [wt_first, wt_first + wt_n)
-    size_t wt_first = 0, wt_n = 0;
-    int wt_c = 0, wt_W = 0;
-    bool auto_precompute = true;
-    std::atomic<bool> lanes_running{false};  // a batch pipeline is driving the lanes: tables are read-only
-    bool set_l2_limit = false;
-    // Lagrange-basis tables, one per domain size 2^k: window table over L = IFFT_G1(SRS[..2^k]) so that
-    // evaluation-form commitments are ONE MSM on the evaluations themselves (no Fr NTT on the path)
-    struct LagTable { Affine* table = nullptr; size_t n = 0; int c = 0, W = 0; uint64_t last_use = 0; uint32_t calls = 0; } lag[29];
-    uint64_t lag_clock = 0;
-    DevBuf batch_bytes;  // blob bytes of the batch in flight (commit_and_prove_blobs)
-    // twiddles
-    Fr* tw = nullptr;
-    int logN = 0;
-    // timer
-    cudaEvent_t t0 = nullptr, t1 = nullptr;
-    // device-side hashing of long Fiat-Shamir transcripts (fs.cu k_fs_midstate_long): its stream, the mapped host block the
-    // kernel reports through ([state 8 x cap | done cap | cancel 1] words) and the device-side argument arrays
-    cudaStream_t hash_st = nullptr;
-    cudaEvent_t ev_hash_uploaded = nullptr;
-    uint32_t* fsl_host = nullptr;
-    std::atomic<bool> lanes_block{false};  // lanes of the running large-blob batch sleep on a blocking event (lane_wait)
-    DevBuf fsl_args;
-    // upload stream + double-buffer fences of msm_srs_host_pipelined
-    cudaStream_t copy_st = nullptr;
-    cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr};
-    // timeline trace (kzgb_trace_begin / kzgb_trace_end, include/kzg_bn254_b200_bench.h): device events and host time
-    // stamps of every MSM of every lane, for reading pipeline stalls without a system profiler
-    struct TraceRec { int lane, kind; cudaEvent_t ev; double host_ms; };
-    std::atomic<bool> trace_on{false};
-    std::mutex trace_mu;
-    std::vector<TraceRec> trace;
-    cudaEvent_t trace_base = nullptr;
-    std::chrono::steady_clock::time_point trace_host0;
-};
-
-namespace {
-
-std::mutex g_err_mu;
-// -1: choose per call, 0: host SHA-256 pool, 1: device kernel (verify_batch_rlc challenges)
-std::atomic<int> g_fs_device{-1};
-// 1: evaluation-form commitments use a Lagrange-basis window table (built on first use per size), 0: Fr-IFFT + monomial table
-// -1: auto, 0: one blob at a time, > 0: blobs per group in the small-blob batch path
-std::atomic<int> g_group{-1};
-// points per chunk of the streamed SRS ingest (0 = 2^22); tests shrink it to cross chunk boundaries
-std::atomic<long> g_srs_chunk{0};
-std::atomic<int> g_group_members{1};  // largest kzgb_group alive in this process
-std::atomic<int> g_lagrange{1};
-std::atomic<int> g_lagrange_after{2};       // build the Lagrange table of a size at its k-th evaluation-form use
-std::atomic<long> g_lagrange_budget_mib{0}; // 0 = half of the device memory
-// kzgb_set_option knobs that used to be environment switches (0 / -1 = the library's own choice)
-std::atomic<int> g_lanes{0};            // lanes of the blob-batch pipelines
-std::atomic<int> g_hash_threads{0};     // host SHA-256 pool threads per batch call
-std::atomic<int> g_lane_wait{-1};       // -1 auto, 0 spin on the stream, 1 poll with short sleeps
-std::atomic<int> g_stream_priority{1};  // 1: bucket accumulation on a low-priority stream of its own
-std::atomic<int> g_l2_fetch_64{1};
-std::atomic<int> g_device_hash{-1};        // blobs of a large-blob batch whose transcript is hashed on the device: -1 auto, 0 none, k > 0 the last k
-std::atomic<int> g_hash_trace{0};         // option "hash_trace": 1 = every multi-buffer group reports its wall and CPU time on stderr
-std::atomic<int> g_hash_nice{1};          // 1: the SHA-256 pool threads of a batch call run at the lowest nice level
-std::atomic<int> g_hash_mb{-1};            // AVX-512 multi-buffer SHA-256 for deep large-blob batches: -1 auto, 0 never, 1 whenever a group of 16 forms
-std::atomic<int> g_pipelined_upload{1};   // 1: host scalars of MSMs of >= 2^22 points over a window table are uploaded in overlapped chunks
-std::atomic<long> g_batch_keep_mib{4096};  // blob staging buffer of kzgb_commit_and_prove_blobs kept between calls up to this size      // 1: contexts that own their stream set the L2 fetch granularity to 64 B
+static std::mutex g_err_mu;
 int fail(kzgb_ctx* c, int code, const std::string& msg) {
     if (c) { std::lock_guard<std::mutex> lk(g_err_mu); c->err = msg; }
     return code;
 }
-#define CK(ctx, call)                                                                              \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess)                                                                     \
-            return fail(ctx, KZGB_ERR_DEVICE, std::string("CUDA error: ") + cudaGetErrorString(e_) + " at " #call); \
-    } while (0)
+int check_srs_capacity(kzgb_ctx* c, size_t n) {
+    if (n <= c->srs_n) return KZGB_OK;
+    char msg[160];
+    snprintf(msg, sizeof msg, "SRS capacity exceeded: polynomial_len=%zu srs_len=%zu", n, c->srs_n);
+    return fail(c, KZGB_ERR_SRS_CAPACITY, msg);
+}
 
 // The MSM gathers 64-byte points at random from tables far larger than L2: with the default fetch granularity a
 // miss pulls the whole 128-byte line and doubles the DRAM traffic of the accumulation.  The limit is device-wide,
@@ -200,7 +91,7 @@ Fr ninv_mont(int logn) {
     return r;
 }
 // 1 / prod_i (z - w_i) with the zero factor (z = w_m) replaced by 1: prod = z^n - 1, or n / z in the domain
-Fr eval_tinv(const Fr& z, int logn, bool* in_domain = nullptr) {
+Fr eval_tinv(const Fr& z, int logn, bool* in_domain) {
     Fr zn = z, one, r;
     for (int k = 0; k < logn; k++) fe_sqr(zn, zn);
     fe_one(one);
@@ -208,23 +99,6 @@ Fr eval_tinv(const Fr& z, int logn, bool* in_domain = nullptr) {
     fe_sub(zn, zn, one);
     fe_inv(r, zn);
     return r;
-}
-// 32 big-endian bytes (any value) -> Fr Montgomery, reduced mod r
-Fr fr_from_be_bytes(const uint8_t* b) {
-    Fr a;
-    for (int k = 0; k < 8; k++)
-        a.l[7 - k] = ((uint32_t)b[4 * k] << 24) | ((uint32_t)b[4 * k + 1] << 16) | ((uint32_t)b[4 * k + 2] << 8) | b[4 * k + 3];
-    fe_to_mont(a, a);
-    return a;
-}
-template <int F>
-void fe_to_be_bytes(const Fe<F>& mont, uint8_t* out) {
-    Fe<F> c; fe_from_mont(c, mont);
-    for (int k = 0; k < 8; k++) {
-        uint32_t w = c.l[7 - k];
-        out[4 * k] = (uint8_t)(w >> 24); out[4 * k + 1] = (uint8_t)(w >> 16);
-        out[4 * k + 2] = (uint8_t)(w >> 8); out[4 * k + 3] = (uint8_t)w;
-    }
 }
 int log2_exact(size_t n) {
     int k = 0;
@@ -241,14 +115,6 @@ Affine affine_from_abi(const uint64_t xy[8], uint8_t inf) {
     Affine a;
     if (inf) aff_set_inf(a); else memcpy(&a, xy, 64);
     return a;
-}
-// arkworks serialize_compressed (reference primitives/src/helpers.rs:458-460)
-void serialize_compressed(const Affine& a, uint8_t out[32]) {
-    memset(out, 0, 32);
-    if (aff_is_inf(a)) { out[31] = 0x40; return; }
-    Fq xc; fe_from_mont(xc, a.x);
-    memcpy(out, xc.l, 32);
-    if (fe_lexicographically_largest(a.y)) out[31] |= 0x80;  // y > -y  <=>  y > (p-1)/2
 }
 void to_gnark_be(const Affine& a, uint8_t out[32]) {
     if (aff_is_inf(a)) { memset(out, 0, 32); out[0] = 0x40; return; }
@@ -450,7 +316,7 @@ void lagrange_release(kzgb_ctx* c) {
 // Fr-IFFT + monomial path, documented in include/kzg_bn254_b200.h.
 // Returns KZGB_OK with no table (t.table == nullptr) when the policy says "not yet", the feature is off or memory is short.
 // Called under the context lock, never while lane threads run.
-int ensure_lagrange(kzgb_ctx* c, int logn, uint32_t weight = 1, bool force = false) {
+int ensure_lagrange(kzgb_ctx* c, int logn, uint32_t weight, bool force) {
     if (logn < 1 || logn > 28) return KZGB_OK;
     kzgb_ctx::LagTable& t = c->lag[logn];
     t.last_use = ++c->lag_clock;
@@ -516,10 +382,26 @@ int srs_install(kzgb_ctx* c, Affine* dev_points, size_t n) {
 }
 
 // ---------------------------------------------------------------- MSM
-struct MsmJob {
-    MsmPlan plan;
-    bool active = false;
-};
+// Launch plan p on lane L in the lane's workspace and queue the copies of its window sums (and, for the statistics, of
+// the length of its sorted list) to the host; msm_finish picks them up.
+int msm_enqueue_plan(kzgb_ctx* c, Lane& L, const MsmPlan& p, const Fr* d_scalars, bool canonical, const Affine* table,
+                     MsmJob* job) {
+    CK(c, L.msm_ws.reserve(msm_workspace_bytes(p)));
+    MsmWorkspace ws;
+    msm_workspace_carve(p, L.msm_ws.p, &ws);
+    lane_collect_acc(L);
+    trace_mark(c, L, 0, L.st);
+    cudaEvent_t tr1 = trace_event(c, L, 1), tr2 = trace_event(c, L, 2);
+    msm_launch(p, ws, d_scalars, canonical, table, L.st, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1, L.st_acc, L.ev_fork, L.ev_join);
+    trace_mark(c, L, 3, L.st);
+    trace_mark(c, L, 10, nullptr);
+    L.ev_pending = !tr1;
+    CK(c, cudaMemcpyAsync(L.h_entries, ws.hist + p.nbuckets, 4, cudaMemcpyDeviceToHost, L.st));
+    CK(c, cudaMemcpyAsync(L.h_sets, ws.set_sums, sizeof(XYZZ) * p.sets, cudaMemcpyDeviceToHost, L.st));
+    job->plan = p;
+    job->active = true;
+    return KZGB_OK;
+}
 
 // Enqueue an MSM on lane L.  bases == nullptr: over the SRS range [first, first+n).
 // lag != nullptr: over the Lagrange-basis table of the domain of size n instead.
@@ -552,25 +434,25 @@ int msm_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_scalars, bool canonical, size_
         table = var_bases;
     }
     if ((uint64_t)n * p.W >= 0xfff00000ull) return fail(c, KZGB_ERR_GENERIC, "MSM too large for one launch");
-    CK(c, L.msm_ws.reserve(msm_workspace_bytes(p)));
-    MsmWorkspace ws;
-    msm_workspace_carve(p, L.msm_ws.p, &ws);
-    lane_collect_acc(L);
-    trace_mark(c, L, 0, L.st);
-    cudaEvent_t tr1 = trace_event(c, L, 1), tr2 = trace_event(c, L, 2);
-    msm_launch(p, ws, d_scalars, canonical, table, L.st, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1, L.st_acc, L.ev_fork, L.ev_join);
-    trace_mark(c, L, 3, L.st);
-    trace_mark(c, L, 10, nullptr);
-    L.ev_pending = !tr1;
-    CK(c, cudaMemcpyAsync(L.h_entries, ws.hist + p.nbuckets, 4, cudaMemcpyDeviceToHost, L.st));
-    CK(c, cudaMemcpyAsync(L.h_sets, ws.set_sums, sizeof(XYZZ) * p.sets, cudaMemcpyDeviceToHost, L.st));
-    job->plan = p;
-    job->active = true;
-    return KZGB_OK;
+    return msm_enqueue_plan(c, L, p, d_scalars, canonical, table, job);
 }
 
-bool lane_wait_polls();
-int lane_wait_mode();
+// 0: spin on the stream, 1: poll an event with short sleeps, 2: block on an event (option "lane_wait"; -1 = auto: spin
+// unless the lane threads of the ranks on this host outnumber half of its hardware threads, then poll)
+int lane_wait_mode() {
+    const int opt = g_lane_wait.load();
+    if (opt >= 0) return opt;
+    static int mode = -1;
+    if (mode < 0) {
+        unsigned hw = std::thread::hardware_concurrency();
+        int local = g_group_members.load();  // GPUs driven by this process (kzgb_group)
+        if (const char* w = getenv("LOCAL_WORLD_SIZE")) { int v = atoi(w); if (v > local) local = v; }  // torchrun: ranks on this host
+        mode = ((unsigned)local * 4u > hw / 2u) ? 1 : 0;
+    }
+    return mode;
+}
+bool lane_wait_polls() { return lane_wait_mode() != 0; }
+
 // Wait for everything queued on the lane.  Spinning by default (a blocking-sync event costs ~0.3 ms per
 // MSM in wake-up latency).  When the ranks on this host have more lane threads than spare cores, spinning
 // lanes starve the SHA-256 pool (8 GPUs x 4 lanes on 32 cores): poll with short sleeps instead.
@@ -691,21 +573,7 @@ int msm_enqueue_batched(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t n_per,
         table = c->wtable;
     }
     if ((uint64_t)n_per * batch * p.W >= 0xfff00000ull) return fail(c, KZGB_ERR_GENERIC, "MSM too large for one launch");
-    CK(c, L.msm_ws.reserve(msm_workspace_bytes(p)));
-    MsmWorkspace ws;
-    msm_workspace_carve(p, L.msm_ws.p, &ws);
-    lane_collect_acc(L);
-    trace_mark(c, L, 0, L.st);
-    cudaEvent_t tr1 = trace_event(c, L, 1), tr2 = trace_event(c, L, 2);
-    msm_launch(p, ws, d_scalars, false, table, L.st, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1, L.st_acc, L.ev_fork, L.ev_join);
-    trace_mark(c, L, 3, L.st);
-    trace_mark(c, L, 10, nullptr);
-    L.ev_pending = !tr1;
-    CK(c, cudaMemcpyAsync(L.h_entries, ws.hist + p.nbuckets, 4, cudaMemcpyDeviceToHost, L.st));
-    CK(c, cudaMemcpyAsync(L.h_sets, ws.set_sums, sizeof(XYZZ) * p.sets, cudaMemcpyDeviceToHost, L.st));
-    job->plan = p;
-    job->active = true;
-    return KZGB_OK;
+    return msm_enqueue_plan(c, L, p, d_scalars, false, table, job);
 }
 int msm_finish_batched(kzgb_ctx* c, Lane& L, const MsmJob& job, size_t batch, Affine* outs) {
     if (!job.active) { for (size_t k = 0; k < batch; k++) aff_set_inf(outs[k]); return KZGB_OK; }
@@ -757,85 +625,6 @@ int proof_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z
     return msm_enqueue(c, L, (Fr*)L.work.p, false, 0, n, nullptr, job);
 }
 
-// ---------------------------------------------------------------- Fiat-Shamir on the host
-const uint8_t FR_MOD_BE[32] = {0x30, 0x64, 0x4e, 0x72, 0xe1, 0x31, 0xa0, 0x29, 0xb8, 0x50, 0x45, 0xb6, 0x81, 0x81, 0x58, 0x5d,
-                               0x28, 0x33, 0xe8, 0x48, 0x79, 0xb9, 0x70, 0x91, 0x43, 0xe1, 0xf5, 0x93, 0xf0, 0x00, 0x00, 0x01};
-
-// Absorb tag || u64_be(n) || n canonical 32-byte evaluations (zero padded) -- everything of the
-// compute_challenge transcript (helpers.rs:424-456) except the trailing commitment.
-void challenge_midstate(Sha256& sh, const uint8_t* blob, size_t len, size_t n) {
-    static const char TAG[] = "EIGENDA_FSBLOBVERIFY_V1_";
-    sh.reset();
-    sh.update(TAG, 24);
-    uint8_t nb[8];
-    for (int i = 0; i < 8; i++) nb[i] = (uint8_t)((uint64_t)n >> (56 - 8 * i));
-    sh.update(nb, 8);
-    size_t full = len / 32;
-    size_t run_start = 0;
-    for (size_t i = 0; i < full; i++) {
-        const uint8_t* ch = blob + 32 * i;
-        if (ch[0] < 0x30 || memcmp(ch, FR_MOD_BE, 32) < 0) continue;  // canonical: hash in place
-        if (i > run_start) sh.update(blob + 32 * run_start, 32 * (i - run_start));
-        Fr v = fr_from_be_bytes(ch);  // to_fr_array reduces mod r (helpers.rs:32-34)
-        uint8_t red[32];
-        fe_to_be_bytes(v, red);
-        sh.update(red, 32);
-        run_start = i + 1;
-    }
-    if (full > run_start) sh.update(blob + 32 * run_start, 32 * (full - run_start));
-    size_t done = full;
-    if (len % 32) {  // trailing partial chunk, right-padded with zeros (helpers.rs:47-51)
-        uint8_t last[32];
-        memset(last, 0, 32);
-        memcpy(last, blob + 32 * full, len % 32);
-        Fr v = fr_from_be_bytes(last);
-        uint8_t red[32];
-        fe_to_be_bytes(v, red);
-        sh.update(red, 32);
-        done++;
-    }
-    static const uint8_t zeros[4096] = {0};
-    size_t pad = (n - done) * 32;
-    while (pad) { size_t t = pad < sizeof(zeros) ? pad : sizeof(zeros); sh.update(zeros, t); pad -= t; }
-}
-Fr challenge_finish(Sha256 sh, const Affine& commitment) {
-    uint8_t cb[32], dg[32];
-    serialize_compressed(commitment, cb);
-    sh.update(cb, 32);
-    sh.finish(dg);
-    return fr_from_be_bytes(dg);  // hash_to_field_element (helpers.rs:382-390)
-}
-
-// 0: spin on the stream, 1: poll an event with short sleeps, 2: block on an event (option "lane_wait"; -1 = auto: spin
-// unless the lane threads of the ranks on this host outnumber half of its hardware threads, then poll)
-int lane_wait_mode() {
-    const int opt = g_lane_wait.load();
-    if (opt >= 0) return opt;
-    static int mode = -1;
-    if (mode < 0) {
-        unsigned hw = std::thread::hardware_concurrency();
-        int local = g_group_members.load();  // GPUs driven by this process (kzgb_group)
-        if (const char* w = getenv("LOCAL_WORLD_SIZE")) { int v = atoi(w); if (v > local) local = v; }  // torchrun: ranks on this host
-        mode = ((unsigned)local * 4u > hw / 2u) ? 1 : 0;
-    }
-    return mode;
-}
-bool lane_wait_polls() { return lane_wait_mode() != 0; }
-
-// Host threads for the SHA-256 pool of one context.  One transcript hash is sequential (~9 ms per 16 MiB
-// with SHA-NI).  Measured on the 8-GPU box (32 hardware threads): one thread per blob, even
-// oversubscribed, beats a pool sized to this rank's share of the cores (1545 vs 1222 blobs/s) -- at
-// 8 GPUs the job is bound by the host's aggregate SHA-256 rate (2.1 GB of transcripts per step).
-size_t hash_pool_threads() {
-    if (int v = g_hash_threads.load()) return (size_t)v;
-    unsigned hw = std::thread::hardware_concurrency();
-    if (hw == 0) hw = 8;
-    size_t pool = std::min<size_t>(hw > 4 ? hw - 2 : 2, 32);
-    // the members of a kzgb_group hash at the same time: share the cores (ranks of a torchrun job are separate
-    // processes; measured there, one thread per blob even oversubscribed beats a share of the cores)
-    size_t members = (size_t)std::max(1, g_group_members.load());
-    return std::max<size_t>(2, pool / members);
-}
 
 size_t blob_poly_len(size_t len) { return next_pow2((len + 31) / 32); }  // Rust: 0usize.next_power_of_two() == 1
 
@@ -852,13 +641,6 @@ int blob_to_evals(kzgb_ctx* c, Lane& L, const uint8_t* blob_host, const uint8_t*
     return KZGB_OK;
 }
 
-struct Guard {
-    kzgb_ctx* c;
-    int prev = -1;
-    std::unique_lock<std::mutex> lk;
-    explicit Guard(kzgb_ctx* ctx) : c(ctx), lk(ctx->mu) { cudaGetDevice(&prev); cudaSetDevice(ctx->device); }
-    ~Guard() { if (prev >= 0) cudaSetDevice(prev); }
-};
 
 // Streamed ingest of `n` compressed points: `read(dst, first, count)` fills a pinned staging buffer with
 // points [first, first+count); the read of chunk k+1 overlaps the H2D copy and the decompression kernel of
@@ -1166,11 +948,7 @@ int kzgb_srs_precompute_range(kzgb_ctx* c, size_t first, size_t count, int windo
 int kzgb_srs_prepare_lagrange(kzgb_ctx* c, size_t n) {
     Guard g(c);
     if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_FFT, "length provided is not a power of 2");
-    if (n > c->srs_n) {
-        char msg[160];
-        snprintf(msg, sizeof msg, "SRS capacity exceeded: polynomial_len=%zu srs_len=%zu", n, c->srs_n);
-        return fail(c, KZGB_ERR_SRS_CAPACITY, msg);
-    }
+    if (int rc = check_srs_capacity(c, n)) return rc;
     int logn = log2_exact(n);
     int rc = ensure_lagrange(c, logn, 1, true);
     if (rc) return rc;
@@ -1343,11 +1121,7 @@ static int commit_evals_host(kzgb_ctx* c, const uint64_t* evals, size_t n, uint6
 
 int kzgb_commit_eval(kzgb_ctx* c, const uint64_t* evals, size_t n, uint64_t out_xy[8], uint8_t* out_inf) {
     Guard g(c);
-    if (n > c->srs_n) {  // kzg.rs:89-94
-        char msg[160];
-        snprintf(msg, sizeof msg, "SRS capacity exceeded: polynomial_len=%zu srs_len=%zu", n, c->srs_n);
-        return fail(c, KZGB_ERR_SRS_CAPACITY, msg);
-    }
+    if (int rc = check_srs_capacity(c, n)) return rc;  // kzg.rs:89-94
     if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_FFT, "length provided is not a power of 2");  // kzg.rs:265-269
     int rc = ensure_lagrange(c, log2_exact(n));
     if (rc) return rc;
@@ -1364,11 +1138,7 @@ int kzgb_commit_blob(kzgb_ctx* c, const uint8_t* blob, size_t len, uint64_t out_
     Lane& L = c->lanes[0];
     size_t n = blob_poly_len(len);
     if (n > ((size_t)1 << 28)) return fail(c, KZGB_ERR_GENERIC, "Input size exceeds maximum polynomial size");
-    if (n > c->srs_n) {
-        char msg[160];
-        snprintf(msg, sizeof msg, "SRS capacity exceeded: polynomial_len=%zu srs_len=%zu", n, c->srs_n);
-        return fail(c, KZGB_ERR_SRS_CAPACITY, msg);
-    }
+    if (int rc = check_srs_capacity(c, n)) return rc;
     int rc = ensure_lagrange(c, log2_exact(n));
     if (rc) return rc;
     rc = blob_to_evals(c, L, blob, nullptr, len, n);
@@ -1390,11 +1160,7 @@ int kzgb_g1_ifft(kzgb_ctx* c, size_t n, uint64_t* out_xy, uint8_t* out_inf) {
     if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_FFT, "length provided is not a power of 2");
     Guard g(c);
     Lane& L = c->lanes[0];
-    if (n > c->srs_n) {
-        char msg[160];
-        snprintf(msg, sizeof msg, "SRS capacity exceeded: polynomial_len=%zu srs_len=%zu", n, c->srs_n);
-        return fail(c, KZGB_ERR_SRS_CAPACITY, msg);
-    }
+    if (int rc = check_srs_capacity(c, n)) return rc;
     if (n > ((size_t)1 << 28)) return fail(c, KZGB_ERR_GENERIC, "power must be <= 28");
     int logn = log2_exact(n);
     int rc = ensure_twiddles(c, logn);
@@ -1418,11 +1184,7 @@ int kzgb_compute_proof(kzgb_ctx* c, const uint64_t* evals, size_t n, const uint6
     Guard g(c);
     Lane& L = c->lanes[0];
     if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_FFT, "length provided is not a power of 2");
-    if (n > c->srs_n) {
-        char msg[160];
-        snprintf(msg, sizeof msg, "SRS capacity exceeded: polynomial_len=%zu srs_len=%zu", n, c->srs_n);
-        return fail(c, KZGB_ERR_SRS_CAPACITY, msg);
-    }
+    if (int rc = check_srs_capacity(c, n)) return rc;
     int rc = ensure_lagrange(c, log2_exact(n));
     if (rc) return rc;
     CK(c, L.evals.reserve(n * sizeof(Fr)));
@@ -1487,11 +1249,7 @@ int kzgb_compute_blob_proof(kzgb_ctx* c, const uint8_t* blob, size_t len, const 
     if (!aff_on_curve(C)) return fail(c, KZGB_ERR_NOT_ON_CURVE, "G1 point not on curve");  // helpers.rs:694-699
     size_t n = blob_poly_len(len);
     if (len == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");  // helpers.rs:554-558 via :482
-    if (n > c->srs_n) {
-        char msg[160];
-        snprintf(msg, sizeof msg, "SRS capacity exceeded: polynomial_len=%zu srs_len=%zu", n, c->srs_n);
-        return fail(c, KZGB_ERR_SRS_CAPACITY, msg);
-    }
+    if (int rc = check_srs_capacity(c, n)) return rc;
     int rc = ensure_lagrange(c, log2_exact(n));
     if (rc) return rc;
     rc = blob_to_evals(c, L, blob, nullptr, len, n);  // H2D + conversion run while the host hashes
@@ -1580,686 +1338,6 @@ int kzgb_verify_blob_proof_g1(kzgb_ctx* c, const uint8_t* blob, size_t len, cons
     return kzgb_verify_proof_g1(c, c_xy, c_inf, proof_xy, proof_inf, (const uint64_t*)y.l, out_xy, out_inf);
 }
 
-// ------------------------------------------------------------------------------- blob batches
-constexpr size_t FSL_CAP = 4096;  // transcripts one batch call can hand to the device
-// Who hashes the Fiat-Shamir transcripts of a large-blob batch (everything but the commitment: challenge_midstate).
-//  * single stream: one SHA-NI thread per blob, ~9 ms per 16 MiB, the first challenges ready after 9 ms -- the default
-//    whenever the pool keeps up with the GPU (16 spare cores next to one GPU: 29 GB/s against 6 GB/s of blobs);
-//  * multi-buffer: groups of 16 equal-size blobs hashed in lockstep on AVX-512 (sha256_mb16_blocks), about twice the bytes
-//    per second of a core, the 16 midstates arrive together (71-80 ms for 16 MiB blobs) -- for deep batches on a host
-//    whose single-stream pool is slower than the GPU (8 ranks on 32 hardware threads: 36 GB/s against 49 GB/s;
-//    profiles/r02_scale8.txt: 2184 -> 2857 blobs/s);
-//  * device: the last k blobs on the GPU next to the MSMs, one warp (0.45 s, 16 % of a blob's MSM work in issue slots) or
-//    one lane (0.9 s: a warp instruction occupies the 16-wide integer ALU for two cycles and the lane does schedule and
-//    rounds alone; half a percent) per transcript -- only a batch several hundred blobs deep hides that latency.
-struct HashPlan {
-    bool mb = false;        // multi-buffer groups on the host
-    size_t mb_threads = 0;  // host threads in multi-buffer mode
-    size_t dev_k = 0;       // transcripts hashed on the device (the last dev_k blobs)
-    bool dev_lanes = false; // k_fs_midstate_lanes instead of k_fs_midstate_long
-};
-bool hash_mb_eligible(size_t len) { const size_t n = len / 32; return len % 32 == 0 && n >= 1024 && (n & (n - 1)) == 0; }
-HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible) {
-    HashPlan hp;
-    if (count < 2) return hp;
-    double bytes = 0;
-    for (size_t i = 0; i < count; i++) bytes += (double)lens[i];
-    const double per_blob = bytes / (double)count;
-    unsigned hw = std::thread::hardware_concurrency();
-    if (hw == 0) hw = 8;
-    int procs = g_group_members.load();
-    if (const char* w = getenv("LOCAL_WORLD_SIZE")) { int v = atoi(w); if (v > procs) procs = v; }
-    const double share = std::max(1.0, (double)hw / procs);                                          // hardware threads of this context
-    const double rate_ni = 1.2e9 * std::max(1.0, std::min<double>((double)hash_pool_threads(), share));  // B/s, HT siblings both hashing
-    const double t_gpu = 2.75e-3 * per_blob / (double)(16u << 20);  // commit + proof of one blob
-    // eligible blobs: exactly 32 * 2^j bytes, j >= 10 (the multi-buffer and device kernels hash whole 64-byte blocks)
-    size_t eligible_total = 0, eligible_tail = 0;
-    for (size_t i = 0; i < count; i++) eligible_total += hash_mb_eligible(lens[i]);
-    while (eligible_tail < count && eligible_tail < FSL_CAP && hash_mb_eligible(lens[count - 1 - eligible_tail])) eligible_tail++;
-    const int mb_opt = g_hash_mb.load();
-    // "keeps up" = the single-stream pool needs at most half of this context's hardware threads for the duration of the GPU work:
-    // the other half belongs to the lanes and the driver (measured on 4 hardware threads per rank: 291 blobs/s single stream, 367 multi-buffer)
-    const bool ni_keeps_up = bytes / rate_ni <= 0.5 * count * t_gpu;
-    if (sha256_has_mb16() && mb_opt != 0 && eligible_total >= 16 && (mb_opt == 1 || (!ni_keeps_up && eligible_total >= 32))) {
-        hp.mb = true;
-        const int ht = g_hash_threads.load();
-        hp.mb_threads = (size_t)std::max(1.0, ht > 0 ? (double)ht : share - 1.0);  // one hardware thread of the share stays with the lanes
-    }
-    const int dev_opt = device_possible ? g_device_hash.load() : 0;
-    if (dev_opt > 0) { hp.dev_k = std::min<size_t>((size_t)dev_opt, eligible_tail); hp.dev_lanes = fs_midstate_lanes() != 0; return hp; }
-    if (dev_opt == 0 || !eligible_tail) return hp;
-    const double rate_host = hp.mb ? 2.4e9 * (double)hp.mb_threads : rate_ni;
-    double best = std::max(count * t_gpu, bytes / rate_host);
-    for (int lanes = 0; lanes < 2; lanes++) {
-        if (fs_midstate_lanes() >= 0 && lanes != fs_midstate_lanes()) continue;
-        const double t_dev = (lanes ? 0.95 : 0.45) * per_blob / (double)(16u << 20), dev_cost = lanes ? 0.006 : 0.16;
-        for (size_t k = 1; k <= eligible_tail; k++) {
-            // GPU busy time; host time for the front of the batch; the device's share lands at t_dev and its proofs follow
-            const double t = std::max({(count + dev_cost * k) * t_gpu, (double)(count - k) * per_blob / rate_host, t_dev + k * t_gpu * 0.5});
-            if (t < best * 0.97) { best = t; hp.dev_k = k; hp.dev_lanes = lanes != 0; }
-        }
-    }
-    return hp;
-}
-// a 32-byte big-endian value >= r inside a transcript block -> its canonical residue (to_fr_array, helpers.rs:32-34)
-void hash_fix_block(uint8_t block[64]) {
-    for (int h = 0; h < 64; h += 32) {
-        uint8_t* ch = block + h;
-        if (ch[0] < 0x30 || memcmp(ch, FR_MOD_BE, 32) < 0) continue;
-        Fr v = fr_from_be_bytes(ch);
-        fe_to_be_bytes(v, ch);
-    }
-}
-// Midstates of up to 16 blobs of exactly 32 n bytes each after tag || u64_be(n) || chunks 0 .. n-2 (all whole blocks),
-// hashed in lockstep; out[m] = 8 state words.  Unused slots repeat blob 0.
-void challenge_midstates_mb16(const uint8_t* const* blobs, size_t members, size_t n, uint32_t out[16][8]) {
-    static const uint32_t iv[8] = {0x6a09e667, 0xbb67ae85, 0x3c6ef372, 0xa54ff53a, 0x510e527f, 0x9b05688c, 0x1f83d9ab, 0x5be0cd19};
-    alignas(64) uint8_t first[16][64];
-    const uint8_t* p[16];
-    for (size_t m = 0; m < 16; m++) {
-        const uint8_t* blob = blobs[m < members ? m : 0];
-        memcpy(first[m], "EIGENDA_FSBLOBVERIFY_V1_", 24);
-        for (int i = 0; i < 8; i++) first[m][24 + i] = (uint8_t)((uint64_t)n >> (56 - 8 * i));
-        memcpy(first[m] + 32, blob, 32);
-        if (first[m][32] >= 0x30 && memcmp(first[m] + 32, FR_MOD_BE, 32) >= 0) { Fr v = fr_from_be_bytes(first[m] + 32); fe_to_be_bytes(v, first[m] + 32); }
-        memcpy(out[m], iv, 32);
-        p[m] = first[m];
-    }
-    sha256_mb16_blocks(out, p, 1, nullptr);
-    for (size_t m = 0; m < 16; m++) p[m] = blobs[m < members ? m : 0] + 32;  // block b >= 1 holds chunks 2b - 1, 2b
-    sha256_mb16_blocks(out, p, n / 2 - 1, hash_fix_block);
-}
-
-static int batch_impl(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
-                      size_t count, uint8_t* commitments32, uint8_t* proofs32) {
-    if (count == 0) return KZGB_OK;
-    size_t max_n = 0;
-    for (size_t i = 0; i < count; i++) {
-        size_t n = blob_poly_len(lens[i]);
-        if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
-        if (n > c->srs_n) {
-            char msg[160];
-            snprintf(msg, sizeof msg, "SRS capacity exceeded: polynomial_len=%zu srs_len=%zu", n, c->srs_n);
-            return fail(c, KZGB_ERR_SRS_CAPACITY, msg);
-        }
-        max_n = std::max(max_n, n);
-    }
-    // Small blobs (<= 2^17 Fr): runs of equal-size blobs are processed as groups, every kernel of a phase
-    // launched ONCE for the whole group (batched conversion, evaluation/quotient and MSM with one bucket set
-    // per blob) -- one blob at a time they are latency-bound (bucket-reduction tail, host hand-off per MSM).
-    const int group_opt = g_group.load();
-    std::vector<std::pair<size_t, size_t>> groups;  // (first blob, blobs)
-    if (group_opt != 0 && count >= 2 && max_n <= ((size_t)1 << 17) && c->auto_precompute && c->srs_n <= ((size_t)1 << 22)) {
-        for (size_t i = 0; i < count;) {
-            size_t n = blob_poly_len(lens[i]);
-            size_t cap = group_opt > 0 ? (size_t)group_opt : std::max<size_t>(1, ((size_t)1 << 21) / n);
-            cap = std::min<size_t>(cap, 64);
-            size_t j = i + 1;
-            while (j < count && j - i < cap && blob_poly_len(lens[j]) == n) j++;
-            groups.emplace_back(i, j - i);
-            i = j;
-        }
-    }
-    // lanes in flight: 3 keep the GPU full on 16 MiB blobs; small blobs are latency-bound per lane
-    // (bucket reduction, host hand-offs), so they get more
-    // Large-blob batches: 6 lanes whose threads SLEEP on a blocking event while their MSM runs (measured against 4 spinning
-    // lanes: 342 -> 353 blobs/s e2e with 16 hardware threads, and the only form that leaves a rank of the 8-GPU box -- 4
-    // hardware threads -- its cores for hashing: profiles/r02_host_hashing.txt, r02_scale8.txt).  The wake-up latency of a blocking event (~0.1-0.3 ms) hides
-    // behind the other lanes; single calls and the latency-bound small-blob groups keep spinning.
-    const int lanes_env = g_lanes.load();
-    // (a rank short of cores -- lane_wait auto = poll -- with a shallow batch is the exception: 4 polling lanes, measured 316
-    // against 288 blobs/s at 16 blobs per step on 4 hardware threads)
-    const bool deep = groups.empty() && count >= 4 && (count >= 32 || !lane_wait_polls());
-    int want_lanes = lanes_env > 0 ? lanes_env : (deep ? 6 : (max_n >= ((size_t)1 << 18) ? 4 : 6));
-    if (!groups.empty() && lanes_env <= 0) want_lanes = 3;
-    struct LanesBlock {
-        kzgb_ctx* c;
-        LanesBlock(kzgb_ctx* ctx, bool on) : c(ctx) { c->lanes_block.store(on); }
-        ~LanesBlock() { c->lanes_block.store(false); }
-    } lanes_block(c, deep);
-    int n_lanes = (int)std::min<size_t>(groups.empty() ? count : groups.size(), (size_t)std::min(want_lanes, MAX_LANES));
-    int rc = ensure_lanes(c, n_lanes);
-    if (rc) return rc;
-    rc = ensure_twiddles(c, log2_exact(max_n));
-    if (rc) return rc;
-    bool all_lagrange = true;
-    for (size_t i = 0; i < count; i++) {
-        int logn = log2_exact(blob_poly_len(lens[i]));
-        rc = ensure_lagrange(c, logn);
-        if (rc) return rc;
-        if (!c->lag[logn].table) all_lagrange = false;
-    }
-    if (!all_lagrange && c->auto_precompute && (!c->wtable || c->wt_first != 0 || max_n > c->wt_n) && c->srs_n <= ((size_t)1 << 22)) {
-        rc = do_precompute(c, 0, std::min(c->srs_n, next_pow2(max_n)), 0);
-        if (rc && rc != KZGB_ERR_DEVICE) return rc;
-    }
-    for (size_t gi = 0; gi < groups.size(); gi++) {  // the batched MSM needs a window table for every size
-        size_t n = blob_poly_len(lens[groups[gi].first]);
-        int logn = log2_exact(n);
-        bool lag_ok = c->lag[logn].table && g_lagrange.load();
-        if (!lag_ok && !(c->wtable && c->wt_first == 0 && n <= c->wt_n)) { groups.clear(); break; }
-    }
-
-    // Blob bytes stay resident on the device between a blob's commit and its proof (one H2D per blob).
-    std::vector<size_t> byte_off(count, 0);
-    bool resident = false;
-    if (!blobs_dev && groups.empty()) {
-        size_t total = 0;
-        for (size_t i = 0; i < count; i++) { byte_off[i] = total; total += (lens[i] + 255) & ~(size_t)255; }
-        if (total <= ((size_t)16 << 30) && c->batch_bytes.reserve(total) == cudaSuccess) resident = true;
-        else cudaGetLastError();
-    }
-
-    // Transcript midstates (everything but the commitment): a pool of host threads from the front of the batch and, when
-    // the host cannot keep up with the GPU, one warp per transcript on the device for the blobs at its end
-    // (device_hash_share).  Whoever delivers a midstate first installs it; the lanes take proofs as they become ready.
-    std::vector<Sha256> mid(count);
-    std::vector<uint8_t> ready(count, 0);
-    std::mutex mu;
-    std::condition_variable cv;
-    bool failed = false;
-    const HashPlan hplan = groups.empty() ? hash_plan(lens, count, blobs_dev || resident) : HashPlan();
-    const size_t dev_k = hplan.dev_k;
-    const size_t dev_first = count - dev_k;
-    std::atomic<bool> dev_failed{false}, dev_stop{false};
-    volatile uint32_t* fsl_done = nullptr;
-    uint32_t* fsl_state = nullptr;
-    volatile uint32_t* fsl_cancel = nullptr;
-    if (dev_k) {
-        cudaError_t e = cudaSuccess;
-        if (!c->hash_st) {
-            int lo = 0, hi = 0;
-            cudaDeviceGetStreamPriorityRange(&lo, &hi);
-            e = cudaStreamCreateWithPriority(&c->hash_st, cudaStreamNonBlocking, hi);  // its few blocks must become resident at once
-            if (e == cudaSuccess) e = cudaEventCreateWithFlags(&c->ev_hash_uploaded, cudaEventDisableTiming);
-            if (e == cudaSuccess) e = cudaHostAlloc((void**)&c->fsl_host, (9 * FSL_CAP + 16) * 4, cudaHostAllocMapped);
-        }
-        if (e == cudaSuccess) e = c->fsl_args.reserve(FSL_CAP * 16);
-        if (e == cudaSuccess) {
-            fsl_state = c->fsl_host;
-            fsl_done = c->fsl_host + 8 * FSL_CAP;
-            fsl_cancel = c->fsl_host + 9 * FSL_CAP;
-            for (size_t j = 0; j < dev_k; j++) fsl_done[j] = 0;
-            *fsl_cancel = 0;
-            std::vector<const uint8_t*> ptrs(dev_k);
-            std::vector<uint32_t> ns(dev_k);
-            for (size_t j = 0; j < dev_k && e == cudaSuccess; j++) {
-                const size_t i = dev_first + j;
-                ns[j] = (uint32_t)(lens[i] / 32);
-                if (blobs_dev) ptrs[j] = blobs_dev[i];
-                else {  // host blobs: the device's share goes up first, on the hashing stream
-                    uint8_t* slot = (uint8_t*)c->batch_bytes.p + byte_off[i];
-                    e = cudaMemcpyAsync(slot, blobs_host[i], lens[i], cudaMemcpyHostToDevice, c->hash_st);
-                    ptrs[j] = slot;
-                }
-            }
-            const uint8_t** d_ptrs = (const uint8_t**)c->fsl_args.p;
-            uint32_t* d_ns = (uint32_t*)((char*)c->fsl_args.p + FSL_CAP * 8);
-            if (e == cudaSuccess) e = cudaEventRecord(c->ev_hash_uploaded, c->hash_st);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(d_ptrs, ptrs.data(), dev_k * 8, cudaMemcpyHostToDevice, c->hash_st);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(d_ns, ns.data(), dev_k * 4, cudaMemcpyHostToDevice, c->hash_st);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(c->hash_st);  // the argument vectors die with this scope
-            if (e == cudaSuccess) {
-                fs_midstate_long_launch(d_ptrs, d_ns, (uint32_t)dev_k, fsl_state, (uint32_t*)fsl_done, (const uint32_t*)fsl_cancel, hplan.dev_lanes, c->hash_st);
-                e = cudaGetLastError();
-            }
-        }
-        if (e != cudaSuccess) { cudaGetLastError(); dev_failed.store(true); }  // the host pool takes the whole batch
-    }
-    // the last 32-byte chunk of a blob of exactly 32 n bytes, reduced mod r as to_fr_array does
-    auto install_device_midstate = [&](size_t i, const uint32_t* st) {
-        const size_t n = lens[i] / 32;
-        Sha256 sh;
-        sh.reset();
-        memcpy(sh.h, st, 32);
-        sh.total = 32 * (uint64_t)n;  // tag (24) + u64 (8) + chunks 0 .. n-2
-        const uint8_t* ch = blobs_host[i] + 32 * (n - 1);
-        if (ch[0] < 0x30 || memcmp(ch, FR_MOD_BE, 32) < 0) sh.update(ch, 32);
-        else { Fr v = fr_from_be_bytes(ch); uint8_t red[32]; fe_to_be_bytes(v, red); sh.update(red, 32); }
-        std::lock_guard<std::mutex> lk(mu);
-        if (!ready[i]) { mid[i] = sh; ready[i] = 1; }
-    };
-    std::thread dev_poller;
-    if (dev_k && !dev_failed.load()) {
-        dev_poller = std::thread([&]() {
-            std::vector<uint8_t> seen(dev_k, 0);
-            size_t remaining = dev_k;
-            while (remaining && !dev_stop.load()) {
-                bool any = false;
-                for (size_t j = 0; j < dev_k; j++) {
-                    if (seen[j] || !fsl_done[j]) continue;
-                    std::atomic_thread_fence(std::memory_order_acquire);
-                    uint32_t st[8];
-                    for (int w = 0; w < 8; w++) st[w] = fsl_state[8 * j + w];
-                    install_device_midstate(dev_first + j, st);
-                    seen[j] = 1; remaining--; any = true;
-                }
-                if (any) cv.notify_all();
-                else { struct timespec ts = {0, 100000}; nanosleep(&ts, nullptr); }
-            }
-        });
-    }
-    // Hash tasks in blob order: one blob on a single stream, or a group of up to 16 equal-size blobs in lockstep.
-    struct HashTask { size_t first, members; };
-    std::vector<HashTask> tasks;
-    for (size_t i = 0; i < count;) {
-        size_t j = i + 1;
-        if (hplan.mb && i < dev_first && hash_mb_eligible(lens[i])) {
-            while (j < dev_first && j - i < 16 && lens[j] == lens[i]) j++;
-            if (j - i < 8) j = i + 1;  // a group under half full hashes no faster than its members one by one
-        }
-        tasks.push_back({i, j - i});
-        i = j;
-    }
-    std::atomic<size_t> next_hash{0};
-    size_t n_hash = std::max<size_t>(1, std::min<size_t>(tasks.size(), hplan.mb ? hplan.mb_threads : hash_pool_threads()));
-    std::vector<std::thread> hashers;
-    for (size_t t = 0; t < n_hash; t++) {
-        hashers.emplace_back([&]() {
-            // The pool is pure throughput work; the lane threads next to it are latency work (every microsecond a lane
-            // wakes up late is a microsecond its stream may run dry).  Where both share a few cores (8 ranks on 32
-            // hardware threads) the hashers yield to them: lowest nice level for this thread only.
-            if (g_hash_nice.load()) setpriority(PRIO_PROCESS, (id_t)syscall(SYS_gettid), 19);
-            for (;;) {
-                size_t ti = next_hash.fetch_add(1);
-                if (ti >= tasks.size()) return;
-                const size_t i = tasks[ti].first, members = tasks[ti].members;
-                if (members > 1) {
-                    uint32_t st[16][8];
-                    struct timespec w0, w1, c0, c1;
-                    const bool trace = g_hash_trace.load() != 0;
-                    if (trace) { clock_gettime(CLOCK_MONOTONIC, &w0); clock_gettime(CLOCK_THREAD_CPUTIME_ID, &c0); }
-                    challenge_midstates_mb16(blobs_host + i, members, lens[i] / 32, st);
-                    if (trace) {  // option "hash_trace": wall and CPU time of the group -- tells a descheduled pool from a slow one
-                        clock_gettime(CLOCK_MONOTONIC, &w1); clock_gettime(CLOCK_THREAD_CPUTIME_ID, &c1);
-                        fprintf(stderr, "[hash] group at blob %zu (%zu members): wall %.1f ms, cpu %.1f ms\n", i, members,
-                                (w1.tv_sec - w0.tv_sec) * 1e3 + (w1.tv_nsec - w0.tv_nsec) * 1e-6, (c1.tv_sec - c0.tv_sec) * 1e3 + (c1.tv_nsec - c0.tv_nsec) * 1e-6);
-                    }
-                    for (size_t m = 0; m < members; m++) install_device_midstate(i + m, st[m]);
-                    cv.notify_all();
-                    continue;
-                }
-                if (i >= dev_first) {  // the device's share: only if the device path failed
-                    std::unique_lock<std::mutex> lk(mu);
-                    cv.wait(lk, [&] { return ready[i] != 0 || failed || dev_failed.load() || dev_stop.load(); });
-                    if (ready[i] || failed || dev_stop.load()) continue;
-                }
-                Sha256 sh;
-                challenge_midstate(sh, blobs_host[i], lens[i], blob_poly_len(lens[i]));
-                { std::lock_guard<std::mutex> lk(mu); if (!ready[i]) { mid[i] = sh; ready[i] = 1; } }
-                cv.notify_all();
-            }
-        });
-    }
-    // every exit path below: stop the device hashing, then wait for it (it reads the blob bytes)
-    struct DevHashJoin {
-        std::thread& poller; std::atomic<bool>& stop; volatile uint32_t* cancel; cudaStream_t st; std::condition_variable& cv;
-        ~DevHashJoin() {
-            stop.store(true);
-            if (cancel) *cancel = 1;
-            cv.notify_all();
-            if (poller.joinable()) poller.join();
-            if (st) cudaStreamSynchronize(st);
-        }
-    } dev_hash_join{dev_poller, dev_stop, fsl_cancel, dev_k ? c->hash_st : nullptr, cv};
-
-    std::vector<int> lane_rc(n_lanes, KZGB_OK);
-    struct LanesRunning {  // from here on the lane threads only READ the context's tables (msm_enqueue builds none)
-        kzgb_ctx* c;
-        explicit LanesRunning(kzgb_ctx* ctx) : c(ctx) { c->lanes_running.store(true); }
-        ~LanesRunning() { c->lanes_running.store(false); }
-    } lanes_running(c);
-    if (!groups.empty()) {
-        // ---- small blobs: groups of equal-size blobs, each phase of a group is ONE batched launch set ----
-        std::atomic<size_t> next_group{0};
-        auto group_main = [&](int li) {
-            cudaSetDevice(c->device);
-            Lane& L = c->lanes[li];
-            std::vector<Affine> pts;
-            std::vector<Fr> zt;
-            for (;;) {
-                size_t gi = next_group.fetch_add(1);
-                if (gi >= groups.size()) return;
-                { std::lock_guard<std::mutex> lk(mu); if (failed) return; }
-                const size_t i0 = groups[gi].first, b = groups[gi].second;
-                const size_t n = blob_poly_len(lens[i0]);
-                const int logn = log2_exact(n);
-                const kzgb_ctx::LagTable* lag = (c->lag[logn].table && g_lagrange.load()) ? &c->lag[logn] : nullptr;
-                Fr ninv = ninv_mont(logn);
-                int r = KZGB_OK;
-                auto ck = [&](cudaError_t e, const char* what) {
-                    if (!r && e != cudaSuccess) r = fail(c, KZGB_ERR_DEVICE, std::string("CUDA error: ") + cudaGetErrorString(e) + " at " + what);
-                };
-                ck(L.evals.reserve(b * n * sizeof(Fr)), "evals");
-                ck(L.work.reserve(b * n * sizeof(Fr)), "work");
-                ck(L.small.reserve((3 * b + 8) * sizeof(Fr)), "small");
-                ck(L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)b) * sizeof(Fr)), "eval scratch");
-                if (!lag) ck(L.ntt_scratch.reserve(b * n * sizeof(Fr)), "ntt scratch");
-                if (!blobs_dev) ck(L.bytes.reserve(b * n * 32), "bytes");
-                bool full = true;  // every blob fills its polynomial: one conversion launch for the group
-                for (size_t k = 0; k < b; k++) full = full && lens[i0 + k] == n * 32;
-                bool dev_run = blobs_dev && full;  // device blobs back to back: one conversion launch too
-                for (size_t k = 0; k < b && dev_run; k++) dev_run = blobs_dev[i0 + k] == blobs_dev[i0] + k * n * 32;
-                if (dev_run) bytes_to_fr_launch(blobs_dev[i0], (uint64_t)b * n * 32, (Fr*)L.evals.p, (uint32_t)(b * n), L.st);
-                for (size_t k = 0; k < b && !r && !dev_run; k++) {
-                    const uint8_t* src = blobs_dev ? blobs_dev[i0 + k] : nullptr;
-                    if (!src) {
-                        uint8_t* dst = (uint8_t*)L.bytes.p + k * n * 32;
-                        ck(cudaMemcpyAsync(dst, blobs_host[i0 + k], lens[i0 + k], cudaMemcpyHostToDevice, L.st), "H2D copy of a blob");
-                        src = dst;
-                    }
-                    if (!full || blobs_dev) bytes_to_fr_launch(src, lens[i0 + k], (Fr*)L.evals.p + k * n, (uint32_t)n, L.st);
-                }
-                if (!r && full && !blobs_dev) bytes_to_fr_launch((const uint8_t*)L.bytes.p, (uint64_t)b * n * 32, (Fr*)L.evals.p, (uint32_t)(b * n), L.st);
-                // commitments
-                MsmJob job;
-                pts.resize(b);
-                if (!r) {
-                    const Fr* sc = (const Fr*)L.evals.p;
-                    if (!lag) {
-                        ck(cudaMemcpyAsync(L.work.p, L.evals.p, b * n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st), "copy");
-                        ntt_launch((Fr*)L.work.p, logn, (uint32_t)b, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-                        sc = (const Fr*)L.work.p;
-                    }
-                    if (!r) r = msm_enqueue_batched(c, L, sc, n, b, lag, &job);
-                }
-                if (!r) r = msm_finish_batched(c, L, job, b, pts.data());
-                if (!r) {
-                    for (size_t k = 0; k < b; k++) serialize_compressed(pts[k], commitments32 + 32 * (i0 + k));
-                    // challenges: the transcript midstates come from the hashing pool
-                    zt.resize(2 * b);
-                    {
-                        std::unique_lock<std::mutex> lk(mu);
-                        for (size_t k = 0; k < b; k++) cv.wait(lk, [&] { return ready[i0 + k] != 0 || failed; });
-                        if (failed) return;
-                    }
-                    bool any_in_domain = false;
-                    for (size_t k = 0; k < b; k++) {
-                        zt[k] = challenge_finish(mid[i0 + k], pts[k]);
-                        zt[b + k] = eval_tinv(zt[k], logn, &any_in_domain);
-                    }
-                    Fr* d_z = (Fr*)L.small.p;  // [z x b | tinv x b | y x b]
-                    ck(cudaMemcpyAsync(d_z, zt.data(), 2 * b * sizeof(Fr), cudaMemcpyHostToDevice, L.st), "H2D of the challenges");
-                    eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_z, d_z + b, c->tw, c->logN, &ninv,
-                                         (Fr*)L.eval_scratch.p, (Fr*)L.work.p, d_z + 2 * b, L.st, !any_in_domain);
-                    if (!lag) ntt_launch((Fr*)L.work.p, logn, (uint32_t)b, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-                    if (!r) r = msm_enqueue_batched(c, L, (const Fr*)L.work.p, n, b, lag, &job);
-                    if (!r) r = msm_finish_batched(c, L, job, b, pts.data());
-                }
-                if (r) {
-                    std::lock_guard<std::mutex> lk(mu);
-                    lane_rc[li] = r; failed = true;
-                    cv.notify_all();
-                    return;
-                }
-                for (size_t k = 0; k < b; k++) serialize_compressed(pts[k], proofs32 + 32 * (i0 + k));
-            }
-        };
-        std::vector<std::thread> lane_threads;
-        for (int li = 1; li < n_lanes; li++) lane_threads.emplace_back(group_main, li);
-        group_main(0);
-        for (auto& t : lane_threads) t.join();
-        next_hash.store(tasks.size());
-        for (auto& t : hashers) t.join();
-        for (int li = 0; li < n_lanes; li++) if (lane_rc[li]) return lane_rc[li];
-        return KZGB_OK;
-    }
-
-    // Task scheduler.  commit(i) needs nothing; proof(i) needs commit(i) and the transcript midstate of
-    // blob i (host SHA-256, ~9 ms for 16 MiB).  A lane takes the lowest ready proof, else the next
-    // commit, so the GPU never idles behind the hashing pool.
-    std::vector<uint8_t> commit_done(count, 0), proof_taken(count, 0);
-    std::vector<Affine> commits(count);
-    size_t next_commit = 0, proofs_taken = 0, proof_scan = 0;
-    auto lane_main = [&](int li) {
-        cudaSetDevice(c->device);
-        Lane& L = c->lanes[li];
-        for (;;) {
-            size_t i = 0;
-            bool is_proof = false;
-            {
-                std::unique_lock<std::mutex> lk(mu);
-                for (;;) {
-                    if (failed) return;
-                    while (proof_scan < count && proof_taken[proof_scan]) proof_scan++;
-                    bool found = false;
-                    for (size_t k = proof_scan; k < count && k < next_commit; k++) {
-                        if (!proof_taken[k] && commit_done[k] && ready[k]) { i = k; found = true; break; }
-                    }
-                    if (found) {
-                        proof_taken[i] = 1; proofs_taken++; is_proof = true;
-                        if (proofs_taken == count) cv.notify_all();  // lanes with nothing left to take can leave
-                        break;
-                    }
-                    if (next_commit < count) { i = next_commit++; break; }
-                    if (proofs_taken == count) return;
-                    cv.wait(lk);
-                }
-            }
-            size_t len = lens[i], n = blob_poly_len(len);
-            const uint8_t* dev_bytes = blobs_dev ? blobs_dev[i] : nullptr;
-            int r = KZGB_OK;
-            if (!dev_bytes && resident) {
-                uint8_t* slot = (uint8_t*)c->batch_bytes.p + byte_off[i];
-                if (i >= dev_first && !dev_failed.load()) {  // went up on the hashing stream
-                    if (!is_proof && cudaStreamWaitEvent(L.st, c->ev_hash_uploaded, 0) != cudaSuccess)
-                        r = fail(c, KZGB_ERR_DEVICE, "CUDA error: cudaStreamWaitEvent failed");
-                } else if (!is_proof && len) {
-                    if (cudaMemcpyAsync(slot, blobs_host[i], len, cudaMemcpyHostToDevice, L.st) != cudaSuccess)
-                        r = fail(c, KZGB_ERR_DEVICE, "CUDA error: H2D copy of a blob failed");
-                }
-                dev_bytes = slot;
-            }
-            MsmJob job;
-            Affine out;
-            if (!r) r = blob_to_evals(c, L, blobs_host[i], dev_bytes, len, n);
-            if (!r && !is_proof) r = commit_evals_enqueue(c, L, (Fr*)L.evals.p, n, &job);
-            if (!r && is_proof) {
-                Fr z = challenge_finish(mid[i], commits[i]);
-                r = proof_enqueue(c, L, (Fr*)L.evals.p, n, z, &job);
-            }
-            if (!r) r = msm_finish(c, L, job, &out);
-            if (r) {
-                std::lock_guard<std::mutex> lk(mu);
-                lane_rc[li] = r; failed = true;
-                cv.notify_all();
-                return;
-            }
-            if (is_proof) {
-                serialize_compressed(out, proofs32 + 32 * i);
-            } else {
-                serialize_compressed(out, commitments32 + 32 * i);
-                { std::lock_guard<std::mutex> lk(mu); commits[i] = out; commit_done[i] = 1; }
-                cv.notify_all();
-            }
-        }
-    };
-    std::vector<std::thread> lane_threads;
-    for (int li = 1; li < n_lanes; li++) lane_threads.emplace_back(lane_main, li);
-    lane_main(0);
-    for (auto& t : lane_threads) t.join();
-    next_hash.store(tasks.size());
-    for (auto& t : hashers) t.join();
-    if (c->batch_bytes.cap > ((size_t)g_batch_keep_mib.load() << 20)) c->batch_bytes.release();  // bounded residency between calls
-    for (int li = 0; li < n_lanes; li++) if (lane_rc[li]) return lane_rc[li];
-    return KZGB_OK;
-}
-
-int kzgb_commit_and_prove_blobs(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,
-                                uint8_t* commitments32, uint8_t* proofs32) {
-    Guard g(c);
-    return batch_impl(c, nullptr, blobs, lens, count, commitments32, proofs32);
-}
-int kzgb_commit_and_prove_blobs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
-                                    const size_t* lens, size_t count, uint8_t* commitments32, uint8_t* proofs32) {
-    Guard g(c);
-    return batch_impl(c, blobs_dev, blobs_host, lens, count, commitments32, proofs32);
-}
-
-// ------------------------------------------------------------------------------- batch verification (RLC)
-int kzgb_verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,
-                          const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
-                          const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8], uint8_t* rhs_inf) {
-    Guard g(c);
-    Lane& L = c->lanes[0];
-    const size_t m = count;
-    Affine inf_pt; aff_set_inf(inf_pt);
-    if (m == 0) { affine_to_abi(inf_pt, lhs_xy, lhs_inf); affine_to_abi(inf_pt, rhs_xy, rhs_inf); return KZGB_OK; }
-    std::vector<Affine> Cs(m), Ps(m);
-    for (size_t i = 0; i < m; i++) {
-        Cs[i] = affine_from_abi(commitments_xy + 8 * i, commitments_inf ? commitments_inf[i] : 0);
-        Ps[i] = affine_from_abi(proofs_xy + 8 * i, proofs_inf ? proofs_inf[i] : 0);
-    }
-    // validate_g1_point on all 2m points (batch.rs:30-37) -- on the GPU
-    CK(c, L.bases.reserve((2 * m + 1) * sizeof(Affine)));
-    CK(c, L.small.reserve(64 * sizeof(Fr)));
-    Affine* d_bases = (Affine*)L.bases.p;  // [C_0..C_{m-1}, pi_0..pi_{m-1}, G]
-    CK(c, cudaMemcpyAsync(d_bases, Cs.data(), m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
-    CK(c, cudaMemcpyAsync(d_bases + m, Ps.data(), m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
-    uint32_t* d_err = (uint32_t*)((Fr*)L.small.p + 32);
-    CK(c, cudaMemsetAsync(d_err, 0xff, 32, L.st));
-    g1_validate_launch(d_bases, (uint32_t)(2 * m), d_err, L.st);
-    uint32_t herr = 0;
-    CK(c, cudaMemcpyAsync(&herr, d_err, 4, cudaMemcpyDeviceToHost, L.st));
-    CK(c, cudaStreamSynchronize(L.st));
-    if (herr != 0xffffffffu) return fail(c, KZGB_ERR_NOT_ON_CURVE, "G1 point not on curve");
-
-    // per-blob challenge (host SHA pool) and evaluation (GPU, batched over blobs of equal length)
-    std::vector<size_t> ns(m);
-    size_t max_n = 0;
-    for (size_t i = 0; i < m; i++) {
-        if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
-        ns[i] = blob_poly_len(lens[i]);
-        max_n = std::max(max_n, ns[i]);
-    }
-    int rc = ensure_twiddles(c, log2_exact(max_n));
-    if (rc) return rc;
-    std::vector<Fr> zs(m), ys(m);
-    // Thousands of small transcripts: hash them on the GPU, one thread per blob, from the evaluations that
-    // are resident anyway (fs.cu).  Otherwise a host SHA-256 pool (one transcript per blob) runs while the
-    // blobs are uploaded and converted.
-    const int fs_opt = g_fs_device.load();
-    const bool fs_device = fs_opt >= 0 ? fs_opt != 0 : (m >= 256 && max_n <= ((size_t)1 << 13));
-    std::atomic<size_t> next{fs_device ? m : 0};
-    std::vector<std::thread> hashers;
-    {
-        size_t nt = fs_device ? 0 : std::max<size_t>(1, std::min<size_t>(m, hash_pool_threads() + 1));
-        for (size_t t = 0; t < nt; t++)
-            hashers.emplace_back([&]() {
-                for (;;) {
-                    size_t i = next.fetch_add(1);
-                    if (i >= m) return;
-                    Sha256 sh;
-                    challenge_midstate(sh, blobs[i], lens[i], ns[i]);
-                    zs[i] = challenge_finish(sh, Cs[i]);
-                }
-            });
-    }
-    struct Joiner {
-        std::vector<std::thread>& t;
-        std::atomic<size_t>& next;
-        size_t m;
-        bool joined = false;
-        void join() { if (!joined) { for (auto& x : t) x.join(); joined = true; } }
-        ~Joiner() { next.store(m); join(); }  // error paths: stop handing out work, then wait
-    } joiner{hashers, next, m};
-    const size_t budget_elems = (size_t)1 << 24;  // evaluations resident per GPU batch
-    size_t i0 = 0;
-    while (i0 < m) {
-        size_t n = ns[i0], i1 = i0;
-        while (i1 < m && ns[i1] == n && (i1 - i0 + 1) * n <= std::max(budget_elems, n) && i1 - i0 < 65535) i1++;  // b is a gridDim.y
-        size_t b = i1 - i0;
-        int logn = log2_exact(n);
-        CK(c, L.evals.reserve(b * n * sizeof(Fr)));
-        CK(c, L.bytes.reserve(b * n * 32));
-        CK(c, L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)b) * sizeof(Fr)));
-        CK(c, L.work.reserve(5 * b * sizeof(Fr)));
-        bool full = (uint64_t)b * n < 0xffffffffull;  // every blob fills its polynomial: one conversion launch
-        for (size_t k = 0; k < b && full; k++) full = lens[i0 + k] == n * 32;
-        for (size_t k = 0; k < b;) {
-            uint8_t* dst = (uint8_t*)L.bytes.p + k * n * 32;
-            size_t run = 1;  // blobs that are adjacent in host memory go up in one copy
-            while (full && k + run < b && blobs[i0 + k + run] == blobs[i0 + k] + run * n * 32) run++;
-            size_t bytes = full ? run * n * 32 : lens[i0 + k];
-            CK(c, cudaMemcpyAsync(dst, blobs[i0 + k], bytes, cudaMemcpyHostToDevice, L.st));
-            if (!full) bytes_to_fr_launch(dst, lens[i0 + k], (Fr*)L.evals.p + k * n, (uint32_t)n, L.st);
-            k += run;
-        }
-        if (full) bytes_to_fr_launch((const uint8_t*)L.bytes.p, (uint64_t)b * n * 32, (Fr*)L.evals.p, (uint32_t)(b * n), L.st);
-        joiner.join();  // the challenges z_i are needed from here on
-        Fr* d_z = (Fr*)L.work.p;
-        Fr* d_t = d_z + b;
-        Fr* d_y = d_t + b;
-        Fr ninv = ninv_mont(logn);
-        std::vector<Fr> tinvs;
-        std::vector<uint8_t> cbytes;
-        bool any_in_domain = false;
-        uint32_t* d_in_domain = nullptr;  // challenges hashed on the device: the device says which z are roots of the domain
-        if (fs_device) {
-            uint8_t* d_c32 = (uint8_t*)(d_y + b);
-            cbytes.resize(b * 32);
-            for (size_t k = 0; k < b; k++) serialize_compressed(Cs[i0 + k], &cbytes[32 * k]);
-            CK(c, cudaMemcpyAsync(d_c32, cbytes.data(), b * 32, cudaMemcpyHostToDevice, L.st));
-            d_in_domain = (uint32_t*)(d_c32 + 32 * b);
-            fs_challenges_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_c32, &ninv, d_z, d_t, L.st, d_in_domain);
-            CK(c, cudaMemcpyAsync(&zs[i0], d_z, b * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
-        } else {
-            tinvs.resize(b);
-            for (size_t k = 0; k < b; k++) tinvs[k] = eval_tinv(zs[i0 + k], logn, &any_in_domain);
-            CK(c, cudaMemcpyAsync(d_z, &zs[i0], b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-            CK(c, cudaMemcpyAsync(d_t, tinvs.data(), b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-        }
-        eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_z, d_t, c->tw, c->logN, &ninv,
-                             (Fr*)L.eval_scratch.p, nullptr, d_y, L.st, !fs_device && !any_in_domain, d_in_domain);
-        CK(c, cudaMemcpyAsync(&ys[i0], d_y, b * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
-        CK(c, cudaStreamSynchronize(L.st));
-        CK(c, cudaGetLastError());
-        i0 = i1;
-    }
-    // r = SHA-256(transcript) mod r (batch.rs:76-168): bytes 24..32 stay zero, count at 32..40
-    std::vector<uint8_t> tr(40 + m * 136, 0);
-    memcpy(tr.data(), "EIGENDA_RCKZGBATCH___V1_", 24);
-    for (int k = 0; k < 8; k++) tr[32 + k] = (uint8_t)((uint64_t)m >> (56 - 8 * k));
-    size_t off = 40;
-    for (size_t i = 0; i < m; i++) { for (int k = 0; k < 8; k++) tr[off + k] = (uint8_t)((uint64_t)ns[i] >> (56 - 8 * k)); off += 8; }
-    for (size_t i = 0; i < m; i++) {
-        serialize_compressed(Cs[i], &tr[off]); off += 32;
-        fe_to_be_bytes(zs[i], &tr[off]); off += 32;
-        fe_to_be_bytes(ys[i], &tr[off]); off += 32;
-        serialize_compressed(Ps[i], &tr[off]); off += 32;
-    }
-    uint8_t dg[32];
-    sha256(tr.data(), tr.size(), dg);
-    Fr r = fr_from_be_bytes(dg);
-
-    // scalars on the GPU: [r^i | r^i z_i | -(sum r^i y_i)]
-    CK(c, L.work.reserve((4 * m + 8) * sizeof(Fr)));
-    Fr* d_sc = (Fr*)L.work.p;          // 2m + 1 scalars
-    Fr* d_zy = d_sc + 2 * m + 1;       // z then y (m each)
-    Fr* d_dot = d_zy + 2 * m;
-    CK(c, cudaMemcpyAsync(d_zy, zs.data(), m * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-    CK(c, cudaMemcpyAsync(d_zy + m, ys.data(), m * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-    fr_powers_launch(d_sc, (uint32_t)m, &r, L.st);                      // helpers.rs:298-314
-    fr_mul_vec_launch(d_sc + m, d_sc, d_zy, (uint32_t)m, L.st);         // r^i z_i (batch.rs:239)
-    fr_dot_launch(d_dot, d_sc, d_zy + m, (uint32_t)m, L.st);            // sum r^i y_i
-    CK(c, cudaMemcpyAsync(&L.h_fr[2], d_dot, sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
-    CK(c, cudaStreamSynchronize(L.st));
-    fe_neg(L.h_fr[2], L.h_fr[2]);
-    CK(c, cudaMemcpyAsync(d_sc + 2 * m, &L.h_fr[2], sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-    Affine G;
-    fe_one(G.x); fe_dbl(G.y, G.x);
-    CK(c, cudaMemcpy(d_bases + 2 * m, &G, sizeof(Affine), cudaMemcpyHostToDevice));
-    // lhs = sum r^i pi_i (batch.rs:228); rhs = sum r^i (C_i - y_i G) + sum r^i z_i pi_i (batch.rs:245-249),
-    // the m generator multiplications folded into ONE extra base: -(sum r^i y_i) * G  (same group element)
-    Affine lhs, rhs;
-    rc = msm_blocking(c, L, d_sc, false, 0, m, d_bases + m, &lhs);
-    if (rc) return rc;
-    rc = msm_blocking(c, L, d_sc, false, 0, 2 * m + 1, d_bases, &rhs);
-    if (rc) return rc;
-    affine_to_abi(lhs, lhs_xy, lhs_inf);
-    affine_to_abi(rhs, rhs_xy, rhs_inf);
-    return KZGB_OK;
-}
 
 // ------------------------------------------------------------------------------- codecs / validation
 int kzgb_g1_serialize_compressed(const uint64_t xy[8], uint8_t inf, uint8_t out32[32]) {

@@ -1,4 +1,4 @@
-// Internal launcher interface between the host orchestration (capi.cu) and the kernel
+// Internal launcher interface between the host orchestration (capi.cu, batch.cu) and the kernel
 // translation units.  Everything here takes DEVICE pointers and a stream; nothing blocks.
 #pragma once
 #include <cuda_runtime.h>

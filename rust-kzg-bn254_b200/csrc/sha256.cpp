@@ -97,7 +97,7 @@ bool sha256_has_shani() {
 // stream is bound by the latency chain of its 32 sha256rnds2 per block (1.8 GB/s on one core of this box, 2.4 GB/s per
 // core with both hardware threads hashing); here a round is 6 rotates + 4 ternary logic ops + 7 additions for SIXTEEN
 // blocks, so one core sustains about twice that -- at the price of latency: the sixteen digests arrive together.  Used by
-// the blob-batch pipeline when a deep batch meets a host whose SHA-NI pool cannot keep up with the GPU (capi.cu batch_impl).
+// the blob-batch pipeline when a deep batch meets a host whose SHA-NI pool cannot keep up with the GPU (batch.cu HashStage).
 // ---------------------------------------------------------------------------------------------------------------
 #define KZ_MB_TARGET __attribute__((target("avx512f,avx512bw,avx512vl")))
 

@@ -1,7 +1,8 @@
-// Test-only shim: exposes the HOST path of csrc/field.cuh + csrc/ec.cuh + sha256 to Python so the
+// Test-only shim: exposes the HOST path of csrc/field.cuh + csrc/ec.cuh + sha256 + the transcript to Python so the
 // exact formulas the kernels use (same source, compiled for the host) can be checked on CPU.
 #include "../../rust-kzg-bn254_b200/csrc/ec.cuh"
 #include "../../rust-kzg-bn254_b200/csrc/sha256.hpp"
+#include "../../rust-kzg-bn254_b200/csrc/transcript.hpp"
 using namespace kzgb;
 extern "C" {
 void t_fq_mul(uint32_t* r, const uint32_t* a, const uint32_t* b) { fe_mul(*(Fq*)r, *(const Fq*)a, *(const Fq*)b); }
@@ -49,5 +50,26 @@ void t_sha256_state(const uint8_t* msg, size_t nblk, uint32_t* out) {
     Sha256 s;
     s.update(msg, 64 * nblk);
     for (int j = 0; j < 8; j++) out[j] = s.h[j];
+}
+// Fiat-Shamir transcript midstates, each finished by SHA-256 padding alone (out: 32-byte digests).
+void t_challenge_midstate(const uint8_t* blob, size_t len, size_t n, uint8_t* out) {
+    Sha256 s;
+    challenge_midstate(s, blob, len, n);
+    s.finish(out);
+}
+// `members` blobs of 32 n bytes back to back, hashed in lockstep, each midstate finished by challenge_midstate_resume
+void t_challenge_midstates_mb16(const uint8_t* blobs, size_t members, size_t n, uint8_t* out) {
+    const uint8_t* p[16];
+    for (size_t m = 0; m < members; m++) p[m] = blobs + 32 * n * m;
+    uint32_t st[16][8];
+    challenge_midstates_mb16(p, members, n, st);
+    for (size_t m = 0; m < members; m++) challenge_midstate_resume(st[m], p[m], n).finish(out + 32 * m);
+}
+// the single-stream state after chunks 0 .. n-2 (what the device hands over), finished by challenge_midstate_resume:
+// for even n those chunks end on a block boundary, so the one zero chunk of padding stays in the buffer, out of h
+void t_challenge_midstate_resumed(const uint8_t* blob, size_t n, uint8_t* out) {
+    Sha256 s;
+    challenge_midstate(s, blob, 32 * (n - 1), n);
+    challenge_midstate_resume(s.h, blob, n).finish(out);
 }
 }

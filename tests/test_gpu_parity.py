@@ -487,7 +487,7 @@ def test_device_hashed_transcripts_equal_host_hashed(pkg):
 
 
 def test_multibuffer_hashed_transcripts_equal_single_stream(pkg):
-    """Host transcripts hashed 16 at a time on AVX-512 (sha256.cpp sha256_mb16_blocks via capi.cu challenge_midstates_mb16),
+    """Host transcripts hashed 16 at a time on AVX-512 (sha256.cpp sha256_mb16_blocks via transcript.cpp challenge_midstates_mb16),
     forced on: same commitments and proofs as the single-stream pool and as the oracle's compute_challenge.  37 blobs =
     two full groups + a group of 5 that falls back to single streams; values >= r in block 0, in the middle, in the last
     chunk (which the host appends after the lockstep part) and a ragged blob that splits a run."""

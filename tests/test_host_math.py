@@ -20,8 +20,9 @@ MONT = 1 << 256
 def hm():
     src = os.path.join(HERE, "native", "host_math_test.cpp")
     out = os.path.join(HERE, "native", "libhostmath_test.so")
-    sha = os.path.join(ROOT, "rust-kzg-bn254_b200", "csrc", "sha256.cpp")
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-x", "c++", "-o", out, src, sha])
+    csrc = os.path.join(ROOT, "rust-kzg-bn254_b200", "csrc")
+    sha, transcript = os.path.join(csrc, "sha256.cpp"), os.path.join(csrc, "transcript.cpp")
+    subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-x", "c++", "-o", out, src, sha, transcript])
     return C.CDLL(out)
 
 
@@ -246,3 +247,54 @@ def test_safegcd_inverse_matches_bigint(hm):
         for a in vals:
             assert call1(fn, a * MONT % mod) == pow(a, -1, mod) * MONT % mod, hex(a)
         assert call1(fn, 0) == 0
+
+
+def _transcript_blobs(count, n, seed):
+    """count blobs of n random 32-byte chunks, each with values >= r in block 0 (chunk 0), in the middle and in the last
+    chunk, plus an all-0xff chunk; the other chunks are random bytes, so about a fifth of them are >= r as well."""
+    rnd = random.Random(seed)
+    blobs = []
+    for k in range(count):
+        chunks = [rnd.getrandbits(256).to_bytes(32, "big") for _ in range(n)]
+        chunks[0] = (o.R + rnd.randrange(1 << 200)).to_bytes(32, "big")
+        chunks[n // 2 + k] = (o.R + k).to_bytes(32, "big")
+        chunks[n - 1] = ((1 << 256) - 1 - k).to_bytes(32, "big")
+        chunks[1 + k] = b"\xff" * 32
+        blobs.append(b"".join(chunks))
+    return blobs
+
+
+def _transcript_digest(blob, n):
+    """The compute_challenge transcript without the commitment, every chunk as a field element (helpers.rs:32-34)."""
+    chunks = [(int.from_bytes(blob[i : i + 32], "big") % o.R).to_bytes(32, "big") for i in range(0, len(blob), 32)]
+    return hashlib.sha256(b"EIGENDA_FSBLOBVERIFY_V1_" + n.to_bytes(8, "big") + b"".join(chunks)).digest()
+
+
+@pytest.mark.parametrize("members", [16, 9])
+def test_multibuffer_transcript_midstates_equal_single_stream(hm, members):
+    """The multi-buffer hashing of the blob-batch pipeline (transcript.cpp challenge_midstates_mb16, a full and a partial
+    group of equal-size blobs), each finished by challenge_midstate_resume, equals challenge_midstate of the blob and the
+    transcript hashed here from the reduced chunks."""
+    if not hm.t_has_mb16():
+        pytest.skip("no AVX-512 on this host")
+    n = 1024
+    blobs = _transcript_blobs(members, n, seed=members)
+    out = C.create_string_buffer(32 * members)
+    hm.t_challenge_midstates_mb16(b"".join(blobs), C.c_size_t(members), C.c_size_t(n), out)
+    for m, blob in enumerate(blobs):
+        single = C.create_string_buffer(32)
+        hm.t_challenge_midstate(blob, C.c_size_t(len(blob)), C.c_size_t(n), single)
+        assert single.raw == _transcript_digest(blob, n), m
+        assert out.raw[32 * m : 32 * m + 32] == single.raw, m
+
+
+def test_resumed_transcript_midstate_equals_single_stream(hm):
+    """The host half of the device-hashed share: a state taken after chunks 0 .. n-2 and finished by
+    challenge_midstate_resume (which appends the last chunk reduced mod r) equals challenge_midstate."""
+    n = 1024
+    for blob in _transcript_blobs(3, n, seed=3):
+        single, resumed = C.create_string_buffer(32), C.create_string_buffer(32)
+        hm.t_challenge_midstate(blob, C.c_size_t(len(blob)), C.c_size_t(n), single)
+        hm.t_challenge_midstate_resumed(blob, C.c_size_t(n), resumed)
+        assert single.raw == _transcript_digest(blob, n)
+        assert resumed.raw == single.raw
