@@ -164,17 +164,13 @@ int plan_batch(Batch& b) {
         int logn = log2_exact(blob_poly_len(lens[i]));
         rc = ensure_lagrange(c, logn);
         if (rc) return rc;
-        if (!c->lag[logn].table) all_lagrange = false;
+        if (!lagrange_table(c, logn)) all_lagrange = false;
     }
-    if (!all_lagrange && c->auto_precompute && (!c->wtable || c->wt_first != 0 || b.max_n > c->wt_n) && c->srs_n <= ((size_t)1 << 22)) {
-        rc = do_precompute(c, 0, std::min(c->srs_n, next_pow2(b.max_n)), 0);
-        if (rc && rc != KZGB_ERR_DEVICE) return rc;
-    }
+    rc = all_lagrange ? KZGB_OK : ensure_window_table(c, 0, b.max_n);  // built here: the lanes only read the tables
+    if (rc) return rc;
     for (size_t gi = 0; gi < b.groups.size(); gi++) {  // the batched MSM needs a window table for every size
         size_t n = blob_poly_len(lens[b.groups[gi].first]);
-        int logn = log2_exact(n);
-        bool lag_ok = c->lag[logn].table && g_lagrange.load();
-        if (!lag_ok && !(c->wtable && c->wt_first == 0 && n <= c->wt_n)) { b.groups.clear(); break; }
+        if (!lagrange_table(c, log2_exact(n)) && !wtable_covers(c, 0, n)) { b.groups.clear(); break; }
     }
     return KZGB_OK;
 }
@@ -399,7 +395,7 @@ int group_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next_group, i
         const size_t i0 = b.groups[gi].first, bn = b.groups[gi].second;
         const size_t n = blob_poly_len(lens[i0]);
         const int logn = log2_exact(n);
-        const kzgb_ctx::LagTable* lag = (c->lag[logn].table && g_lagrange.load()) ? &c->lag[logn] : nullptr;
+        const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
         Fr ninv = ninv_mont(logn);
         int r = KZGB_OK;
         auto ck = [&](cudaError_t e, const char* what) {
@@ -638,17 +634,10 @@ int kzgb_verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs, const size_t
     }
     // validate_g1_point on all 2m points (batch.rs:30-37) -- on the GPU
     CK(c, L.bases.reserve((2 * m + 1) * sizeof(Affine)));
-    CK(c, L.small.reserve(64 * sizeof(Fr)));
     Affine* d_bases = (Affine*)L.bases.p;  // [C_0..C_{m-1}, pi_0..pi_{m-1}, G]
     CK(c, cudaMemcpyAsync(d_bases, Cs.data(), m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
     CK(c, cudaMemcpyAsync(d_bases + m, Ps.data(), m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
-    uint32_t* d_err = (uint32_t*)((Fr*)L.small.p + 32);
-    CK(c, cudaMemsetAsync(d_err, 0xff, 32, L.st));
-    g1_validate_launch(d_bases, (uint32_t)(2 * m), d_err, L.st);
-    uint32_t herr = 0;
-    CK(c, cudaMemcpyAsync(&herr, d_err, 4, cudaMemcpyDeviceToHost, L.st));
-    CK(c, cudaStreamSynchronize(L.st));
-    if (herr != 0xffffffffu) return fail(c, KZGB_ERR_NOT_ON_CURVE, "G1 point not on curve");
+    if (int rc = validate_points_dev(c, L, d_bases, 2 * m)) return rc;
 
     // per-blob challenge (host SHA pool) and evaluation (GPU, batched over blobs of equal length)
     std::vector<size_t> ns(m);

@@ -126,7 +126,7 @@ void to_gnark_be(const Affine& a, uint8_t out[32]) {
 int choose_c_var(size_t n) {
     int best = 4; double bc = 1e300;
     for (int c = 4; c <= 20; c++) {
-        int W = (255 + c - 1) / c;
+        int W = window_count(c);
         if (W > MAX_SETS) continue;
         double cost = (double)n * W * 10.0 + (double)W * (double)(1u << (c - 1)) * 40.0;
         if (cost < bc) { bc = cost; best = c; }
@@ -140,7 +140,7 @@ int choose_c_fixed(size_t n) {
     // 51.5 GB table at 2^26 points -- what 180 GB of HBM is for).
     const int c_max = n > ((size_t)1 << 20) ? 22 : 17;
     for (int c = 4; c <= c_max; c++) {
-        int W = (255 + c - 1) / c;
+        int W = window_count(c);
         double cost = (double)n * W * 10.0 + (double)(1u << (c - 1)) * 140.0;  // the bucket tail is latency-bound
         if (cost < bc) { bc = cost; best = c; }
     }
@@ -195,6 +195,11 @@ int ensure_lanes(kzgb_ctx* c, int want) {
     }
     return KZGB_OK;
 }
+cudaError_t drain_lanes(kzgb_ctx* c) {  // waits for every lane's stream, up to the first error
+    for (int i = 0; i < c->n_lanes; i++)
+        if (cudaError_t e = cudaStreamSynchronize(c->lanes[i].st)) return e;
+    return cudaSuccess;
+}
 // called once the lane's stream has drained: duration of the accumulate kernel and the additions it performed
 void lane_collect_acc(Lane& L) {
     if (L.ev_pending) {
@@ -233,7 +238,7 @@ int ensure_twiddles(kzgb_ctx* c, int logn) {
     int want = std::max(logn, 1);
     if (c->srs_n) want = std::max(want, log2_exact(next_pow2(c->srs_n)) > 28 ? 28 : log2_exact(next_pow2(c->srs_n)));
     if (want > 28) return fail(c, KZGB_ERR_GENERIC, "power must be <= 28");
-    for (int i = 0; i < c->n_lanes; i++) CK(c, cudaStreamSynchronize(c->lanes[i].st));
+    CK(c, drain_lanes(c));
     if (c->tw) { cudaFree(c->tw); c->tw = nullptr; }
     CK(c, cudaMalloc((void**)&c->tw, sizeof(Fr) * ((size_t)1 << (want - 1))));
     Fr w = root_of_unity_mont(want);
@@ -244,17 +249,22 @@ int ensure_twiddles(kzgb_ctx* c, int logn) {
 }
 
 // ---------------------------------------------------------------- SRS tables
+// A table of `bytes` fits in the free device memory plus the `reusable` bytes of the one it replaces, 2 GiB to spare.
+int check_table_fits(kzgb_ctx* c, size_t bytes, size_t reusable) {
+    size_t free_b = 0, total_b = 0;
+    CK(c, cudaMemGetInfo(&free_b, &total_b));
+    if (bytes + (2ull << 30) > free_b + reusable)
+        return fail(c, KZGB_ERR_DEVICE, "not enough device memory for the fixed-base window tables");
+    return KZGB_OK;
+}
 // Window table over `points` (n affine points on the device): table[w*n + i] = 2^(c*w) * points[i].
-int build_window_table(kzgb_ctx* c, const Affine* points, size_t n, int cb, size_t reusable_bytes, Affine** out, int* W_out) {
+int build_window_table(kzgb_ctx* c, const Affine* points, size_t n, int cb, Affine** out, int* W_out) {
     if (cb < 2 || cb > 24) return fail(c, KZGB_ERR_GENERIC, "window_bits out of range");
-    int W = (255 + cb - 1) / cb;
+    int W = window_count(cb);
     if ((uint64_t)W * n >= ((uint64_t)1 << 31))  // sorted refs are 31 bits + sign (msm.cu k_scatter)
         return fail(c, KZGB_ERR_GENERIC, "window table too large: windows x points must stay below 2^31 (use more window bits)");
     size_t bytes = (size_t)W * n * sizeof(Affine);
-    size_t free_b = 0, total_b = 0;
-    CK(c, cudaMemGetInfo(&free_b, &total_b));
-    if (bytes + (2ull << 30) > free_b + reusable_bytes)
-        return fail(c, KZGB_ERR_DEVICE, "not enough device memory for the fixed-base window tables");
+    if (int rc = check_table_fits(c, bytes, 0)) return rc;
     Lane& L = c->lanes[0];
     Affine* table = nullptr;
     CK(c, cudaMalloc((void**)&table, bytes));
@@ -281,21 +291,28 @@ int do_precompute(kzgb_ctx* c, size_t first, size_t count, int window_bits) {
     if (count == 0) return KZGB_OK;
     int cb = window_bits > 0 ? window_bits : choose_c_fixed(count);
     if (cb < 2 || cb > 24) return fail(c, KZGB_ERR_GENERIC, "window_bits out of range");
-    for (int i = 0; i < c->n_lanes; i++) CK(c, cudaStreamSynchronize(c->lanes[i].st));
+    CK(c, drain_lanes(c));
     size_t reusable = c->wtable ? (size_t)c->wt_W * c->wt_n * sizeof(Affine) : 0;
-    {
-        size_t need = (size_t)((255 + cb - 1) / cb) * count * sizeof(Affine), free_b = 0, total_b = 0;
-        CK(c, cudaMemGetInfo(&free_b, &total_b));
-        if (need + (2ull << 30) > free_b + reusable)
-            return fail(c, KZGB_ERR_DEVICE, "not enough device memory for the fixed-base window tables");
-    }
-    if (c->wtable) { cudaFree(c->wtable); c->wtable = nullptr; c->wt_n = 0; c->wt_first = 0; }
+    if (int rc = check_table_fits(c, (size_t)window_count(cb) * count * sizeof(Affine), reusable)) return rc;
+    drop_window_table(c);
     Affine* table = nullptr;
     int W = 0;
-    int rc = build_window_table(c, c->srs + first, count, cb, 0, &table, &W);
+    int rc = build_window_table(c, c->srs + first, count, cb, &table, &W);
     if (rc) return rc;
     c->wtable = table; c->wt_first = first; c->wt_n = count; c->wt_c = cb; c->wt_W = W;
     return KZGB_OK;
+}
+
+void drop_window_table(kzgb_ctx* c) {
+    if (c->wtable) { cudaFree(c->wtable); c->wtable = nullptr; c->wt_n = 0; c->wt_first = 0; }
+}
+bool wtable_covers(const kzgb_ctx* c, size_t first, size_t n) { return c->wtable && first >= c->wt_first && first + n <= c->wt_first + c->wt_n; }
+// Lazy build of the monomial window table over [0, next_pow2(first + n)) when none covers [first, first + n); SRS above
+// 2^22 points get one only on request.  Short of device memory (KZGB_ERR_DEVICE) the MSMs run on the variable-base plan.
+int ensure_window_table(kzgb_ctx* c, size_t first, size_t n) {
+    if (!c->auto_precompute || wtable_covers(c, first, n) || c->srs_n > ((size_t)1 << 22)) return KZGB_OK;
+    int rc = do_precompute(c, 0, std::min(c->srs_n, next_pow2(first + n)), 0);
+    return rc == KZGB_ERR_DEVICE ? KZGB_OK : rc;
 }
 
 void lagrange_release(kzgb_ctx* c) {
@@ -330,7 +347,7 @@ int ensure_lagrange(kzgb_ctx* c, int logn, uint32_t weight, bool force) {
         size_t free_b = 0, total_b = 0;
         CK(c, cudaMemGetInfo(&free_b, &total_b));
         size_t budget = g_lagrange_budget_mib.load() > 0 ? (size_t)g_lagrange_budget_mib.load() << 20 : total_b / 2;
-        const size_t need = (size_t)((255 + cb_plan - 1) / cb_plan) * n * sizeof(Affine);
+        const size_t need = (size_t)window_count(cb_plan) * n * sizeof(Affine);
         if (need > budget) return KZGB_OK;
         for (;;) {
             size_t held = 0;
@@ -341,14 +358,14 @@ int ensure_lagrange(kzgb_ctx* c, int logn, uint32_t weight, bool force) {
                 if (!lru || o.last_use < lru->last_use) lru = &o;
             }
             if (held + need <= budget || !lru) break;
-            for (int i = 0; i < c->n_lanes; i++) CK(c, cudaStreamSynchronize(c->lanes[i].st));
+            CK(c, drain_lanes(c));
             cudaFree(lru->table);
             lru->table = nullptr; lru->n = 0; lru->calls = 0;
         }
     }
     int rc = ensure_twiddles(c, logn);
     if (rc) return rc;
-    for (int i = 0; i < c->n_lanes; i++) CK(c, cudaStreamSynchronize(c->lanes[i].st));
+    CK(c, drain_lanes(c));
     Lane& L = c->lanes[0];
     DevBuf work, pts;
     if (work.reserve(n * sizeof(XYZZ)) != cudaSuccess || pts.reserve(n * sizeof(Affine)) != cudaSuccess) {
@@ -363,7 +380,7 @@ int ensure_lagrange(kzgb_ctx* c, int logn, uint32_t weight, bool force) {
     if (e != cudaSuccess) { pts.release(); CK(c, e); }
     Affine* table = nullptr;
     int W = 0, cb = cb_plan;  // an explicit window override of the monomial table carries over
-    rc = build_window_table(c, (const Affine*)pts.p, n, cb, 0, &table, &W);
+    rc = build_window_table(c, (const Affine*)pts.p, n, cb, &table, &W);
     pts.release();
     if (rc == KZGB_ERR_DEVICE) { cudaGetLastError(); return KZGB_OK; }  // short of memory: stay on the monomial path
     if (rc) return rc;
@@ -371,10 +388,15 @@ int ensure_lagrange(kzgb_ctx* c, int logn, uint32_t weight, bool force) {
     return KZGB_OK;
 }
 
+// The table that serves evaluation-form MSMs of size 2^logn; none while option "lagrange" is off, even if one is resident.
+const kzgb_ctx::LagTable* lagrange_table(const kzgb_ctx* c, int logn) {
+    return logn >= 1 && logn <= 28 && c->lag[logn].table && g_lagrange.load() ? &c->lag[logn] : nullptr;
+}
+
 int srs_install(kzgb_ctx* c, Affine* dev_points, size_t n) {
-    for (int i = 0; i < c->n_lanes; i++) cudaStreamSynchronize(c->lanes[i].st);
+    drain_lanes(c);
     if (c->srs) cudaFree(c->srs);
-    if (c->wtable) { cudaFree(c->wtable); c->wtable = nullptr; c->wt_n = 0; c->wt_first = 0; }
+    drop_window_table(c);
     lagrange_release(c);
     c->srs = dev_points;
     c->srs_n = n;
@@ -415,14 +437,10 @@ int msm_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_scalars, bool canonical, size_
         table = lag->table;
     } else if (!var_bases) {
         if (first > c->srs_n || n > c->srs_n - first) return fail(c, KZGB_ERR_GENERIC, "MSM range exceeds the SRS");
-        auto covered = [&]() { return c->wtable && first >= c->wt_first && first + n <= c->wt_first + c->wt_n; };
-        // lazily built on the first use -- never from the lane threads of a running batch (they only read the tables)
-        if (c->auto_precompute && !covered() && c->srs_n <= ((size_t)1 << 22) && !c->lanes_running.load()) {
-            size_t want = std::min(c->srs_n, next_pow2(first + n));
-            int rc = do_precompute(c, 0, want, 0);
-            if (rc && rc != KZGB_ERR_DEVICE) return rc;
+        if (!c->lanes_running.load()) {  // never from the lane threads of a running batch (they only read the tables)
+            if (int rc = ensure_window_table(c, first, n)) return rc;
         }
-        if (covered()) {
+        if (wtable_covers(c, first, n)) {
             p = msm_make_plan((uint32_t)n, c->wt_c, true, (uint32_t)c->wt_n, (uint32_t)(first - c->wt_first));
             table = c->wtable;
         } else {
@@ -510,11 +528,10 @@ int msm_blocking(kzgb_ctx* c, Lane& L, const Fr* d_scalars, bool canonical, size
 // Returns KZGB_OK with *done = false when the shape does not qualify (no table over the range, or too small to matter).
 int msm_srs_host_pipelined(kzgb_ctx* c, Lane& L, const uint64_t* scalars, size_t first, size_t n, Affine* out, bool* done) {
     *done = false;
-    if (n < ((size_t)1 << 22) || !g_pipelined_upload.load()) return KZGB_OK;
-    if (!(c->wtable && first >= c->wt_first && first + n <= c->wt_first + c->wt_n)) return KZGB_OK;
+    if (n < ((size_t)1 << 22) || !g_pipelined_upload.load() || !wtable_covers(c, first, n)) return KZGB_OK;
     const size_t S = n >= ((size_t)1 << 24) ? 8 : 4;
     const size_t per = ((n + S - 1) / S + 31) & ~(size_t)31;
-    if ((uint64_t)per * ((255 + c->wt_c - 1) / c->wt_c) >= 0xfff00000ull) return KZGB_OK;
+    if ((uint64_t)per * window_count(c->wt_c) >= 0xfff00000ull) return KZGB_OK;
     if (!c->copy_st) {
         CK(c, cudaStreamCreateWithFlags(&c->copy_st, cudaStreamNonBlocking));
         for (int k = 0; k < 2; k++) {
@@ -568,7 +585,7 @@ int msm_enqueue_batched(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t n_per,
         p = msm_make_plan((uint32_t)(n_per * batch), lag->c, true, (uint32_t)lag->n, 0, (uint32_t)batch);
         table = lag->table;
     } else {
-        if (!c->wtable || c->wt_first != 0 || n_per > c->wt_n) return fail(c, KZGB_ERR_GENERIC, "batched MSM needs a fixed-base table");
+        if (!wtable_covers(c, 0, n_per)) return fail(c, KZGB_ERR_GENERIC, "batched MSM needs a fixed-base table");
         p = msm_make_plan((uint32_t)(n_per * batch), c->wt_c, true, (uint32_t)c->wt_n, 0, (uint32_t)batch);
         table = c->wtable;
     }
@@ -588,8 +605,8 @@ int msm_finish_batched(kzgb_ctx* c, Lane& L, const MsmJob& job, size_t batch, Af
 // d_evals (n Fr, Montgomery) -> commitment.  Uses L.work / L.ntt_scratch.
 int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJob* job) {
     int logn = log2_exact(n);
-    if (logn <= 28 && c->lag[logn].table && g_lagrange.load())  // Lagrange-basis table resident: the evaluations ARE the scalars
-        return msm_enqueue(c, L, d_evals, false, 0, n, nullptr, job, &c->lag[logn]);
+    if (const kzgb_ctx::LagTable* lag = lagrange_table(c, logn))  // the evaluations ARE the scalars
+        return msm_enqueue(c, L, d_evals, false, 0, n, nullptr, job, lag);
     int rc = ensure_twiddles(c, logn);
     if (rc) return rc;
     CK(c, L.work.reserve(n * sizeof(Fr)));
@@ -601,28 +618,37 @@ int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJ
     return msm_enqueue(c, L, (Fr*)L.work.p, false, 0, n, nullptr, job);
 }
 
-// quotient of d_evals at z (device, Montgomery) into L.work, then commit it.  y stays in L.small[2].
-int proof_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z_mont, MsmJob* job) {
-    int logn = log2_exact(n);
-    int rc = ensure_twiddles(c, logn);
-    if (rc) return rc;
-    CK(c, L.work.reserve(n * sizeof(Fr)));
-    CK(c, L.ntt_scratch.reserve(n * sizeof(Fr)));
+// y = p(z) into L.small[2] and, unless d_quotient is nullptr, the quotient; the twiddles of size n must be resident.
+int eval_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z, Fr* d_quotient) {
+    const int logn = log2_exact(n);
     CK(c, L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, 1) * sizeof(Fr)));
     CK(c, L.small.reserve(64 * sizeof(Fr)));
     Fr* d_z = (Fr*)L.small.p;  // [z, tinv, y]
-    Fr* d_y = d_z + 2;
-    L.h_fr[0] = z_mont;
+    L.h_fr[0] = z;
     bool in_domain = false;
-    L.h_fr[1] = eval_tinv(z_mont, logn, &in_domain);
+    L.h_fr[1] = eval_tinv(z, logn, &in_domain);
     CK(c, cudaMemcpyAsync(d_z, &L.h_fr[0], 2 * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
     Fr ninv = ninv_mont(logn);
     eval_quotient_launch(d_evals, (uint32_t)n, logn, 1, d_z, d_z + 1, c->tw, c->logN, &ninv, (Fr*)L.eval_scratch.p,
-                         (Fr*)L.work.p, d_y, L.st, !in_domain);
-    if (c->lag[logn].table && g_lagrange.load())  // quotient in evaluation form against the Lagrange-basis table
-        return msm_enqueue(c, L, (Fr*)L.work.p, false, 0, n, nullptr, job, &c->lag[logn]);
-    ntt_launch((Fr*)L.work.p, logn, 1, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-    return msm_enqueue(c, L, (Fr*)L.work.p, false, 0, n, nullptr, job);
+                         d_quotient, d_z + 2, L.st, !in_domain);
+    return KZGB_OK;
+}
+// Waits for the lane and returns the y of the last eval_enqueue.
+int eval_read_y(kzgb_ctx* c, Lane& L, Fr* y) {
+    CK(c, cudaMemcpyAsync(&L.h_fr[3], (Fr*)L.small.p + 2, sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
+    CK(c, cudaStreamSynchronize(L.st));
+    CK(c, cudaGetLastError());
+    *y = L.h_fr[3];
+    return KZGB_OK;
+}
+
+// quotient of d_evals at z (device, Montgomery) into L.work, then commit it.  y stays in L.small[2].
+int proof_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z_mont, MsmJob* job) {
+    if (int rc = ensure_twiddles(c, log2_exact(n))) return rc;
+    CK(c, L.work.reserve(n * sizeof(Fr)));
+    CK(c, L.ntt_scratch.reserve(n * sizeof(Fr)));
+    if (int rc = eval_enqueue(c, L, d_evals, n, z_mont, (Fr*)L.work.p)) return rc;
+    return commit_evals_enqueue(c, L, (Fr*)L.work.p, n, job);  // the quotient is in evaluation form
 }
 
 
@@ -641,6 +667,18 @@ int blob_to_evals(kzgb_ctx* c, Lane& L, const uint8_t* blob_host, const uint8_t*
     return KZGB_OK;
 }
 
+// KZGB_ERR_NOT_ON_CURVE unless each of the n points at d_pts (device) is on the curve or the identity.  Waits for the lane.
+int validate_points_dev(kzgb_ctx* c, Lane& L, const Affine* d_pts, size_t n) {
+    CK(c, L.small.reserve(64 * sizeof(Fr)));
+    uint32_t* d_err = (uint32_t*)((Fr*)L.small.p + 32);
+    CK(c, cudaMemsetAsync(d_err, 0xff, 32, L.st));
+    g1_validate_launch(d_pts, (uint32_t)n, d_err, L.st);
+    uint32_t herr = 0;
+    CK(c, cudaMemcpyAsync(&herr, d_err, 4, cudaMemcpyDeviceToHost, L.st));
+    CK(c, cudaStreamSynchronize(L.st));
+    if (herr != 0xffffffffu) return fail(c, KZGB_ERR_NOT_ON_CURVE, "G1 point not on curve");
+    return KZGB_OK;
+}
 
 // Streamed ingest of `n` compressed points: `read(dst, first, count)` fills a pinned staging buffer with
 // points [first, first+count); the read of chunk k+1 overlaps the H2D copy and the decompression kernel of
@@ -757,7 +795,7 @@ void kzgb_ctx_destroy(kzgb_ctx* c) {
     cudaSetDevice(c->device);
     for (int i = 0; i < c->n_lanes; i++) { cudaStreamSynchronize(c->lanes[i].st); lane_destroy(c->lanes[i]); }
     if (c->srs) cudaFree(c->srs);
-    if (c->wtable) cudaFree(c->wtable);
+    drop_window_table(c);
     lagrange_release(c);
     if (c->tw) cudaFree(c->tw);
     c->batch_bytes.release();
@@ -780,7 +818,7 @@ const char* kzgb_last_error(const kzgb_ctx* c) { return c ? c->err.c_str() : "nu
 
 int kzgb_sync(kzgb_ctx* c) {
     Guard g(c);
-    for (int i = 0; i < c->n_lanes; i++) CK(c, cudaStreamSynchronize(c->lanes[i].st));
+    CK(c, drain_lanes(c));
     return KZGB_OK;
 }
 
@@ -882,7 +920,7 @@ int kzgb_srs_clone(kzgb_ctx* dst, kzgb_ctx* src) {
     int src_dev = 0;
     {
         Guard gs(src);
-        for (int i = 0; i < src->n_lanes; i++) CK(src, cudaStreamSynchronize(src->lanes[i].st));
+        CK(src, drain_lanes(src));
         n = src->srs_n; from = src->srs; src_dev = src->device;
     }
     Guard g(dst);
@@ -929,8 +967,8 @@ int kzgb_srs_precompute(kzgb_ctx* c, size_t max_n, int window_bits) {
     Guard g(c);
     if (window_bits < 0) {  // disable fixed-base tables (variable-base mode over the monomial points)
         c->auto_precompute = false;
-        for (int i = 0; i < c->n_lanes; i++) cudaStreamSynchronize(c->lanes[i].st);
-        if (c->wtable) { cudaFree(c->wtable); c->wtable = nullptr; c->wt_n = 0; c->wt_first = 0; }
+        drain_lanes(c);
+        drop_window_table(c);
         lagrange_release(c);
         return KZGB_OK;
     }
@@ -1207,25 +1245,16 @@ int kzgb_evaluate_polynomial(kzgb_ctx* c, const uint64_t* evals, size_t n, const
     Guard g(c);
     Lane& L = c->lanes[0];
     if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_INVALID_INPUT_LENGTH, "polynomial length must be a power of two");
-    int logn = log2_exact(n);
-    int rc = ensure_twiddles(c, logn);
+    int rc = ensure_twiddles(c, log2_exact(n));
     if (rc) return rc;
     CK(c, L.evals.reserve(n * sizeof(Fr)));
-    CK(c, L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, 1) * sizeof(Fr)));
-    CK(c, L.small.reserve(64 * sizeof(Fr)));
     CK(c, cudaMemcpyAsync(L.evals.p, evals, n * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-    memcpy(L.h_fr[0].l, z_mont, 32);
-    bool in_domain = false;
-    L.h_fr[1] = eval_tinv(L.h_fr[0], logn, &in_domain);
-    Fr* d_z = (Fr*)L.small.p;
-    CK(c, cudaMemcpyAsync(d_z, &L.h_fr[0], 2 * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-    Fr ninv = ninv_mont(logn);
-    eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, 1, d_z, d_z + 1, c->tw, c->logN, &ninv,
-                         (Fr*)L.eval_scratch.p, nullptr, d_z + 2, L.st, !in_domain);
-    CK(c, cudaMemcpyAsync(&L.h_fr[3], d_z + 2, sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
-    CK(c, cudaStreamSynchronize(L.st));
-    CK(c, cudaGetLastError());
-    memcpy(y_out, &L.h_fr[3], 32);
+    Fr z, y;
+    memcpy(z.l, z_mont, 32);
+    rc = eval_enqueue(c, L, (Fr*)L.evals.p, n, z, nullptr);
+    if (!rc) rc = eval_read_y(c, L, &y);
+    if (rc) return rc;
+    memcpy(y_out, y.l, 32);
     return KZGB_OK;
 }
 
@@ -1311,28 +1340,17 @@ int kzgb_verify_blob_proof_g1(kzgb_ctx* c, const uint8_t* blob, size_t len, cons
     {
         Guard g(c);
         Lane& L = c->lanes[0];
-        const int logn = log2_exact(n);
-        int rc = ensure_twiddles(c, logn);
+        int rc = ensure_twiddles(c, log2_exact(n));
         if (rc) return rc;
         rc = blob_to_evals(c, L, blob, nullptr, len, n);
         if (rc) return rc;
         Sha256 sh;
         challenge_midstate(sh, blob, len, n);
-        L.h_fr[0] = challenge_finish(sh, C);
-        CK(c, L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, 1) * sizeof(Fr)));
-        CK(c, L.small.reserve(64 * sizeof(Fr)));
-        bool in_domain = false;
-        L.h_fr[1] = eval_tinv(L.h_fr[0], logn, &in_domain);
-        Fr* d_z = (Fr*)L.small.p;
-        CK(c, cudaMemcpyAsync(d_z, &L.h_fr[0], 2 * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-        Fr ninv = ninv_mont(logn);
-        eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, 1, d_z, d_z + 1, c->tw, c->logN, &ninv, (Fr*)L.eval_scratch.p,
-                             nullptr, d_z + 2, L.st, !in_domain);
-        CK(c, cudaMemcpyAsync(&L.h_fr[3], d_z + 2, sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
-        CK(c, cudaStreamSynchronize(L.st));
-        CK(c, cudaGetLastError());
-        y = L.h_fr[3];
-        if (z_out) memcpy(z_out, L.h_fr[0].l, 32);
+        const Fr z = challenge_finish(sh, C);
+        rc = eval_enqueue(c, L, (Fr*)L.evals.p, n, z, nullptr);
+        if (!rc) rc = eval_read_y(c, L, &y);
+        if (rc) return rc;
+        if (z_out) memcpy(z_out, z.l, 32);
         if (y_out) memcpy(y_out, y.l, 32);
     }
     return kzgb_verify_proof_g1(c, c_xy, c_inf, proof_xy, proof_inf, (const uint64_t*)y.l, out_xy, out_inf);
@@ -1355,16 +1373,8 @@ int kzgb_validate_g1_points(kzgb_ctx* c, const uint64_t* xy, const uint8_t* inf,
     std::vector<Affine> pts(n);
     for (size_t i = 0; i < n; i++) pts[i] = affine_from_abi(xy + 8 * i, inf ? inf[i] : 0);
     CK(c, L.bases.reserve(n * sizeof(Affine)));
-    CK(c, L.small.reserve(64 * sizeof(Fr)));
-    uint32_t* d_err = (uint32_t*)((Fr*)L.small.p + 32);
     CK(c, cudaMemcpyAsync(L.bases.p, pts.data(), n * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
-    CK(c, cudaMemsetAsync(d_err, 0xff, 32, L.st));
-    g1_validate_launch((Affine*)L.bases.p, (uint32_t)n, d_err, L.st);
-    uint32_t herr = 0;
-    CK(c, cudaMemcpyAsync(&herr, d_err, 4, cudaMemcpyDeviceToHost, L.st));
-    CK(c, cudaStreamSynchronize(L.st));
-    if (herr != 0xffffffffu) return fail(c, KZGB_ERR_NOT_ON_CURVE, "G1 point not on curve");
-    return KZGB_OK;
+    return validate_points_dev(c, L, (const Affine*)L.bases.p, n);
 }
 
 // ------------------------------------------------------------------------------- measurement hooks
@@ -1466,7 +1476,7 @@ int kzgb_timer_end(kzgb_ctx* c, double* ms_out) {
 }
 int kzgb_trace_begin(kzgb_ctx* c) {
     Guard g(c);
-    for (int i = 0; i < c->n_lanes; i++) CK(c, cudaStreamSynchronize(c->lanes[i].st));
+    CK(c, drain_lanes(c));
     for (auto& r : c->trace) if (r.ev) cudaEventDestroy(r.ev);
     c->trace.clear();
     if (!c->trace_base) CK(c, cudaEventCreate(&c->trace_base));

@@ -151,9 +151,15 @@ Affine affine_from_abi(const uint64_t xy[8], uint8_t inf);
 
 // ---- lanes and tables
 int ensure_lanes(kzgb_ctx* c, int want);
+cudaError_t drain_lanes(kzgb_ctx* c);
 int ensure_twiddles(kzgb_ctx* c, int logn);
 int ensure_lagrange(kzgb_ctx* c, int logn, uint32_t weight = 1, bool force = false);
+const kzgb_ctx::LagTable* lagrange_table(const kzgb_ctx* c, int logn);
+int check_table_fits(kzgb_ctx* c, size_t bytes, size_t reusable);
 int do_precompute(kzgb_ctx* c, size_t first, size_t count, int window_bits);
+void drop_window_table(kzgb_ctx* c);
+bool wtable_covers(const kzgb_ctx* c, size_t first, size_t n);
+int ensure_window_table(kzgb_ctx* c, size_t first, size_t n);
 bool lane_wait_polls();
 
 // ---- MSM and polynomial pieces (enqueue on the lane, finish waits for it)
@@ -168,7 +174,10 @@ int msm_enqueue_batched(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t n_per,
                         const kzgb_ctx::LagTable* lag, MsmJob* job);
 int msm_finish_batched(kzgb_ctx* c, Lane& L, const MsmJob& job, size_t batch, Affine* outs);
 int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJob* job);
+int eval_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z, Fr* d_quotient);
+int eval_read_y(kzgb_ctx* c, Lane& L, Fr* y);
 int proof_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z_mont, MsmJob* job);
 int blob_to_evals(kzgb_ctx* c, Lane& L, const uint8_t* blob_host, const uint8_t* blob_dev, size_t len, size_t n);
+int validate_points_dev(kzgb_ctx* c, Lane& L, const Affine* d_pts, size_t n);
 
 }  // namespace kzgb

@@ -17,6 +17,7 @@ extern std::atomic<uint64_t> g_launch_count;
 // With a fixed-base table (precomputed 2^(c*w) * P_i for every window w) all windows
 // share ONE bucket set; without it (variable bases) every window has its own set and
 // the host finishes with a Horner combine.
+inline int window_count(int c) { return (255 + c - 1) / c; }  // W of a c-bit plan or window table
 struct MsmPlan {
     int c;             // window bits
     int W;             // number of windows

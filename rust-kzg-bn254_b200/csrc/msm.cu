@@ -577,7 +577,7 @@ void msm_set_acc_waves(int waves) { g_acc_waves.store(waves < 1 ? 1 : (waves > 6
 MsmPlan msm_make_plan(uint32_t n, int c, bool fixed_base, uint32_t table_stride, uint32_t base_offset, uint32_t batch) {
     MsmPlan p;
     p.c = c;
-    p.W = (255 + c - 1) / c;
+    p.W = window_count(c);
     p.batch_n = (fixed_base && batch > 0) ? n / batch : 0;  // `batch` independent MSMs over the same table, one bucket set each
     p.sets = fixed_base ? (p.batch_n ? (int)batch : 1) : p.W;
     p.nbuckets = (uint32_t)p.sets << (c - 1);

@@ -649,6 +649,29 @@ def test_lagrange_table_and_monomial_paths_agree(pkg, ref_srs_points):
         lib.kzgb_set_option(b"lagrange", 1)
 
 
+def test_batch_with_lagrange_off_builds_the_monomial_table(pkg):
+    """A Lagrange table built before option "lagrange" is turned off does not serve the blob batch: the batch builds
+    the monomial window table (it would otherwise run every MSM on the variable-base plan over the raw SRS points)
+    and gives the bytes of the same batch with the option on."""
+    import ctypes as C
+
+    rnd = random.Random(31)
+    blobs = [pkg.Blob.from_raw_data(bytes(rnd.getrandbits(8) for _ in range(31 * 64 - k))) for k in (0, 3, 0, 9)]  # n = 64
+    lib = pkg.lib
+    eng = pkg.Engine(0)
+    srs = pkg.SRS.from_gnark_bytes(g.g1_point_bytes(), engine=eng)
+    srs.prepare_lagrange(64)
+    try:
+        assert lib.kzgb_set_option(b"lagrange", 0) == 0
+        off = pkg.KZG.commit_and_prove_blobs(blobs, srs)
+        cb, cw, ct = C.c_int(0), C.c_int(0), C.c_size_t(0)
+        eng.check(lib.kzgb_msm_config(eng.h, C.byref(cb), C.byref(cw), C.byref(ct)))
+        assert ct.value >= 64
+    finally:
+        lib.kzgb_set_option(b"lagrange", 1)
+    assert off == pkg.KZG.commit_and_prove_blobs(blobs, srs)
+
+
 def test_lagrange_table_tau_trick_large(pkg):
     """n = 2^16 on the synthetic SRS: commitment through the Lagrange table == p(tau) G, proof == ((p(tau)-y)/(tau-z)) G."""
     n = 1 << 16
