@@ -175,6 +175,14 @@ int kzgb_commit_and_prove_blobs(kzgb_ctx* ctx, const uint8_t* const* blobs, cons
  * SHA-256 transcript; pass them in `blobs_host`). */
 int kzgb_commit_and_prove_blobs_dev(kzgb_ctx* ctx, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
                                     const size_t* lens, size_t count, uint8_t* commitments32, uint8_t* proofs32);
+/* KZG::commit_blob (kzg.rs:182-185) for `count` blobs, pipelined; no proofs, no transcripts.  out_xy: count x 8 words
+ * (x||y Montgomery), out_inf: count flags (may be NULL).  Blob i's point and every error are those of kzgb_commit_blob
+ * on blob i alone; all blobs are checked before any work starts.  count == 0 writes nothing. */
+int kzgb_commit_blobs(kzgb_ctx* ctx, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                      uint64_t* out_xy, uint8_t* out_inf);
+/* Same with the blob bytes in device memory (no host copy needed: nothing is hashed). */
+int kzgb_commit_blobs_dev(kzgb_ctx* ctx, const uint8_t* const* blobs_dev, const size_t* lens, size_t count,
+                          uint64_t* out_xy, uint8_t* out_inf);
 
 /* ---- batch verification, everything before the pairing (verifier/src/batch.rs:16-249) ------ */
 /* Per-blob challenge z_i and evaluation y_i (helpers.rs:613-662), RLC scalar r and its powers
@@ -284,6 +292,10 @@ int kzgb_group_srs_precompute_ranges(kzgb_group* group, size_t n, int window_bit
  * byte-identical to the single-context call. */
 int kzgb_group_commit_and_prove_blobs(kzgb_group* group, const uint8_t* const* blobs, const size_t* lens, size_t count,
                                       uint8_t* commitments32, uint8_t* proofs32);
+/* kzgb_commit_blobs cut into contiguous shares of about equal bytes, one per member; identical to the one-context call.
+ * Each member checks its own share before it starts. */
+int kzgb_group_commit_blobs(kzgb_group* group, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                            uint64_t* out_xy, uint8_t* out_inf);
 /* kzgb_msm_srs with the points cut into G contiguous ranges; the partial sums are added on the host. */
 int kzgb_group_msm_srs(kzgb_group* group, const uint64_t* scalars_mont, size_t n, uint64_t out_xy[8], uint8_t* out_inf);
 

@@ -83,6 +83,16 @@ def _blobs_to_abi(blobs: Sequence["Blob"]):
     return keep, ptrs, lens
 
 
+def _commit_blobs(call, blobs: Sequence["Blob"]) -> List[Affine]:
+    """Runs call(blob pointers, lengths, count, out_xy, out_inf) of a kzgb_*commit_blobs entry point; returns the points."""
+    count = len(blobs)
+    keep, ptrs, lens = _blobs_to_abi(blobs)  # keep: the buffers ptrs points into
+    xy = C.create_string_buffer(64 * count if count else 1)
+    inf = C.create_string_buffer(count if count else 1)
+    call(ptrs, lens, count, xy, inf)
+    return g1_from_abi(xy.raw[: 64 * count], inf.raw[:count])
+
+
 def _next_pow2(n: int) -> int:
     return 1 if n <= 1 else 1 << (n - 1).bit_length()
 
@@ -199,6 +209,10 @@ class Group:
         ps = C.create_string_buffer(32 * count if count else 1)
         self.check(lib.kzgb_group_commit_and_prove_blobs(self.h, ptrs, lens, count, cs, ps))
         return ([cs.raw[32 * i : 32 * i + 32] for i in range(count)], [ps.raw[32 * i : 32 * i + 32] for i in range(count)])
+
+    def commit_blobs(self, blobs: Sequence["Blob"]) -> List[Affine]:
+        """KZG::commit_blob for every blob (prover/src/kzg.rs:182-185), the batch cut by blob across the members."""
+        return _commit_blobs(lambda *a: self.check(lib.kzgb_group_commit_blobs(self.h, *a)), blobs)
 
     def commit_coeff_form(self, polynomial: "PolynomialCoeffForm") -> Affine:
         """KZG::commit_coeff_form with the points cut into one range per GPU (prover/src/kzg.rs:107-125)."""
@@ -539,6 +553,12 @@ class KZG:
         """kzg.rs:182-185."""
         e = srs.engine
         return e._point_call(lambda h, *a: lib.kzgb_commit_blob(h, blob.blob_data, len(blob.blob_data), *a))
+
+    @staticmethod
+    def commit_blobs(blobs: Sequence[Blob], srs: SRS) -> List[Affine]:
+        """commit_blob (kzg.rs:182-185) for every blob, pipelined inside the library; no proofs, no transcripts."""
+        e = srs.engine
+        return _commit_blobs(lambda *a: e.check(lib.kzgb_commit_blobs(e.h, *a)), blobs)
 
     def compute_proof(self, polynomial: PolynomialEvalForm, z_fr: int, srs: SRS) -> Affine:
         """kzg.rs:215-234 (+ compute_proof_impl :128-178)."""

@@ -68,6 +68,8 @@ SIGNATURES = {
         C.c_int,
         [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf],
     ),
+    "kzgb_commit_blobs": (C.c_int, [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf]),
+    "kzgb_commit_blobs_dev": (C.c_int, [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf]),
     "kzgb_verify_batch_rlc": (
         C.c_int,
         [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf,
@@ -106,6 +108,7 @@ SIGNATURES = {
     "kzgb_group_srs_prepare_lagrange": (C.c_int, [grp_p, C.c_size_t]),
     "kzgb_group_srs_precompute_ranges": (C.c_int, [grp_p, C.c_size_t, C.c_int]),
     "kzgb_group_commit_and_prove_blobs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf]),
+    "kzgb_group_commit_blobs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf]),
     "kzgb_group_msm_srs": (C.c_int, [grp_p, buf, C.c_size_t, buf, C.POINTER(C.c_uint8)]),
 }
 

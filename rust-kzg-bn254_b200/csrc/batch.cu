@@ -1,5 +1,6 @@
 // The blob-batch pipelines: kzgb_commit_and_prove_blobs{,_dev} -- commitment and proof of many blobs on several lanes
-// while a hashing stage produces the Fiat-Shamir transcripts -- and kzgb_verify_batch_rlc.
+// while a hashing stage produces the Fiat-Shamir transcripts --, kzgb_commit_blobs{,_dev} -- the commitments alone, on
+// the same plan and lanes -- and kzgb_verify_batch_rlc.
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
@@ -100,15 +101,18 @@ HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible) {
 }
 
 // ---------------------------------------------------------------- planning
-// One kzgb_commit_and_prove_blobs{,_dev} call: its arguments and the plan made for them.
+// One kzgb_commit_and_prove_blobs{,_dev} or kzgb_commit_blobs{,_dev} call: its arguments and the plan made for them.
 struct Batch {
     kzgb_ctx* c;
     const uint8_t* const* blobs_dev;   // nullptr: the blobs are only on the host
-    const uint8_t* const* blobs_host;  // the transcripts are hashed from these
+    const uint8_t* const* blobs_host;  // the transcripts are hashed from these (commit-only with blobs_dev: nullptr)
     const size_t* lens;
     size_t count;
     uint8_t* commitments32;
     uint8_t* proofs32;
+    bool commit_only = false;  // kzgb_commit_blobs: commitments into out_xy / out_inf, no proofs
+    uint64_t* out_xy = nullptr;
+    uint8_t* out_inf = nullptr;
     size_t max_n = 0;
     std::vector<std::pair<size_t, size_t>> groups;  // small blobs: (first blob, blobs); empty: one blob per task
     int n_lanes = 0;
@@ -117,14 +121,20 @@ struct Batch {
     bool resident = false;
 };
 
-// Validation, groups, lanes and the tables every size of the batch needs.
+// Validation, groups, lanes and the tables every size of the batch needs.  A commit-only batch checks every blob as
+// kzgb_commit_blob does (a blob of length 0 commits the zero polynomial of size 1); with proofs, length 0 is
+// compute_blob_proof's error.
 int plan_batch(Batch& b) {
     kzgb_ctx* c = b.c;
     const size_t* lens = b.lens;
     const size_t count = b.count;
     for (size_t i = 0; i < count; i++) {
-        if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
-        if (int rc = check_srs_capacity(c, blob_poly_len(lens[i]))) return rc;
+        if (b.commit_only) {
+            if (int rc = check_commit_blob_len(c, blob_poly_len(lens[i]))) return rc;
+        } else {
+            if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
+            if (int rc = check_srs_capacity(c, blob_poly_len(lens[i]))) return rc;
+        }
         b.max_n = std::max(b.max_n, blob_poly_len(lens[i]));
     }
     // Small blobs (<= 2^17 Fr): runs of equal-size blobs are processed as groups, every kernel of a phase
@@ -380,10 +390,81 @@ int run_lanes(const Batch& b, F lane_main) {
     return KZGB_OK;
 }
 
+// The commitment phase of one group: bn blobs of one size n from blob i0, ONE batched launch set; pts[k] is the
+// commitment of blob i0 + k.  With proofs to follow, or without a Lagrange table, the blob bytes become Montgomery
+// evaluations in L.evals (which the proof phase reads).  A commit-only group over a Lagrange table hands the bytes to
+// the MSM's first pass instead: laid out at a stride of 32 n with zero-filled tails (device blobs that already are
+// back to back and full are read in place), so that one launch covers the group.
+int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
+    kzgb_ctx* c = b.c;
+    const uint8_t* const* blobs_dev = b.blobs_dev;
+    const size_t* lens = b.lens;
+    const size_t n = blob_poly_len(lens[i0]);
+    const int logn = log2_exact(n);
+    const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
+    const bool from_bytes = b.commit_only && lag;
+    Fr ninv = ninv_mont(logn);
+    int r = KZGB_OK;
+    auto ck = [&](cudaError_t e, const char* what) {
+        if (!r && e != cudaSuccess) r = fail(c, KZGB_ERR_DEVICE, std::string("CUDA error: ") + cudaGetErrorString(e) + " at " + what);
+    };
+    bool full = true;  // every blob fills its polynomial: one conversion launch for the group
+    for (size_t k = 0; k < bn; k++) full = full && lens[i0 + k] == n * 32;
+    bool dev_run = blobs_dev && full;  // device blobs back to back: one conversion launch too
+    for (size_t k = 0; k < bn && dev_run; k++) dev_run = blobs_dev[i0 + k] == blobs_dev[i0] + k * n * 32;
+    if (!from_bytes) {
+        ck(L.evals.reserve(bn * n * sizeof(Fr)), "evals");
+        ck(L.work.reserve(bn * n * sizeof(Fr)), "work");
+    }
+    if (!b.commit_only) {  // the proof phase's buffers
+        ck(L.small.reserve((3 * bn + 8) * sizeof(Fr)), "small");
+        ck(L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)bn) * sizeof(Fr)), "eval scratch");
+    }
+    if (!lag) ck(L.ntt_scratch.reserve(bn * n * sizeof(Fr)), "ntt scratch");
+    if (from_bytes ? !dev_run : !blobs_dev) ck(L.bytes.reserve(bn * n * 32), "bytes");
+    MsmJob job;
+    if (from_bytes) {
+        for (size_t k = 0; k < bn && !r && !dev_run; k++) {
+            uint8_t* dst = (uint8_t*)L.bytes.p + k * n * 32;
+            const size_t len = lens[i0 + k];
+            if (len) {
+                if (blobs_dev) ck(cudaMemcpyAsync(dst, blobs_dev[i0 + k], len, cudaMemcpyDeviceToDevice, L.st), "D2D copy of a blob");
+                else ck(cudaMemcpyAsync(dst, b.blobs_host[i0 + k], len, cudaMemcpyHostToDevice, L.st), "H2D copy of a blob");
+            }
+            if (len < n * 32) ck(cudaMemsetAsync(dst + len, 0, n * 32 - len, L.st), "zero fill");
+        }
+        const uint8_t* src = dev_run ? blobs_dev[i0] : (const uint8_t*)L.bytes.p;
+        if (!r) r = commit_blob_enqueue(c, L, src, (uint64_t)bn * n * 32, n, bn, lag, &job);
+        if (!r) r = msm_finish_batched(c, L, job, bn, pts);
+        return r;
+    }
+    if (dev_run) bytes_to_fr_launch(blobs_dev[i0], (uint64_t)bn * n * 32, (Fr*)L.evals.p, (uint32_t)(bn * n), L.st);
+    for (size_t k = 0; k < bn && !r && !dev_run; k++) {
+        const uint8_t* src = blobs_dev ? blobs_dev[i0 + k] : nullptr;
+        if (!src) {
+            uint8_t* dst = (uint8_t*)L.bytes.p + k * n * 32;
+            ck(cudaMemcpyAsync(dst, b.blobs_host[i0 + k], lens[i0 + k], cudaMemcpyHostToDevice, L.st), "H2D copy of a blob");
+            src = dst;
+        }
+        if (!full || blobs_dev) bytes_to_fr_launch(src, lens[i0 + k], (Fr*)L.evals.p + k * n, (uint32_t)n, L.st);
+    }
+    if (!r && full && !blobs_dev) bytes_to_fr_launch((const uint8_t*)L.bytes.p, (uint64_t)bn * n * 32, (Fr*)L.evals.p, (uint32_t)(bn * n), L.st);
+    if (!r) {
+        const Fr* sc = (const Fr*)L.evals.p;
+        if (!lag) {
+            ck(cudaMemcpyAsync(L.work.p, L.evals.p, bn * n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st), "copy");
+            ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+            sc = (const Fr*)L.work.p;
+        }
+        if (!r) r = msm_enqueue_batched(c, L, sc, n, bn, lag, &job);
+    }
+    if (!r) r = msm_finish_batched(c, L, job, bn, pts);
+    return r;
+}
+
 // Small blobs: groups of equal-size blobs, each phase of a group is ONE batched launch set.
 int group_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next_group, int li) {
     kzgb_ctx* c = b.c;
-    const uint8_t* const* blobs_dev = b.blobs_dev;
     const size_t* lens = b.lens;
     Lane& L = c->lanes[li];
     std::vector<Affine> pts;
@@ -397,44 +478,12 @@ int group_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next_group, i
         const int logn = log2_exact(n);
         const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
         Fr ninv = ninv_mont(logn);
-        int r = KZGB_OK;
+        pts.resize(bn);
+        int r = group_commit(b, L, i0, bn, pts.data());
         auto ck = [&](cudaError_t e, const char* what) {
             if (!r && e != cudaSuccess) r = fail(c, KZGB_ERR_DEVICE, std::string("CUDA error: ") + cudaGetErrorString(e) + " at " + what);
         };
-        ck(L.evals.reserve(bn * n * sizeof(Fr)), "evals");
-        ck(L.work.reserve(bn * n * sizeof(Fr)), "work");
-        ck(L.small.reserve((3 * bn + 8) * sizeof(Fr)), "small");
-        ck(L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)bn) * sizeof(Fr)), "eval scratch");
-        if (!lag) ck(L.ntt_scratch.reserve(bn * n * sizeof(Fr)), "ntt scratch");
-        if (!blobs_dev) ck(L.bytes.reserve(bn * n * 32), "bytes");
-        bool full = true;  // every blob fills its polynomial: one conversion launch for the group
-        for (size_t k = 0; k < bn; k++) full = full && lens[i0 + k] == n * 32;
-        bool dev_run = blobs_dev && full;  // device blobs back to back: one conversion launch too
-        for (size_t k = 0; k < bn && dev_run; k++) dev_run = blobs_dev[i0 + k] == blobs_dev[i0] + k * n * 32;
-        if (dev_run) bytes_to_fr_launch(blobs_dev[i0], (uint64_t)bn * n * 32, (Fr*)L.evals.p, (uint32_t)(bn * n), L.st);
-        for (size_t k = 0; k < bn && !r && !dev_run; k++) {
-            const uint8_t* src = blobs_dev ? blobs_dev[i0 + k] : nullptr;
-            if (!src) {
-                uint8_t* dst = (uint8_t*)L.bytes.p + k * n * 32;
-                ck(cudaMemcpyAsync(dst, b.blobs_host[i0 + k], lens[i0 + k], cudaMemcpyHostToDevice, L.st), "H2D copy of a blob");
-                src = dst;
-            }
-            if (!full || blobs_dev) bytes_to_fr_launch(src, lens[i0 + k], (Fr*)L.evals.p + k * n, (uint32_t)n, L.st);
-        }
-        if (!r && full && !blobs_dev) bytes_to_fr_launch((const uint8_t*)L.bytes.p, (uint64_t)bn * n * 32, (Fr*)L.evals.p, (uint32_t)(bn * n), L.st);
-        // commitments
         MsmJob job;
-        pts.resize(bn);
-        if (!r) {
-            const Fr* sc = (const Fr*)L.evals.p;
-            if (!lag) {
-                ck(cudaMemcpyAsync(L.work.p, L.evals.p, bn * n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st), "copy");
-                ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-                sc = (const Fr*)L.work.p;
-            }
-            if (!r) r = msm_enqueue_batched(c, L, sc, n, bn, lag, &job);
-        }
-        if (!r) r = msm_finish_batched(c, L, job, bn, pts.data());
         if (!r) {
             for (size_t k = 0; k < bn; k++) serialize_compressed(pts[k], b.commitments32 + 32 * (i0 + k));
             // challenges: the transcript midstates come from the hashing stage
@@ -557,6 +606,66 @@ int commit_and_prove(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t
     return rc;
 }
 
+// ---------------------------------------------------------------- commitments only
+// Small blobs: the groups' commitment phase and nothing else.
+int commit_group_lane(const Batch& b, std::atomic<size_t>& next_group, std::atomic<bool>& failed, int li) {
+    Lane& L = b.c->lanes[li];
+    std::vector<Affine> pts;
+    for (;;) {
+        const size_t gi = next_group.fetch_add(1);
+        if (gi >= b.groups.size() || failed.load()) return KZGB_OK;
+        const size_t i0 = b.groups[gi].first, bn = b.groups[gi].second;
+        pts.resize(bn);
+        if (int r = group_commit(b, L, i0, bn, pts.data())) { failed.store(true); return r; }
+        for (size_t k = 0; k < bn; k++) affine_to_abi(pts[k], b.out_xy + 8 * (i0 + k), b.out_inf ? b.out_inf + i0 + k : nullptr);
+    }
+}
+
+// Large blobs: every task is "commit blob i", taken in blob order.  A blob is read once, so it goes up into the lane's
+// own buffer; over a Lagrange table the MSM reads its bytes, otherwise they are converted, inverse-transformed and
+// committed over the monomial table (commit_evals_enqueue).
+int commit_task_lane(const Batch& b, std::atomic<size_t>& next, std::atomic<bool>& failed, int li) {
+    kzgb_ctx* c = b.c;
+    Lane& L = c->lanes[li];
+    for (;;) {
+        const size_t i = next.fetch_add(1);
+        if (i >= b.count || failed.load()) return KZGB_OK;
+        const size_t len = b.lens[i], n = blob_poly_len(len);
+        const kzgb_ctx::LagTable* lag = lagrange_table(c, log2_exact(n));
+        const uint8_t* blob_host = b.blobs_dev ? nullptr : b.blobs_host[i];
+        const uint8_t* dev_bytes = b.blobs_dev ? b.blobs_dev[i] : nullptr;
+        MsmJob job;
+        Affine out;
+        int r = KZGB_OK;
+        if (lag) {
+            if (!dev_bytes) {
+                r = blob_upload(c, L, blob_host, len);
+                dev_bytes = (const uint8_t*)L.bytes.p;
+            }
+            if (!r) r = commit_blob_enqueue(c, L, dev_bytes, len, n, 1, lag, &job);
+        } else {
+            r = blob_to_evals(c, L, blob_host, dev_bytes, len, n);
+            if (!r) r = commit_evals_enqueue(c, L, (Fr*)L.evals.p, n, &job);
+        }
+        if (!r) r = msm_finish(c, L, job, &out);
+        if (r) { failed.store(true); return r; }
+        affine_to_abi(out, b.out_xy + 8 * i, b.out_inf ? b.out_inf + i : nullptr);
+    }
+}
+
+int commit_blobs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
+                 size_t count, uint64_t* out_xy, uint8_t* out_inf) {
+    if (count == 0) return KZGB_OK;
+    Batch b{c, blobs_dev, blobs_host, lens, count, nullptr, nullptr, true, out_xy, out_inf};
+    int rc = plan_batch(b);
+    if (rc) return rc;
+    std::atomic<size_t> next{0};
+    std::atomic<bool> failed{false};
+    return run_lanes(b, [&](int li) {
+        return b.groups.empty() ? commit_task_lane(b, next, failed, li) : commit_group_lane(b, next, failed, li);
+    });
+}
+
 // The random linear combination of m validated and evaluated openings (batch.rs:76-249): d_bases holds C_0 .. C_{m-1},
 // pi_0 .. pi_{m-1} and room for one more point.
 int rlc_combine(kzgb_ctx* c, Lane& L, const std::vector<Affine>& Cs, const std::vector<Affine>& Ps,
@@ -617,6 +726,16 @@ int kzgb_commit_and_prove_blobs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev
                                     const size_t* lens, size_t count, uint8_t* commitments32, uint8_t* proofs32) {
     Guard g(c);
     return commit_and_prove(c, blobs_dev, blobs_host, lens, count, commitments32, proofs32);
+}
+int kzgb_commit_blobs(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count, uint64_t* out_xy,
+                      uint8_t* out_inf) {
+    Guard g(c);
+    return commit_blobs(c, nullptr, blobs, lens, count, out_xy, out_inf);
+}
+int kzgb_commit_blobs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const size_t* lens, size_t count,
+                          uint64_t* out_xy, uint8_t* out_inf) {
+    Guard g(c);
+    return commit_blobs(c, blobs_dev, nullptr, lens, count, out_xy, out_inf);
 }
 // ------------------------------------------------------------------------------- batch verification (RLC)
 int kzgb_verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,

@@ -41,6 +41,10 @@ int check_srs_capacity(kzgb_ctx* c, size_t n) {
     snprintf(msg, sizeof msg, "SRS capacity exceeded: polynomial_len=%zu srs_len=%zu", n, c->srs_n);
     return fail(c, KZGB_ERR_SRS_CAPACITY, msg);
 }
+int check_commit_blob_len(kzgb_ctx* c, size_t n) {
+    if (n > ((size_t)1 << 28)) return fail(c, KZGB_ERR_GENERIC, "Input size exceeds maximum polynomial size");
+    return check_srs_capacity(c, n);
+}
 
 // The MSM gathers 64-byte points at random from tables far larger than L2: with the default fetch granularity a
 // miss pulls the whole 128-byte line and doubles the DRAM traffic of the accumulation.  The limit is device-wide,
@@ -406,15 +410,17 @@ int srs_install(kzgb_ctx* c, Affine* dev_points, size_t n) {
 // ---------------------------------------------------------------- MSM
 // Launch plan p on lane L in the lane's workspace and queue the copies of its window sums (and, for the statistics, of
 // the length of its sorted list) to the host; msm_finish picks them up.
+// d_blob != nullptr: the scalars are read from blob_len bytes of blob data instead (msm_launch_blob).
 int msm_enqueue_plan(kzgb_ctx* c, Lane& L, const MsmPlan& p, const Fr* d_scalars, bool canonical, const Affine* table,
-                     MsmJob* job) {
+                     MsmJob* job, const uint8_t* d_blob = nullptr, uint64_t blob_len = 0) {
     CK(c, L.msm_ws.reserve(msm_workspace_bytes(p)));
     MsmWorkspace ws;
     msm_workspace_carve(p, L.msm_ws.p, &ws);
     lane_collect_acc(L);
     trace_mark(c, L, 0, L.st);
     cudaEvent_t tr1 = trace_event(c, L, 1), tr2 = trace_event(c, L, 2);
-    msm_launch(p, ws, d_scalars, canonical, table, L.st, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1, L.st_acc, L.ev_fork, L.ev_join);
+    if (d_blob) msm_launch_blob(p, ws, d_blob, blob_len, table, L.st, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1, L.st_acc, L.ev_fork, L.ev_join);
+    else msm_launch(p, ws, d_scalars, canonical, table, L.st, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1, L.st_acc, L.ev_fork, L.ev_join);
     trace_mark(c, L, 3, L.st);
     trace_mark(c, L, 10, nullptr);
     L.ev_pending = !tr1;
@@ -592,6 +598,16 @@ int msm_enqueue_batched(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t n_per,
     if ((uint64_t)n_per * batch * p.W >= 0xfff00000ull) return fail(c, KZGB_ERR_GENERIC, "MSM too large for one launch");
     return msm_enqueue_plan(c, L, p, d_scalars, false, table, job);
 }
+// Commitments of `batch` blobs over the Lagrange table `lag` of their size n, in ONE MSM whose first pass reads the
+// blob bytes (no Montgomery form in between): blob k at d_bytes + 32 n k, len bytes in all, zero past len.  The
+// result is read with msm_finish_batched (or msm_finish when batch == 1).
+int commit_blob_enqueue(kzgb_ctx* c, Lane& L, const uint8_t* d_bytes, uint64_t len, size_t n, size_t batch,
+                        const kzgb_ctx::LagTable* lag, MsmJob* job) {
+    if (batch > (size_t)MAX_SETS) return fail(c, KZGB_ERR_GENERIC, "too many MSMs in one batch");
+    const MsmPlan p = msm_make_plan((uint32_t)(n * batch), lag->c, true, (uint32_t)lag->n, 0, (uint32_t)batch);
+    if ((uint64_t)n * batch * p.W >= 0xfff00000ull) return fail(c, KZGB_ERR_GENERIC, "MSM too large for one launch");
+    return msm_enqueue_plan(c, L, p, nullptr, false, lag->table, job, d_bytes, len);
+}
 int msm_finish_batched(kzgb_ctx* c, Lane& L, const MsmJob& job, size_t batch, Affine* outs) {
     if (!job.active) { for (size_t k = 0; k < batch; k++) aff_set_inf(outs[k]); return KZGB_OK; }
     int rc = lane_wait(c, L);
@@ -654,13 +670,19 @@ int proof_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z
 
 size_t blob_poly_len(size_t len) { return next_pow2((len + 31) / 32); }  // Rust: 0usize.next_power_of_two() == 1
 
+// blob bytes on the host -> L.bytes
+int blob_upload(kzgb_ctx* c, Lane& L, const uint8_t* blob_host, size_t len) {
+    CK(c, L.bytes.reserve(len ? len : 32));
+    if (len) CK(c, cudaMemcpyAsync(L.bytes.p, blob_host, len, cudaMemcpyHostToDevice, L.st));
+    return KZGB_OK;
+}
+
 // blob bytes on the host -> L.evals (n Fr Montgomery)
 int blob_to_evals(kzgb_ctx* c, Lane& L, const uint8_t* blob_host, const uint8_t* blob_dev, size_t len, size_t n) {
     CK(c, L.evals.reserve(n * sizeof(Fr)));
     const uint8_t* src = blob_dev;
     if (!src) {
-        CK(c, L.bytes.reserve(len ? len : 32));
-        if (len) CK(c, cudaMemcpyAsync(L.bytes.p, blob_host, len, cudaMemcpyHostToDevice, L.st));
+        if (int rc = blob_upload(c, L, blob_host, len)) return rc;
         src = (const uint8_t*)L.bytes.p;
     }
     bytes_to_fr_launch(src, len, (Fr*)L.evals.p, (uint32_t)n, L.st);
@@ -1175,8 +1197,7 @@ int kzgb_commit_blob(kzgb_ctx* c, const uint8_t* blob, size_t len, uint64_t out_
     Guard g(c);
     Lane& L = c->lanes[0];
     size_t n = blob_poly_len(len);
-    if (n > ((size_t)1 << 28)) return fail(c, KZGB_ERR_GENERIC, "Input size exceeds maximum polynomial size");
-    if (int rc = check_srs_capacity(c, n)) return rc;
+    if (int rc = check_commit_blob_len(c, n)) return rc;
     int rc = ensure_lagrange(c, log2_exact(n));
     if (rc) return rc;
     rc = blob_to_evals(c, L, blob, nullptr, len, n);

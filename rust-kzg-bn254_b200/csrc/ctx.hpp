@@ -130,6 +130,8 @@ int fail(kzgb_ctx* c, int code, const std::string& msg);
     } while (0)
 // KZGB_ERR_SRS_CAPACITY unless a polynomial of n coefficients fits the loaded SRS (kzg.rs:89-94)
 int check_srs_capacity(kzgb_ctx* c, size_t n);
+// kzgb_commit_blob's checks of a blob whose polynomial has n elements: at most 2^28 (polynomial.rs), then check_srs_capacity
+int check_commit_blob_len(kzgb_ctx* c, size_t n);
 
 // Holds the context's lock and makes its device current for the length of an entry point.
 struct Guard {
@@ -173,10 +175,13 @@ int msm_blocking(kzgb_ctx* c, Lane& L, const Fr* d_scalars, bool canonical, size
 int msm_enqueue_batched(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t n_per, size_t batch,
                         const kzgb_ctx::LagTable* lag, MsmJob* job);
 int msm_finish_batched(kzgb_ctx* c, Lane& L, const MsmJob& job, size_t batch, Affine* outs);
+int commit_blob_enqueue(kzgb_ctx* c, Lane& L, const uint8_t* d_bytes, uint64_t len, size_t n, size_t batch,
+                        const kzgb_ctx::LagTable* lag, MsmJob* job);
 int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJob* job);
 int eval_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z, Fr* d_quotient);
 int eval_read_y(kzgb_ctx* c, Lane& L, Fr* y);
 int proof_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z_mont, MsmJob* job);
+int blob_upload(kzgb_ctx* c, Lane& L, const uint8_t* blob_host, size_t len);
 int blob_to_evals(kzgb_ctx* c, Lane& L, const uint8_t* blob_host, const uint8_t* blob_dev, size_t len, size_t n);
 int validate_points_dev(kzgb_ctx* c, Lane& L, const Affine* d_pts, size_t n);
 

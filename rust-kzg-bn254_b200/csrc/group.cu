@@ -58,6 +58,21 @@ void share(size_t n, int G, int i, size_t align, size_t* first, size_t* count) {
     *first = a; *count = b - a;
 }
 
+// cut points of a blob batch: member i takes blobs [cut[i], cut[i+1]) with about 1/G of the bytes
+std::vector<size_t> byte_balanced_cut(const size_t* lens, size_t count, int G) {
+    size_t total = 0;
+    for (size_t k = 0; k < count; k++) total += lens[k];
+    std::vector<size_t> cut(G + 1, count);
+    cut[0] = 0;
+    size_t acc = 0, k = 0;
+    for (int i = 1; i < G; i++) {
+        const size_t target = (size_t)((__uint128_t)total * i / G);
+        while (k < count && acc + lens[k] / 2 < target) acc += lens[k++];
+        cut[i] = k;
+    }
+    return cut;
+}
+
 int replicate_from_member0(kzgb_group* g) {
     return for_members(g, [&](int i) { return i == 0 ? KZGB_OK : kzgb_srs_clone(g->ctx[i], g->ctx[0]); });
 }
@@ -170,22 +185,24 @@ int kzgb_group_commit_and_prove_blobs(kzgb_group* g, const uint8_t* const* blobs
                                       uint8_t* commitments32, uint8_t* proofs32) {
     std::lock_guard<std::mutex> lk(g->mu);
     if (count == 0) return KZGB_OK;
-    const int G = (int)g->ctx.size();
-    // cut points: member i takes blobs [cut[i], cut[i+1]) with about 1/G of the bytes each
-    size_t total = 0;
-    for (size_t k = 0; k < count; k++) total += lens[k];
-    std::vector<size_t> cut(G + 1, count);
-    cut[0] = 0;
-    size_t acc = 0, k = 0;
-    for (int i = 1; i < G; i++) {
-        const size_t target = (size_t)((__uint128_t)total * i / G);
-        while (k < count && acc + lens[k] / 2 < target) acc += lens[k++];
-        cut[i] = k;
-    }
+    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
     return for_members(g, [&](int i) {
         const size_t a = cut[i], b = cut[i + 1];
         if (a >= b) return (int)KZGB_OK;
         return kzgb_commit_and_prove_blobs(g->ctx[i], blobs + a, lens + a, b - a, commitments32 + 32 * a, proofs32 + 32 * a);
+    });
+}
+
+// KZG::commit_blob (prover/src/kzg.rs:182-185) for `count` blobs, cut as kzgb_group_commit_and_prove_blobs cuts them.
+int kzgb_group_commit_blobs(kzgb_group* g, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                            uint64_t* out_xy, uint8_t* out_inf) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    if (count == 0) return KZGB_OK;
+    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
+    return for_members(g, [&](int i) {
+        const size_t a = cut[i], b = cut[i + 1];
+        if (a >= b) return (int)KZGB_OK;
+        return kzgb_commit_blobs(g->ctx[i], blobs + a, lens + a, b - a, out_xy + 8 * a, out_inf ? out_inf + a : nullptr);
     });
 }
 

@@ -75,6 +75,40 @@ void msm_launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scal
                         cudaEvent_t ev_join = nullptr);
 void msm_launch_reduce(const MsmPlan& p, const MsmWorkspace& ws, const XYZZ* buckets, cudaStream_t st);
 void msm_merge_buckets(XYZZ* dst, const XYZZ* src, uint32_t nbuckets, cudaStream_t st);
+// msm_launch with the scalars read from blob bytes (blob_element below, reduced mod r) by the first sort pass: for
+// commitments over a Lagrange table, where the evaluations of the blob are the scalars and nothing needs their
+// Montgomery form.  A batched plan reads blob k at blob + 32 * batch_n * k.
+void msm_launch_blob(const MsmPlan& p, const MsmWorkspace& ws, const uint8_t* blob, uint64_t len_bytes,
+                     const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin = nullptr,
+                     cudaEvent_t ev_acc_end = nullptr, cudaStream_t st_acc = nullptr, cudaEvent_t ev_fork = nullptr,
+                     cudaEvent_t ev_join = nullptr);
+
+// Element i of blob bytes (primitives/src/helpers.rs:40-57): the 32 big-endian bytes at offset 32 i as a 256-bit
+// integer, the last partial chunk right-padded with zeros, zero past len.  Not reduced mod r.
+__device__ __forceinline__ Fr blob_element(const uint8_t* __restrict__ in, uint64_t len, uint32_t i) {
+    const uint64_t off = (uint64_t)i * 32;
+    Fr v;
+    if (off >= len) { fe_zero(v); return v; }
+    uint32_t be[8];
+    if (off + 32 <= len && ((uintptr_t)in & 15) == 0) {
+        const uint4* q = reinterpret_cast<const uint4*>(in + off);
+        uint4 a = __ldg(q), b = __ldg(q + 1);
+        be[0] = a.x; be[1] = a.y; be[2] = a.z; be[3] = a.w;
+        be[4] = b.x; be[5] = b.y; be[6] = b.z; be[7] = b.w;
+    } else {
+        for (int k = 0; k < 8; k++) {
+            uint32_t w = 0;
+            for (int j = 0; j < 4; j++) {
+                uint64_t p = off + 4 * k + j;
+                uint32_t byte = p < len ? in[p] : 0u;
+                w |= byte << (8 * j);
+            }
+            be[k] = w;
+        }
+    }
+    for (int k = 0; k < 8; k++) v.l[7 - k] = __byte_perm(be[k], 0, 0x0123);
+    return v;
+}
 
 // ---- SRS ------------------------------------------------------------------------
 // gnark big-endian compressed points -> affine Montgomery (n < 2^30 per launch).  err[0] must be preset to

@@ -4,6 +4,7 @@
 //
 // Pipeline (all on one stream, no host sync):
 //   1. k_digits_hist     scalar -> canonical -> W signed c-bit digits; histogram of bucket keys
+//                        (k_digits_hist_blob: the same from blob bytes, for commit-only blob batches)
 //   2. k_scan            exclusive scan of the histogram (bucket offsets)
 //   3. k_scatter         counting-sort scatter: point refs grouped by bucket (order inside a
 //                        bucket is irrelevant: group addition is commutative and exact)
@@ -47,12 +48,9 @@ __device__ __forceinline__ uint32_t signed_digit(const uint32_t* l, int w, int c
     return d;
 }
 
-__global__ void __launch_bounds__(256) k_digits_hist(const Fr* __restrict__ scalars, bool canonical, MsmPlan p,
-                                                      Fr* __restrict__ canon, uint32_t* __restrict__ hist) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= p.n) return;
-    Fr s = fe_load_ro(&scalars[i]);
-    if (!canonical) fe_from_mont(s, s);
+// canonical scalar i -> canon[i], and its digits into the bucket histogram
+__device__ __forceinline__ void digits_hist(const Fr& s, uint32_t i, const MsmPlan& p, Fr* __restrict__ canon,
+                                            uint32_t* __restrict__ hist) {
     fe_store(&canon[i], s);
     uint32_t half = 1u << (p.c - 1);
     uint32_t carry = 0;
@@ -64,6 +62,49 @@ __global__ void __launch_bounds__(256) k_digits_hist(const Fr* __restrict__ scal
             atomicAdd(&hist[key], 1u);
         }
     }
+}
+
+__global__ void __launch_bounds__(256) k_digits_hist(const Fr* __restrict__ scalars, bool canonical, MsmPlan p,
+                                                      Fr* __restrict__ canon, uint32_t* __restrict__ hist) {
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= p.n) return;
+    Fr s = fe_load_ro(&scalars[i]);
+    if (!canonical) fe_from_mont(s, s);
+    digits_hist(s, i, p, canon, hist);
+}
+
+// x -= m when x >= m (8 little-endian limbs)
+__device__ __forceinline__ void sub_if_geq(uint32_t* x, const uint32_t* m) {
+    uint32_t t[8];
+    uint32_t borrow = 0;
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+        const uint64_t d = (uint64_t)x[k] - m[k] - borrow;
+        t[k] = (uint32_t)d;
+        borrow = (uint32_t)(d >> 63);
+    }
+#pragma unroll
+    for (int k = 0; k < 8; k++) x[k] = borrow ? x[k] : t[k];
+}
+
+// The first sort pass over blob bytes (msm_launch_blob): scalar i is blob_element(i) mod r.  Every 256-bit value is
+// below 6r, so subtracting 4r, 2r and r where they fit leaves the canonical value.
+__global__ void __launch_bounds__(256) k_digits_hist_blob(const uint8_t* __restrict__ blob, uint64_t len, MsmPlan p,
+                                                           Fr* __restrict__ canon, uint32_t* __restrict__ hist) {
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= p.n) return;
+    Fr s = blob_element(blob, len, i);
+    uint32_t r[8], r2[8], r4[8];
+    FeConst<FR>::mod(r);
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+        r2[k] = (r[k] << 1) | (k ? r[k - 1] >> 31 : 0u);
+        r4[k] = (r[k] << 2) | (k ? r[k - 1] >> 30 : 0u);
+    }
+    sub_if_geq(s.l, r4);
+    sub_if_geq(s.l, r2);
+    sub_if_geq(s.l, r);
+    digits_hist(s, i, p, canon, hist);
 }
 
 // Exclusive scan of the bucket histogram, 32 counters per thread held in registers (8 x 128-bit
@@ -658,16 +699,22 @@ void msm_launch(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scalars, boo
     msm_launch_reduce(p, ws, ws.buckets, st);
 }
 
-// sort + accumulate + stitch: afterwards ws.buckets holds the sum of every bucket (identity where empty)
-void msm_launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scalars, bool scalars_canonical,
-                        const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin, cudaEvent_t ev_acc_end,
-                        cudaStream_t st_acc, cudaEvent_t ev_fork, cudaEvent_t ev_join) {
+// sort + accumulate + stitch: afterwards ws.buckets holds the sum of every bucket (identity where empty).  The scalars
+// come from `scalars`, or from blob bytes when blob != nullptr.
+static void launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scalars, bool scalars_canonical,
+                           const uint8_t* blob, uint64_t blob_len, const Affine* table, cudaStream_t st,
+                           cudaEvent_t ev_acc_begin, cudaEvent_t ev_acc_end, cudaStream_t st_acc, cudaEvent_t ev_fork,
+                           cudaEvent_t ev_join) {
     const bool split = st_acc && ev_fork && ev_join;
     cudaStream_t sa = split ? st_acc : st;
     cudaMemsetAsync(ws.hist, 0, ((size_t)p.nbuckets + 1) * 4, st);
     const uint32_t sb = (uint32_t)g_sort_block.load();
     uint32_t gb = (p.n + sb - 1) / sb;
-    if (p.n) { k_digits_hist<<<gb, sb, 0, st>>>(scalars, scalars_canonical, p, ws.canon, ws.hist); g_launch_count += 2; }
+    if (p.n) {
+        if (blob) k_digits_hist_blob<<<gb, sb, 0, st>>>(blob, blob_len, p, ws.canon, ws.hist);
+        else k_digits_hist<<<gb, sb, 0, st>>>(scalars, scalars_canonical, p, ws.canon, ws.hist);
+        g_launch_count += 2;
+    }
     {
         uint32_t ntiles = (p.nbuckets + SCAN_TILE - 1) / SCAN_TILE;
         k_scan_tiles<<<ntiles, SCAN_THREADS, 0, st>>>(ws.hist, ws.cursor, p.nbuckets, ws.tile_tot, ntiles == 1);
@@ -708,6 +755,19 @@ void msm_launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scal
     }
     KZ_DBG("bucket_fix");
     g_launch_count += 3;  // accumulate, bucket_fix, bucket_fix_long
+}
+
+void msm_launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scalars, bool scalars_canonical,
+                        const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin, cudaEvent_t ev_acc_end,
+                        cudaStream_t st_acc, cudaEvent_t ev_fork, cudaEvent_t ev_join) {
+    launch_buckets(p, ws, scalars, scalars_canonical, nullptr, 0, table, st, ev_acc_begin, ev_acc_end, st_acc, ev_fork, ev_join);
+}
+
+void msm_launch_blob(const MsmPlan& p, const MsmWorkspace& ws, const uint8_t* blob, uint64_t len_bytes,
+                     const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin, cudaEvent_t ev_acc_end,
+                     cudaStream_t st_acc, cudaEvent_t ev_fork, cudaEvent_t ev_join) {
+    launch_buckets(p, ws, nullptr, false, blob, len_bytes, table, st, ev_acc_begin, ev_acc_end, st_acc, ev_fork, ev_join);
+    msm_launch_reduce(p, ws, ws.buckets, st);
 }
 
 // bucket sums -> ws.set_sums (one XYZZ point per bucket set)

@@ -18,32 +18,8 @@ __global__ void __launch_bounds__(256) k_bytes_to_fr(const uint8_t* __restrict__
                                                       uint32_t n) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    uint64_t off = (uint64_t)i * 32;
-    Fr v;
-    if (off >= len) {
-        fe_zero(v);
-        fe_store(&out[i], v);
-        return;
-    }
-    uint32_t be[8];
-    if (off + 32 <= len && ((uintptr_t)in & 15) == 0) {
-        const uint4* q = reinterpret_cast<const uint4*>(in + off);
-        uint4 a = __ldg(q), b = __ldg(q + 1);
-        be[0] = a.x; be[1] = a.y; be[2] = a.z; be[3] = a.w;
-        be[4] = b.x; be[5] = b.y; be[6] = b.z; be[7] = b.w;
-    } else {
-        for (int k = 0; k < 8; k++) {
-            uint32_t w = 0;
-            for (int j = 0; j < 4; j++) {
-                uint64_t p = off + 4 * k + j;
-                uint32_t byte = p < len ? in[p] : 0u;  // trailing partial chunk is right-padded with zeros
-                w |= byte << (8 * j);
-            }
-            be[k] = w;
-        }
-    }
-    for (int k = 0; k < 8; k++) v.l[7 - k] = bswap32(be[k]);
-    fe_to_mont(v, v);  // also reduces any 256-bit value mod r
+    Fr v = blob_element(in, len, i);
+    if ((uint64_t)i * 32 < len) fe_to_mont(v, v);  // also reduces any 256-bit value mod r
     fe_store(&out[i], v);
 }
 

@@ -50,6 +50,10 @@ extern "C" {
                                    out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_commit_and_prove_blobs(ctx: *mut kzgb_ctx, blobs: *const *const u8, lens: *const usize, count: usize,
                                        commitments32: *mut u8, proofs32: *mut u8) -> c_int;
+    pub fn kzgb_commit_blobs(ctx: *mut kzgb_ctx, blobs: *const *const u8, lens: *const usize, count: usize, out_xy: *mut u64,
+                             out_inf: *mut u8) -> c_int;
+    pub fn kzgb_commit_blobs_dev(ctx: *mut kzgb_ctx, blobs_dev: *const *const u8, lens: *const usize, count: usize,
+                                 out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_verify_proof_g1(ctx: *mut kzgb_ctx, c_xy: *const u64, c_inf: u8, proof_xy: *const u64, proof_inf: u8, y: *const u64,
                                 out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_verify_blob_proof_g1(ctx: *mut kzgb_ctx, blob: *const u8, len: usize, c_xy: *const u64, c_inf: u8, proof_xy: *const u64,
@@ -66,6 +70,8 @@ extern "C" {
     pub fn kzgb_group_srs_precompute_ranges(group: *mut kzgb_group, n: usize, window_bits: c_int) -> c_int;
     pub fn kzgb_group_commit_and_prove_blobs(group: *mut kzgb_group, blobs: *const *const u8, lens: *const usize, count: usize,
                                              commitments32: *mut u8, proofs32: *mut u8) -> c_int;
+    pub fn kzgb_group_commit_blobs(group: *mut kzgb_group, blobs: *const *const u8, lens: *const usize, count: usize,
+                                   out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_group_msm_srs(group: *mut kzgb_group, scalars: *const u64, n: usize, out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_verify_batch_rlc(ctx: *mut kzgb_ctx, blobs: *const *const u8, lens: *const usize, count: usize,
                                  commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,

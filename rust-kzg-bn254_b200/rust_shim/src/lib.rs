@@ -337,6 +337,36 @@ impl KZG {
             if rc != 0 { Err(to_err(ctx, rc, d.len().div_ceil(32).next_power_of_two(), srs.g1.len())) } else { Ok(unpack_point(&xy, inf)) }
         })
     }
+    /// Addition next to the reference's API: `commit_blob` for every blob in ONE call, for callers that check blobs
+    /// against the commitments of their certificates.  The batch is cut by bytes across the GPUs of the box
+    /// (`kzgb_group_commit_blobs`) and pipelined on each; no proofs, no transcripts.  Point i is `commit_blob` of blob
+    /// i, and an error is the one `commit_blob` reports for the first blob the library rejects.
+    pub fn commit_blobs(&self, blobs: &[Blob], srs: &SRS) -> Result<Vec<G1Affine>, KzgError> {
+        let ptrs: Vec<*const u8> = blobs.iter().map(|b| b.data().as_ptr()).collect();
+        let lens: Vec<usize> = blobs.iter().map(|b| b.data().len()).collect();
+        let mut xy = vec![0u64; 8 * blobs.len()];
+        let mut inf = vec![0u8; blobs.len()];
+        let gpu = gpu_for(srs)?;
+        let rc = unsafe {
+            ffi::kzgb_group_commit_blobs(gpu.group, ptrs.as_ptr(), lens.as_ptr(), blobs.len(), xy.as_mut_ptr(), inf.as_mut_ptr())
+        };
+        if rc != 0 {
+            let poly_lens = lens.iter().map(|l| l.div_ceil(32).next_power_of_two());
+            let srs_len = srs.g1.len();
+            return Err(match rc {
+                ffi::KZGB_ERR_SRS_CAPACITY => {
+                    let polynomial_len = poly_lens.clone().find(|&n| n > srs_len).unwrap_or(0);
+                    KzgError::SrsCapacityExceeded { polynomial_len, srs_len }
+                }
+                // the group's message names the member; commit_blob's does not
+                ffi::KZGB_ERR_GENERIC if poly_lens.clone().any(|n| n > 1 << 28) => {
+                    KzgError::GenericError("Input size exceeds maximum polynomial size".to_string())
+                }
+                _ => group_err(gpu.group, rc),
+            });
+        }
+        Ok((0..blobs.len()).map(|i| unpack_point(xy[8 * i..8 * i + 8].try_into().unwrap(), inf[i])).collect())
+    }
     pub fn compute_proof(&self, polynomial: &PolynomialEvalForm, z_fr: &Fr, srs: &SRS) -> Result<G1Affine, KzgError> {
         if polynomial.len() != self.expanded_roots_of_unity.len() {
             return Err(KzgError::GenericError("inconsistent length between blob and root of unities".to_string()));
