@@ -434,8 +434,8 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
             if (len < n * 32) ck(cudaMemsetAsync(dst + len, 0, n * 32 - len, L.st), "zero fill");
         }
         const uint8_t* src = dev_run ? blobs_dev[i0] : (const uint8_t*)L.bytes.p;
-        if (!r) r = commit_blob_enqueue(c, L, src, (uint64_t)bn * n * 32, n, bn, lag, &job);
-        if (!r) r = msm_finish_batched(c, L, job, bn, pts);
+        if (!r) r = msm_enqueue(c, L, {nullptr, src, (uint64_t)bn * n * 32}, n, bn, lag, nullptr, 0, &job);
+        if (!r) r = msm_finish(c, L, job, pts);
         return r;
     }
     if (dev_run) bytes_to_fr_launch(blobs_dev[i0], (uint64_t)bn * n * 32, (Fr*)L.evals.p, (uint32_t)(bn * n), L.st);
@@ -456,9 +456,9 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
             ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
             sc = (const Fr*)L.work.p;
         }
-        if (!r) r = msm_enqueue_batched(c, L, sc, n, bn, lag, &job);
+        if (!r) r = msm_enqueue(c, L, {sc}, n, bn, lag, nullptr, 0, &job);
     }
-    if (!r) r = msm_finish_batched(c, L, job, bn, pts);
+    if (!r) r = msm_finish(c, L, job, pts);
     return r;
 }
 
@@ -503,8 +503,8 @@ int group_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next_group, i
             eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)bn, d_z, d_z + bn, c->tw, c->logN, &ninv,
                                  (Fr*)L.eval_scratch.p, (Fr*)L.work.p, d_z + 2 * bn, L.st, !any_in_domain);
             if (!lag) ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-            if (!r) r = msm_enqueue_batched(c, L, (const Fr*)L.work.p, n, bn, lag, &job);
-            if (!r) r = msm_finish_batched(c, L, job, bn, pts.data());
+            if (!r) r = msm_enqueue(c, L, {(const Fr*)L.work.p}, n, bn, lag, nullptr, 0, &job);
+            if (!r) r = msm_finish(c, L, job, pts.data());
         }
         if (r) { hs.fail(); return r; }
         for (size_t k = 0; k < bn; k++) serialize_compressed(pts[k], b.proofs32 + 32 * (i0 + k));
@@ -642,7 +642,7 @@ int commit_task_lane(const Batch& b, std::atomic<size_t>& next, std::atomic<bool
                 r = blob_upload(c, L, blob_host, len);
                 dev_bytes = (const uint8_t*)L.bytes.p;
             }
-            if (!r) r = commit_blob_enqueue(c, L, dev_bytes, len, n, 1, lag, &job);
+            if (!r) r = msm_enqueue(c, L, {nullptr, dev_bytes, len}, n, 1, lag, nullptr, 0, &job);
         } else {
             r = blob_to_evals(c, L, blob_host, dev_bytes, len, n);
             if (!r) r = commit_evals_enqueue(c, L, (Fr*)L.evals.p, n, &job);
@@ -707,9 +707,9 @@ int rlc_combine(kzgb_ctx* c, Lane& L, const std::vector<Affine>& Cs, const std::
     CK(c, cudaMemcpy(d_bases + 2 * m, &G, sizeof(Affine), cudaMemcpyHostToDevice));
     // lhs = sum r^i pi_i (batch.rs:228); rhs = sum r^i (C_i - y_i G) + sum r^i z_i pi_i (batch.rs:245-249),
     // the m generator multiplications folded into ONE extra base: -(sum r^i y_i) * G  (same group element)
-    int rc = msm_blocking(c, L, d_sc, false, 0, m, d_bases + m, lhs);
+    int rc = msm_blocking(c, L, d_sc, 0, m, d_bases + m, lhs);
     if (rc) return rc;
-    return msm_blocking(c, L, d_sc, false, 0, 2 * m + 1, d_bases, rhs);
+    return msm_blocking(c, L, d_sc, 0, 2 * m + 1, d_bases, rhs);
 }
 
 }  // namespace

@@ -226,7 +226,7 @@ cudaEvent_t trace_mark(kzgb_ctx* c, const Lane& L, int kind, cudaStream_t st) {
     c->trace.push_back({lane_index(c, L), kind, ev, host});
     return ev;
 }
-// an event the caller records itself (accumulate begin / end inside msm_launch)
+// an event the caller records itself (accumulate begin / end inside msm_launch_buckets)
 cudaEvent_t trace_event(kzgb_ctx* c, const Lane& L, int kind) {
     if (!c->trace_on.load()) return nullptr;
     cudaEvent_t ev = nullptr;
@@ -408,19 +408,43 @@ int srs_install(kzgb_ctx* c, Affine* dev_points, size_t n) {
 }
 
 // ---------------------------------------------------------------- MSM
-// Launch plan p on lane L in the lane's workspace and queue the copies of its window sums (and, for the statistics, of
-// the length of its sorted list) to the host; msm_finish picks them up.
-// d_blob != nullptr: the scalars are read from blob_len bytes of blob data instead (msm_launch_blob).
-int msm_enqueue_plan(kzgb_ctx* c, Lane& L, const MsmPlan& p, const Fr* d_scalars, bool canonical, const Affine* table,
-                     MsmJob* job, const uint8_t* d_blob = nullptr, uint64_t blob_len = 0) {
+// Enqueue an MSM job on lane L and queue the copies of its set sums (and, for the statistics, of the length of its
+// sorted list) to the host; msm_finish picks them up.  The one place that chooses plan and table: a Lagrange table, a
+// monomial window table covering the SRS range (built lazily for a single MSM while no batch drives the lanes: lane
+// threads only read the tables), else the variable-base plan over the points themselves.
+int msm_enqueue(kzgb_ctx* c, Lane& L, const MsmScalars& scalars, size_t n, size_t batch, const kzgb_ctx::LagTable* lag,
+                const Affine* var_bases, size_t first, MsmJob* job) {
+    job->results = batch;
+    if (n == 0 || batch == 0) { job->active = false; return KZGB_OK; }
+    if (batch > (size_t)MAX_SETS) return fail(c, KZGB_ERR_GENERIC, "too many MSMs in one batch");
+    const Affine* table = nullptr;  // fixed-base window table
+    int cb = 0;
+    size_t stride = 0, offset = 0;
+    if (lag) {
+        table = lag->table; cb = lag->c; stride = lag->n;
+    } else if (!var_bases) {
+        if (first > c->srs_n || n > c->srs_n - first) return fail(c, KZGB_ERR_GENERIC, "MSM range exceeds the SRS");
+        if (batch == 1 && !c->lanes_running.load())
+            if (int rc = ensure_window_table(c, first, n)) return rc;
+        if (wtable_covers(c, first, n)) { table = c->wtable; cb = c->wt_c; stride = c->wt_n; offset = first - c->wt_first; }
+    }
+    MsmPlan p;
+    if (table) {
+        p = msm_make_plan((uint32_t)(n * batch), cb, true, (uint32_t)stride, (uint32_t)offset, batch > 1 ? (uint32_t)batch : 0);
+    } else {
+        if (batch > 1) return fail(c, KZGB_ERR_GENERIC, "batched MSM needs a fixed-base table");
+        p = msm_make_plan((uint32_t)n, choose_c_var(n), false, 0, 0);
+        table = var_bases ? var_bases : c->srs + first;
+    }
+    if ((uint64_t)n * batch * p.W >= 0xfff00000ull) return fail(c, KZGB_ERR_GENERIC, "MSM too large for one launch");
     CK(c, L.msm_ws.reserve(msm_workspace_bytes(p)));
     MsmWorkspace ws;
     msm_workspace_carve(p, L.msm_ws.p, &ws);
     lane_collect_acc(L);
     trace_mark(c, L, 0, L.st);
     cudaEvent_t tr1 = trace_event(c, L, 1), tr2 = trace_event(c, L, 2);
-    if (d_blob) msm_launch_blob(p, ws, d_blob, blob_len, table, L.st, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1, L.st_acc, L.ev_fork, L.ev_join);
-    else msm_launch(p, ws, d_scalars, canonical, table, L.st, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1, L.st_acc, L.ev_fork, L.ev_join);
+    msm_launch_buckets(p, ws, scalars, table, {L.st, L.st_acc, L.ev_fork, L.ev_join, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1});
+    msm_launch_reduce(p, ws, ws.buckets, L.st);
     trace_mark(c, L, 3, L.st);
     trace_mark(c, L, 10, nullptr);
     L.ev_pending = !tr1;
@@ -429,36 +453,6 @@ int msm_enqueue_plan(kzgb_ctx* c, Lane& L, const MsmPlan& p, const Fr* d_scalars
     job->plan = p;
     job->active = true;
     return KZGB_OK;
-}
-
-// Enqueue an MSM on lane L.  bases == nullptr: over the SRS range [first, first+n).
-// lag != nullptr: over the Lagrange-basis table of the domain of size n instead.
-int msm_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_scalars, bool canonical, size_t first, size_t n,
-                const Affine* var_bases, MsmJob* job, const kzgb_ctx::LagTable* lag = nullptr) {
-    if (n == 0) { job->active = false; return KZGB_OK; }
-    MsmPlan p;
-    const Affine* table;
-    if (lag) {
-        p = msm_make_plan((uint32_t)n, lag->c, true, (uint32_t)lag->n, 0);
-        table = lag->table;
-    } else if (!var_bases) {
-        if (first > c->srs_n || n > c->srs_n - first) return fail(c, KZGB_ERR_GENERIC, "MSM range exceeds the SRS");
-        if (!c->lanes_running.load()) {  // never from the lane threads of a running batch (they only read the tables)
-            if (int rc = ensure_window_table(c, first, n)) return rc;
-        }
-        if (wtable_covers(c, first, n)) {
-            p = msm_make_plan((uint32_t)n, c->wt_c, true, (uint32_t)c->wt_n, (uint32_t)(first - c->wt_first));
-            table = c->wtable;
-        } else {
-            p = msm_make_plan((uint32_t)n, choose_c_var(n), false, 0, 0);
-            table = c->srs + first;
-        }
-    } else {
-        p = msm_make_plan((uint32_t)n, choose_c_var(n), false, 0, 0);
-        table = var_bases;
-    }
-    if ((uint64_t)n * p.W >= 0xfff00000ull) return fail(c, KZGB_ERR_GENERIC, "MSM too large for one launch");
-    return msm_enqueue_plan(c, L, p, d_scalars, canonical, table, job);
 }
 
 // 0: spin on the stream, 1: poll an event with short sleeps, 2: block on an event (option "lane_wait"; -1 = auto: spin
@@ -500,27 +494,31 @@ int lane_wait(kzgb_ctx* c, Lane& L) {
     CK(c, cudaGetLastError());
     return KZGB_OK;
 }
-// Wait for the lane and finish on the host: Horner over the window sums, then to affine.
-int msm_finish(kzgb_ctx* c, Lane& L, const MsmJob& job, Affine* out) {
-    if (!job.active) { aff_set_inf(*out); return KZGB_OK; }
+// Wait for the lane and finish on the host.  A job of one MSM combines its plan's sets by Horner (the W window sums of a
+// variable-base plan, the single set of a fixed-base one); a batched job has one set per MSM.  Then to affine.
+int msm_finish(kzgb_ctx* c, Lane& L, const MsmJob& job, Affine* outs) {
+    if (!job.active) { for (size_t k = 0; k < job.results; k++) aff_set_inf(outs[k]); return KZGB_OK; }
     { int rc = lane_wait(c, L); if (rc) return rc; }
     trace_mark(c, L, 11, nullptr);
     lane_collect_acc(L);
     const MsmPlan& p = job.plan;
-    XYZZ acc = L.h_sets[p.sets - 1];
-    for (int w = p.sets - 2; w >= 0; w--) {
-        for (int k = 0; k < p.c; k++) xyzz_dbl(acc, acc);
-        xyzz_add(acc, L.h_sets[w]);
+    if (job.results == 1) {
+        XYZZ acc = L.h_sets[p.sets - 1];
+        for (int w = p.sets - 2; w >= 0; w--) {
+            for (int k = 0; k < p.c; k++) xyzz_dbl(acc, acc);
+            xyzz_add(acc, L.h_sets[w]);
+        }
+        xyzz_to_affine(outs[0], acc);
+    } else {
+        for (int k = 0; k < p.sets; k++) xyzz_to_affine(outs[k], L.h_sets[k]);
     }
-    xyzz_to_affine(*out, acc);
     trace_mark(c, L, 12, nullptr);
     return KZGB_OK;
 }
 
-int msm_blocking(kzgb_ctx* c, Lane& L, const Fr* d_scalars, bool canonical, size_t first, size_t n,
-                 const Affine* var_bases, Affine* out) {
+int msm_blocking(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t first, size_t n, const Affine* var_bases, Affine* out) {
     MsmJob job;
-    int rc = msm_enqueue(c, L, d_scalars, canonical, first, n, var_bases, &job);
+    int rc = msm_enqueue(c, L, {d_scalars}, n, 1, nullptr, var_bases, first, &job);
     if (rc) return rc;
     return msm_finish(c, L, job, out);
 }
@@ -564,7 +562,7 @@ int msm_srs_host_pipelined(kzgb_ctx* c, Lane& L, const uint64_t* scalars, size_t
         CK(c, cudaEventRecord(c->ev_copied[b], c->copy_st));
         CK(c, cudaStreamWaitEvent(L.st, c->ev_copied[b], 0));
         const MsmPlan p = msm_make_plan((uint32_t)cnt, c->wt_c, true, (uint32_t)c->wt_n, (uint32_t)(first + off - c->wt_first));
-        msm_launch_buckets(p, ws, stage[b], false, c->wtable, L.st, nullptr, nullptr, L.st_acc, L.ev_fork, L.ev_join);
+        msm_launch_buckets(p, ws, {stage[b]}, c->wtable, {L.st, L.st_acc, L.ev_fork, L.ev_join});
         CK(c, cudaEventRecord(c->ev_consumed[b], L.st));
         if (k == 0) CK(c, cudaMemcpyAsync(total, ws.buckets, (size_t)p0.nbuckets * sizeof(XYZZ), cudaMemcpyDeviceToDevice, L.st));
         else msm_merge_buckets(total, ws.buckets, p0.nbuckets, L.st);
@@ -577,52 +575,12 @@ int msm_srs_host_pipelined(kzgb_ctx* c, Lane& L, const uint64_t* scalars, size_t
     return KZGB_OK;
 }
 
-// `batch` independent fixed-base MSMs of n_per scalars each in ONE set of launches (one bucket set per
-// MSM): d_scalars holds batch * n_per scalars back to back.  Over the Lagrange-basis table `lag`, or the
-// monomial window table when lag == nullptr.  Small polynomials are latency-bound one at a time (bucket
-// reduction tail, host hand-off per MSM); batched they fill the GPU.
-int msm_enqueue_batched(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t n_per, size_t batch,
-                        const kzgb_ctx::LagTable* lag, MsmJob* job) {
-    if (n_per == 0 || batch == 0) { job->active = false; return KZGB_OK; }
-    if (batch > (size_t)MAX_SETS) return fail(c, KZGB_ERR_GENERIC, "too many MSMs in one batch");
-    const Affine* table;
-    MsmPlan p;
-    if (lag) {
-        p = msm_make_plan((uint32_t)(n_per * batch), lag->c, true, (uint32_t)lag->n, 0, (uint32_t)batch);
-        table = lag->table;
-    } else {
-        if (!wtable_covers(c, 0, n_per)) return fail(c, KZGB_ERR_GENERIC, "batched MSM needs a fixed-base table");
-        p = msm_make_plan((uint32_t)(n_per * batch), c->wt_c, true, (uint32_t)c->wt_n, 0, (uint32_t)batch);
-        table = c->wtable;
-    }
-    if ((uint64_t)n_per * batch * p.W >= 0xfff00000ull) return fail(c, KZGB_ERR_GENERIC, "MSM too large for one launch");
-    return msm_enqueue_plan(c, L, p, d_scalars, false, table, job);
-}
-// Commitments of `batch` blobs over the Lagrange table `lag` of their size n, in ONE MSM whose first pass reads the
-// blob bytes (no Montgomery form in between): blob k at d_bytes + 32 n k, len bytes in all, zero past len.  The
-// result is read with msm_finish_batched (or msm_finish when batch == 1).
-int commit_blob_enqueue(kzgb_ctx* c, Lane& L, const uint8_t* d_bytes, uint64_t len, size_t n, size_t batch,
-                        const kzgb_ctx::LagTable* lag, MsmJob* job) {
-    if (batch > (size_t)MAX_SETS) return fail(c, KZGB_ERR_GENERIC, "too many MSMs in one batch");
-    const MsmPlan p = msm_make_plan((uint32_t)(n * batch), lag->c, true, (uint32_t)lag->n, 0, (uint32_t)batch);
-    if ((uint64_t)n * batch * p.W >= 0xfff00000ull) return fail(c, KZGB_ERR_GENERIC, "MSM too large for one launch");
-    return msm_enqueue_plan(c, L, p, nullptr, false, lag->table, job, d_bytes, len);
-}
-int msm_finish_batched(kzgb_ctx* c, Lane& L, const MsmJob& job, size_t batch, Affine* outs) {
-    if (!job.active) { for (size_t k = 0; k < batch; k++) aff_set_inf(outs[k]); return KZGB_OK; }
-    int rc = lane_wait(c, L);
-    if (rc) return rc;
-    lane_collect_acc(L);
-    for (size_t k = 0; k < batch; k++) xyzz_to_affine(outs[k], L.h_sets[k]);
-    return KZGB_OK;
-}
-
 // ---------------------------------------------------------------- polynomial pipeline pieces
 // d_evals (n Fr, Montgomery) -> commitment.  Uses L.work / L.ntt_scratch.
 int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJob* job) {
     int logn = log2_exact(n);
     if (const kzgb_ctx::LagTable* lag = lagrange_table(c, logn))  // the evaluations ARE the scalars
-        return msm_enqueue(c, L, d_evals, false, 0, n, nullptr, job, lag);
+        return msm_enqueue(c, L, {d_evals}, n, 1, lag, nullptr, 0, job);
     int rc = ensure_twiddles(c, logn);
     if (rc) return rc;
     CK(c, L.work.reserve(n * sizeof(Fr)));
@@ -631,7 +589,7 @@ int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJ
         CK(c, cudaMemcpyAsync(L.work.p, d_evals, n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st));
     Fr ninv = ninv_mont(logn);
     ntt_launch((Fr*)L.work.p, logn, 1, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-    return msm_enqueue(c, L, (Fr*)L.work.p, false, 0, n, nullptr, job);
+    return msm_enqueue(c, L, {(Fr*)L.work.p}, n, 1, nullptr, nullptr, 0, job);
 }
 
 // y = p(z) into L.small[2] and, unless d_quotient is nullptr, the quotient; the twiddles of size n must be resident.
@@ -1029,7 +987,7 @@ int kzgb_msm_srs_range(kzgb_ctx* c, const uint64_t* scalars, size_t first, size_
     if (!done) {
         CK(c, L.work.reserve(n * sizeof(Fr)));
         CK(c, cudaMemcpyAsync(L.work.p, scalars, n * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-        rc = msm_blocking(c, L, (Fr*)L.work.p, false, first, n, nullptr, &r);
+        rc = msm_blocking(c, L, (Fr*)L.work.p, first, n, nullptr, &r);
     }
     if (rc) return rc;
     affine_to_abi(r, out_xy, out_inf);
@@ -1041,7 +999,7 @@ int kzgb_msm_srs_range_dev(kzgb_ctx* c, const uint64_t* scalars_dev, size_t firs
     Lane& L = c->lanes[0];
     if (first > c->srs_n || n > c->srs_n - first) return fail(c, KZGB_ERR_SERIALIZATION, "polynomial length is not correct");
     Affine r;
-    int rc = msm_blocking(c, L, (const Fr*)scalars_dev, false, first, n, nullptr, &r);
+    int rc = msm_blocking(c, L, (const Fr*)scalars_dev, first, n, nullptr, &r);
     if (rc) return rc;
     affine_to_abi(r, out_xy, out_inf);
     return KZGB_OK;
@@ -1077,7 +1035,7 @@ int kzgb_msm_var(kzgb_ctx* c, const uint64_t* bases_xy, const uint8_t* bases_inf
         CK(c, cudaMemcpyAsync(L.bases.p, bases_xy, m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
     }
     CK(c, cudaMemcpyAsync(L.work.p, scalars, m * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-    int rc = msm_blocking(c, L, (Fr*)L.work.p, false, 0, m, (const Affine*)L.bases.p, &r);
+    int rc = msm_blocking(c, L, (Fr*)L.work.p, 0, m, (const Affine*)L.bases.p, &r);
     if (rc) return rc;
     affine_to_abi(r, out_xy, out_inf);
     return KZGB_OK;
@@ -1431,13 +1389,13 @@ int kzgb_bench_msm(kzgb_ctx* c, size_t n, int reps, double* ms_total, double* ms
     Fr base = fr_from_u64(0x9e3779b97f4a7c15ull);
     fr_powers_launch((Fr*)L.evals.p, (uint32_t)n, &base, L.st);
     Affine r;
-    int rc = msm_blocking(c, L, (Fr*)L.evals.p, false, 0, n, nullptr, &r);  // warm-up (+ lazy table build)
+    int rc = msm_blocking(c, L, (Fr*)L.evals.p, 0, n, nullptr, &r);  // warm-up (+ lazy table build)
     if (rc) return rc;
     double acc0 = L.acc_ms;
     uint64_t l0 = L.acc_launches;
     CK(c, cudaEventRecord(c->t0, L.st));
     for (int i = 0; i < reps; i++) {
-        rc = msm_blocking(c, L, (Fr*)L.evals.p, false, 0, n, nullptr, &r);
+        rc = msm_blocking(c, L, (Fr*)L.evals.p, 0, n, nullptr, &r);
         if (rc) return rc;
     }
     CK(c, cudaEventRecord(c->t1, L.st));
@@ -1569,8 +1527,6 @@ int kzgb_set_option(const char* name, long value) {
     if (!strcmp(name, "lagrange_budget_mib")) { g_lagrange_budget_mib.store(value < 0 ? 0 : value); return KZGB_OK; }
     if (!strcmp(name, "acc_waves")) { msm_set_acc_waves((int)value); return KZGB_OK; }
     if (!strcmp(name, "msm_debug_sync")) { msm_set_debug_sync((int)value); return KZGB_OK; }
-    if (!strcmp(name, "acc_regs")) { msm_set_experiment((int)value, -1); return KZGB_OK; }
-    if (!strcmp(name, "sort_block")) { msm_set_experiment(-1, (int)value); return KZGB_OK; }
     return KZGB_ERR_GENERIC;
 }
 

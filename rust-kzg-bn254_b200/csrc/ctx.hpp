@@ -167,16 +167,15 @@ bool lane_wait_polls();
 // ---- MSM and polynomial pieces (enqueue on the lane, finish waits for it)
 struct MsmJob {
     MsmPlan plan;
+    size_t results = 0;  // MSMs in the job: msm_finish writes outs[0 .. results)
     bool active = false;
 };
-int msm_finish(kzgb_ctx* c, Lane& L, const MsmJob& job, Affine* out);
-int msm_blocking(kzgb_ctx* c, Lane& L, const Fr* d_scalars, bool canonical, size_t first, size_t n,
-                 const Affine* var_bases, Affine* out);
-int msm_enqueue_batched(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t n_per, size_t batch,
-                        const kzgb_ctx::LagTable* lag, MsmJob* job);
-int msm_finish_batched(kzgb_ctx* c, Lane& L, const MsmJob& job, size_t batch, Affine* outs);
-int commit_blob_enqueue(kzgb_ctx* c, Lane& L, const uint8_t* d_bytes, uint64_t len, size_t n, size_t batch,
-                        const kzgb_ctx::LagTable* lag, MsmJob* job);
+// `batch` MSMs of n scalars each (scalar k * n + i belongs to MSM k), over the Lagrange table `lag`, else over the
+// variable bases var_bases[0 .. n), else over the SRS points [first, first + n).  batch > 1 needs a fixed-base table.
+int msm_enqueue(kzgb_ctx* c, Lane& L, const MsmScalars& scalars, size_t n, size_t batch, const kzgb_ctx::LagTable* lag,
+                const Affine* var_bases, size_t first, MsmJob* job);
+int msm_finish(kzgb_ctx* c, Lane& L, const MsmJob& job, Affine* outs);
+int msm_blocking(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t first, size_t n, const Affine* var_bases, Affine* out);
 int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJob* job);
 int eval_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z, Fr* d_quotient);
 int eval_read_y(kzgb_ctx* c, Lane& L, Fr* y);

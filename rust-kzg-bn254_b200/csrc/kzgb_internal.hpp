@@ -56,32 +56,32 @@ MsmPlan msm_make_plan(uint32_t n, int c, bool fixed_base, uint32_t table_stride,
 // waves of accumulate blocks (4 blocks of 128 threads per SM and wave) the sorted list is cut into; default 4
 void msm_set_acc_waves(int waves);
 void msm_set_debug_sync(int on);
-void msm_set_experiment(int acc_regs, int sort_block);
 
-// scalars: n Fr (Montgomery unless scalars_canonical).  Result: ws.set_sums[0..sets) on the device.
-// The optional events bracket the bucket-accumulation kernel (roofline timing).
-void msm_launch(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scalars, bool scalars_canonical,
-                const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin = nullptr,
-                cudaEvent_t ev_acc_end = nullptr, cudaStream_t st_acc = nullptr, cudaEvent_t ev_fork = nullptr,
-                cudaEvent_t ev_join = nullptr);
-// st_acc (optional): a second, lower-priority stream for the bucket accumulation, fenced against `st`
-// with ev_fork / ev_join.
-// The two halves of msm_launch: sort + accumulate + stitch (ws.buckets = the sum of every bucket), and the
-// bucket reduction of any bucket array of the plan's shape.  Large MSMs whose scalars arrive from the host in
-// chunks run the first half per chunk, fold the bucket sums together (msm_merge_buckets) and reduce once.
-void msm_launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scalars, bool scalars_canonical,
-                        const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin = nullptr,
-                        cudaEvent_t ev_acc_end = nullptr, cudaStream_t st_acc = nullptr, cudaEvent_t ev_fork = nullptr,
-                        cudaEvent_t ev_join = nullptr);
+// The n scalars of a plan, from exactly one source:
+//   mont  n Fr in Montgomery form;
+//   blob  blob bytes (blob_element below, reduced mod r by the first sort pass): for commitments over a Lagrange
+//         table, where the evaluations of the blob are the scalars and nothing needs their Montgomery form.  A
+//         batched plan reads blob k at blob + 32 * batch_n * k.
+struct MsmScalars {
+    const Fr* mont = nullptr;
+    const uint8_t* blob = nullptr;
+    uint64_t blob_len = 0;
+};
+// Where an MSM runs.  Everything goes to st, except the bucket accumulation: that goes to st_acc, a second,
+// lower-priority stream fenced against st with fork / join, when all three are set.  acc_begin / acc_end, when
+// set, bracket the accumulation kernel (roofline timing).
+struct MsmStreams {
+    cudaStream_t st = nullptr, st_acc = nullptr;
+    cudaEvent_t fork = nullptr, join = nullptr, acc_begin = nullptr, acc_end = nullptr;
+};
+// An MSM is two halves: sort + accumulate + stitch (ws.buckets = the sum of every bucket, the identity where
+// empty), then the reduction of any bucket array of the plan's shape into ws.set_sums[0..sets) on the device.
+// Large MSMs whose scalars arrive from the host in chunks run the first half per chunk, fold the bucket sums
+// together (msm_merge_buckets) and reduce once.
+void msm_launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const MsmScalars& scalars, const Affine* table,
+                        const MsmStreams& s);
 void msm_launch_reduce(const MsmPlan& p, const MsmWorkspace& ws, const XYZZ* buckets, cudaStream_t st);
 void msm_merge_buckets(XYZZ* dst, const XYZZ* src, uint32_t nbuckets, cudaStream_t st);
-// msm_launch with the scalars read from blob bytes (blob_element below, reduced mod r) by the first sort pass: for
-// commitments over a Lagrange table, where the evaluations of the blob are the scalars and nothing needs their
-// Montgomery form.  A batched plan reads blob k at blob + 32 * batch_n * k.
-void msm_launch_blob(const MsmPlan& p, const MsmWorkspace& ws, const uint8_t* blob, uint64_t len_bytes,
-                     const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin = nullptr,
-                     cudaEvent_t ev_acc_end = nullptr, cudaStream_t st_acc = nullptr, cudaEvent_t ev_fork = nullptr,
-                     cudaEvent_t ev_join = nullptr);
 
 // Element i of blob bytes (primitives/src/helpers.rs:40-57): the 32 big-endian bytes at offset 32 i as a 256-bit
 // integer, the last partial chunk right-padded with zeros, zero past len.  Not reduced mod r.

@@ -64,12 +64,12 @@ __device__ __forceinline__ void digits_hist(const Fr& s, uint32_t i, const MsmPl
     }
 }
 
-__global__ void __launch_bounds__(256) k_digits_hist(const Fr* __restrict__ scalars, bool canonical, MsmPlan p,
-                                                      Fr* __restrict__ canon, uint32_t* __restrict__ hist) {
+__global__ void __launch_bounds__(256) k_digits_hist(const Fr* __restrict__ scalars, MsmPlan p, Fr* __restrict__ canon,
+                                                      uint32_t* __restrict__ hist) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= p.n) return;
     Fr s = fe_load_ro(&scalars[i]);
-    if (!canonical) fe_from_mont(s, s);
+    fe_from_mont(s, s);
     digits_hist(s, i, p, canon, hist);
 }
 
@@ -87,7 +87,7 @@ __device__ __forceinline__ void sub_if_geq(uint32_t* x, const uint32_t* m) {
     for (int k = 0; k < 8; k++) x[k] = borrow ? x[k] : t[k];
 }
 
-// The first sort pass over blob bytes (msm_launch_blob): scalar i is blob_element(i) mod r.  Every 256-bit value is
+// The first sort pass over blob bytes (MsmScalars::blob): scalar i is blob_element(i) mod r.  Every 256-bit value is
 // below 6r, so subtracting 4r, 2r and r where they fit leaves the canonical value.
 __global__ void __launch_bounds__(256) k_digits_hist_blob(const uint8_t* __restrict__ blob, uint64_t len, MsmPlan p,
                                                            Fr* __restrict__ canon, uint32_t* __restrict__ hist) {
@@ -252,9 +252,9 @@ __device__ __forceinline__ bool xyzz_madd_relaxed_nonempty(XYZZ& acc, const Affi
 // Thread t owns sorted entries [t*chunk, (t+1)*chunk).  A bucket run that lies entirely inside the chunk is
 // written to buckets[b]; the run cut by the chunk's start goes to partial[2t], the one cut by its end to
 // partial[2t+1] (k_bucket_fix adds them up).
-__device__ __forceinline__ void accumulate_body(const uint32_t* __restrict__ sorted, const uint32_t* __restrict__ offsets,
-                                                const Affine* __restrict__ table, uint32_t nb, uint32_t acc_threads,
-                                                uint32_t chunk, XYZZ* __restrict__ buckets, XYZZ* __restrict__ partial) {
+__global__ void __launch_bounds__(128, 4) k_accumulate(const uint32_t* __restrict__ sorted, const uint32_t* __restrict__ offsets,
+                                                        const Affine* __restrict__ table, uint32_t nb, uint32_t acc_threads,
+                                                        uint32_t chunk, XYZZ* __restrict__ buckets, XYZZ* __restrict__ partial) {
     uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= acc_threads) return;
     const uint32_t M = offsets[nb];
@@ -297,19 +297,6 @@ __device__ __forceinline__ void accumulate_body(const uint32_t* __restrict__ sor
     }
     bool complete = (run_begin >= start) && (next <= end);
     flush(complete ? &buckets[b] : (run_begin <= start) ? &partial[2 * t] : &partial[2 * t + 1]);
-}
-__global__ void __launch_bounds__(128, 4) k_accumulate(const uint32_t* __restrict__ sorted, const uint32_t* __restrict__ offsets,
-                                                        const Affine* __restrict__ table, uint32_t nb, uint32_t acc_threads,
-                                                        uint32_t chunk, XYZZ* __restrict__ buckets, XYZZ* __restrict__ partial) {
-    accumulate_body(sorted, offsets, table, nb, acc_threads, chunk, buckets, partial);
-}
-// EXPERIMENT (option "acc_regs"): the same body under a hard register cap, so that four blocks leave part of the
-// register file free and the short sort kernels of the other lanes can be resident NEXT TO the accumulation
-template <int MAXR>
-__global__ void __maxnreg__(MAXR) k_accumulate_capped(const uint32_t* __restrict__ sorted, const uint32_t* __restrict__ offsets,
-                                                       const Affine* __restrict__ table, uint32_t nb, uint32_t acc_threads,
-                                                       uint32_t chunk, XYZZ* __restrict__ buckets, XYZZ* __restrict__ partial) {
-    accumulate_body(sorted, offsets, table, nb, acc_threads, chunk, buckets, partial);
 }
 
 // Buckets whose entries span more than LONG_SPAN chunks (hot buckets: equal scalars, a top window with a
@@ -599,12 +586,7 @@ __global__ void __launch_bounds__(32) k_reduce_final(const XYZZ* __restrict__ gr
 
 // ---------------------------------------------------------------------------------
 static std::atomic<int> g_acc_waves{4};
-static std::atomic<int> g_acc_regs{0}, g_sort_block{256};
-void msm_set_experiment(int acc_regs, int sort_block) {
-    if (acc_regs >= 0) g_acc_regs.store(acc_regs);
-    if (sort_block == 64 || sort_block == 128 || sort_block == 256) g_sort_block.store(sort_block);
-}
-static std::atomic<int> g_debug_sync{0};  // option "msm_debug_sync": synchronise and report after every kernel of msm_launch
+static std::atomic<int> g_debug_sync{0};  // option "msm_debug_sync": synchronise and report after every kernel of an MSM
 void msm_set_debug_sync(int on) { g_debug_sync.store(on); }
 #define KZ_DBG(name)                                                                                         \
     do {                                                                                                     \
@@ -677,7 +659,7 @@ void msm_workspace_carve(const MsmPlan& p, void* base, MsmWorkspace* ws) {
 }
 
 // dst[k] += src[k]: bucket sums of a further point sub-range folded into the running totals (msm_launch_buckets
-// of the chunks of one large MSM whose scalars arrive piecewise, capi.cu msm_host_scalars_pipelined)
+// of the chunks of one large MSM whose scalars arrive piecewise, capi.cu msm_srs_host_pipelined)
 __global__ void __launch_bounds__(128) k_merge_buckets(XYZZ* __restrict__ dst, const XYZZ* __restrict__ src, uint32_t n) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -692,27 +674,17 @@ void msm_merge_buckets(XYZZ* dst, const XYZZ* src, uint32_t nbuckets, cudaStream
     g_launch_count++;
 }
 
-void msm_launch(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scalars, bool scalars_canonical,
-                const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin, cudaEvent_t ev_acc_end,
-                cudaStream_t st_acc, cudaEvent_t ev_fork, cudaEvent_t ev_join) {
-    msm_launch_buckets(p, ws, scalars, scalars_canonical, table, st, ev_acc_begin, ev_acc_end, st_acc, ev_fork, ev_join);
-    msm_launch_reduce(p, ws, ws.buckets, st);
-}
-
-// sort + accumulate + stitch: afterwards ws.buckets holds the sum of every bucket (identity where empty).  The scalars
-// come from `scalars`, or from blob bytes when blob != nullptr.
-static void launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scalars, bool scalars_canonical,
-                           const uint8_t* blob, uint64_t blob_len, const Affine* table, cudaStream_t st,
-                           cudaEvent_t ev_acc_begin, cudaEvent_t ev_acc_end, cudaStream_t st_acc, cudaEvent_t ev_fork,
-                           cudaEvent_t ev_join) {
-    const bool split = st_acc && ev_fork && ev_join;
-    cudaStream_t sa = split ? st_acc : st;
+// sort + accumulate + stitch: afterwards ws.buckets holds the sum of every bucket (identity where empty)
+void msm_launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const MsmScalars& scalars, const Affine* table,
+                        const MsmStreams& s) {
+    const cudaStream_t st = s.st;
+    const bool split = s.st_acc && s.fork && s.join;
+    const cudaStream_t sa = split ? s.st_acc : st;
     cudaMemsetAsync(ws.hist, 0, ((size_t)p.nbuckets + 1) * 4, st);
-    const uint32_t sb = (uint32_t)g_sort_block.load();
-    uint32_t gb = (p.n + sb - 1) / sb;
+    const uint32_t gb = (p.n + 255) / 256;
     if (p.n) {
-        if (blob) k_digits_hist_blob<<<gb, sb, 0, st>>>(blob, blob_len, p, ws.canon, ws.hist);
-        else k_digits_hist<<<gb, sb, 0, st>>>(scalars, scalars_canonical, p, ws.canon, ws.hist);
+        if (scalars.blob) k_digits_hist_blob<<<gb, 256, 0, st>>>(scalars.blob, scalars.blob_len, p, ws.canon, ws.hist);
+        else k_digits_hist<<<gb, 256, 0, st>>>(scalars.mont, p, ws.canon, ws.hist);
         g_launch_count += 2;
     }
     {
@@ -725,24 +697,14 @@ static void launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* s
             g_launch_count += 2;
         }
     }
-    if (p.n) k_scatter<<<gb, sb, 0, st>>>(ws.canon, p, ws.cursor, ws.sorted);
+    if (p.n) k_scatter<<<gb, 256, 0, st>>>(ws.canon, p, ws.cursor, ws.sorted);
     KZ_DBG("sort");
-    if (split) { cudaEventRecord(ev_fork, st); cudaStreamWaitEvent(sa, ev_fork, 0); }
-    if (ev_acc_begin) cudaEventRecord(ev_acc_begin, sa);
-    {
-        const dim3 ga((p.acc_threads + 127) / 128);
-#define KZ_ACC(K) K<<<ga, 128, 0, sa>>>(ws.sorted, ws.hist, table, p.nbuckets, p.acc_threads, p.chunk, ws.buckets, ws.partial)
-        switch (g_acc_regs.load()) {
-            case 120: KZ_ACC(k_accumulate_capped<120>); break;
-            case 112: KZ_ACC(k_accumulate_capped<112>); break;
-            case 104: KZ_ACC(k_accumulate_capped<104>); break;
-            case 96: KZ_ACC(k_accumulate_capped<96>); break;
-            default: KZ_ACC(k_accumulate); break;
-        }
-#undef KZ_ACC
-    }
-    if (ev_acc_end) cudaEventRecord(ev_acc_end, sa);
-    if (split) { cudaEventRecord(ev_join, sa); cudaStreamWaitEvent(st, ev_join, 0); }
+    if (split) { cudaEventRecord(s.fork, st); cudaStreamWaitEvent(sa, s.fork, 0); }
+    if (s.acc_begin) cudaEventRecord(s.acc_begin, sa);
+    k_accumulate<<<(p.acc_threads + 127) / 128, 128, 0, sa>>>(ws.sorted, ws.hist, table, p.nbuckets, p.acc_threads, p.chunk,
+                                                             ws.buckets, ws.partial);
+    if (s.acc_end) cudaEventRecord(s.acc_end, sa);
+    if (split) { cudaEventRecord(s.join, sa); cudaStreamWaitEvent(st, s.join, 0); }
     KZ_DBG("accumulate");
     {
         const uint32_t long_cap = p.acc_threads / LONG_SPAN + 4;  // a long bucket owns >= LONG_SPAN chunks
@@ -755,19 +717,6 @@ static void launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* s
     }
     KZ_DBG("bucket_fix");
     g_launch_count += 3;  // accumulate, bucket_fix, bucket_fix_long
-}
-
-void msm_launch_buckets(const MsmPlan& p, const MsmWorkspace& ws, const Fr* scalars, bool scalars_canonical,
-                        const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin, cudaEvent_t ev_acc_end,
-                        cudaStream_t st_acc, cudaEvent_t ev_fork, cudaEvent_t ev_join) {
-    launch_buckets(p, ws, scalars, scalars_canonical, nullptr, 0, table, st, ev_acc_begin, ev_acc_end, st_acc, ev_fork, ev_join);
-}
-
-void msm_launch_blob(const MsmPlan& p, const MsmWorkspace& ws, const uint8_t* blob, uint64_t len_bytes,
-                     const Affine* table, cudaStream_t st, cudaEvent_t ev_acc_begin, cudaEvent_t ev_acc_end,
-                     cudaStream_t st_acc, cudaEvent_t ev_fork, cudaEvent_t ev_join) {
-    launch_buckets(p, ws, nullptr, false, blob, len_bytes, table, st, ev_acc_begin, ev_acc_end, st_acc, ev_fork, ev_join);
-    msm_launch_reduce(p, ws, ws.buckets, st);
 }
 
 // bucket sums -> ws.set_sums (one XYZZ point per bucket set)

@@ -1,6 +1,6 @@
 #!/bin/bash
 # Headline pipeline under kzgb_set_option settings: one line per setting (resident blobs/s, e2e blobs/s, isolated accumulate ms).
-# usage: bash scripts/sweep_opts.sh "acc_regs=120" "acc_regs=112 sort_block=128" ...
+# usage: bash scripts/sweep_opts.sh "acc_waves=2" "lanes=4 stream_priority=0" ...
 mkdir -p gpurun_out
 out=gpurun_out/sweep_opts.txt
 : > $out

@@ -418,6 +418,42 @@ def test_batch_groups_of_equal_size_blobs(pkg, ref_srs, ref_srs_points):
         assert first[1][i] == o.g1_serialize_compressed(ko.compute_blob_proof(bo, c, ref_srs_points))
 
 
+def test_batch_groups_trace_every_msm(pkg):
+    """The grouped small-blob path records the whole kzgb_trace_begin / kzgb_trace_end timeline of every MSM on
+    every lane: sort begins (0), accumulate begins / ends (1, 2), MSM ends (3), enqueued (10), lane woke up (11),
+    result finished (12)."""
+    import ctypes as C
+
+    rnd = random.Random(21)
+    blobs = [pkg.Blob.from_raw_data(bytes(rnd.getrandbits(8) for _ in range(31 * 64))) for _ in range(12)]
+    lib = pkg.lib
+    eng = pkg.Engine(0)
+    srs = pkg.SRS.from_gnark_bytes(g.g1_point_bytes(), engine=eng)
+    cap = 1024
+    buf = (C.c_double * (4 * cap))()
+    nrec = C.c_size_t(0)
+    try:
+        assert lib.kzgb_set_option(b"group", 4) == 0  # 3 groups of 4 blobs, one lane each
+        eng.check(lib.kzgb_trace_begin(eng.h))
+        pkg.KZG.commit_and_prove_blobs(blobs, srs)
+        eng.check(lib.kzgb_trace_end(eng.h, buf, cap, C.byref(nrec)))
+    finally:
+        lib.kzgb_set_option(b"group", -1)
+    assert 0 < nrec.value <= cap
+    recs = [(int(buf[4 * i]), int(buf[4 * i + 1])) for i in range(nrec.value)]
+    msms = []
+    for lane in sorted({r[0] for r in recs}):
+        kinds = [k for ln, k in recs if ln == lane]
+        assert kinds[0] == 0, (lane, kinds)
+        for k in kinds:
+            if k == 0:
+                msms.append(set())
+            msms[-1].add(k)
+    assert len(msms) == 2 * 3  # a commitment MSM and a proof MSM per group
+    for m in msms:
+        assert m == {0, 1, 2, 3, 10, 11, 12}, m
+
+
 def test_device_hashed_transcripts_equal_host_hashed(pkg):
     """Long-transcript hashing on the device (fs.cu k_fs_midstate_long, one warp per blob, from the resident blob bytes)
     forced on for the tail of a batch: same commitments and proofs as the host SHA-256 pool and as the oracle's
