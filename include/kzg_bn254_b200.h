@@ -102,6 +102,11 @@ int kzgb_srs_clone(kzgb_ctx* dst, kzgb_ctx* src);
  * Fr-IFFT + the monomial table.  Err KZGB_ERR_FFT / KZGB_ERR_SRS_CAPACITY as kzgb_g1_ifft; KZGB_ERR_DEVICE if the
  * table cannot be built (switched off, above 2^22, over the budget). */
 int kzgb_srs_prepare_lagrange(kzgb_ctx* ctx, size_t n);
+/* Build the per-size table of kzgb_compute_proofs_all_roots ahead of the first call: s_hat = DFT_2n of SRS[..n-1]
+ * reversed and zero-padded (2n x 64 B, 64 MiB at n = 2^19; one forward G1 NTT of 2n points).  Kept until the SRS
+ * changes; the first call of a size builds it when the caller does not.  Errors as kzgb_compute_proofs_all_roots;
+ * KZGB_ERR_GENERIC for n > 2^22, where nothing is kept and every call builds its own. */
+int kzgb_srs_prepare_all_roots(kzgb_ctx* ctx, size_t n);
 
 /* ---- MSM (ark-ec VariableBaseMSM::msm call sites) ---------------------------------------- */
 /* sum scalars[i] * SRS[i], i < n.  Replaces G1Projective::msm(&srs.g1[..n], coeffs) in
@@ -155,6 +160,11 @@ int kzgb_g1_ifft(kzgb_ctx* ctx, size_t n, uint64_t* out_xy, uint8_t* out_inf);
  * caller-supplied z (Montgomery).  Optionally returns y = p(z) (Montgomery) if y_out != NULL. */
 int kzgb_compute_proof(kzgb_ctx* ctx, const uint64_t* evals_mont, size_t n, const uint64_t z_mont[4],
                        uint64_t out_xy[8], uint8_t* out_inf, uint64_t y_out[4]);
+/* KZG::compute_proof_with_known_z_fr_index (kzg.rs:187-207) at EVERY index: out proof i (x||y Montgomery, n x 8 words;
+ * out_inf n flags, may be NULL) is the point kzgb_compute_proof(evals, n, w^i) returns.  FK20: one Toeplitz product in G1
+ * (two G1 FFTs + 2n scalar multiplications) instead of n MSMs.  Errors and their order as kzgb_compute_proof: KZGB_ERR_FFT
+ * (n not 2^k), KZGB_ERR_SRS_CAPACITY (n > srs_len), GenericError "power must be <= 28" (2n > 2^28), KZGB_ERR_DEVICE. */
+int kzgb_compute_proofs_all_roots(kzgb_ctx* ctx, const uint64_t* evals_mont, size_t n, uint64_t* out_xy, uint8_t* out_inf);
 /* helpers::evaluate_polynomial_in_evaluation_form (primitives/src/helpers.rs:475-535). */
 int kzgb_evaluate_polynomial(kzgb_ctx* ctx, const uint64_t* evals_mont, size_t n, const uint64_t z_mont[4],
                              uint64_t y_out[4]);

@@ -517,6 +517,11 @@ class SRS:
         equivalent of the g1_ifft that KZG::commit_eval_form runs on every call (prover/src/kzg.rs:98)."""
         self.engine.check(lib.kzgb_srs_prepare_lagrange(self.engine.h, n))
 
+    def prepare_all_roots(self, n: int) -> None:
+        """Resident table of :meth:`KZG.compute_proofs_at_all_roots` for polynomials of n elements (n <= 2^22), built
+        now instead of by the first call of that size."""
+        self.engine.check(lib.kzgb_srs_prepare_all_roots(self.engine.h, n))
+
 
 class KZG:
     """prover/src/kzg.rs:25-309."""
@@ -575,6 +580,18 @@ class KZG:
         if z is None:
             raise KzgError("GenericError", "Root of unity not found")
         return self.compute_proof(polynomial, z, srs)
+
+    def compute_proofs_at_all_roots(self, polynomial: PolynomialEvalForm, srs: SRS) -> List[Affine]:
+        """compute_proof_with_known_z_fr_index (kzg.rs:187-207) at every index 0 .. n-1 in one call (FK20 on the GPU):
+        element i is the proof at the i-th root of unity."""
+        if len(polynomial) != len(self.expanded_roots_of_unity):
+            raise KzgError("GenericError", "inconsistent length between blob and root of unities")
+        e = srs.engine
+        n = len(polynomial)
+        xy = C.create_string_buffer(64 * n)
+        inf = C.create_string_buffer(n)
+        e.check(lib.kzgb_compute_proofs_all_roots(e.h, fr_to_mont_bytes(polynomial.evaluations), n, xy, inf))
+        return g1_from_abi(xy.raw, inf.raw)
 
     def g1_ifft(self, length: int, srs: SRS) -> List[Affine]:
         """kzg.rs:263-285."""

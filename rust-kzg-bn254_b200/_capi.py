@@ -42,6 +42,7 @@ SIGNATURES = {
     "kzgb_srs_get_affine_mont": (C.c_int, [ctx_p, C.c_size_t, C.c_size_t, buf, buf]),
     "kzgb_srs_precompute": (C.c_int, [ctx_p, C.c_size_t, C.c_int]),
     "kzgb_srs_prepare_lagrange": (C.c_int, [ctx_p, C.c_size_t]),
+    "kzgb_srs_prepare_all_roots": (C.c_int, [ctx_p, C.c_size_t]),
     "kzgb_msm_srs": (C.c_int, [ctx_p, buf, C.c_size_t, buf, u8p]),
     "kzgb_msm_srs_range": (C.c_int, [ctx_p, buf, C.c_size_t, C.c_size_t, buf, u8p]),
     "kzgb_msm_srs_range_dev": (C.c_int, [ctx_p, buf, C.c_size_t, C.c_size_t, buf, u8p]),
@@ -57,6 +58,7 @@ SIGNATURES = {
     "kzgb_commit_blob": (C.c_int, [ctx_p, buf, C.c_size_t, buf, u8p]),
     "kzgb_g1_ifft": (C.c_int, [ctx_p, C.c_size_t, buf, buf]),
     "kzgb_compute_proof": (C.c_int, [ctx_p, buf, C.c_size_t, buf, buf, u8p, buf]),
+    "kzgb_compute_proofs_all_roots": (C.c_int, [ctx_p, buf, C.c_size_t, buf, buf]),
     "kzgb_evaluate_polynomial": (C.c_int, [ctx_p, buf, C.c_size_t, buf, buf]),
     "kzgb_compute_challenge": (C.c_int, [ctx_p, buf, C.c_size_t, buf, C.c_uint8, buf]),
     "kzgb_compute_blob_proof": (C.c_int, [ctx_p, buf, C.c_size_t, buf, C.c_uint8, buf, u8p]),

@@ -397,11 +397,52 @@ const kzgb_ctx::LagTable* lagrange_table(const kzgb_ctx* c, int logn) {
     return logn >= 1 && logn <= 28 && c->lag[logn].table && g_lagrange.load() ? &c->lag[logn] : nullptr;
 }
 
+// ---------------------------------------------------------------- proofs at every root: the s_hat tables (allroots.cu)
+void allroots_release(kzgb_ctx* c) {
+    for (auto& t : c->allroots) { if (t) cudaFree(t); t = nullptr; }
+}
+
+// Canonical 1: g1_ntt_finish_launch converts to affine without scaling.
+Fr fr_one_canon() { Fr one; fe_zero(one); one.l[0] = 1; return one; }
+
+// s_hat = DFT_2n(r), r_t = SRS[n-2-t] (t <= n-2) zero-padded to 2n: 2n affine points in natural order.  work: 2n XYZZ.
+// The twiddles of size 2n must be resident.
+void allroots_shat_launch(kzgb_ctx* c, int logn, XYZZ* work, Affine* out, cudaStream_t st) {
+    const Fr one = fr_one_canon();
+    allroots_embed_launch(c->srs, logn, work, st);
+    g1_ntt_stages_launch(work, logn + 1, false, c->tw, c->logN, st);
+    g1_ntt_finish_launch(work, out, logn + 1, &one, st);
+}
+
+// The s_hat table of the domain 2^logn, built on first use (2n x 64 B: 64 MiB at 2^19, one forward G1 NTT of 2n points)
+// and kept until the SRS changes; *out = nullptr above 2^22, where each call builds its own (the cut-off of the Lagrange
+// tables).  Uses lane 0's work buffer; the twiddles of size 2n must be resident.  Called under the context lock, so
+// never while a batch pipeline drives the lanes.
+int ensure_allroots(kzgb_ctx* c, int logn, const Affine** out) {
+    *out = nullptr;
+    if (logn > ALLROOTS_MAX_LOG) return KZGB_OK;
+    if (!c->allroots[logn]) {
+        Lane& L = c->lanes[0];
+        const size_t m = (size_t)2 << logn;
+        CK(c, L.work.reserve(m * sizeof(XYZZ)));
+        Affine* table = nullptr;
+        CK(c, cudaMalloc((void**)&table, m * sizeof(Affine)));
+        allroots_shat_launch(c, logn, (XYZZ*)L.work.p, table, L.st);
+        cudaError_t e = cudaStreamSynchronize(L.st);
+        if (e == cudaSuccess) e = cudaGetLastError();
+        if (e != cudaSuccess) { cudaFree(table); CK(c, e); }
+        c->allroots[logn] = table;
+    }
+    *out = c->allroots[logn];
+    return KZGB_OK;
+}
+
 int srs_install(kzgb_ctx* c, Affine* dev_points, size_t n) {
     drain_lanes(c);
     if (c->srs) cudaFree(c->srs);
     drop_window_table(c);
     lagrange_release(c);
+    allroots_release(c);
     c->srs = dev_points;
     c->srs_n = n;
     return KZGB_OK;
@@ -777,6 +818,7 @@ void kzgb_ctx_destroy(kzgb_ctx* c) {
     if (c->srs) cudaFree(c->srs);
     drop_window_table(c);
     lagrange_release(c);
+    allroots_release(c);
     if (c->tw) cudaFree(c->tw);
     c->batch_bytes.release();
     if (c->t0) cudaEventDestroy(c->t0);
@@ -1218,6 +1260,68 @@ int kzgb_compute_proof(kzgb_ctx* c, const uint64_t* evals, size_t n, const uint6
     if (y_out) memcpy(y_out, &L.h_fr[3], 32);
     affine_to_abi(r, out_xy, out_inf);
     return KZGB_OK;
+}
+
+// KZG::compute_proof_with_known_z_fr_index (kzg.rs:187-207) at every index of the domain, by FK20 (allroots.cu), on lane 0:
+// c = IFFT_n(evals) and c_hat = DFT_2n(c || 0) on the Fr side; u = IDFT_2n((c_hat / 2n) (.) s_hat), H_i = u_{i+n-1} and
+// pi = DFT_n(H) in G1, kept in XYZZ until the one conversion to affine.  shat == nullptr: built here into *own.
+static int proofs_all_roots(kzgb_ctx* c, const uint64_t* evals, int logn, const Affine* shat, DevBuf* own, uint64_t* out_xy,
+                            uint8_t* out_inf) {
+    Lane& L = c->lanes[0];
+    const size_t n = (size_t)1 << logn, m = 2 * n;
+    CK(c, L.evals.reserve(m * sizeof(Fr)));
+    CK(c, L.ntt_scratch.reserve(m * sizeof(Fr)));
+    CK(c, L.work.reserve(m * sizeof(XYZZ)));
+    CK(c, L.bases.reserve(n * sizeof(XYZZ)));
+    Fr* f = (Fr*)L.evals.p;
+    XYZZ* u = (XYZZ*)L.work.p;
+    XYZZ* H = (XYZZ*)L.bases.p;
+    if (!shat) {
+        CK(c, own->reserve(m * sizeof(Affine)));
+        allroots_shat_launch(c, logn, u, (Affine*)own->p, L.st);
+        shat = (const Affine*)own->p;
+    }
+    CK(c, cudaMemcpyAsync(f, evals, n * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+    CK(c, cudaMemsetAsync(f + n, 0, n * sizeof(Fr), L.st));
+    const Fr ninv = ninv_mont(logn), inv2n = ninv_mont(logn + 1), one = fr_one_canon();
+    ntt_launch(f, logn, 1, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+    ntt_launch(f, logn + 1, 1, false, c->tw, c->logN, &inv2n, (Fr*)L.ntt_scratch.p, L.st);
+    allroots_hadamard_launch(f, &inv2n, shat, u, logn + 1, L.st);  // the 1/2n of the inverse transform, on the scalars
+    g1_ntt_stages_launch(u, logn + 1, true, c->tw, c->logN, L.st);
+    allroots_extract_launch(u, H, logn, L.st);
+    g1_ntt_stages_launch(H, logn, false, c->tw, c->logN, L.st);
+    g1_ntt_finish_launch(H, (Affine*)L.work.p, logn, &one, L.st);  // u is consumed: its buffer takes the proofs
+    std::vector<Affine> host(n);
+    CK(c, cudaMemcpyAsync(host.data(), L.work.p, n * sizeof(Affine), cudaMemcpyDeviceToHost, L.st));
+    CK(c, cudaStreamSynchronize(L.st));
+    CK(c, cudaGetLastError());
+    for (size_t i = 0; i < n; i++) affine_to_abi(host[i], out_xy + 8 * i, out_inf ? out_inf + i : nullptr);
+    return KZGB_OK;
+}
+
+int kzgb_compute_proofs_all_roots(kzgb_ctx* c, const uint64_t* evals, size_t n, uint64_t* out_xy, uint8_t* out_inf) {
+    Guard g(c);
+    if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_FFT, "length provided is not a power of 2");
+    if (int rc = check_srs_capacity(c, n)) return rc;
+    const int logn = log2_exact(n);
+    if (int rc = ensure_twiddles(c, logn + 1)) return rc;
+    const Affine* shat = nullptr;
+    if (int rc = ensure_allroots(c, logn, &shat)) return rc;
+    DevBuf own;  // s_hat of a domain above 2^22, for this call only
+    int rc = proofs_all_roots(c, evals, logn, shat, &own, out_xy, out_inf);
+    own.release();
+    return rc;
+}
+
+int kzgb_srs_prepare_all_roots(kzgb_ctx* c, size_t n) {
+    Guard g(c);
+    if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_FFT, "length provided is not a power of 2");
+    if (int rc = check_srs_capacity(c, n)) return rc;
+    const int logn = log2_exact(n);
+    if (logn > ALLROOTS_MAX_LOG) return fail(c, KZGB_ERR_GENERIC, "all-roots table not kept above 2^22 (each call builds its own)");
+    if (int rc = ensure_twiddles(c, logn + 1)) return rc;
+    const Affine* shat = nullptr;
+    return ensure_allroots(c, logn, &shat);
 }
 
 int kzgb_evaluate_polynomial(kzgb_ctx* c, const uint64_t* evals, size_t n, const uint64_t z_mont[4], uint64_t y_out[4]) {

@@ -14,6 +14,7 @@ namespace kzgb {
 
 constexpr int MAX_LANES = 8;
 constexpr int MAX_SETS = 96;
+constexpr int ALLROOTS_MAX_LOG = 22;  // largest domain 2^k whose kzgb_compute_proofs_all_roots table is kept
 
 struct DevBuf {
     void* p = nullptr;
@@ -68,6 +69,9 @@ struct kzgb_ctx {
     // evaluation-form commitments are ONE MSM on the evaluations themselves (no Fr NTT on the path)
     struct LagTable { kzgb::Affine* table = nullptr; size_t n = 0; int c = 0, W = 0; uint64_t last_use = 0; uint32_t calls = 0; } lag[29];
     uint64_t lag_clock = 0;
+    // kzgb_compute_proofs_all_roots: s_hat = DFT_2n of the reversed SRS prefix, 2n affine points per domain 2^k, built by
+    // the first call of that size (or kzgb_srs_prepare_all_roots) and dropped with the SRS
+    kzgb::Affine* allroots[kzgb::ALLROOTS_MAX_LOG + 1] = {};
     kzgb::DevBuf batch_bytes;  // blob bytes of the batch in flight (commit_and_prove_blobs)
     // twiddles
     kzgb::Fr* tw = nullptr;

@@ -213,6 +213,39 @@ KZ_HD void xyzz_mul_small(XYZZ& r, const XYZZ& p, uint32_t k) {
     r = acc;
 }
 
+// r = k * p for a canonical (non-Montgomery) scalar k < 2^254, signed 4-bit windows: K = k + 0x88..8 (64 nibbles of 8)
+// has base-16 digits e_i with k = sum (e_i - 8) 16^i, so each digit lies in [-8, 7] with no carry pass.  A table of
+// 1p .. 8p (one doubling, six additions; local memory, indexed by the digit), then 252 doublings and at most 64
+// additions -- against ~127 additions for plain double-and-add.  Exact for every input (k = 0, p = identity).
+KZ_HD void xyzz_mul_scalar_w4(XYZZ& r, const XYZZ& p, const Fr& k) {
+    XYZZ tab[8];
+    tab[0] = p;
+    xyzz_dbl(tab[1], p);
+    for (int j = 2; j < 8; j++) { tab[j] = tab[j - 1]; xyzz_add(tab[j], p); }
+    uint32_t K[8];
+    uint64_t carry = 0;
+    for (int w = 0; w < 8; w++) {
+        carry += (uint64_t)k.l[w] + 0x88888888u;
+        K[w] = (uint32_t)carry;
+        carry >>= 32;
+    }
+    XYZZ acc; xyzz_set_inf(acc);
+    for (int w = 7; w >= 0; w--) {
+        for (int q = 7; q >= 0; q--) {
+            for (int d = 0; d < 4; d++) xyzz_dbl(acc, acc);  // returns at once while acc is the identity
+            const int v = (int)((K[w] >> (4 * q)) & 15u) - 8;
+            if (v > 0) {
+                xyzz_add(acc, tab[v - 1]);
+            } else if (v < 0) {
+                XYZZ t;
+                xyzz_neg(t, tab[-v - 1]);
+                xyzz_add(acc, t);
+            }
+        }
+    }
+    r = acc;
+}
+
 // Affine from XYZZ given inv = 1/ZZZ:  1/Z = inv*ZZ, x = X/Z^2, y = Y*inv
 KZ_HD void xyzz_to_affine_with_inv(Affine& r, const XYZZ& p, const Fq& inv_zzz) {
     Fq zi, zi2;

@@ -135,11 +135,23 @@ void ntt_launch(Fr* data, int logn, uint32_t batch, bool inverse, const Fr* tw, 
 // 0: shared-memory tile passes (default), 1: warp-resident passes (registers + shuffles + bulk copy)
 void ntt_set_kernel(int which);
 
-// ---- G1 inverse NTT (KZG::g1_ifft, prover/src/kzg.rs:263-285) --------------------------
-// srs: 2^logn affine points; work: 2^logn XYZZ scratch; out: 2^logn affine points (natural order).
-// ninv_canon_host: 1/n as a CANONICAL (non-Montgomery) scalar.
+// ---- G1 NTTs (g1ntt.cu) -------------------------------------------------------------
+// in place on 2^logn XYZZ points: natural order in, bit-reversed out, unscaled (forward w^t or inverse w^-t)
+void g1_ntt_stages_launch(XYZZ* pts, int logn, bool inverse, const Fr* tw, int logN, cudaStream_t st);
+// out[bitrev(i)] = affine(scale * pts[i]): natural order; scale_canon_host CANONICAL (non-Montgomery)
+void g1_ntt_finish_launch(const XYZZ* pts, Affine* out, int logn, const Fr* scale_canon_host, cudaStream_t st);
+// KZG::g1_ifft (prover/src/kzg.rs:263-285): srs: 2^logn affine points; work: 2^logn XYZZ scratch; out: 2^logn affine
+// points (natural order).  ninv_canon_host: 1/n as a CANONICAL (non-Montgomery) scalar.
 void g1_intt_launch(const Affine* srs, int logn, XYZZ* work, Affine* out, const Fr* tw, int logN,
                     const Fr* ninv_canon_host, cudaStream_t st);
+
+// ---- proofs at every root of the domain (allroots.cu, FK20) ------------------------------
+// out[t] = SRS[n-2-t] for t <= n-2, the identity up to 2n (out: 2n XYZZ, n = 2^logn)
+void allroots_embed_launch(const Affine* srs, int logn, XYZZ* out, cudaStream_t st);
+// u[k] = (chat[k] * scale) * shat[k] for k < 2^logm (chat Montgomery, shat affine)
+void allroots_hadamard_launch(const Fr* chat, const Fr* scale_mont_host, const Affine* shat, XYZZ* u, int logm, cudaStream_t st);
+// H[i] = u[bitrev_{logn+1}(i + n - 1)] for i <= n-2, H[n-1] = identity (H: n XYZZ)
+void allroots_extract_launch(const XYZZ* u, XYZZ* H, int logn, cudaStream_t st);
 
 // ---- polynomial glue ------------------------------------------------------------
 // bytes (big-endian 32 B chunks, last chunk zero-right-padded) -> n Fr Montgomery (zero padded to n)

@@ -33,6 +33,7 @@ extern "C" {
     pub fn kzgb_srs_load_cache(ctx: *mut kzgb_ctx, path: *const c_char, points_to_load: u32) -> c_int;
     pub fn kzgb_srs_precompute(ctx: *mut kzgb_ctx, max_n: usize, window_bits: c_int) -> c_int;
     pub fn kzgb_srs_prepare_lagrange(ctx: *mut kzgb_ctx, n: usize) -> c_int;
+    pub fn kzgb_srs_prepare_all_roots(ctx: *mut kzgb_ctx, n: usize) -> c_int;
     pub fn kzgb_srs_load_affine_mont(ctx: *mut kzgb_ctx, xy: *const u64, inf: *const u8, n: usize) -> c_int;
     pub fn kzgb_srs_len(ctx: *const kzgb_ctx) -> usize;
     pub fn kzgb_srs_get_affine_mont(ctx: *mut kzgb_ctx, start: usize, count: usize, out_xy: *mut u64, out_inf: *mut u8) -> c_int;
@@ -46,6 +47,8 @@ extern "C" {
     pub fn kzgb_g1_ifft(ctx: *mut kzgb_ctx, n: usize, out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_compute_proof(ctx: *mut kzgb_ctx, evals: *const u64, n: usize, z: *const u64, out_xy: *mut u64,
                               out_inf: *mut u8, y_out: *mut u64) -> c_int;
+    pub fn kzgb_compute_proofs_all_roots(ctx: *mut kzgb_ctx, evals: *const u64, n: usize, out_xy: *mut u64,
+                                         out_inf: *mut u8) -> c_int;
     pub fn kzgb_compute_blob_proof(ctx: *mut kzgb_ctx, blob: *const u8, len: usize, c_xy: *const u64, c_inf: u8,
                                    out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_commit_and_prove_blobs(ctx: *mut kzgb_ctx, blobs: *const *const u8, lens: *const usize, count: usize,

@@ -230,6 +230,14 @@ impl SRS<'_> {
         let rc = unsafe { ffi::kzgb_group_srs_prepare_lagrange(gpu.group, n) };
         if rc != 0 { Err(group_err(gpu.group, rc)) } else { Ok(()) }
     }
+    /// Builds the resident table of `KZG::compute_proofs_at_all_roots` for polynomials of `n` elements (n <= 2^22) now
+    /// instead of on the first call of that size.
+    pub fn prepare_all_roots(&self, n: usize) -> Result<(), KzgError> {
+        with_ctx(self, |ctx| {
+            let rc = unsafe { ffi::kzgb_srs_prepare_all_roots(ctx, n) };
+            if rc != 0 { Err(to_err(ctx, rc, n, self.g1.len())) } else { Ok(()) }
+        })
+    }
     /// Writes the decompressed points so that a later process can skip the per-point square root
     /// (`kzgb_srs_load_cache` checks every point to be on the curve instead).
     pub fn save_cache(&self, path: &str) -> Result<(), KzgError> {
@@ -386,6 +394,22 @@ impl KZG {
             .get_nth_root_of_unity(index as usize)
             .ok_or_else(|| KzgError::GenericError("Root of unity not found".to_string()))?;
         self.compute_proof(polynomial, z, srs)
+    }
+    /// `compute_proof_with_known_z_fr_index` (prover/src/kzg.rs:187-207) at every index 0 .. n-1 in one call (FK20 on
+    /// the GPU: two G1 FFTs and 2n scalar multiplications instead of n MSMs); element i is the proof at the i-th root.
+    pub fn compute_proofs_at_all_roots(&self, polynomial: &PolynomialEvalForm, srs: &SRS) -> Result<Vec<G1Affine>, KzgError> {
+        if polynomial.len() != self.expanded_roots_of_unity.len() {
+            return Err(KzgError::GenericError("inconsistent length between blob and root of unities".to_string()));
+        }
+        let ev = polynomial.evaluations();
+        let n = ev.len();
+        let mut xy = vec![0u64; 8 * n];
+        let mut inf = vec![0u8; n];
+        with_ctx(srs, |ctx| {
+            let rc = unsafe { ffi::kzgb_compute_proofs_all_roots(ctx, fr_words(ev), n, xy.as_mut_ptr(), inf.as_mut_ptr()) };
+            if rc != 0 { return Err(to_err(ctx, rc, n, srs.g1.len())); }
+            Ok((0..n).map(|i| unpack_point(xy[8 * i..8 * i + 8].try_into().unwrap(), inf[i])).collect())
+        })
     }
     pub fn g1_ifft(&self, length: usize, srs: &SRS) -> Result<Vec<G1Affine>, KzgError> {
         if !length.is_power_of_two() {
