@@ -176,7 +176,8 @@ int kzgb_compute_blob_proof(kzgb_ctx* ctx, const uint8_t* blob, size_t len, cons
                             uint64_t out_xy[8], uint8_t* out_inf);
 
 /* ---- batches (blob-sharded hot path) ------------------------------------------------------ */
-/* commit_blob + compute_blob_proof for `count` blobs, pipelined (H2D, GPU, host SHA-256 overlap).
+/* commit_blob + compute_blob_proof for `count` blobs, pipelined (H2D, GPU, host SHA-256 overlap).  The batch has no
+ * per-instance roots of unity, so the reference's roots-length check (kzg.rs:135-139) is not made.
  * commitments / proofs: count x 32 B arkworks `serialize_compressed` bytes (the encoding the
  * reference feeds to its transcripts, helpers.rs:457-461).  Blob pointers are HOST memory. */
 int kzgb_commit_and_prove_blobs(kzgb_ctx* ctx, const uint8_t* const* blobs, const size_t* lens, size_t count,
@@ -193,6 +194,22 @@ int kzgb_commit_blobs(kzgb_ctx* ctx, const uint8_t* const* blobs, const size_t* 
 /* Same with the blob bytes in device memory (no host copy needed: nothing is hashed). */
 int kzgb_commit_blobs_dev(kzgb_ctx* ctx, const uint8_t* const* blobs_dev, const size_t* lens, size_t count,
                           uint64_t* out_xy, uint8_t* out_inf);
+/* KZG::compute_blob_proof (kzg.rs:288-309) for `count` blobs with caller-supplied commitments, pipelined (H2D, GPU, host
+ * SHA-256 overlap); no commitment is computed.  commitments_xy: count x 8 words (x||y Montgomery), commitments_inf: count
+ * flags (may be NULL).  out_xy / out_inf as kzgb_commit_blobs.  Proof i and every error are those of
+ * kzgb_compute_blob_proof on (blob i, commitment i) alone: blob by blob in index order, the commitment on the curve
+ * (KZGB_ERR_NOT_ON_CURVE; the identity is valid), the length not 0 (GenericError "Length of data after padding is 0"),
+ * the SRS large enough (KZGB_ERR_SRS_CAPACITY); the error of the lowest-index blob that fails is returned before any
+ * work starts and the outputs are left untouched.  count == 0 writes nothing.  Like kzgb_commit_and_prove_blobs, the
+ * batch has no per-instance roots of unity, so the reference's roots-length check (kzg.rs:135-139) is not made. */
+int kzgb_compute_blob_proofs(kzgb_ctx* ctx, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                             const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                             uint64_t* out_xy, uint8_t* out_inf);
+/* Same with the blob bytes in device memory; host copies are still needed for the SHA-256 transcripts (pass them in
+ * `blobs_host`, as for kzgb_commit_and_prove_blobs_dev). */
+int kzgb_compute_blob_proofs_dev(kzgb_ctx* ctx, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
+                                 const size_t* lens, size_t count, const uint64_t* commitments_xy,
+                                 const uint8_t* commitments_inf, uint64_t* out_xy, uint8_t* out_inf);
 
 /* ---- batch verification, everything before the pairing (verifier/src/batch.rs:16-249) ------ */
 /* Per-blob challenge z_i and evaluation y_i (helpers.rs:613-662), RLC scalar r and its powers
@@ -244,13 +261,14 @@ int kzgb_validate_g1_points(kzgb_ctx* ctx, const uint64_t* xy, const uint8_t* in
  *   "ntt_kernel"           Fr (I)NTT implementation: 0 passes through shared-memory tiles, 1 warp-resident passes (registers, warp
  *                          shuffles, bulk asynchronous tile loads), -1 (default) by shape (1 for large batches of transforms of
  *                          <= 2^13, where it is 27 % faster; 0 elsewhere, where it is up to 12 % faster) -- same results
- *   "hash_mb"              -1 (default): kzgb_commit_and_prove_blobs hashes the transcripts of a large-blob batch sixteen at a time on
+ *   "hash_mb"              -1 (default): kzgb_commit_and_prove_blobs (and kzgb_compute_blob_proofs, where the groups the batch forms
+ *                          also hash faster than the pool, behind a single-stream head) hashes the transcripts of a large-blob batch sixteen at a time on
  *                          AVX-512 (multi-buffer SHA-256: ~2x the bytes per second of a core's SHA-NI, the 16 digests arrive together)
  *                          when the single-stream pool of this context's share of the host is slower than the GPU and >= 32 blobs
  *                          of exactly 32 * 2^j bytes are in the batch; 0: never; 1: whenever a group of >= 8 forms
  *   "hash_nice"            1 (default): the SHA-256 pool threads of a batch call run at nice 19, so a waking lane thread preempts them
  *   "hash_trace"           1: every multi-buffer group reports its wall and CPU time on stderr
- *   "device_hash"          -1 (default): kzgb_commit_and_prove_blobs decides how many transcripts of a large-blob batch are
+ *   "device_hash"          -1 (default): kzgb_commit_and_prove_blobs / kzgb_compute_blob_proofs decide how many transcripts of a large-blob batch are
  *                          hashed on the device next to the host pool (none unless the host cannot keep up even with "hash_mb" and
  *                          the batch is several hundred blobs deep); 0: none; k > 0: the last k eligible blobs
  *   "device_hash_lanes"    device kernel for those: 0 one warp per transcript (0.45 s, 16 % of a blob's MSM work each), 1 one lane per
@@ -306,6 +324,12 @@ int kzgb_group_commit_and_prove_blobs(kzgb_group* group, const uint8_t* const* b
  * Each member checks its own share before it starts. */
 int kzgb_group_commit_blobs(kzgb_group* group, const uint8_t* const* blobs, const size_t* lens, size_t count,
                             uint64_t* out_xy, uint8_t* out_inf);
+/* kzgb_compute_blob_proofs cut into contiguous shares of about equal bytes, one per member; identical to the one-context
+ * call.  Each member checks its own share before it starts (so on an error, members with valid shares may have written
+ * their proofs). */
+int kzgb_group_compute_blob_proofs(kzgb_group* group, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                                   const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                                   uint64_t* out_xy, uint8_t* out_inf);
 /* kzgb_msm_srs with the points cut into G contiguous ranges; the partial sums are added on the host. */
 int kzgb_group_msm_srs(kzgb_group* group, const uint64_t* scalars_mont, size_t n, uint64_t out_xy[8], uint8_t* out_inf);
 

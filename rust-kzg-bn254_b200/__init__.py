@@ -93,6 +93,20 @@ def _commit_blobs(call, blobs: Sequence["Blob"]) -> List[Affine]:
     return g1_from_abi(xy.raw[: 64 * count], inf.raw[:count])
 
 
+def _compute_blob_proofs(call, blobs: Sequence["Blob"], commitments: Sequence[Affine]) -> List[Affine]:
+    """Runs call(blob pointers, lengths, count, commitments_xy, commitments_inf, out_xy, out_inf) of a
+    kzgb_*compute_blob_proofs entry point; returns the proofs."""
+    if len(blobs) != len(commitments):
+        raise KzgError("GenericError", "length's of the input are not the same")
+    count = len(blobs)
+    keep, ptrs, lens = _blobs_to_abi(blobs)  # keep: the buffers ptrs points into
+    cxy, cinf = g1_to_abi(commitments)
+    xy = C.create_string_buffer(64 * count if count else 1)
+    inf = C.create_string_buffer(count if count else 1)
+    call(ptrs, lens, count, cxy, cinf, xy, inf)
+    return g1_from_abi(xy.raw[: 64 * count], inf.raw[:count])
+
+
 def _next_pow2(n: int) -> int:
     return 1 if n <= 1 else 1 << (n - 1).bit_length()
 
@@ -213,6 +227,11 @@ class Group:
     def commit_blobs(self, blobs: Sequence["Blob"]) -> List[Affine]:
         """KZG::commit_blob for every blob (prover/src/kzg.rs:182-185), the batch cut by blob across the members."""
         return _commit_blobs(lambda *a: self.check(lib.kzgb_group_commit_blobs(self.h, *a)), blobs)
+
+    def compute_blob_proofs(self, blobs: Sequence["Blob"], commitments: Sequence[Affine]) -> List[Affine]:
+        """KZG::compute_blob_proof for every (blob, commitment) pair (prover/src/kzg.rs:288-309), the batch cut by blob
+        across the members."""
+        return _compute_blob_proofs(lambda *a: self.check(lib.kzgb_group_compute_blob_proofs(self.h, *a)), blobs, commitments)
 
     def commit_coeff_form(self, polynomial: "PolynomialCoeffForm") -> Affine:
         """KZG::commit_coeff_form with the points cut into one range per GPU (prover/src/kzg.rs:107-125)."""
@@ -614,6 +633,13 @@ class KZG:
         return e._point_call(
             lambda h, *a: lib.kzgb_compute_blob_proof(h, blob.blob_data, len(blob.blob_data), xy, inf[0], *a)
         )
+
+    @staticmethod
+    def compute_blob_proofs(blobs: Sequence[Blob], commitments: Sequence[Affine], srs: SRS) -> List[Affine]:
+        """compute_blob_proof (kzg.rs:288-309) for every (blob, commitment) pair, pipelined inside the library; the
+        commitments are the caller's, none is computed."""
+        e = srs.engine
+        return _compute_blob_proofs(lambda *a: e.check(lib.kzgb_compute_blob_proofs(e.h, *a)), blobs, commitments)
 
     # -- fused hot path: commit + proof for a batch of blobs (sharded by blob across GPUs) ---
     @staticmethod

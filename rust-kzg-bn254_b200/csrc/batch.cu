@@ -1,6 +1,7 @@
 // The blob-batch pipelines: kzgb_commit_and_prove_blobs{,_dev} -- commitment and proof of many blobs on several lanes
 // while a hashing stage produces the Fiat-Shamir transcripts --, kzgb_commit_blobs{,_dev} -- the commitments alone, on
-// the same plan and lanes -- and kzgb_verify_batch_rlc.
+// the same plan and lanes --, kzgb_compute_blob_proofs{,_dev} -- the proofs alone, against the caller's commitments --
+// and kzgb_verify_batch_rlc.
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
@@ -54,10 +55,13 @@ constexpr size_t FSL_CAP = 4096;  // transcripts one batch call can hand to the 
 struct HashPlan {
     bool mb = false;        // multi-buffer groups on the host
     size_t mb_threads = 0;  // host threads in multi-buffer mode
+    size_t head = 0;        // multi-buffer mode: blobs [0, head) are hashed single-stream before the first group
     size_t dev_k = 0;       // transcripts hashed on the device (the last dev_k blobs)
     bool dev_lanes = false; // k_fs_midstate_lanes instead of k_fs_midstate_long
 };
-HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible) {
+// proof_only (kzgb_compute_blob_proofs): no commit phase hides the first transcripts, and a blob's whole GPU work follows
+// its transcript.
+HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible, bool proof_only) {
     HashPlan hp;
     if (count < 2) return hp;
     double bytes = 0;
@@ -69,7 +73,11 @@ HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible) {
     if (const char* w = getenv("LOCAL_WORLD_SIZE")) { int v = atoi(w); if (v > procs) procs = v; }
     const double share = std::max(1.0, (double)hw / procs);                                          // hardware threads of this context
     const double rate_ni = 1.2e9 * std::max(1.0, std::min<double>((double)hash_pool_threads(), share));  // B/s, HT siblings both hashing
-    const double t_gpu = 2.75e-3 * per_blob / (double)(16u << 20);  // commit + proof of one blob
+    // GPU time of one blob: commit + proof, or (proof_only) the proof alone: 1.6e-3 s = 1 / 622 blobs/s, the rate of
+    // kzgb_compute_blob_proofs_dev at 64 x 2^19 Fr with the single-stream pool keeping up (scripts/blob_proofs_bench.py,
+    // B200 at 1000 W, 16 hardware threads; the ~9 ms to the first transcript included)
+    const double t_gpu = (proof_only ? 1.6e-3 : 2.75e-3) * per_blob / (double)(16u << 20);
+    const double after_hash = proof_only ? 1.0 : 0.5;  // the share of t_gpu that waits for the blob's transcript
     // eligible blobs: exactly 32 * 2^j bytes, j >= 10 (the multi-buffer and device kernels hash whole 64-byte blocks)
     size_t eligible_total = 0, eligible_tail = 0;
     for (size_t i = 0; i < count; i++) eligible_total += hash_mb_eligible(lens[i]);
@@ -78,10 +86,17 @@ HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible) {
     // "keeps up" = the single-stream pool needs at most half of this context's hardware threads for the duration of the GPU work:
     // the other half belongs to the lanes and the driver (measured on 4 hardware threads per rank: 291 blobs/s single stream, 367 multi-buffer)
     const bool ni_keeps_up = bytes / rate_ni <= 0.5 * count * t_gpu;
-    if (sha256_has_mb16() && mb_opt != 0 && eligible_total >= 16 && (mb_opt == 1 || (!ni_keeps_up && eligible_total >= 32))) {
+    const int ht = g_hash_threads.load();
+    const size_t mb_threads = (size_t)std::max(1.0, ht > 0 ? (double)ht : share - 1.0);  // one hardware thread of the share stays with the lanes
+    // proof_only: multi-buffer only where the groups the batch forms hash faster than the pool (64 blobs are 4 groups,
+    // 4 threads: 418 blobs/s against 622 single-stream on 16 hardware threads)
+    const bool mb_faster = !proof_only || 2.4e9 * (double)std::min(mb_threads, eligible_total / 16) > rate_ni;
+    if (sha256_has_mb16() && mb_opt != 0 && eligible_total >= 16 && (mb_opt == 1 || (!ni_keeps_up && mb_faster && eligible_total >= 32))) {
         hp.mb = true;
-        const int ht = g_hash_threads.load();
-        hp.mb_threads = (size_t)std::max(1.0, ht > 0 ? (double)ht : share - 1.0);  // one hardware thread of the share stays with the lanes
+        hp.mb_threads = mb_threads;
+        // the 16 midstates of a group arrive together after 71-80 ms (16 MiB blobs): without a commit phase the lanes would
+        // idle that long, so every hashing thread first hashes one blob of the head single-stream (~9 ms)
+        if (proof_only) hp.head = std::min(count, hp.mb_threads);
     }
     const int dev_opt = device_possible ? g_device_hash.load() : 0;
     if (dev_opt > 0) { hp.dev_k = std::min<size_t>((size_t)dev_opt, eligible_tail); hp.dev_lanes = fs_midstate_lanes() != 0; return hp; }
@@ -93,7 +108,7 @@ HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible) {
         const double t_dev = (lanes ? 0.95 : 0.45) * per_blob / (double)(16u << 20), dev_cost = lanes ? 0.006 : 0.16;
         for (size_t k = 1; k <= eligible_tail; k++) {
             // GPU busy time; host time for the front of the batch; the device's share lands at t_dev and its proofs follow
-            const double t = std::max({(count + dev_cost * k) * t_gpu, (double)(count - k) * per_blob / rate_host, t_dev + k * t_gpu * 0.5});
+            const double t = std::max({(count + dev_cost * k) * t_gpu, (double)(count - k) * per_blob / rate_host, t_dev + k * t_gpu * after_hash});
             if (t < best * 0.97) { best = t; hp.dev_k = k; hp.dev_lanes = lanes != 0; }
         }
     }
@@ -101,7 +116,8 @@ HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible) {
 }
 
 // ---------------------------------------------------------------- planning
-// One kzgb_commit_and_prove_blobs{,_dev} or kzgb_commit_blobs{,_dev} call: its arguments and the plan made for them.
+// One kzgb_commit_and_prove_blobs{,_dev}, kzgb_commit_blobs{,_dev} or kzgb_compute_blob_proofs{,_dev} call: its arguments
+// and the plan made for them.
 struct Batch {
     kzgb_ctx* c;
     const uint8_t* const* blobs_dev;   // nullptr: the blobs are only on the host
@@ -113,6 +129,8 @@ struct Batch {
     bool commit_only = false;  // kzgb_commit_blobs: commitments into out_xy / out_inf, no proofs
     uint64_t* out_xy = nullptr;
     uint8_t* out_inf = nullptr;
+    bool prove_only = false;      // kzgb_compute_blob_proofs: proofs against `commits` into out_xy / out_inf, no commit phase
+    std::vector<Affine> commits;  // prove_only: the caller's commitments
     size_t max_n = 0;
     std::vector<std::pair<size_t, size_t>> groups;  // small blobs: (first blob, blobs); empty: one blob per task
     int n_lanes = 0;
@@ -123,7 +141,7 @@ struct Batch {
 
 // Validation, groups, lanes and the tables every size of the batch needs.  A commit-only batch checks every blob as
 // kzgb_commit_blob does (a blob of length 0 commits the zero polynomial of size 1); with proofs, length 0 is
-// compute_blob_proof's error.
+// compute_blob_proof's error, and a proof-only batch checks each commitment first, as kzgb_compute_blob_proof does.
 int plan_batch(Batch& b) {
     kzgb_ctx* c = b.c;
     const size_t* lens = b.lens;
@@ -132,6 +150,7 @@ int plan_batch(Batch& b) {
         if (b.commit_only) {
             if (int rc = check_commit_blob_len(c, blob_poly_len(lens[i]))) return rc;
         } else {
+            if (b.prove_only && !aff_on_curve(b.commits[i])) return fail(c, KZGB_ERR_NOT_ON_CURVE, "G1 point not on curve");
             if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
             if (int rc = check_srs_capacity(c, blob_poly_len(lens[i]))) return rc;
         }
@@ -218,6 +237,12 @@ public:
         failed = true;
         cv.notify_all();
     }
+    // Waits for the midstates of blobs [first, first + n); false: a lane failed.
+    bool wait_ready(size_t first, size_t n) {
+        std::unique_lock<std::mutex> lk(mu);
+        for (size_t k = 0; k < n; k++) cv.wait(lk, [&] { return ready[first + k] != 0 || failed; });
+        return !failed;
+    }
     // blob i went up to c->batch_bytes on the hashing stream (ev_hash_uploaded)
     bool uploaded_here(size_t i) const { return i >= dev_first && !dev_failed.load(); }
 
@@ -251,7 +276,7 @@ HashStage::HashStage(const Batch& batch, const HashPlan& hp)
     if (dev_k && !dev_failed.load()) poller = std::thread(&HashStage::poll_device, this);
     for (size_t i = 0; i < b.count;) {
         size_t j = i + 1;
-        if (hp.mb && i < dev_first && hash_mb_eligible(b.lens[i])) {
+        if (hp.mb && i >= hp.head && i < dev_first && hash_mb_eligible(b.lens[i])) {
             while (j < dev_first && j - i < 16 && b.lens[j] == b.lens[i]) j++;
             if (j - i < 8) j = i + 1;  // a group under half full hashes no faster than its members one by one
         }
@@ -390,11 +415,38 @@ int run_lanes(const Batch& b, F lane_main) {
     return KZGB_OK;
 }
 
+// Where proof i goes: arkworks-compressed bytes (commit_and_prove), or the affine ABI (compute_blob_proofs).
+void put_proof(const Batch& b, size_t i, const Affine& p) {
+    if (b.prove_only) affine_to_abi(p, b.out_xy + 8 * i, b.out_inf ? b.out_inf + i : nullptr);
+    else serialize_compressed(p, b.proofs32 + 32 * i);
+}
+
+// The bytes of the bn blobs from blob i0 (all of n elements) at a stride of 32 n with zero-filled tails, so that one launch
+// covers the group: device blobs that already are back to back and full are read in place, the others are gathered
+// into L.bytes.
+int group_bytes(const Batch& b, Lane& L, size_t i0, size_t bn, const uint8_t** src) {
+    kzgb_ctx* c = b.c;
+    const uint8_t* const* blobs_dev = b.blobs_dev;
+    const size_t n = blob_poly_len(b.lens[i0]);
+    bool dev_run = blobs_dev != nullptr;
+    for (size_t k = 0; k < bn && dev_run; k++) dev_run = b.lens[i0 + k] == n * 32 && blobs_dev[i0 + k] == blobs_dev[i0] + k * n * 32;
+    if (dev_run) { *src = blobs_dev[i0]; return KZGB_OK; }
+    CK(c, L.bytes.reserve(bn * n * 32));
+    for (size_t k = 0; k < bn; k++) {
+        uint8_t* dst = (uint8_t*)L.bytes.p + k * n * 32;
+        const size_t len = b.lens[i0 + k];
+        if (len && blobs_dev) CK(c, cudaMemcpyAsync(dst, blobs_dev[i0 + k], len, cudaMemcpyDeviceToDevice, L.st));
+        else if (len) CK(c, cudaMemcpyAsync(dst, b.blobs_host[i0 + k], len, cudaMemcpyHostToDevice, L.st));
+        if (len < n * 32) CK(c, cudaMemsetAsync(dst + len, 0, n * 32 - len, L.st));
+    }
+    *src = (const uint8_t*)L.bytes.p;
+    return KZGB_OK;
+}
+
 // The commitment phase of one group: bn blobs of one size n from blob i0, ONE batched launch set; pts[k] is the
 // commitment of blob i0 + k.  With proofs to follow, or without a Lagrange table, the blob bytes become Montgomery
 // evaluations in L.evals (which the proof phase reads).  A commit-only group over a Lagrange table hands the bytes to
-// the MSM's first pass instead: laid out at a stride of 32 n with zero-filled tails (device blobs that already are
-// back to back and full are read in place), so that one launch covers the group.
+// the MSM's first pass instead (group_bytes).
 int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
     kzgb_ctx* c = b.c;
     const uint8_t* const* blobs_dev = b.blobs_dev;
@@ -402,7 +454,14 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
     const size_t n = blob_poly_len(lens[i0]);
     const int logn = log2_exact(n);
     const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
-    const bool from_bytes = b.commit_only && lag;
+    MsmJob job;
+    if (b.commit_only && lag) {
+        const uint8_t* src = nullptr;
+        int r = group_bytes(b, L, i0, bn, &src);
+        if (!r) r = msm_enqueue(c, L, {nullptr, src, (uint64_t)bn * n * 32}, n, bn, lag, nullptr, 0, &job);
+        if (!r) r = msm_finish(c, L, job, pts);
+        return r;
+    }
     Fr ninv = ninv_mont(logn);
     int r = KZGB_OK;
     auto ck = [&](cudaError_t e, const char* what) {
@@ -412,32 +471,10 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
     for (size_t k = 0; k < bn; k++) full = full && lens[i0 + k] == n * 32;
     bool dev_run = blobs_dev && full;  // device blobs back to back: one conversion launch too
     for (size_t k = 0; k < bn && dev_run; k++) dev_run = blobs_dev[i0 + k] == blobs_dev[i0] + k * n * 32;
-    if (!from_bytes) {
-        ck(L.evals.reserve(bn * n * sizeof(Fr)), "evals");
-        ck(L.work.reserve(bn * n * sizeof(Fr)), "work");
-    }
-    if (!b.commit_only) {  // the proof phase's buffers
-        ck(L.small.reserve((3 * bn + 8) * sizeof(Fr)), "small");
-        ck(L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)bn) * sizeof(Fr)), "eval scratch");
-    }
+    ck(L.evals.reserve(bn * n * sizeof(Fr)), "evals");
+    ck(L.work.reserve(bn * n * sizeof(Fr)), "work");
     if (!lag) ck(L.ntt_scratch.reserve(bn * n * sizeof(Fr)), "ntt scratch");
-    if (from_bytes ? !dev_run : !blobs_dev) ck(L.bytes.reserve(bn * n * 32), "bytes");
-    MsmJob job;
-    if (from_bytes) {
-        for (size_t k = 0; k < bn && !r && !dev_run; k++) {
-            uint8_t* dst = (uint8_t*)L.bytes.p + k * n * 32;
-            const size_t len = lens[i0 + k];
-            if (len) {
-                if (blobs_dev) ck(cudaMemcpyAsync(dst, blobs_dev[i0 + k], len, cudaMemcpyDeviceToDevice, L.st), "D2D copy of a blob");
-                else ck(cudaMemcpyAsync(dst, b.blobs_host[i0 + k], len, cudaMemcpyHostToDevice, L.st), "H2D copy of a blob");
-            }
-            if (len < n * 32) ck(cudaMemsetAsync(dst + len, 0, n * 32 - len, L.st), "zero fill");
-        }
-        const uint8_t* src = dev_run ? blobs_dev[i0] : (const uint8_t*)L.bytes.p;
-        if (!r) r = msm_enqueue(c, L, {nullptr, src, (uint64_t)bn * n * 32}, n, bn, lag, nullptr, 0, &job);
-        if (!r) r = msm_finish(c, L, job, pts);
-        return r;
-    }
+    if (!blobs_dev) ck(L.bytes.reserve(bn * n * 32), "bytes");
     if (dev_run) bytes_to_fr_launch(blobs_dev[i0], (uint64_t)bn * n * 32, (Fr*)L.evals.p, (uint32_t)(bn * n), L.st);
     for (size_t k = 0; k < bn && !r && !dev_run; k++) {
         const uint8_t* src = blobs_dev ? blobs_dev[i0 + k] : nullptr;
@@ -462,52 +499,70 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
     return r;
 }
 
-// Small blobs: groups of equal-size blobs, each phase of a group is ONE batched launch set.
+// The proof phase of one group whose transcript midstates are ready and whose Montgomery evaluations are in L.evals: the
+// challenges of blobs i0 .. i0 + bn - 1 against the commitments cs[0 .. bn), ONE batched evaluation / quotient launch set
+// with a challenge per blob and ONE batched MSM of the quotients; pts[k] is the proof of blob i0 + k.
+int group_prove(const Batch& b, const HashStage& hs, Lane& L, size_t i0, size_t bn, const Affine* cs, Affine* pts) {
+    kzgb_ctx* c = b.c;
+    const size_t n = blob_poly_len(b.lens[i0]);
+    const int logn = log2_exact(n);
+    const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
+    Fr ninv = ninv_mont(logn);
+    CK(c, L.small.reserve((3 * bn + 8) * sizeof(Fr)));
+    CK(c, L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)bn) * sizeof(Fr)));
+    CK(c, L.work.reserve(bn * n * sizeof(Fr)));
+    if (!lag) CK(c, L.ntt_scratch.reserve(bn * n * sizeof(Fr)));
+    std::vector<Fr> zt(2 * bn);
+    bool any_in_domain = false;
+    for (size_t k = 0; k < bn; k++) {
+        zt[k] = challenge_finish(hs.mid[i0 + k], cs[k]);
+        zt[bn + k] = eval_tinv(zt[k], logn, &any_in_domain);
+    }
+    Fr* d_z = (Fr*)L.small.p;  // [z x bn | tinv x bn | y x bn]
+    CK(c, cudaMemcpyAsync(d_z, zt.data(), 2 * bn * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+    eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)bn, d_z, d_z + bn, c->tw, c->logN, &ninv,
+                         (Fr*)L.eval_scratch.p, (Fr*)L.work.p, d_z + 2 * bn, L.st, !any_in_domain);
+    if (!lag) ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+    MsmJob job;
+    int r = msm_enqueue(c, L, {(const Fr*)L.work.p}, n, bn, lag, nullptr, 0, &job);
+    if (!r) r = msm_finish(c, L, job, pts);
+    return r;
+}
+
+// Small blobs: groups of equal-size blobs, each phase of a group is ONE batched launch set.  A proof-only group has no
+// commitment phase: its blob bytes (group_bytes) become Montgomery evaluations in one conversion launch and the
+// commitments are the caller's.
 int group_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next_group, int li) {
     kzgb_ctx* c = b.c;
-    const size_t* lens = b.lens;
     Lane& L = c->lanes[li];
-    std::vector<Affine> pts;
-    std::vector<Fr> zt;
+    std::vector<Affine> commits, pts;
     for (;;) {
         size_t gi = next_group.fetch_add(1);
         if (gi >= b.groups.size()) return KZGB_OK;
         { std::lock_guard<std::mutex> lk(hs.mu); if (hs.failed) return KZGB_OK; }
         const size_t i0 = b.groups[gi].first, bn = b.groups[gi].second;
-        const size_t n = blob_poly_len(lens[i0]);
-        const int logn = log2_exact(n);
-        const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
-        Fr ninv = ninv_mont(logn);
+        const size_t n = blob_poly_len(b.lens[i0]);
+        int r = KZGB_OK;
+        const Affine* cs = nullptr;
+        if (b.prove_only) {
+            const uint8_t* src = nullptr;
+            r = group_bytes(b, L, i0, bn, &src);
+            if (!r && L.evals.reserve(bn * n * sizeof(Fr)) != cudaSuccess) r = fail(c, KZGB_ERR_DEVICE, "CUDA error: evals");
+            if (!r) bytes_to_fr_launch(src, (uint64_t)bn * n * 32, (Fr*)L.evals.p, (uint32_t)(bn * n), L.st);
+            cs = b.commits.data() + i0;
+        } else {
+            commits.resize(bn);
+            r = group_commit(b, L, i0, bn, commits.data());
+            if (!r) for (size_t k = 0; k < bn; k++) serialize_compressed(commits[k], b.commitments32 + 32 * (i0 + k));
+            cs = commits.data();
+        }
         pts.resize(bn);
-        int r = group_commit(b, L, i0, bn, pts.data());
-        auto ck = [&](cudaError_t e, const char* what) {
-            if (!r && e != cudaSuccess) r = fail(c, KZGB_ERR_DEVICE, std::string("CUDA error: ") + cudaGetErrorString(e) + " at " + what);
-        };
-        MsmJob job;
         if (!r) {
-            for (size_t k = 0; k < bn; k++) serialize_compressed(pts[k], b.commitments32 + 32 * (i0 + k));
-            // challenges: the transcript midstates come from the hashing stage
-            zt.resize(2 * bn);
-            {
-                std::unique_lock<std::mutex> lk(hs.mu);
-                for (size_t k = 0; k < bn; k++) hs.cv.wait(lk, [&] { return hs.ready[i0 + k] != 0 || hs.failed; });
-                if (hs.failed) return KZGB_OK;
-            }
-            bool any_in_domain = false;
-            for (size_t k = 0; k < bn; k++) {
-                zt[k] = challenge_finish(hs.mid[i0 + k], pts[k]);
-                zt[bn + k] = eval_tinv(zt[k], logn, &any_in_domain);
-            }
-            Fr* d_z = (Fr*)L.small.p;  // [z x bn | tinv x bn | y x bn]
-            ck(cudaMemcpyAsync(d_z, zt.data(), 2 * bn * sizeof(Fr), cudaMemcpyHostToDevice, L.st), "H2D of the challenges");
-            eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)bn, d_z, d_z + bn, c->tw, c->logN, &ninv,
-                                 (Fr*)L.eval_scratch.p, (Fr*)L.work.p, d_z + 2 * bn, L.st, !any_in_domain);
-            if (!lag) ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-            if (!r) r = msm_enqueue(c, L, {(const Fr*)L.work.p}, n, bn, lag, nullptr, 0, &job);
-            if (!r) r = msm_finish(c, L, job, pts.data());
+            if (!hs.wait_ready(i0, bn)) return KZGB_OK;  // the transcript midstates come from the hashing stage
+            r = group_prove(b, hs, L, i0, bn, cs, pts.data());
         }
         if (r) { hs.fail(); return r; }
-        for (size_t k = 0; k < bn; k++) serialize_compressed(pts[k], b.proofs32 + 32 * (i0 + k));
+        for (size_t k = 0; k < bn; k++) put_proof(b, i0 + k, pts[k]);
     }
 }
 
@@ -597,7 +652,7 @@ int commit_and_prove(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t
     int rc = plan_batch(b);
     if (rc) return rc;
     stage_blob_bytes(b);
-    const HashPlan hplan = b.groups.empty() ? hash_plan(lens, count, blobs_dev || b.resident) : HashPlan();
+    const HashPlan hplan = b.groups.empty() ? hash_plan(lens, count, blobs_dev || b.resident, false) : HashPlan();
     {
         HashStage hs(b, hplan);
         rc = b.groups.empty() ? run_tasks(b, hs) : run_groups(b, hs);
@@ -664,6 +719,59 @@ int commit_blobs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* co
     return run_lanes(b, [&](int li) {
         return b.groups.empty() ? commit_task_lane(b, next, failed, li) : commit_group_lane(b, next, failed, li);
     });
+}
+
+// ---------------------------------------------------------------- proofs only
+// Large blobs: every task is "prove blob i", taken in blob order.  A blob is read once, so it goes up into the lane's own
+// buffer (unless the device's share of the hashing has staged it already) and is converted while its transcript is
+// hashed.  Then the challenge with the caller's commitment, the quotient and its MSM.
+int prove_task_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next, int li) {
+    kzgb_ctx* c = b.c;
+    Lane& L = c->lanes[li];
+    for (;;) {
+        const size_t i = next.fetch_add(1);
+        if (i >= b.count) return KZGB_OK;
+        const size_t len = b.lens[i], n = blob_poly_len(len);
+        const uint8_t* dev_bytes = b.blobs_dev ? b.blobs_dev[i] : nullptr;
+        int r = KZGB_OK;
+        if (!dev_bytes && hs.uploaded_here(i)) {
+            if (cudaStreamWaitEvent(L.st, c->ev_hash_uploaded, 0) != cudaSuccess)
+                r = fail(c, KZGB_ERR_DEVICE, "CUDA error: cudaStreamWaitEvent failed");
+            dev_bytes = (const uint8_t*)c->batch_bytes.p + b.byte_off[i];
+        }
+        if (!r) r = blob_to_evals(c, L, b.blobs_host[i], dev_bytes, len, n);
+        if (!r && !hs.wait_ready(i, 1)) return KZGB_OK;
+        MsmJob job;
+        Affine out;
+        if (!r) r = proof_enqueue(c, L, (Fr*)L.evals.p, n, challenge_finish(hs.mid[i], b.commits[i]), &job);
+        if (!r) r = msm_finish(c, L, job, &out);
+        if (r) { hs.fail(); return r; }
+        put_proof(b, i, out);
+    }
+}
+
+int compute_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
+                        size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf, uint64_t* out_xy,
+                        uint8_t* out_inf) {
+    if (count == 0) return KZGB_OK;
+    Batch b{c, blobs_dev, blobs_host, lens, count, nullptr, nullptr, false, out_xy, out_inf};
+    b.prove_only = true;
+    b.commits.resize(count);
+    for (size_t i = 0; i < count; i++) b.commits[i] = affine_from_abi(commitments_xy + 8 * i, commitments_inf ? commitments_inf[i] : 0);
+    int rc = plan_batch(b);
+    if (rc) return rc;
+    HashPlan hplan = b.groups.empty() ? hash_plan(lens, count, true, true) : HashPlan();
+    if (hplan.dev_k && !blobs_dev) {  // the device hashes blobs it holds: stage the host blobs
+        stage_blob_bytes(b);
+        if (!b.resident) hplan.dev_k = 0;
+    }
+    {
+        HashStage hs(b, hplan);
+        std::atomic<size_t> next{0};
+        rc = run_lanes(b, [&](int li) { return b.groups.empty() ? prove_task_lane(b, hs, next, li) : group_lane(b, hs, next, li); });
+    }
+    if (b.resident && c->batch_bytes.cap > ((size_t)g_batch_keep_mib.load() << 20)) c->batch_bytes.release();
+    return rc;
 }
 
 // The random linear combination of m validated and evaluated openings (batch.rs:76-249): d_bases holds C_0 .. C_{m-1},
@@ -736,6 +844,17 @@ int kzgb_commit_blobs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const si
                           uint64_t* out_xy, uint8_t* out_inf) {
     Guard g(c);
     return commit_blobs(c, blobs_dev, nullptr, lens, count, out_xy, out_inf);
+}
+int kzgb_compute_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                             const uint64_t* commitments_xy, const uint8_t* commitments_inf, uint64_t* out_xy, uint8_t* out_inf) {
+    Guard g(c);
+    return compute_blob_proofs(c, nullptr, blobs, lens, count, commitments_xy, commitments_inf, out_xy, out_inf);
+}
+int kzgb_compute_blob_proofs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
+                                 const size_t* lens, size_t count, const uint64_t* commitments_xy,
+                                 const uint8_t* commitments_inf, uint64_t* out_xy, uint8_t* out_inf) {
+    Guard g(c);
+    return compute_blob_proofs(c, blobs_dev, blobs_host, lens, count, commitments_xy, commitments_inf, out_xy, out_inf);
 }
 // ------------------------------------------------------------------------------- batch verification (RLC)
 int kzgb_verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,

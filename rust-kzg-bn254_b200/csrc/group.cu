@@ -206,6 +206,23 @@ int kzgb_group_commit_blobs(kzgb_group* g, const uint8_t* const* blobs, const si
     });
 }
 
+// KZG::compute_blob_proof (prover/src/kzg.rs:288-309) for `count` blobs with the caller's commitments, cut as
+// kzgb_group_commit_and_prove_blobs cuts them.
+int kzgb_group_compute_blob_proofs(kzgb_group* g, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                                   const uint64_t* commitments_xy, const uint8_t* commitments_inf, uint64_t* out_xy,
+                                   uint8_t* out_inf) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    if (count == 0) return KZGB_OK;
+    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
+    return for_members(g, [&](int i) {
+        const size_t a = cut[i], b = cut[i + 1];
+        if (a >= b) return (int)KZGB_OK;
+        return kzgb_compute_blob_proofs(g->ctx[i], blobs + a, lens + a, b - a, commitments_xy + 8 * a,
+                                        commitments_inf ? commitments_inf + a : nullptr, out_xy + 8 * a,
+                                        out_inf ? out_inf + a : nullptr);
+    });
+}
+
 // ---- one large MSM over the SRS, sharded by point range -------------------------------------------------------
 // KZG::commit_coeff_form (prover/src/kzg.rs:107-125) for polynomials too large for one GPU's liking: member i
 // computes sum_{j in share i} s_j SRS_j (fixed-base over its range table when kzgb_group_srs_precompute_ranges was

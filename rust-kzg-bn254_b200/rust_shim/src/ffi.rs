@@ -75,6 +75,9 @@ extern "C" {
                                              commitments32: *mut u8, proofs32: *mut u8) -> c_int;
     pub fn kzgb_group_commit_blobs(group: *mut kzgb_group, blobs: *const *const u8, lens: *const usize, count: usize,
                                    out_xy: *mut u64, out_inf: *mut u8) -> c_int;
+    pub fn kzgb_group_compute_blob_proofs(group: *mut kzgb_group, blobs: *const *const u8, lens: *const usize, count: usize,
+                                          commitments_xy: *const u64, commitments_inf: *const u8, out_xy: *mut u64,
+                                          out_inf: *mut u8) -> c_int;
     pub fn kzgb_group_msm_srs(group: *mut kzgb_group, scalars: *const u64, n: usize, out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_verify_batch_rlc(ctx: *mut kzgb_ctx, blobs: *const *const u8, lens: *const usize, count: usize,
                                  commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,

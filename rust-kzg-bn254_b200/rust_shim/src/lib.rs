@@ -437,6 +437,43 @@ impl KZG {
             if rc != 0 { Err(to_err(ctx, rc, n, srs.g1.len())) } else { Ok(unpack_point(&xy, inf)) }
         })
     }
+    /// Addition next to the reference's API: `compute_blob_proof` for every (blob, commitment) pair in ONE call, for
+    /// callers that already hold the commitments.  The batch is cut by bytes across the GPUs of the box
+    /// (`kzgb_group_compute_blob_proofs`) and pipelined on each; no commitment is computed.  Proof i is
+    /// `compute_blob_proof(blob i, commitment i)`, and an error is the one `compute_blob_proof` reports for the first
+    /// pair the library rejects (without the per-instance roots-length check, which a batch of sizes has no use for).
+    pub fn compute_blob_proofs(&self, blobs: &[Blob], commitments: &[G1Affine], srs: &SRS) -> Result<Vec<G1Affine>, KzgError> {
+        if blobs.len() != commitments.len() {
+            return Err(KzgError::GenericError("length's of the input are not the same".to_string()));
+        }
+        let ptrs: Vec<*const u8> = blobs.iter().map(|b| b.data().as_ptr()).collect();
+        let lens: Vec<usize> = blobs.iter().map(|b| b.data().len()).collect();
+        let (cxy, cinf) = pack_points(commitments);
+        let mut xy = vec![0u64; 8 * blobs.len()];
+        let mut inf = vec![0u8; blobs.len()];
+        let gpu = gpu_for(srs)?;
+        let rc = unsafe {
+            ffi::kzgb_group_compute_blob_proofs(gpu.group, ptrs.as_ptr(), lens.as_ptr(), blobs.len(), cxy.as_ptr(), cinf.as_ptr(),
+                                                xy.as_mut_ptr(), inf.as_mut_ptr())
+        };
+        if rc != 0 {
+            // the library fails on the lowest-index pair that does not pass compute_blob_proof's checks; the group's
+            // message names the member, so the error is rebuilt from that pair as compute_blob_proof reports it
+            let srs_len = srs.g1.len();
+            for (len, commitment) in lens.iter().zip(commitments) {
+                helpers::validate_g1_point(commitment)?;
+                if *len == 0 {
+                    return Err(KzgError::GenericError("Length of data after padding is 0".to_string()));
+                }
+                let polynomial_len = len.div_ceil(32).next_power_of_two();
+                if polynomial_len > srs_len {
+                    return Err(KzgError::SrsCapacityExceeded { polynomial_len, srs_len });
+                }
+            }
+            return Err(group_err(gpu.group, rc));
+        }
+        Ok((0..blobs.len()).map(|i| unpack_point(xy[8 * i..8 * i + 8].try_into().unwrap(), inf[i])).collect())
+    }
 }
 
 impl KZG {
