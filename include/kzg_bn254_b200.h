@@ -231,7 +231,8 @@ int kzgb_validate_g1_points(kzgb_ctx* ctx, const uint64_t* xy, const uint8_t* in
 
 /* Process-wide switches that never change results, only which exact code path produces them:
  *   "fs_device"            -1 auto (default), 0 host SHA-256 pool, 1 device kernel for the per-blob
- *                          Fiat-Shamir challenges of kzgb_verify_batch_rlc (auto: >= 256 blobs of <= 2^13 Fr)
+ *                          Fiat-Shamir challenges of kzgb_verify_batch_rlc and kzgb_verify_blob_proofs_g1{,_dev}
+ *                          (auto: >= 256 blobs of <= 2^13 Fr)
  *   "acc_waves"            waves of bucket-accumulation blocks the sorted list is cut into (default 4; any value >= 1
  *                          gives the same result -- tests use it to move the chunk boundaries)
  *   "fs_force_generic"     1: the device-hashed challenges of kzgb_verify_batch_rlc are all flagged "in the domain", so the
@@ -290,6 +291,25 @@ int kzgb_verify_proof_g1(kzgb_ctx* ctx, const uint64_t c_xy[8], uint8_t c_inf, c
 int kzgb_verify_blob_proof_g1(kzgb_ctx* ctx, const uint8_t* blob, size_t len, const uint64_t c_xy[8], uint8_t c_inf,
                               const uint64_t proof_xy[8], uint8_t proof_inf, uint64_t out_xy[8], uint8_t* out_inf,
                               uint64_t z_out[4], uint64_t y_out[4]);
+/* verify_blob_kzg_proof (verify.rs:77-115) up to the pairing for `count` blobs.  out i / z i / y i are what
+ * kzgb_verify_blob_proof_g1 returns for (blob i, commitment i, proof i) alone: out = C_i - [y_i] G1 (count x 8 words,
+ * x||y Montgomery; out_inf count flags, may be NULL), z_i = compute_challenge(blob i, C_i), y_i = p_i(z_i) (count x 4
+ * words Montgomery each, either may be NULL).  Checks, blob by blob in index order: C_i and proof_i on the curve
+ * (KZGB_ERR_NOT_ON_CURVE; the identity is valid), length not 0 (GenericError "Length of data after padding is 0"),
+ * polynomial length <= 2^28 (GenericError "Input size exceeds maximum polynomial size").  The error of the lowest-index
+ * blob that fails is returned before any work starts, and the outputs are left untouched.  count == 0 writes nothing.
+ * No SRS is needed.  commitments_inf / proofs_inf may be NULL (no identity among them).  The challenges are hashed as
+ * kzgb_verify_batch_rlc hashes them (option "fs_device"); C_i - [y_i] G1 is one GPU thread per blob. */
+int kzgb_verify_blob_proofs_g1(kzgb_ctx* ctx, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                               const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                               const uint64_t* proofs_xy, const uint8_t* proofs_inf,
+                               uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out);
+/* Same with the blob bytes in device memory.  Host copies are still needed for the SHA-256 transcripts (blobs_host),
+ * as for kzgb_compute_blob_proofs_dev. */
+int kzgb_verify_blob_proofs_g1_dev(kzgb_ctx* ctx, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
+                                   const size_t* lens, size_t count, const uint64_t* commitments_xy,
+                                   const uint8_t* commitments_inf, const uint64_t* proofs_xy, const uint8_t* proofs_inf,
+                                   uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out);
 
 /* ---- multi-GPU: one handle over several GPUs of one box (SURVEY.md 8e) ------------------------------------
  * The path shards by blob (batches) and by point range (one large MSM) and has no exchange step besides adding
@@ -330,6 +350,13 @@ int kzgb_group_commit_blobs(kzgb_group* group, const uint8_t* const* blobs, cons
 int kzgb_group_compute_blob_proofs(kzgb_group* group, const uint8_t* const* blobs, const size_t* lens, size_t count,
                                    const uint64_t* commitments_xy, const uint8_t* commitments_inf,
                                    uint64_t* out_xy, uint8_t* out_inf);
+/* kzgb_verify_blob_proofs_g1 cut into contiguous shares of about equal bytes, one per member; identical to the one-context
+ * call.  Each member checks its own share before it starts (so on an error, members with valid shares may have written
+ * their outputs). */
+int kzgb_group_verify_blob_proofs_g1(kzgb_group* group, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                                     const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                                     const uint64_t* proofs_xy, const uint8_t* proofs_inf,
+                                     uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out);
 /* kzgb_msm_srs with the points cut into G contiguous ranges; the partial sums are added on the host. */
 int kzgb_group_msm_srs(kzgb_group* group, const uint64_t* scalars_mont, size_t n, uint64_t out_xy[8], uint8_t* out_inf);
 

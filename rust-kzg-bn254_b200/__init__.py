@@ -107,6 +107,24 @@ def _compute_blob_proofs(call, blobs: Sequence["Blob"], commitments: Sequence[Af
     return g1_from_abi(xy.raw[: 64 * count], inf.raw[:count])
 
 
+def _verify_blob_proofs(call, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]):
+    """Runs call(blob pointers, lengths, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, out_xy, out_inf,
+    z_out, y_out) of a kzgb_*verify_blob_proofs_g1 entry point; returns (C_i - [y_i] G1, z_i, y_i) for every blob."""
+    if not (len(commitments) == len(blobs) and len(proofs) == len(blobs)):
+        raise KzgError("GenericError", "length's of the input are not the same")
+    count = len(blobs)
+    keep, ptrs, lens = _blobs_to_abi(blobs)  # keep: the buffers ptrs points into
+    cxy, cinf = g1_to_abi(commitments)
+    pxy, pinf = g1_to_abi(proofs)
+    xy = C.create_string_buffer(64 * count if count else 1)
+    inf = C.create_string_buffer(count if count else 1)
+    z = C.create_string_buffer(32 * count if count else 1)
+    y = C.create_string_buffer(32 * count if count else 1)
+    call(ptrs, lens, count, cxy, cinf, pxy, pinf, xy, inf, z, y)
+    outs = g1_from_abi(xy.raw[: 64 * count], inf.raw[:count])
+    return list(zip(outs, fr_from_mont_bytes(z.raw[: 32 * count]), fr_from_mont_bytes(y.raw[: 32 * count])))
+
+
 def _next_pow2(n: int) -> int:
     return 1 if n <= 1 else 1 << (n - 1).bit_length()
 
@@ -232,6 +250,14 @@ class Group:
         """KZG::compute_blob_proof for every (blob, commitment) pair (prover/src/kzg.rs:288-309), the batch cut by blob
         across the members."""
         return _compute_blob_proofs(lambda *a: self.check(lib.kzgb_group_compute_blob_proofs(self.h, *a)), blobs, commitments)
+
+    def verify_blob_kzg_proofs_g1(
+        self, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]
+    ) -> List[Tuple[Affine, int, int]]:
+        """verify_blob_kzg_proofs_g1 with the batch cut by blob across the members."""
+        return _verify_blob_proofs(
+            lambda *a: self.check(lib.kzgb_group_verify_blob_proofs_g1(self.h, *a)), blobs, commitments, proofs
+        )
 
     def commit_coeff_form(self, polynomial: "PolynomialCoeffForm") -> Affine:
         """KZG::commit_coeff_form with the points cut into one range per GPU (prover/src/kzg.rs:107-125)."""
@@ -700,6 +726,16 @@ def verify_blob_kzg_proof_g1(blob: "Blob", commitment: Affine, proof: Affine, en
     z, y = C.create_string_buffer(32), C.create_string_buffer(32)
     e.check(lib.kzgb_verify_blob_proof_g1(e.h, blob.blob_data, len(blob.blob_data), cxy, cinf[0], pxy, pinf[0], out, C.byref(inf), z, y))
     return g1_from_abi(out.raw, bytes([inf.value]))[0], fr_from_mont_bytes(z.raw)[0], fr_from_mont_bytes(y.raw)[0]
+
+
+def verify_blob_kzg_proofs_g1(
+    blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine], engine: Optional[Engine] = None
+) -> List[Tuple[Affine, int, int]]:
+    """verifier/src/verify.rs:77-115 up to the pairing for every (blob, commitment, proof) triple in one call: entry i is
+    what ``verify_blob_kzg_proof_g1`` returns for triple i alone, ``(commitment - [y] G1, z, y)``; the pairing of each
+    (``pairings_verify(out, G2, proof, [tau - z] G2)``) stays in the reference's code and gives one bool per blob."""
+    e = engine or default_engine()
+    return _verify_blob_proofs(lambda *a: e.check(lib.kzgb_verify_blob_proofs_g1(e.h, *a)), blobs, commitments, proofs)
 
 
 def verify_blob_kzg_proof_batch_rlc(

@@ -99,6 +99,15 @@ SIGNATURES = {
     "kzgb_msm_config": (C.c_int, [ctx_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_size_t)]),
     "kzgb_verify_proof_g1": (C.c_int, [ctx_p, buf, C.c_uint8, buf, C.c_uint8, buf, buf, u8p]),
     "kzgb_verify_blob_proof_g1": (C.c_int, [ctx_p, buf, C.c_size_t, buf, C.c_uint8, buf, C.c_uint8, buf, u8p, buf, buf]),
+    "kzgb_verify_blob_proofs_g1": (
+        C.c_int,
+        [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf, buf, buf, buf, buf, buf],
+    ),
+    "kzgb_verify_blob_proofs_g1_dev": (
+        C.c_int,
+        [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf, buf, buf,
+         buf, buf, buf],
+    ),
     "kzgb_trace_begin": (C.c_int, [ctx_p]),
     "kzgb_trace_end": (C.c_int, [ctx_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "kzgb_srs_precompute_range": (C.c_int, [ctx_p, C.c_size_t, C.c_size_t, C.c_int]),
@@ -120,6 +129,9 @@ SIGNATURES = {
     "kzgb_group_commit_and_prove_blobs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf]),
     "kzgb_group_commit_blobs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf]),
     "kzgb_group_compute_blob_proofs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf]),
+    "kzgb_group_verify_blob_proofs_g1": (
+        C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf, buf, buf, buf, buf]
+    ),
     "kzgb_group_msm_srs": (C.c_int, [grp_p, buf, C.c_size_t, buf, C.POINTER(C.c_uint8)]),
 }
 

@@ -1,7 +1,7 @@
 // The blob-batch pipelines: kzgb_commit_and_prove_blobs{,_dev} -- commitment and proof of many blobs on several lanes
 // while a hashing stage produces the Fiat-Shamir transcripts --, kzgb_commit_blobs{,_dev} -- the commitments alone, on
 // the same plan and lanes --, kzgb_compute_blob_proofs{,_dev} -- the proofs alone, against the caller's commitments --
-// and kzgb_verify_batch_rlc.
+// and the verifier's calls, kzgb_verify_blob_proofs_g1{,_dev} and kzgb_verify_batch_rlc, over one per-blob stage.
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
@@ -774,6 +774,157 @@ int compute_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint
     return rc;
 }
 
+// ---------------------------------------------------------------- verification
+// The per-blob front half of every verification (helpers.rs:613-662) on lane L: zs[i] = compute_challenge(blob i, Cs[i])
+// and ys[i] = p_i(zs[i]) for m blobs of ns[i] = blob_poly_len(lens[i]) > 0 elements.  The blobs are evaluated in rounds
+// of equal-size runs; after_round(i0, b, d_y) runs at the end of each round, with y_{i0} .. y_{i0+b-1} resident at d_y,
+// to enqueue more work on L.st before the round's synchronise.  blobs_dev (may be null): the blob bytes on the device,
+// read in place; the transcripts are hashed from blobs_host either way.
+template <class F>
+int blob_evals_stage(kzgb_ctx* c, Lane& L, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
+                     const size_t* lens, const std::vector<size_t>& ns, const std::vector<Affine>& Cs, std::vector<Fr>& zs,
+                     std::vector<Fr>& ys, F after_round) {
+    const size_t m = ns.size();
+    const size_t max_n = *std::max_element(ns.begin(), ns.end());
+    int rc = ensure_twiddles(c, log2_exact(max_n));
+    if (rc) return rc;
+    // Thousands of small transcripts: hash them on the GPU, one thread per blob, from the evaluations that
+    // are resident anyway (fs.cu).  Otherwise a host SHA-256 pool (one transcript per blob) runs while the
+    // blobs are uploaded and converted.
+    const int fs_opt = g_fs_device.load();
+    const bool fs_device = fs_opt >= 0 ? fs_opt != 0 : (m >= 256 && max_n <= ((size_t)1 << 13));
+    std::atomic<size_t> next{fs_device ? m : 0};
+    std::vector<std::thread> hashers;
+    {
+        size_t nt = fs_device ? 0 : std::max<size_t>(1, std::min<size_t>(m, hash_pool_threads() + 1));
+        for (size_t t = 0; t < nt; t++)
+            hashers.emplace_back([&]() {
+                for (;;) {
+                    size_t i = next.fetch_add(1);
+                    if (i >= m) return;
+                    Sha256 sh;
+                    challenge_midstate(sh, blobs_host[i], lens[i], ns[i]);
+                    zs[i] = challenge_finish(sh, Cs[i]);
+                }
+            });
+    }
+    struct Joiner {
+        std::vector<std::thread>& t;
+        std::atomic<size_t>& next;
+        size_t m;
+        bool joined = false;
+        void join() { if (!joined) { for (auto& x : t) x.join(); joined = true; } }
+        ~Joiner() { next.store(m); join(); }  // error paths: stop handing out work, then wait
+    } joiner{hashers, next, m};
+    const size_t budget_elems = (size_t)1 << 24;  // evaluations resident per GPU batch
+    size_t i0 = 0;
+    while (i0 < m) {
+        size_t n = ns[i0], i1 = i0;
+        while (i1 < m && ns[i1] == n && (i1 - i0 + 1) * n <= std::max(budget_elems, n) && i1 - i0 < 65535) i1++;  // b is a gridDim.y
+        size_t b = i1 - i0;
+        int logn = log2_exact(n);
+        CK(c, L.evals.reserve(b * n * sizeof(Fr)));
+        if (!blobs_dev) CK(c, L.bytes.reserve(b * n * 32));
+        CK(c, L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)b) * sizeof(Fr)));
+        CK(c, L.work.reserve(5 * b * sizeof(Fr)));
+        bool full = (uint64_t)b * n < 0xffffffffull;  // every blob fills its polynomial: one conversion launch
+        for (size_t k = 0; k < b && full; k++) full = lens[i0 + k] == n * 32;
+        const uint8_t* const* src = blobs_dev ? blobs_dev : blobs_host;
+        for (size_t k = 0; k < b;) {
+            size_t run = 1;  // blobs that are adjacent in memory go up in one copy, or are converted in one launch
+            while (full && k + run < b && src[i0 + k + run] == src[i0 + k] + run * n * 32) run++;
+            size_t bytes = full ? run * n * 32 : lens[i0 + k];
+            Fr* evals = (Fr*)L.evals.p + k * n;
+            if (blobs_dev) {
+                bytes_to_fr_launch(src[i0 + k], bytes, evals, (uint32_t)(full ? run * n : n), L.st);
+            } else {
+                uint8_t* dst = (uint8_t*)L.bytes.p + k * n * 32;
+                CK(c, cudaMemcpyAsync(dst, src[i0 + k], bytes, cudaMemcpyHostToDevice, L.st));
+                if (!full) bytes_to_fr_launch(dst, lens[i0 + k], evals, (uint32_t)n, L.st);
+            }
+            k += run;
+        }
+        if (full && !blobs_dev) bytes_to_fr_launch((const uint8_t*)L.bytes.p, (uint64_t)b * n * 32, (Fr*)L.evals.p, (uint32_t)(b * n), L.st);
+        joiner.join();  // the challenges z_i are needed from here on
+        Fr* d_z = (Fr*)L.work.p;
+        Fr* d_t = d_z + b;
+        Fr* d_y = d_t + b;
+        Fr ninv = ninv_mont(logn);
+        std::vector<Fr> tinvs;
+        std::vector<uint8_t> cbytes;
+        bool any_in_domain = false;
+        uint32_t* d_in_domain = nullptr;  // challenges hashed on the device: the device says which z are roots of the domain
+        if (fs_device) {
+            uint8_t* d_c32 = (uint8_t*)(d_y + b);
+            cbytes.resize(b * 32);
+            for (size_t k = 0; k < b; k++) serialize_compressed(Cs[i0 + k], &cbytes[32 * k]);
+            CK(c, cudaMemcpyAsync(d_c32, cbytes.data(), b * 32, cudaMemcpyHostToDevice, L.st));
+            d_in_domain = (uint32_t*)(d_c32 + 32 * b);
+            fs_challenges_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_c32, &ninv, d_z, d_t, L.st, d_in_domain);
+            CK(c, cudaMemcpyAsync(&zs[i0], d_z, b * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
+        } else {
+            tinvs.resize(b);
+            for (size_t k = 0; k < b; k++) tinvs[k] = eval_tinv(zs[i0 + k], logn, &any_in_domain);
+            CK(c, cudaMemcpyAsync(d_z, &zs[i0], b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+            CK(c, cudaMemcpyAsync(d_t, tinvs.data(), b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+        }
+        eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_z, d_t, c->tw, c->logN, &ninv,
+                             (Fr*)L.eval_scratch.p, nullptr, d_y, L.st, !fs_device && !any_in_domain, d_in_domain);
+        CK(c, cudaMemcpyAsync(&ys[i0], d_y, b * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
+        rc = after_round(i0, b, (const Fr*)d_y);
+        if (rc) return rc;
+        CK(c, cudaStreamSynchronize(L.st));
+        CK(c, cudaGetLastError());
+        i0 = i1;
+    }
+    return KZGB_OK;
+}
+
+// verify_blob_kzg_proof (verify.rs:77-115) up to the pairing for `count` blobs on lane 0: every blob checked as
+// kzgb_verify_blob_proof_g1 checks it, in index order, then the stage and one k_commit_minus_value launch per round.
+int verify_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
+                       size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
+                       const uint8_t* proofs_inf, uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out) {
+    if (count == 0) return KZGB_OK;
+    std::vector<Affine> Cs(count);
+    std::vector<size_t> ns(count);
+    for (size_t i = 0; i < count; i++) {
+        Cs[i] = affine_from_abi(commitments_xy + 8 * i, commitments_inf ? commitments_inf[i] : 0);
+        const Affine P = affine_from_abi(proofs_xy + 8 * i, proofs_inf ? proofs_inf[i] : 0);
+        if (!aff_on_curve(Cs[i]) || !aff_on_curve(P)) return fail(c, KZGB_ERR_NOT_ON_CURVE, "G1 point not on curve");
+        if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
+        ns[i] = blob_poly_len(lens[i]);
+        if (ns[i] > ((size_t)1 << 28)) return fail(c, KZGB_ERR_GENERIC, "Input size exceeds maximum polynomial size");
+    }
+    Lane& L = c->lanes[0];
+    if (!c->gen_table) {
+        Affine* t = nullptr;
+        CK(c, cudaMalloc(&t, GEN_TABLE_POINTS * sizeof(Affine)));
+        const cudaError_t e = cudaMemcpy(t, generator_window_table(), GEN_TABLE_POINTS * sizeof(Affine), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) cudaFree(t);
+        CK(c, e);
+        c->gen_table = t;
+    }
+    CK(c, L.bases.reserve(2 * count * sizeof(Affine)));
+    Affine* d_c = (Affine*)L.bases.p;  // [C_0 .. C_{count-1} | out_0 .. out_{count-1}]
+    Affine* d_out = d_c + count;
+    CK(c, cudaMemcpyAsync(d_c, Cs.data(), count * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
+    std::vector<Fr> zs(count), ys(count);
+    std::vector<Affine> outs(count);
+    int rc = blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys, [&](size_t i0, size_t b, const Fr* d_y) {
+        commit_minus_value_launch(d_c + i0, d_y, c->gen_table, d_out + i0, (uint32_t)b, L.st);
+        CK(c, cudaMemcpyAsync(&outs[i0], d_out + i0, b * sizeof(Affine), cudaMemcpyDeviceToHost, L.st));
+        return (int)KZGB_OK;
+    });
+    if (rc) return rc;
+    for (size_t i = 0; i < count; i++) {
+        affine_to_abi(outs[i], out_xy + 8 * i, out_inf ? out_inf + i : nullptr);
+        if (z_out) memcpy(z_out + 4 * i, zs[i].l, 32);
+        if (y_out) memcpy(y_out + 4 * i, ys[i].l, 32);
+    }
+    return KZGB_OK;
+}
+
 // The random linear combination of m validated and evaluated openings (batch.rs:76-249): d_bases holds C_0 .. C_{m-1},
 // pi_0 .. pi_{m-1} and room for one more point.
 int rlc_combine(kzgb_ctx* c, Lane& L, const std::vector<Affine>& Cs, const std::vector<Affine>& Ps,
@@ -856,6 +1007,22 @@ int kzgb_compute_blob_proofs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, c
     Guard g(c);
     return compute_blob_proofs(c, blobs_dev, blobs_host, lens, count, commitments_xy, commitments_inf, out_xy, out_inf);
 }
+// ------------------------------------------------------------------------------- per-blob verification, G1 side
+int kzgb_verify_blob_proofs_g1(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                               const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
+                               const uint8_t* proofs_inf, uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out) {
+    Guard g(c);
+    return verify_blob_proofs(c, nullptr, blobs, lens, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, out_xy,
+                              out_inf, z_out, y_out);
+}
+int kzgb_verify_blob_proofs_g1_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
+                                   const size_t* lens, size_t count, const uint64_t* commitments_xy,
+                                   const uint8_t* commitments_inf, const uint64_t* proofs_xy, const uint8_t* proofs_inf,
+                                   uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out) {
+    Guard g(c);
+    return verify_blob_proofs(c, blobs_dev, blobs_host, lens, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf,
+                              out_xy, out_inf, z_out, y_out);
+}
 // ------------------------------------------------------------------------------- batch verification (RLC)
 int kzgb_verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,
                           const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
@@ -877,98 +1044,14 @@ int kzgb_verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs, const size_t
     CK(c, cudaMemcpyAsync(d_bases + m, Ps.data(), m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
     if (int rc = validate_points_dev(c, L, d_bases, 2 * m)) return rc;
 
-    // per-blob challenge (host SHA pool) and evaluation (GPU, batched over blobs of equal length)
     std::vector<size_t> ns(m);
-    size_t max_n = 0;
     for (size_t i = 0; i < m; i++) {
         if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
         ns[i] = blob_poly_len(lens[i]);
-        max_n = std::max(max_n, ns[i]);
     }
-    int rc = ensure_twiddles(c, log2_exact(max_n));
+    std::vector<Fr> zs(m), ys(m);  // per-blob challenges and evaluations: the stage the per-blob verification shares
+    int rc = blob_evals_stage(c, L, nullptr, blobs, lens, ns, Cs, zs, ys, [](size_t, size_t, const Fr*) { return (int)KZGB_OK; });
     if (rc) return rc;
-    std::vector<Fr> zs(m), ys(m);
-    // Thousands of small transcripts: hash them on the GPU, one thread per blob, from the evaluations that
-    // are resident anyway (fs.cu).  Otherwise a host SHA-256 pool (one transcript per blob) runs while the
-    // blobs are uploaded and converted.
-    const int fs_opt = g_fs_device.load();
-    const bool fs_device = fs_opt >= 0 ? fs_opt != 0 : (m >= 256 && max_n <= ((size_t)1 << 13));
-    std::atomic<size_t> next{fs_device ? m : 0};
-    std::vector<std::thread> hashers;
-    {
-        size_t nt = fs_device ? 0 : std::max<size_t>(1, std::min<size_t>(m, hash_pool_threads() + 1));
-        for (size_t t = 0; t < nt; t++)
-            hashers.emplace_back([&]() {
-                for (;;) {
-                    size_t i = next.fetch_add(1);
-                    if (i >= m) return;
-                    Sha256 sh;
-                    challenge_midstate(sh, blobs[i], lens[i], ns[i]);
-                    zs[i] = challenge_finish(sh, Cs[i]);
-                }
-            });
-    }
-    struct Joiner {
-        std::vector<std::thread>& t;
-        std::atomic<size_t>& next;
-        size_t m;
-        bool joined = false;
-        void join() { if (!joined) { for (auto& x : t) x.join(); joined = true; } }
-        ~Joiner() { next.store(m); join(); }  // error paths: stop handing out work, then wait
-    } joiner{hashers, next, m};
-    const size_t budget_elems = (size_t)1 << 24;  // evaluations resident per GPU batch
-    size_t i0 = 0;
-    while (i0 < m) {
-        size_t n = ns[i0], i1 = i0;
-        while (i1 < m && ns[i1] == n && (i1 - i0 + 1) * n <= std::max(budget_elems, n) && i1 - i0 < 65535) i1++;  // b is a gridDim.y
-        size_t b = i1 - i0;
-        int logn = log2_exact(n);
-        CK(c, L.evals.reserve(b * n * sizeof(Fr)));
-        CK(c, L.bytes.reserve(b * n * 32));
-        CK(c, L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)b) * sizeof(Fr)));
-        CK(c, L.work.reserve(5 * b * sizeof(Fr)));
-        bool full = (uint64_t)b * n < 0xffffffffull;  // every blob fills its polynomial: one conversion launch
-        for (size_t k = 0; k < b && full; k++) full = lens[i0 + k] == n * 32;
-        for (size_t k = 0; k < b;) {
-            uint8_t* dst = (uint8_t*)L.bytes.p + k * n * 32;
-            size_t run = 1;  // blobs that are adjacent in host memory go up in one copy
-            while (full && k + run < b && blobs[i0 + k + run] == blobs[i0 + k] + run * n * 32) run++;
-            size_t bytes = full ? run * n * 32 : lens[i0 + k];
-            CK(c, cudaMemcpyAsync(dst, blobs[i0 + k], bytes, cudaMemcpyHostToDevice, L.st));
-            if (!full) bytes_to_fr_launch(dst, lens[i0 + k], (Fr*)L.evals.p + k * n, (uint32_t)n, L.st);
-            k += run;
-        }
-        if (full) bytes_to_fr_launch((const uint8_t*)L.bytes.p, (uint64_t)b * n * 32, (Fr*)L.evals.p, (uint32_t)(b * n), L.st);
-        joiner.join();  // the challenges z_i are needed from here on
-        Fr* d_z = (Fr*)L.work.p;
-        Fr* d_t = d_z + b;
-        Fr* d_y = d_t + b;
-        Fr ninv = ninv_mont(logn);
-        std::vector<Fr> tinvs;
-        std::vector<uint8_t> cbytes;
-        bool any_in_domain = false;
-        uint32_t* d_in_domain = nullptr;  // challenges hashed on the device: the device says which z are roots of the domain
-        if (fs_device) {
-            uint8_t* d_c32 = (uint8_t*)(d_y + b);
-            cbytes.resize(b * 32);
-            for (size_t k = 0; k < b; k++) serialize_compressed(Cs[i0 + k], &cbytes[32 * k]);
-            CK(c, cudaMemcpyAsync(d_c32, cbytes.data(), b * 32, cudaMemcpyHostToDevice, L.st));
-            d_in_domain = (uint32_t*)(d_c32 + 32 * b);
-            fs_challenges_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_c32, &ninv, d_z, d_t, L.st, d_in_domain);
-            CK(c, cudaMemcpyAsync(&zs[i0], d_z, b * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
-        } else {
-            tinvs.resize(b);
-            for (size_t k = 0; k < b; k++) tinvs[k] = eval_tinv(zs[i0 + k], logn, &any_in_domain);
-            CK(c, cudaMemcpyAsync(d_z, &zs[i0], b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-            CK(c, cudaMemcpyAsync(d_t, tinvs.data(), b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-        }
-        eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_z, d_t, c->tw, c->logN, &ninv,
-                             (Fr*)L.eval_scratch.p, nullptr, d_y, L.st, !fs_device && !any_in_domain, d_in_domain);
-        CK(c, cudaMemcpyAsync(&ys[i0], d_y, b * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
-        CK(c, cudaStreamSynchronize(L.st));
-        CK(c, cudaGetLastError());
-        i0 = i1;
-    }
     Affine lhs, rhs;
     rc = rlc_combine(c, L, Cs, Ps, ns, zs, ys, d_bases, &lhs, &rhs);
     if (rc) return rc;

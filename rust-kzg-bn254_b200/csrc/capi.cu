@@ -821,6 +821,7 @@ void kzgb_ctx_destroy(kzgb_ctx* c) {
     allroots_release(c);
     if (c->tw) cudaFree(c->tw);
     c->batch_bytes.release();
+    if (c->gen_table) cudaFree(c->gen_table);
     if (c->t0) cudaEventDestroy(c->t0);
     if (c->t1) cudaEventDestroy(c->t1);
     if (c->copy_st) cudaStreamDestroy(c->copy_st);

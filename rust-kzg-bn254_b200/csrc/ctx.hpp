@@ -73,6 +73,7 @@ struct kzgb_ctx {
     // the first call of that size (or kzgb_srs_prepare_all_roots) and dropped with the SRS
     kzgb::Affine* allroots[kzgb::ALLROOTS_MAX_LOG + 1] = {};
     kzgb::DevBuf batch_bytes;  // blob bytes of the batch in flight (commit_and_prove_blobs)
+    kzgb::Affine* gen_table = nullptr;  // generator_window_table() on this device, uploaded by the first per-blob verification
     // twiddles
     kzgb::Fr* tw = nullptr;
     int logN = 0;

@@ -223,6 +223,25 @@ int kzgb_group_compute_blob_proofs(kzgb_group* g, const uint8_t* const* blobs, c
     });
 }
 
+// verify_blob_kzg_proof (verifier/src/verify.rs:77-115) up to the pairing for `count` blobs, cut as
+// kzgb_group_commit_and_prove_blobs cuts them.
+int kzgb_group_verify_blob_proofs_g1(kzgb_group* g, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                                     const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                                     const uint64_t* proofs_xy, const uint8_t* proofs_inf, uint64_t* out_xy,
+                                     uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    if (count == 0) return KZGB_OK;
+    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
+    return for_members(g, [&](int i) {
+        const size_t a = cut[i], b = cut[i + 1];
+        if (a >= b) return (int)KZGB_OK;
+        return kzgb_verify_blob_proofs_g1(g->ctx[i], blobs + a, lens + a, b - a, commitments_xy + 8 * a,
+                                          commitments_inf ? commitments_inf + a : nullptr, proofs_xy + 8 * a,
+                                          proofs_inf ? proofs_inf + a : nullptr, out_xy + 8 * a, out_inf ? out_inf + a : nullptr,
+                                          z_out ? z_out + 4 * a : nullptr, y_out ? y_out + 4 * a : nullptr);
+    });
+}
+
 // ---- one large MSM over the SRS, sharded by point range -------------------------------------------------------
 // KZG::commit_coeff_form (prover/src/kzg.rs:107-125) for polynomials too large for one GPU's liking: member i
 // computes sum_{j in share i} s_j SRS_j (fixed-base over its range table when kzgb_group_srs_precompute_ranges was

@@ -192,6 +192,14 @@ void fs_midstate_long_launch(const uint8_t* const* blobs_dev, const uint32_t* ns
 // in_domain_out (optional, batch words): 1 where z_k turned out to be a root of the domain.
 void fs_challenges_launch(const Fr* evals, uint32_t n, int logn, uint32_t batch, const uint8_t* commit32_dev,
                           const Fr* ninv_mont_host, Fr* z_out, Fr* tinv_out, cudaStream_t st, uint32_t* in_domain_out = nullptr);
+// j 16^w G1 (affine) at [8 w + j - 1], w < 64, j = 1..8: the generator's signed 4-bit window multiples (verify.cu),
+// computed once per process on the host
+constexpr int GEN_TABLE_POINTS = 512;
+const Affine* generator_window_table();
+// out[i] = C[i] - [y_i] G1 (verify.cu; y Montgomery, one thread per opening, the identity as (0, 0)); gen_table: the
+// points of generator_window_table() on the device
+void commit_minus_value_launch(const Affine* C, const Fr* y_mont, const Affine* gen_table, Affine* out, uint32_t count,
+                               cudaStream_t st);
 // out[i] = base^(first + i) (Montgomery), i < n
 void fr_powers_launch(Fr* out, uint32_t n, const Fr* base_mont_host, cudaStream_t st, uint32_t first = 0);
 // out[i] = a[i] * b[i]

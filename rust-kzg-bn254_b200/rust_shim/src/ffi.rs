@@ -78,6 +78,10 @@ extern "C" {
     pub fn kzgb_group_compute_blob_proofs(group: *mut kzgb_group, blobs: *const *const u8, lens: *const usize, count: usize,
                                           commitments_xy: *const u64, commitments_inf: *const u8, out_xy: *mut u64,
                                           out_inf: *mut u8) -> c_int;
+    pub fn kzgb_group_verify_blob_proofs_g1(group: *mut kzgb_group, blobs: *const *const u8, lens: *const usize, count: usize,
+                                            commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,
+                                            proofs_inf: *const u8, out_xy: *mut u64, out_inf: *mut u8, z_out: *mut u64,
+                                            y_out: *mut u64) -> c_int;
     pub fn kzgb_group_msm_srs(group: *mut kzgb_group, scalars: *const u64, n: usize, out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_verify_batch_rlc(ctx: *mut kzgb_ctx, blobs: *const *const u8, lens: *const usize, count: usize,
                                  commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,

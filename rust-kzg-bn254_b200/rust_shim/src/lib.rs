@@ -535,6 +535,100 @@ pub mod backend {
     }
     static DEFAULT_CTX: Mutex<Option<Ctx>> = Mutex::new(None);
 
+    struct Grp(*mut ffi::kzgb_group);
+    unsafe impl Send for Grp {}
+    impl Drop for Grp {
+        fn drop(&mut self) {
+            unsafe { ffi::kzgb_group_destroy(self.0) }
+        }
+    }
+    /// Every visible GPU (created on first use) for the per-blob verification of a batch, which needs no SRS.
+    static DEFAULT_GROUP: Mutex<Option<Grp>> = Mutex::new(None);
+
+    fn with_default_group<T>(f: impl FnOnce(*mut ffi::kzgb_group) -> T) -> Result<T, KzgError> {
+        let mut guard = DEFAULT_GROUP.lock().unwrap();
+        if guard.is_none() {
+            *guard = Some(Grp(new_group()?));
+        }
+        Ok(f(guard.as_ref().unwrap().0))
+    }
+
+    /// `verify_proof`'s pairing (verifier/src/verify.rs:44-74) on the library's `commit_minus_value` = C - [y] G1:
+    /// e(C - [y] G1, G2) == e(proof, [tau - z] G2).
+    fn pairing_check(commit_minus_value: G1Affine, proof: G1Affine, z: Fr) -> bool {
+        use ark_bn254::G2Affine;
+        use ark_ec::CurveGroup;
+        use rust_kzg_bn254_primitives::consts::G2_TAU;
+        let x_minus_z = (G2_TAU.into_group() - G2Affine::generator() * z).into_affine();
+        helpers::pairings_verify(commit_minus_value, G2Affine::generator(), proof, x_minus_z)
+    }
+
+    fn fr_from_words(w: &[u64]) -> Fr {
+        Fr::new_unchecked(ark_ff::BigInt([w[0], w[1], w[2], w[3]])) // Montgomery limbs, as fr_words passes them
+    }
+
+    /// `verifier::verify::verify_blob_kzg_proof` (verifier/src/verify.rs:77-115): validation, challenge, evaluation and
+    /// C - [y] G1 are one `kzgb_verify_blob_proof_g1` call; the pairing stays the reference's code.
+    pub fn verify_blob_kzg_proof(blob: &Blob, commitment: &G1Affine, proof: &G1Affine) -> Result<bool, KzgError> {
+        let (cxy, cinf) = pack_points(std::slice::from_ref(commitment));
+        let (pxy, pinf) = pack_points(std::slice::from_ref(proof));
+        let (mut out, mut out_inf, mut z) = ([0u64; 8], 0u8, [0u64; 4]);
+        let data = blob.data();
+        let commit_minus_value = with_default_ctx(|ctx| {
+            let rc = unsafe {
+                ffi::kzgb_verify_blob_proof_g1(ctx, data.as_ptr(), data.len(), cxy.as_ptr(), cinf[0], pxy.as_ptr(), pinf[0],
+                                               out.as_mut_ptr(), &mut out_inf, z.as_mut_ptr(), std::ptr::null_mut())
+            };
+            if rc != 0 { Err(to_err(ctx, rc, 0, 0)) } else { Ok(unpack_point(&out, out_inf)) }
+        })??;
+        Ok(pairing_check(commit_minus_value, *proof, fr_from_words(&z)))
+    }
+
+    /// Addition next to the reference's API: `verify_blob_kzg_proof` for every (blob, commitment, proof) triple in ONE
+    /// call, one bool per blob -- what a verifier needs when `verify_blob_kzg_proof_batch` fails and it must find the bad
+    /// blobs.  The G1 side of the batch is cut by bytes across the GPUs of the box (`kzgb_group_verify_blob_proofs_g1`);
+    /// each blob then gets the pairing of verify.rs:44-74.  An error is the one `verify_blob_kzg_proof` reports for the
+    /// first triple the library rejects.
+    pub fn verify_blob_kzg_proofs(blobs: &[Blob], commitments: &[G1Affine], proofs: &[G1Affine]) -> Result<Vec<bool>, KzgError> {
+        if !(commitments.len() == blobs.len() && proofs.len() == blobs.len()) {
+            return Err(KzgError::GenericError("length's of the input are not the same".to_string()));
+        }
+        let m = blobs.len();
+        let ptrs: Vec<*const u8> = blobs.iter().map(|b| b.data().as_ptr()).collect();
+        let lens: Vec<usize> = blobs.iter().map(|b| b.data().len()).collect();
+        let (cxy, cinf) = pack_points(commitments);
+        let (pxy, pinf) = pack_points(proofs);
+        let mut out = vec![0u64; 8 * m];
+        let mut out_inf = vec![0u8; m];
+        let mut z = vec![0u64; 4 * m];
+        with_default_group(|group| {
+            let rc = unsafe {
+                ffi::kzgb_group_verify_blob_proofs_g1(group, ptrs.as_ptr(), lens.as_ptr(), m, cxy.as_ptr(), cinf.as_ptr(),
+                                                      pxy.as_ptr(), pinf.as_ptr(), out.as_mut_ptr(), out_inf.as_mut_ptr(),
+                                                      z.as_mut_ptr(), std::ptr::null_mut())
+            };
+            if rc == 0 {
+                return Ok(());
+            }
+            // the group's message names the member: the error is rebuilt from the first failing triple as the
+            // single-blob call reports it
+            for (len, (c, p)) in lens.iter().zip(commitments.iter().zip(proofs)) {
+                helpers::validate_g1_point(c)?;
+                helpers::validate_g1_point(p)?;
+                if *len == 0 {
+                    return Err(KzgError::GenericError("Length of data after padding is 0".to_string()));
+                }
+                if len.div_ceil(32).next_power_of_two() > 1 << 28 {
+                    return Err(KzgError::GenericError("Input size exceeds maximum polynomial size".to_string()));
+                }
+            }
+            Err(group_err(group, rc))
+        })??;
+        Ok((0..m)
+            .map(|i| pairing_check(unpack_point(out[8 * i..8 * i + 8].try_into().unwrap(), out_inf[i]), proofs[i], fr_from_words(&z[4 * i..4 * i + 4])))
+            .collect())
+    }
+
     fn with_default_ctx<T>(f: impl FnOnce(*mut ffi::kzgb_ctx) -> T) -> Result<T, KzgError> {
         let mut guard = DEFAULT_CTX.lock().unwrap();
         if guard.is_none() {
