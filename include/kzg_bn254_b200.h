@@ -220,6 +220,24 @@ int kzgb_verify_batch_rlc(kzgb_ctx* ctx, const uint8_t* const* blobs, const size
                           const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
                           const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8],
                           uint8_t* rhs_inf);
+/* Same with the blob bytes in device memory, read in place.  Host copies are still needed for the SHA-256 transcripts
+ * (blobs_host), as for kzgb_verify_blob_proofs_g1_dev.  Checks, their order, errors and outputs are the host form's. */
+int kzgb_verify_batch_rlc_dev(kzgb_ctx* ctx, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
+                              const size_t* lens, size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                              const uint64_t* proofs_xy, const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf,
+                              uint64_t rhs_xy[8], uint8_t* rhs_inf);
+/* verify_kzg_proof_batch (batch.rs:185-249) up to the pairing: the random linear combination of kzgb_verify_batch_rlc
+ * over `count` openings the caller has already evaluated (z_i, y_i = p_i(z_i)), with no blob and no per-blob hashing.
+ * zs_mont / ys_mont: count x 4 words Montgomery each, as kzgb_verify_blob_proofs_g1 returns them.  poly_lens[i]: the
+ * padded polynomial length n_i that the transcript hashes (batch.rs:48-54), hashed as given -- for a blob of len bytes,
+ * next_pow2(ceil(len / 32)).  lhs / rhs: as kzgb_verify_batch_rlc defines them.  Checks, all before any work: the 2m
+ * points on the curve as kzgb_verify_batch_rlc checks them (KZGB_ERR_NOT_ON_CURVE), then every z_i and y_i below r
+ * (KZGB_ERR_INVALID_FIELD_ELEMENT: an arkworks Fr always is, and a larger word would hash other bytes than the
+ * reference's).  count == 0 writes the identity to both outputs.  commitments_inf / proofs_inf may be NULL. */
+int kzgb_verify_kzg_proof_batch_rlc(kzgb_ctx* ctx, size_t count, const uint64_t* commitments_xy,
+                                    const uint8_t* commitments_inf, const uint64_t* proofs_xy, const uint8_t* proofs_inf,
+                                    const uint64_t* zs_mont, const uint64_t* ys_mont, const uint64_t* poly_lens,
+                                    uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8], uint8_t* rhs_inf);
 
 /* ---- point codecs (host) ------------------------------------------------------------------ */
 /* arkworks CanonicalSerialize::serialize_compressed of a G1Affine (helpers.rs:458-460). */
@@ -299,7 +317,9 @@ int kzgb_verify_blob_proof_g1(kzgb_ctx* ctx, const uint8_t* blob, size_t len, co
  * polynomial length <= 2^28 (GenericError "Input size exceeds maximum polynomial size").  The error of the lowest-index
  * blob that fails is returned before any work starts, and the outputs are left untouched.  count == 0 writes nothing.
  * No SRS is needed.  commitments_inf / proofs_inf may be NULL (no identity among them).  The challenges are hashed as
- * kzgb_verify_batch_rlc hashes them (option "fs_device"); C_i - [y_i] G1 is one GPU thread per blob. */
+ * kzgb_verify_batch_rlc hashes them (option "fs_device"); C_i - [y_i] G1 is one GPU thread per blob.  out_xy may be NULL
+ * (then out_inf is ignored): only z and y are computed, which is what the RLC over the openings needs
+ * (kzgb_verify_kzg_proof_batch_rlc); checks and errors are the same. */
 int kzgb_verify_blob_proofs_g1(kzgb_ctx* ctx, const uint8_t* const* blobs, const size_t* lens, size_t count,
                                const uint64_t* commitments_xy, const uint8_t* commitments_inf,
                                const uint64_t* proofs_xy, const uint8_t* proofs_inf,
@@ -357,6 +377,16 @@ int kzgb_group_verify_blob_proofs_g1(kzgb_group* group, const uint8_t* const* bl
                                      const uint64_t* commitments_xy, const uint8_t* commitments_inf,
                                      const uint64_t* proofs_xy, const uint8_t* proofs_inf,
                                      uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out);
+/* kzgb_verify_batch_rlc on the group, with the same output words as the one-context call.  The 2m points are checked on
+ * member 0, then the lengths, with the one-context call's order, codes and messages, before any member starts.  Then
+ * each member computes z_i and y_i for its share of the blobs (cut as kzgb_group_verify_blob_proofs_g1 cuts them), and
+ * member 0 combines all m openings (kzgb_verify_kzg_proof_batch_rlc with n_i = next_pow2(ceil(len_i / 32))).  An error
+ * raised inside a member (a device failure) is reported as "member i (device d): <message>"; the outputs are written
+ * only on success. */
+int kzgb_group_verify_batch_rlc(kzgb_group* group, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                                const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
+                                const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8],
+                                uint8_t* rhs_inf);
 /* kzgb_msm_srs with the points cut into G contiguous ranges; the partial sums are added on the host. */
 int kzgb_group_msm_srs(kzgb_group* group, const uint64_t* scalars_mont, size_t n, uint64_t out_xy[8], uint8_t* out_inf);
 

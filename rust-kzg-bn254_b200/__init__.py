@@ -125,6 +125,23 @@ def _verify_blob_proofs(call, blobs: Sequence["Blob"], commitments: Sequence[Aff
     return list(zip(outs, fr_from_mont_bytes(z.raw[: 32 * count]), fr_from_mont_bytes(y.raw[: 32 * count])))
 
 
+def _batch_rlc(call, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]) -> Tuple[Affine, Affine]:
+    """Runs call(blob pointers, lengths, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, lhs_xy, lhs_inf,
+    rhs_xy, rhs_inf) of a kzgb_*verify_batch_rlc entry point; returns (lhs, rhs)."""
+    if not (len(commitments) == len(blobs) and len(proofs) == len(blobs)):
+        raise KzgError("GenericError", "length's of the input are not the same")
+    count = len(blobs)
+    keep, ptrs, lens = _blobs_to_abi(blobs)  # keep: the buffers ptrs points into
+    cxy, cinf = g1_to_abi(commitments)
+    pxy, pinf = g1_to_abi(proofs)
+    lhs = C.create_string_buffer(64)
+    rhs = C.create_string_buffer(64)
+    li = C.c_uint8(0)
+    ri = C.c_uint8(0)
+    call(ptrs, lens, count, cxy, cinf, pxy, pinf, lhs, C.byref(li), rhs, C.byref(ri))
+    return g1_from_abi(lhs.raw, bytes([li.value]))[0], g1_from_abi(rhs.raw, bytes([ri.value]))[0]
+
+
 def _next_pow2(n: int) -> int:
     return 1 if n <= 1 else 1 << (n - 1).bit_length()
 
@@ -258,6 +275,13 @@ class Group:
         return _verify_blob_proofs(
             lambda *a: self.check(lib.kzgb_group_verify_blob_proofs_g1(self.h, *a)), blobs, commitments, proofs
         )
+
+    def verify_blob_kzg_proof_batch_rlc(
+        self, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]
+    ) -> Tuple[Affine, Affine]:
+        """verify_blob_kzg_proof_batch_rlc with the per-blob challenges and evaluations cut by blob across the members and
+        the combination on member 0: the same (lhs, rhs) as the one-context call."""
+        return _batch_rlc(lambda *a: self.check(lib.kzgb_group_verify_batch_rlc(self.h, *a)), blobs, commitments, proofs)
 
     def commit_coeff_form(self, polynomial: "PolynomialCoeffForm") -> Affine:
         """KZG::commit_coeff_form with the points cut into one range per GPU (prover/src/kzg.rs:107-125)."""
@@ -744,16 +768,29 @@ def verify_blob_kzg_proof_batch_rlc(
     """verifier/src/batch.rs:16-249 up to (not including) the pairing: returns the two G1 inputs
     ``(proof_lincomb, rhs_g1)`` of ``pairings_verify`` (batch.rs:253-254), which stays in the
     reference's code."""
-    if not (len(commitments) == len(blobs) and len(proofs) == len(blobs)):
+    e = engine or default_engine()
+    return _batch_rlc(lambda *a: e.check(lib.kzgb_verify_batch_rlc(e.h, *a)), blobs, commitments, proofs)
+
+
+def verify_kzg_proof_batch_rlc(
+    commitments: Sequence[Affine], zs: Sequence[int], ys: Sequence[int], proofs: Sequence[Affine],
+    poly_lens: Sequence[int], engine: Optional[Engine] = None
+) -> Tuple[Affine, Affine]:
+    """verifier/src/batch.rs:185-249 up to the pairing over openings that are already evaluated (y_i = p_i(z_i), e.g. the
+    z and y of ``verify_blob_kzg_proofs_g1``): the ``(proof_lincomb, rhs_g1)`` of ``verify_blob_kzg_proof_batch_rlc``
+    without hashing any blob.  ``poly_lens[i]`` is the padded polynomial length the RLC transcript hashes.  Field elements
+    are taken modulo r, as the reference's ``Fr`` holds them."""
+    if not (len(commitments) == len(zs) == len(ys) == len(proofs) == len(poly_lens)):
         raise KzgError("GenericError", "length's of the input are not the same")
     e = engine or default_engine()
-    count = len(blobs)
-    keep, ptrs, lens = _blobs_to_abi(blobs)  # keep: the buffers ptrs points into
+    count = len(commitments)
     cxy, cinf = g1_to_abi(commitments)
     pxy, pinf = g1_to_abi(proofs)
+    ns = (C.c_uint64 * max(1, count))(*poly_lens)
     lhs = C.create_string_buffer(64)
     rhs = C.create_string_buffer(64)
     li = C.c_uint8(0)
     ri = C.c_uint8(0)
-    e.check(lib.kzgb_verify_batch_rlc(e.h, ptrs, lens, count, cxy, cinf, pxy, pinf, lhs, C.byref(li), rhs, C.byref(ri)))
+    e.check(lib.kzgb_verify_kzg_proof_batch_rlc(e.h, count, cxy, cinf, pxy, pinf, fr_to_mont_bytes(zs), fr_to_mont_bytes(ys),
+                                                ns, lhs, C.byref(li), rhs, C.byref(ri)))
     return g1_from_abi(lhs.raw, bytes([li.value]))[0], g1_from_abi(rhs.raw, bytes([ri.value]))[0]

@@ -85,6 +85,14 @@ SIGNATURES = {
         [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf,
          buf, buf, u8p, buf, u8p],
     ),
+    "kzgb_verify_batch_rlc_dev": (
+        C.c_int,
+        [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf, buf,
+         buf, u8p, buf, u8p],
+    ),
+    "kzgb_verify_kzg_proof_batch_rlc": (
+        C.c_int, [ctx_p, C.c_size_t, buf, buf, buf, buf, buf, buf, buf, buf, u8p, buf, u8p]
+    ),
     "kzgb_g1_serialize_compressed": (C.c_int, [buf, C.c_uint8, buf]),
     "kzgb_g1_to_gnark_be": (C.c_int, [buf, C.c_uint8, buf]),
     "kzgb_validate_g1_points": (C.c_int, [ctx_p, buf, buf, C.c_size_t]),
@@ -131,6 +139,9 @@ SIGNATURES = {
     "kzgb_group_compute_blob_proofs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf]),
     "kzgb_group_verify_blob_proofs_g1": (
         C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf, buf, buf, buf, buf]
+    ),
+    "kzgb_group_verify_batch_rlc": (
+        C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf, buf, u8p, buf, u8p]
     ),
     "kzgb_group_msm_srs": (C.c_int, [grp_p, buf, C.c_size_t, buf, C.POINTER(C.c_uint8)]),
 }

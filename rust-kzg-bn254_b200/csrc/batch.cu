@@ -1,7 +1,8 @@
 // The blob-batch pipelines: kzgb_commit_and_prove_blobs{,_dev} -- commitment and proof of many blobs on several lanes
 // while a hashing stage produces the Fiat-Shamir transcripts --, kzgb_commit_blobs{,_dev} -- the commitments alone, on
 // the same plan and lanes --, kzgb_compute_blob_proofs{,_dev} -- the proofs alone, against the caller's commitments --
-// and the verifier's calls, kzgb_verify_blob_proofs_g1{,_dev} and kzgb_verify_batch_rlc, over one per-blob stage.
+// and the verifier's calls, kzgb_verify_blob_proofs_g1{,_dev} and kzgb_verify_batch_rlc{,_dev}, over one per-blob stage,
+// and kzgb_verify_kzg_proof_batch_rlc, the random linear combination alone over openings the caller has evaluated.
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
@@ -882,6 +883,7 @@ int blob_evals_stage(kzgb_ctx* c, Lane& L, const uint8_t* const* blobs_dev, cons
 
 // verify_blob_kzg_proof (verify.rs:77-115) up to the pairing for `count` blobs on lane 0: every blob checked as
 // kzgb_verify_blob_proof_g1 checks it, in index order, then the stage and one k_commit_minus_value launch per round.
+// out_xy == null: z and y only (no generator table, no k_commit_minus_value).
 int verify_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
                        size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
                        const uint8_t* proofs_inf, uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out) {
@@ -897,28 +899,32 @@ int verify_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8
         if (ns[i] > ((size_t)1 << 28)) return fail(c, KZGB_ERR_GENERIC, "Input size exceeds maximum polynomial size");
     }
     Lane& L = c->lanes[0];
-    if (!c->gen_table) {
-        Affine* t = nullptr;
-        CK(c, cudaMalloc(&t, GEN_TABLE_POINTS * sizeof(Affine)));
-        const cudaError_t e = cudaMemcpy(t, generator_window_table(), GEN_TABLE_POINTS * sizeof(Affine), cudaMemcpyHostToDevice);
-        if (e != cudaSuccess) cudaFree(t);
-        CK(c, e);
-        c->gen_table = t;
+    Affine* d_c = nullptr;  // [C_0 .. C_{count-1} | out_0 .. out_{count-1}]
+    if (out_xy) {
+        if (!c->gen_table) {
+            Affine* t = nullptr;
+            CK(c, cudaMalloc(&t, GEN_TABLE_POINTS * sizeof(Affine)));
+            const cudaError_t e = cudaMemcpy(t, generator_window_table(), GEN_TABLE_POINTS * sizeof(Affine), cudaMemcpyHostToDevice);
+            if (e != cudaSuccess) cudaFree(t);
+            CK(c, e);
+            c->gen_table = t;
+        }
+        CK(c, L.bases.reserve(2 * count * sizeof(Affine)));
+        d_c = (Affine*)L.bases.p;
+        CK(c, cudaMemcpyAsync(d_c, Cs.data(), count * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
     }
-    CK(c, L.bases.reserve(2 * count * sizeof(Affine)));
-    Affine* d_c = (Affine*)L.bases.p;  // [C_0 .. C_{count-1} | out_0 .. out_{count-1}]
-    Affine* d_out = d_c + count;
-    CK(c, cudaMemcpyAsync(d_c, Cs.data(), count * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
+    Affine* d_out = d_c ? d_c + count : nullptr;
     std::vector<Fr> zs(count), ys(count);
-    std::vector<Affine> outs(count);
+    std::vector<Affine> outs(out_xy ? count : 0);
     int rc = blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys, [&](size_t i0, size_t b, const Fr* d_y) {
+        if (!out_xy) return (int)KZGB_OK;
         commit_minus_value_launch(d_c + i0, d_y, c->gen_table, d_out + i0, (uint32_t)b, L.st);
         CK(c, cudaMemcpyAsync(&outs[i0], d_out + i0, b * sizeof(Affine), cudaMemcpyDeviceToHost, L.st));
         return (int)KZGB_OK;
     });
     if (rc) return rc;
     for (size_t i = 0; i < count; i++) {
-        affine_to_abi(outs[i], out_xy + 8 * i, out_inf ? out_inf + i : nullptr);
+        if (out_xy) affine_to_abi(outs[i], out_xy + 8 * i, out_inf ? out_inf + i : nullptr);
         if (z_out) memcpy(z_out + 4 * i, zs[i].l, 32);
         if (y_out) memcpy(y_out + 4 * i, ys[i].l, 32);
     }
@@ -969,6 +975,100 @@ int rlc_combine(kzgb_ctx* c, Lane& L, const std::vector<Affine>& Cs, const std::
     int rc = msm_blocking(c, L, d_sc, 0, m, d_bases + m, lhs);
     if (rc) return rc;
     return msm_blocking(c, L, d_sc, 0, 2 * m + 1, d_bases, rhs);
+}
+
+// The m > 0 openings' points from the ABI into Cs / Ps and onto lane L's d_bases ([C_0..C_{m-1}, pi_0..pi_{m-1}, room for
+// G]), then validate_g1_point on all 2m of them (batch.rs:30-37) on the GPU.
+int upload_rlc_points(kzgb_ctx* c, Lane& L, size_t m, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                      const uint64_t* proofs_xy, const uint8_t* proofs_inf, std::vector<Affine>& Cs, std::vector<Affine>& Ps,
+                      Affine** d_bases) {
+    Cs.resize(m);
+    Ps.resize(m);
+    for (size_t i = 0; i < m; i++) {
+        Cs[i] = affine_from_abi(commitments_xy + 8 * i, commitments_inf ? commitments_inf[i] : 0);
+        Ps[i] = affine_from_abi(proofs_xy + 8 * i, proofs_inf ? proofs_inf[i] : 0);
+    }
+    CK(c, L.bases.reserve((2 * m + 1) * sizeof(Affine)));
+    *d_bases = (Affine*)L.bases.p;
+    CK(c, cudaMemcpyAsync(*d_bases, Cs.data(), m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
+    CK(c, cudaMemcpyAsync(*d_bases + m, Ps.data(), m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
+    return validate_points_dev(c, L, *d_bases, 2 * m);
+}
+
+// verify_blob_kzg_proof_batch (batch.rs:16-249) up to the pairing on lane 0: the 2m points, then the lengths, then the
+// per-blob stage (blobs_dev as blob_evals_stage reads it) and the combination.
+int verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
+                     size_t m, const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
+                     const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8], uint8_t* rhs_inf) {
+    Lane& L = c->lanes[0];
+    Affine lhs, rhs;
+    if (m == 0) {
+        aff_set_inf(lhs);
+        affine_to_abi(lhs, lhs_xy, lhs_inf);
+        affine_to_abi(lhs, rhs_xy, rhs_inf);
+        return KZGB_OK;
+    }
+    std::vector<Affine> Cs, Ps;
+    Affine* d_bases = nullptr;
+    if (int rc = upload_rlc_points(c, L, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, Cs, Ps, &d_bases)) return rc;
+    std::vector<size_t> ns(m);
+    for (size_t i = 0; i < m; i++) {
+        if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
+        ns[i] = blob_poly_len(lens[i]);
+    }
+    std::vector<Fr> zs(m), ys(m);  // per-blob challenges and evaluations: the stage the per-blob verification shares
+    int rc = blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys, [](size_t, size_t, const Fr*) { return (int)KZGB_OK; });
+    if (rc) return rc;
+    rc = rlc_combine(c, L, Cs, Ps, ns, zs, ys, d_bases, &lhs, &rhs);
+    if (rc) return rc;
+    affine_to_abi(lhs, lhs_xy, lhs_inf);
+    affine_to_abi(rhs, rhs_xy, rhs_inf);
+    return KZGB_OK;
+}
+
+// the 4 little-endian words at w hold a value below r
+bool fr_words_reduced(const uint64_t* w) {
+    uint32_t r[8];
+    FeConst<FR>::mod(r);
+    for (int k = 7; k >= 0; k--) {
+        const uint32_t x = (uint32_t)(w[k / 2] >> (32 * (k & 1)));
+        if (x != r[k]) return x < r[k];
+    }
+    return false;
+}
+
+// verify_kzg_proof_batch (batch.rs:185-249) on lane 0 over m openings that are already evaluated: the 2m points, then
+// every z_i and y_i a reduced Montgomery value (< r, as an arkworks Fr always is: a larger word would be hashed as other
+// bytes than the reference hashes), then the combination with the caller's n_i.
+int verify_openings_rlc(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                        const uint64_t* proofs_xy, const uint8_t* proofs_inf, const uint64_t* zs_mont, const uint64_t* ys_mont,
+                        const uint64_t* poly_lens, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8], uint8_t* rhs_inf) {
+    Lane& L = c->lanes[0];
+    Affine lhs, rhs;
+    if (m == 0) {
+        aff_set_inf(lhs);
+        affine_to_abi(lhs, lhs_xy, lhs_inf);
+        affine_to_abi(lhs, rhs_xy, rhs_inf);
+        return KZGB_OK;
+    }
+    std::vector<Affine> Cs, Ps;
+    Affine* d_bases = nullptr;
+    if (int rc = upload_rlc_points(c, L, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, Cs, Ps, &d_bases)) return rc;
+    std::vector<Fr> zs(m), ys(m);
+    std::vector<size_t> ns(m);
+    for (size_t i = 0; i < m; i++) {
+        if (!fr_words_reduced(zs_mont + 4 * i) || !fr_words_reduced(ys_mont + 4 * i))
+            return fail(c, KZGB_ERR_INVALID_FIELD_ELEMENT,
+                        "z or y of opening " + std::to_string(i) + " is not a reduced field element");
+        memcpy(zs[i].l, zs_mont + 4 * i, 32);
+        memcpy(ys[i].l, ys_mont + 4 * i, 32);
+        ns[i] = (size_t)poly_lens[i];
+    }
+    int rc = rlc_combine(c, L, Cs, Ps, ns, zs, ys, d_bases, &lhs, &rhs);
+    if (rc) return rc;
+    affine_to_abi(lhs, lhs_xy, lhs_inf);
+    affine_to_abi(rhs, rhs_xy, rhs_inf);
+    return KZGB_OK;
 }
 
 }  // namespace
@@ -1028,35 +1128,23 @@ int kzgb_verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs, const size_t
                           const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
                           const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8], uint8_t* rhs_inf) {
     Guard g(c);
-    Lane& L = c->lanes[0];
-    const size_t m = count;
-    Affine inf_pt; aff_set_inf(inf_pt);
-    if (m == 0) { affine_to_abi(inf_pt, lhs_xy, lhs_inf); affine_to_abi(inf_pt, rhs_xy, rhs_inf); return KZGB_OK; }
-    std::vector<Affine> Cs(m), Ps(m);
-    for (size_t i = 0; i < m; i++) {
-        Cs[i] = affine_from_abi(commitments_xy + 8 * i, commitments_inf ? commitments_inf[i] : 0);
-        Ps[i] = affine_from_abi(proofs_xy + 8 * i, proofs_inf ? proofs_inf[i] : 0);
-    }
-    // validate_g1_point on all 2m points (batch.rs:30-37) -- on the GPU
-    CK(c, L.bases.reserve((2 * m + 1) * sizeof(Affine)));
-    Affine* d_bases = (Affine*)L.bases.p;  // [C_0..C_{m-1}, pi_0..pi_{m-1}, G]
-    CK(c, cudaMemcpyAsync(d_bases, Cs.data(), m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
-    CK(c, cudaMemcpyAsync(d_bases + m, Ps.data(), m * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
-    if (int rc = validate_points_dev(c, L, d_bases, 2 * m)) return rc;
-
-    std::vector<size_t> ns(m);
-    for (size_t i = 0; i < m; i++) {
-        if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
-        ns[i] = blob_poly_len(lens[i]);
-    }
-    std::vector<Fr> zs(m), ys(m);  // per-blob challenges and evaluations: the stage the per-blob verification shares
-    int rc = blob_evals_stage(c, L, nullptr, blobs, lens, ns, Cs, zs, ys, [](size_t, size_t, const Fr*) { return (int)KZGB_OK; });
-    if (rc) return rc;
-    Affine lhs, rhs;
-    rc = rlc_combine(c, L, Cs, Ps, ns, zs, ys, d_bases, &lhs, &rhs);
-    if (rc) return rc;
-    affine_to_abi(lhs, lhs_xy, lhs_inf);
-    affine_to_abi(rhs, rhs_xy, rhs_inf);
-    return KZGB_OK;
+    return verify_batch_rlc(c, nullptr, blobs, lens, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, lhs_xy,
+                            lhs_inf, rhs_xy, rhs_inf);
+}
+int kzgb_verify_batch_rlc_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
+                              const size_t* lens, size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                              const uint64_t* proofs_xy, const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf,
+                              uint64_t rhs_xy[8], uint8_t* rhs_inf) {
+    Guard g(c);
+    return verify_batch_rlc(c, blobs_dev, blobs_host, lens, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf,
+                            lhs_xy, lhs_inf, rhs_xy, rhs_inf);
+}
+int kzgb_verify_kzg_proof_batch_rlc(kzgb_ctx* c, size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                                    const uint64_t* proofs_xy, const uint8_t* proofs_inf, const uint64_t* zs_mont,
+                                    const uint64_t* ys_mont, const uint64_t* poly_lens, uint64_t lhs_xy[8], uint8_t* lhs_inf,
+                                    uint64_t rhs_xy[8], uint8_t* rhs_inf) {
+    Guard g(c);
+    return verify_openings_rlc(c, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, zs_mont, ys_mont, poly_lens,
+                               lhs_xy, lhs_inf, rhs_xy, rhs_inf);
 }
 }  // extern "C"

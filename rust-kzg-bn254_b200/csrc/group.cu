@@ -242,6 +242,49 @@ int kzgb_group_verify_blob_proofs_g1(kzgb_group* g, const uint8_t* const* blobs,
     });
 }
 
+// verify_blob_kzg_proof_batch (verifier/src/batch.rs:16-249) up to the pairing.  The per-blob challenges and evaluations,
+// nearly all of the work, are cut by bytes across the members; the combination (two MSMs of m and 2m + 1 points) runs
+// on member 0 over all m openings, so the result is the one-context call's.
+int kzgb_group_verify_batch_rlc(kzgb_group* g, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                                const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
+                                const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8],
+                                uint8_t* rhs_inf) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    kzgb_ctx* c0 = g->ctx[0];
+    const size_t m = count;
+    std::vector<uint64_t> zs(4 * m), ys(4 * m), ns(m);
+    if (m) {
+        // the one-context call's checks, in its order: the 2m points (batch.rs:30-37), then the lengths
+        std::vector<uint64_t> xy(16 * m);
+        std::vector<uint8_t> inf(2 * m, 0);
+        memcpy(xy.data(), commitments_xy, 64 * m);
+        memcpy(xy.data() + 8 * m, proofs_xy, 64 * m);
+        if (commitments_inf) memcpy(inf.data(), commitments_inf, m);
+        if (proofs_inf) memcpy(inf.data() + m, proofs_inf, m);
+        int rc = kzgb_validate_g1_points(c0, xy.data(), inf.data(), 2 * m);
+        if (rc) return gfail(g, rc, kzgb_last_error(c0));
+        for (size_t i = 0; i < m; i++) {
+            if (lens[i] == 0) return gfail(g, KZGB_ERR_GENERIC, "Length of data after padding is 0");
+            size_t n = 1;
+            while (n < (lens[i] + 31) / 32) n <<= 1;
+            ns[i] = n;
+        }
+        const std::vector<size_t> cut = byte_balanced_cut(lens, m, (int)g->ctx.size());
+        rc = for_members(g, [&](int i) {
+            const size_t a = cut[i], b = cut[i + 1];
+            if (a >= b) return (int)KZGB_OK;
+            return kzgb_verify_blob_proofs_g1(g->ctx[i], blobs + a, lens + a, b - a, commitments_xy + 8 * a,
+                                              commitments_inf ? commitments_inf + a : nullptr, proofs_xy + 8 * a,
+                                              proofs_inf ? proofs_inf + a : nullptr, nullptr, nullptr, &zs[4 * a], &ys[4 * a]);
+        });
+        if (rc) return rc;
+    }
+    const int rc = kzgb_verify_kzg_proof_batch_rlc(c0, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, zs.data(),
+                                                   ys.data(), ns.data(), lhs_xy, lhs_inf, rhs_xy, rhs_inf);
+    if (rc) return gfail(g, rc, std::string("member 0 (device ") + std::to_string(g->dev[0]) + "): " + kzgb_last_error(c0));
+    return KZGB_OK;
+}
+
 // ---- one large MSM over the SRS, sharded by point range -------------------------------------------------------
 // KZG::commit_coeff_form (prover/src/kzg.rs:107-125) for polynomials too large for one GPU's liking: member i
 // computes sum_{j in share i} s_j SRS_j (fixed-base over its range table when kzgb_group_srs_precompute_ranges was

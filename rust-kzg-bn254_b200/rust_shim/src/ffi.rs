@@ -87,4 +87,16 @@ extern "C" {
                                  commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,
                                  proofs_inf: *const u8, lhs_xy: *mut u64, lhs_inf: *mut u8, rhs_xy: *mut u64,
                                  rhs_inf: *mut u8) -> c_int;
+    pub fn kzgb_verify_batch_rlc_dev(ctx: *mut kzgb_ctx, blobs_dev: *const *const u8, blobs_host: *const *const u8,
+                                     lens: *const usize, count: usize, commitments_xy: *const u64, commitments_inf: *const u8,
+                                     proofs_xy: *const u64, proofs_inf: *const u8, lhs_xy: *mut u64, lhs_inf: *mut u8,
+                                     rhs_xy: *mut u64, rhs_inf: *mut u8) -> c_int;
+    pub fn kzgb_verify_kzg_proof_batch_rlc(ctx: *mut kzgb_ctx, count: usize, commitments_xy: *const u64,
+                                           commitments_inf: *const u8, proofs_xy: *const u64, proofs_inf: *const u8,
+                                           zs_mont: *const u64, ys_mont: *const u64, poly_lens: *const u64,
+                                           lhs_xy: *mut u64, lhs_inf: *mut u8, rhs_xy: *mut u64, rhs_inf: *mut u8) -> c_int;
+    pub fn kzgb_group_verify_batch_rlc(group: *mut kzgb_group, blobs: *const *const u8, lens: *const usize, count: usize,
+                                       commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,
+                                       proofs_inf: *const u8, lhs_xy: *mut u64, lhs_inf: *mut u8, rhs_xy: *mut u64,
+                                       rhs_inf: *mut u8) -> c_int;
 }

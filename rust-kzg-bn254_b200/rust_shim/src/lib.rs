@@ -556,12 +556,13 @@ pub mod backend {
     /// `verify_proof`'s pairing (verifier/src/verify.rs:44-74) on the library's `commit_minus_value` = C - [y] G1:
     /// e(C - [y] G1, G2) == e(proof, [tau - z] G2).
     fn pairing_check(commit_minus_value: G1Affine, proof: G1Affine, z: Fr) -> bool {
-        use ark_bn254::G2Affine;
         use ark_ec::CurveGroup;
-        use rust_kzg_bn254_primitives::consts::G2_TAU;
         let x_minus_z = (G2_TAU.into_group() - G2Affine::generator() * z).into_affine();
         helpers::pairings_verify(commit_minus_value, G2Affine::generator(), proof, x_minus_z)
     }
+
+    use ark_bn254::G2Affine;
+    use rust_kzg_bn254_primitives::consts::G2_TAU;
 
     fn fr_from_words(w: &[u64]) -> Fr {
         Fr::new_unchecked(ark_ff::BigInt([w[0], w[1], w[2], w[3]])) // Montgomery limbs, as fr_words passes them
@@ -666,10 +667,9 @@ pub mod backend {
 
     /// `verifier::batch::verify_blob_kzg_proof_batch` (verifier/src/batch.rs:16-255): the input checks and the final
     /// pairing stay the reference's code; per-blob challenges and evaluations, the RLC scalar and the three linear
-    /// combinations (batch.rs:40-249) are one `kzgb_verify_batch_rlc` call.
+    /// combinations (batch.rs:40-249) are one `kzgb_group_verify_batch_rlc` call, whose per-blob half is cut by bytes
+    /// across the GPUs of the box.
     pub fn verify_blob_kzg_proof_batch(blobs: &[Blob], commitments: &[G1Affine], proofs: &[G1Affine]) -> Result<bool, KzgError> {
-        use ark_bn254::G2Affine;
-        use rust_kzg_bn254_primitives::consts::G2_TAU;
         if !(commitments.len() == blobs.len() && proofs.len() == blobs.len()) {
             return Err(KzgError::GenericError("length's of the input are not the same".to_string()));
         }
@@ -684,14 +684,53 @@ pub mod backend {
         let (cxy, cinf) = pack_points(commitments);
         let (pxy, pinf) = pack_points(proofs);
         let (mut lhs, mut lhs_inf, mut rhs, mut rhs_inf) = ([0u64; 8], 0u8, [0u64; 8], 0u8);
+        let (proof_lincomb, rhs_g1) = with_default_group(|group| {
+            let rc = unsafe {
+                ffi::kzgb_group_verify_batch_rlc(group, ptrs.as_ptr(), lens.as_ptr(), blobs.len(), cxy.as_ptr(), cinf.as_ptr(),
+                                                 pxy.as_ptr(), pinf.as_ptr(), lhs.as_mut_ptr(), &mut lhs_inf, rhs.as_mut_ptr(),
+                                                 &mut rhs_inf)
+            };
+            if rc == 0 {
+                return Ok((unpack_point(&lhs, lhs_inf), unpack_point(&rhs, rhs_inf)));
+            }
+            // the points were validated above; what is left is the one-context call's length check, reported as it
+            // reports it, or a device failure, whose group message names the member
+            if lens.contains(&0) {
+                return Err(KzgError::GenericError("Length of data after padding is 0".to_string()));
+            }
+            Err(group_err(group, rc))
+        })??;
+        // e(sum r^i proof_i, [tau]G2) == e(sum r^i (C_i - [y_i]) + sum r^i z_i proof_i, G2)   (batch.rs:253-254)
+        Ok(helpers::pairings_verify(proof_lincomb, G2_TAU, rhs_g1, G2Affine::generator()))
+    }
+
+    /// Addition next to the reference's API: `verifier::batch::verify_kzg_proof_batch` (verifier/src/batch.rs:185-255)
+    /// over openings the caller has already evaluated, for instance the z and y of `verify_blob_kzg_proofs`' G1 call.  No
+    /// blob is hashed.  `poly_lens[i]` is the padded polynomial length n_i the RLC transcript hashes (batch.rs:48-54).  The
+    /// random linear combination is one `kzgb_verify_kzg_proof_batch_rlc` call; the pairing stays the reference's code.
+    pub fn verify_kzg_proof_batch(commitments: &[G1Affine], zs: &[Fr], ys: &[Fr], proofs: &[G1Affine], poly_lens: &[u64])
+                                  -> Result<bool, KzgError> {
+        let m = commitments.len();
+        if !(zs.len() == m && ys.len() == m && proofs.len() == m && poly_lens.len() == m) {
+            return Err(KzgError::GenericError("length's of the input are not the same".to_string()));
+        }
+        for c in commitments.iter() {
+            helpers::validate_g1_point(c)?;
+        }
+        for p in proofs.iter() {
+            helpers::validate_g1_point(p)?;
+        }
+        let (cxy, cinf) = pack_points(commitments);
+        let (pxy, pinf) = pack_points(proofs);
+        let (mut lhs, mut lhs_inf, mut rhs, mut rhs_inf) = ([0u64; 8], 0u8, [0u64; 8], 0u8);
         let (proof_lincomb, rhs_g1) = with_default_ctx(|ctx| {
             let rc = unsafe {
-                ffi::kzgb_verify_batch_rlc(ctx, ptrs.as_ptr(), lens.as_ptr(), blobs.len(), cxy.as_ptr(), cinf.as_ptr(), pxy.as_ptr(),
-                                           pinf.as_ptr(), lhs.as_mut_ptr(), &mut lhs_inf, rhs.as_mut_ptr(), &mut rhs_inf)
+                ffi::kzgb_verify_kzg_proof_batch_rlc(ctx, m, cxy.as_ptr(), cinf.as_ptr(), pxy.as_ptr(), pinf.as_ptr(), fr_words(zs),
+                                                     fr_words(ys), poly_lens.as_ptr(), lhs.as_mut_ptr(), &mut lhs_inf,
+                                                     rhs.as_mut_ptr(), &mut rhs_inf)
             };
             if rc != 0 { Err(to_err(ctx, rc, 0, 0)) } else { Ok((unpack_point(&lhs, lhs_inf), unpack_point(&rhs, rhs_inf))) }
         })??;
-        // e(sum r^i proof_i, [tau]G2) == e(sum r^i (C_i - [y_i]) + sum r^i z_i proof_i, G2)   (batch.rs:253-254)
         Ok(helpers::pairings_verify(proof_lincomb, G2_TAU, rhs_g1, G2Affine::generator()))
     }
 }
