@@ -331,6 +331,42 @@ int kzgb_verify_blob_proofs_g1_dev(kzgb_ctx* ctx, const uint8_t* const* blobs_de
                                    const uint8_t* commitments_inf, const uint64_t* proofs_xy, const uint8_t* proofs_inf,
                                    uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out);
 
+/* ---- per-opening verification through the pairing (verifier/src/verify.rs:10-115) ---------------------------------
+ * Each opening (C, pi, z, y) is checked as e(C - [y]G1 + [z]pi, G2) * e(-pi, [tau]G2) == 1 -- by bilinearity the bool of
+ * the reference's e(C - [y]G1, G2) == e(pi, [tau - z]G2) -- on the GPU, one thread per opening: the lines of the Miller
+ * loop of both fixed G2 points are precomputed on the host once per context, the final exponentiation runs per opening.
+ * ok[i] is the bool verify_proof / verify_blob_kzg_proof returns for entry i alone, under this context's [tau]G2.
+ * If [z_i]G2 == [tau]G2 for some i (the reference's check of [tau - z]G2 = O, verify.rs:55-59), the call returns
+ * KZGB_ERR_GENERIC "Evaluation point equals trusted setup secret" for the lowest such i.  On any error `ok` is left
+ * untouched.  count == 0 writes nothing; commitments_inf / proofs_inf may be NULL (no identity among them).  No SRS is
+ * needed.  The single final pairing of verify_blob_kzg_proof_batch (kzgb_verify_batch_rlc) is not one of these: it
+ * stays in the reference's code. */
+/* [tau]G2 of this context's pairing checks: x.c0, x.c1, y.c0, y.c1 (4 words each, Montgomery; Fq2 = c0 + c1 u,
+ * u^2 = -1 -- the memory layout of arkworks' G2Affine without its flag).  NULL restores the default, the reference's
+ * G2_TAU (primitives/src/consts.rs:55-64).  Off the twist, the identity, or outside the order-r subgroup:
+ * KZGB_ERR_NOT_ON_CURVE "Invalid trusted setup: G2_TAU not on curve"; the setting is unchanged.  Loading an SRS does
+ * not change it. */
+int kzgb_set_g2_tau(kzgb_ctx* ctx, const uint64_t xy[16]);
+/* verify_proof (verify.rs:10-75) for `count` openings: ok[i] = 1 if the pairing check of (C_i, pi_i, z_i, y_i) holds,
+ * else 0.  zs_mont / ys_mont: count x 4 words Montgomery each.  Checks, all before any work: the 2m points on the curve
+ * as kzgb_verify_kzg_proof_batch_rlc checks them (KZGB_ERR_NOT_ON_CURVE), then every z_i and y_i below r
+ * (KZGB_ERR_INVALID_FIELD_ELEMENT). */
+int kzgb_verify_proofs(kzgb_ctx* ctx, size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                       const uint64_t* proofs_xy, const uint8_t* proofs_inf, const uint64_t* zs_mont,
+                       const uint64_t* ys_mont, uint8_t* ok);
+/* verify_blob_kzg_proof (verify.rs:77-115) for `count` blobs, through the pairing: z_i and y_i as
+ * kzgb_verify_blob_proofs_g1 computes them (hashing as option "fs_device" says), then the pairing check of each opening
+ * while z and y are still on the device.  Checks, their order, codes and messages: those of kzgb_verify_blob_proofs_g1
+ * (points on the curve, length not 0, polynomial length <= 2^28, the lowest failing index first). */
+int kzgb_verify_blob_proofs(kzgb_ctx* ctx, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                            const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                            const uint64_t* proofs_xy, const uint8_t* proofs_inf, uint8_t* ok);
+/* Same with the blob bytes in device memory, read in place; host copies feed the SHA-256 transcripts (blobs_host). */
+int kzgb_verify_blob_proofs_dev(kzgb_ctx* ctx, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
+                                const size_t* lens, size_t count, const uint64_t* commitments_xy,
+                                const uint8_t* commitments_inf, const uint64_t* proofs_xy, const uint8_t* proofs_inf,
+                                uint8_t* ok);
+
 /* ---- multi-GPU: one handle over several GPUs of one box (SURVEY.md 8e) ------------------------------------
  * The path shards by blob (batches) and by point range (one large MSM) and has no exchange step besides adding
  * G partial sums of 64 bytes, which happens on the host: one process, one host thread per GPU for the duration of
@@ -377,6 +413,14 @@ int kzgb_group_verify_blob_proofs_g1(kzgb_group* group, const uint8_t* const* bl
                                      const uint64_t* commitments_xy, const uint8_t* commitments_inf,
                                      const uint64_t* proofs_xy, const uint8_t* proofs_inf,
                                      uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out);
+/* kzgb_verify_blob_proofs cut as kzgb_group_verify_blob_proofs_g1 cuts the batch; identical to the one-context call.  Each
+ * member checks its own share before it starts (so on an error, members with valid shares may have written their
+ * entries of ok). */
+int kzgb_group_verify_blob_proofs(kzgb_group* group, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                                  const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                                  const uint64_t* proofs_xy, const uint8_t* proofs_inf, uint8_t* ok);
+/* kzgb_set_g2_tau on every member; on an error no member's setting changes. */
+int kzgb_group_set_g2_tau(kzgb_group* group, const uint64_t xy[16]);
 /* kzgb_verify_batch_rlc on the group, with the same output words as the one-context call.  The 2m points are checked on
  * member 0, then the lengths, with the one-context call's order, codes and messages, before any member starts.  Then
  * each member computes z_i and y_i for its share of the blobs (cut as kzgb_group_verify_blob_proofs_g1 cuts them), and

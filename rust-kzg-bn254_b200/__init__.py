@@ -125,6 +125,28 @@ def _verify_blob_proofs(call, blobs: Sequence["Blob"], commitments: Sequence[Aff
     return list(zip(outs, fr_from_mont_bytes(z.raw[: 32 * count]), fr_from_mont_bytes(y.raw[: 32 * count])))
 
 
+def _verify_blob_proofs_ok(call, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]) -> List[bool]:
+    """Runs call(blob pointers, lengths, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, ok) of a
+    kzgb_*verify_blob_proofs entry point; returns one bool per blob."""
+    if not (len(commitments) == len(blobs) and len(proofs) == len(blobs)):
+        raise KzgError("GenericError", "length's of the input are not the same")
+    count = len(blobs)
+    keep, ptrs, lens = _blobs_to_abi(blobs)  # keep: the buffers ptrs points into
+    cxy, cinf = g1_to_abi(commitments)
+    pxy, pinf = g1_to_abi(proofs)
+    ok = C.create_string_buffer(count if count else 1)
+    call(ptrs, lens, count, cxy, cinf, pxy, pinf, ok)
+    return [bool(b) for b in ok.raw[:count]]
+
+
+def g2_to_abi(q) -> Optional[bytes]:
+    """An oracle-style G2 point ``((x0, x1), (y0, y1))`` as the 16 Montgomery words of kzgb_set_g2_tau; None stays None."""
+    if q is None:
+        return None
+    (x0, x1), (y0, y1) = q
+    return b"".join((v % P * _MONT % P).to_bytes(32, "little") for v in (x0, x1, y0, y1))
+
+
 def _batch_rlc(call, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]) -> Tuple[Affine, Affine]:
     """Runs call(blob pointers, lengths, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, lhs_xy, lhs_inf,
     rhs_xy, rhs_inf) of a kzgb_*verify_batch_rlc entry point; returns (lhs, rhs)."""
@@ -185,6 +207,11 @@ class Engine:
 
     def launch_count(self) -> int:
         return int(lib.kzgb_launch_count(self.h))
+
+    def set_g2_tau(self, q) -> None:
+        """[tau]G2 of this context's pairing checks (``verify_proofs``, ``verify_blob_kzg_proofs``) as an oracle-style
+        ``((x0, x1), (y0, y1))``; None restores the reference's G2_TAU."""
+        self.check(lib.kzgb_set_g2_tau(self.h, g2_to_abi(q)))
 
 
 class Group:
@@ -275,6 +302,16 @@ class Group:
         return _verify_blob_proofs(
             lambda *a: self.check(lib.kzgb_group_verify_blob_proofs_g1(self.h, *a)), blobs, commitments, proofs
         )
+
+    def verify_blob_kzg_proofs(self, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]) -> List[bool]:
+        """verify_blob_kzg_proofs with the batch cut by blob across the members."""
+        return _verify_blob_proofs_ok(
+            lambda *a: self.check(lib.kzgb_group_verify_blob_proofs(self.h, *a)), blobs, commitments, proofs
+        )
+
+    def set_g2_tau(self, q) -> None:
+        """Engine.set_g2_tau on every member."""
+        self.check(lib.kzgb_group_set_g2_tau(self.h, g2_to_abi(q)))
 
     def verify_blob_kzg_proof_batch_rlc(
         self, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]
@@ -794,3 +831,30 @@ def verify_kzg_proof_batch_rlc(
     e.check(lib.kzgb_verify_kzg_proof_batch_rlc(e.h, count, cxy, cinf, pxy, pinf, fr_to_mont_bytes(zs), fr_to_mont_bytes(ys),
                                                 ns, lhs, C.byref(li), rhs, C.byref(ri)))
     return g1_from_abi(lhs.raw, bytes([li.value]))[0], g1_from_abi(rhs.raw, bytes([ri.value]))[0]
+
+
+def verify_proofs(
+    commitments: Sequence[Affine], proofs: Sequence[Affine], zs: Sequence[int], ys: Sequence[int],
+    engine: Optional[Engine] = None
+) -> List[bool]:
+    """verifier/src/verify.rs:10-75 for every opening (commitment, proof, z, y), the pairing included: entry i is the bool
+    ``verify_proof`` returns for opening i alone under the engine's [tau]G2 (``Engine.set_g2_tau``).  Field elements are
+    taken modulo r, as the reference's ``Fr`` holds them."""
+    if not (len(commitments) == len(proofs) == len(zs) == len(ys)):
+        raise KzgError("GenericError", "length's of the input are not the same")
+    e = engine or default_engine()
+    count = len(commitments)
+    cxy, cinf = g1_to_abi(commitments)
+    pxy, pinf = g1_to_abi(proofs)
+    ok = C.create_string_buffer(count if count else 1)
+    e.check(lib.kzgb_verify_proofs(e.h, count, cxy, cinf, pxy, pinf, fr_to_mont_bytes(zs), fr_to_mont_bytes(ys), ok))
+    return [bool(b) for b in ok.raw[:count]]
+
+
+def verify_blob_kzg_proofs(
+    blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine], engine: Optional[Engine] = None
+) -> List[bool]:
+    """verifier/src/verify.rs:77-115 for every (blob, commitment, proof) triple in one call, the pairing included: entry
+    i is the bool ``verify_blob_kzg_proof`` returns for triple i alone under the engine's [tau]G2."""
+    e = engine or default_engine()
+    return _verify_blob_proofs_ok(lambda *a: e.check(lib.kzgb_verify_blob_proofs(e.h, *a)), blobs, commitments, proofs)

@@ -116,6 +116,13 @@ SIGNATURES = {
         [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf, buf, buf,
          buf, buf, buf],
     ),
+    "kzgb_set_g2_tau": (C.c_int, [ctx_p, buf]),
+    "kzgb_verify_proofs": (C.c_int, [ctx_p, C.c_size_t, buf, buf, buf, buf, buf, buf, buf]),
+    "kzgb_verify_blob_proofs": (C.c_int, [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf, buf, buf]),
+    "kzgb_verify_blob_proofs_dev": (
+        C.c_int,
+        [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf, buf, buf],
+    ),
     "kzgb_trace_begin": (C.c_int, [ctx_p]),
     "kzgb_trace_end": (C.c_int, [ctx_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "kzgb_srs_precompute_range": (C.c_int, [ctx_p, C.c_size_t, C.c_size_t, C.c_int]),
@@ -140,6 +147,8 @@ SIGNATURES = {
     "kzgb_group_verify_blob_proofs_g1": (
         C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf, buf, buf, buf, buf]
     ),
+    "kzgb_group_verify_blob_proofs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf, buf]),
+    "kzgb_group_set_g2_tau": (C.c_int, [grp_p, buf]),
     "kzgb_group_verify_batch_rlc": (
         C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf, buf, u8p, buf, u8p]
     ),

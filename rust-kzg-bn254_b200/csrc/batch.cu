@@ -1,8 +1,9 @@
 // The blob-batch pipelines: kzgb_commit_and_prove_blobs{,_dev} -- commitment and proof of many blobs on several lanes
 // while a hashing stage produces the Fiat-Shamir transcripts --, kzgb_commit_blobs{,_dev} -- the commitments alone, on
 // the same plan and lanes --, kzgb_compute_blob_proofs{,_dev} -- the proofs alone, against the caller's commitments --
-// and the verifier's calls, kzgb_verify_blob_proofs_g1{,_dev} and kzgb_verify_batch_rlc{,_dev}, over one per-blob stage,
-// and kzgb_verify_kzg_proof_batch_rlc, the random linear combination alone over openings the caller has evaluated.
+// and the verifier's calls, kzgb_verify_blob_proofs{,_g1}{,_dev} and kzgb_verify_batch_rlc{,_dev}, over one per-blob stage,
+// kzgb_verify_kzg_proof_batch_rlc, the random linear combination alone over openings the caller has evaluated, and
+// kzgb_verify_proofs, the pairing check of each such opening.
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
@@ -778,7 +779,8 @@ int compute_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint
 // ---------------------------------------------------------------- verification
 // The per-blob front half of every verification (helpers.rs:613-662) on lane L: zs[i] = compute_challenge(blob i, Cs[i])
 // and ys[i] = p_i(zs[i]) for m blobs of ns[i] = blob_poly_len(lens[i]) > 0 elements.  The blobs are evaluated in rounds
-// of equal-size runs; after_round(i0, b, d_y) runs at the end of each round, with y_{i0} .. y_{i0+b-1} resident at d_y,
+// of equal-size runs; after_round(i0, b, d_z, d_y) runs at the end of each round, with z_{i0} .. z_{i0+b-1} resident at
+// d_z and y_{i0} .. y_{i0+b-1} at d_y,
 // to enqueue more work on L.st before the round's synchronise.  blobs_dev (may be null): the blob bytes on the device,
 // read in place; the transcripts are hashed from blobs_host either way.
 template <class F>
@@ -872,7 +874,7 @@ int blob_evals_stage(kzgb_ctx* c, Lane& L, const uint8_t* const* blobs_dev, cons
         eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_z, d_t, c->tw, c->logN, &ninv,
                              (Fr*)L.eval_scratch.p, nullptr, d_y, L.st, !fs_device && !any_in_domain, d_in_domain);
         CK(c, cudaMemcpyAsync(&ys[i0], d_y, b * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
-        rc = after_round(i0, b, (const Fr*)d_y);
+        rc = after_round(i0, b, (const Fr*)d_z, (const Fr*)d_y);
         if (rc) return rc;
         CK(c, cudaStreamSynchronize(L.st));
         CK(c, cudaGetLastError());
@@ -881,14 +883,27 @@ int blob_evals_stage(kzgb_ctx* c, Lane& L, const uint8_t* const* blobs_dev, cons
     return KZGB_OK;
 }
 
-// verify_blob_kzg_proof (verify.rs:77-115) up to the pairing for `count` blobs on lane 0: every blob checked as
-// kzgb_verify_blob_proof_g1 checks it, in index order, then the stage and one k_commit_minus_value launch per round.
-// out_xy == null: z and y only (no generator table, no k_commit_minus_value).
+// generator_window_table() on c's device, uploaded once
+int ensure_gen_table(kzgb_ctx* c) {
+    if (c->gen_table) return KZGB_OK;
+    Affine* t = nullptr;
+    CK(c, cudaMalloc(&t, GEN_TABLE_POINTS * sizeof(Affine)));
+    const cudaError_t e = cudaMemcpy(t, generator_window_table(), GEN_TABLE_POINTS * sizeof(Affine), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) cudaFree(t);
+    CK(c, e);
+    c->gen_table = t;
+    return KZGB_OK;
+}
+
+// verify_blob_kzg_proof (verify.rs:77-115) for `count` blobs on lane 0: every blob checked as kzgb_verify_blob_proof_g1
+// checks it, in index order, then the stage and, per round, one k_commit_minus_value launch (out_xy != null: up to the
+// pairing) or the pairing check of every opening (ok != null: the bools).  Neither: z and y only.
 int verify_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
                        size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
-                       const uint8_t* proofs_inf, uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out) {
+                       const uint8_t* proofs_inf, uint64_t* out_xy, uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out,
+                       uint8_t* ok = nullptr) {
     if (count == 0) return KZGB_OK;
-    std::vector<Affine> Cs(count);
+    std::vector<Affine> Cs(count), Ps(ok ? count : 0);
     std::vector<size_t> ns(count);
     for (size_t i = 0; i < count; i++) {
         Cs[i] = affine_from_abi(commitments_xy + 8 * i, commitments_inf ? commitments_inf[i] : 0);
@@ -897,32 +912,39 @@ int verify_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8
         if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
         ns[i] = blob_poly_len(lens[i]);
         if (ns[i] > ((size_t)1 << 28)) return fail(c, KZGB_ERR_GENERIC, "Input size exceeds maximum polynomial size");
+        if (ok) Ps[i] = P;
     }
     Lane& L = c->lanes[0];
-    Affine* d_c = nullptr;  // [C_0 .. C_{count-1} | out_0 .. out_{count-1}]
-    if (out_xy) {
-        if (!c->gen_table) {
-            Affine* t = nullptr;
-            CK(c, cudaMalloc(&t, GEN_TABLE_POINTS * sizeof(Affine)));
-            const cudaError_t e = cudaMemcpy(t, generator_window_table(), GEN_TABLE_POINTS * sizeof(Affine), cudaMemcpyHostToDevice);
-            if (e != cudaSuccess) cudaFree(t);
-            CK(c, e);
-            c->gen_table = t;
+    Affine* d_c = nullptr;  // [C_0 .. C_{count-1} | out_0 .. out_{count-1}], or [C | pi] for the pairing checks
+    if (out_xy || ok) {
+        if (int rc = ensure_gen_table(c)) return rc;
+        if (ok) {
+            if (int rc = ensure_pairing_tables(c)) return rc;
+            CK(c, L.pairing.reserve(pairing_workspace_bytes((uint32_t)std::min<size_t>(count, 65535))));
         }
         CK(c, L.bases.reserve(2 * count * sizeof(Affine)));
         d_c = (Affine*)L.bases.p;
         CK(c, cudaMemcpyAsync(d_c, Cs.data(), count * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
+        if (ok) CK(c, cudaMemcpyAsync(d_c + count, Ps.data(), count * sizeof(Affine), cudaMemcpyHostToDevice, L.st));
     }
     Affine* d_out = d_c ? d_c + count : nullptr;
     std::vector<Fr> zs(count), ys(count);
     std::vector<Affine> outs(out_xy ? count : 0);
-    int rc = blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys, [&](size_t i0, size_t b, const Fr* d_y) {
+    std::vector<uint8_t> flags(ok ? count : 0);
+    int rc = blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys,
+                              [&](size_t i0, size_t b, const Fr* d_z, const Fr* d_y) {
+        if (ok) {  // a round holds at most 65 535 blobs
+            const uint8_t* d_flags = pairing_check_launch(d_c + i0, d_c + count + i0, d_z, d_y, c->gen_table, c->pair_tab,
+                                                          L.pairing.p, (uint32_t)b, L.st);
+            CK(c, cudaMemcpyAsync(&flags[i0], d_flags, b, cudaMemcpyDeviceToHost, L.st));
+        }
         if (!out_xy) return (int)KZGB_OK;
         commit_minus_value_launch(d_c + i0, d_y, c->gen_table, d_out + i0, (uint32_t)b, L.st);
         CK(c, cudaMemcpyAsync(&outs[i0], d_out + i0, b * sizeof(Affine), cudaMemcpyDeviceToHost, L.st));
         return (int)KZGB_OK;
     });
     if (rc) return rc;
+    if (ok) return pairing_finish(c, flags, ok);
     for (size_t i = 0; i < count; i++) {
         if (out_xy) affine_to_abi(outs[i], out_xy + 8 * i, out_inf ? out_inf + i : nullptr);
         if (z_out) memcpy(z_out + 4 * i, zs[i].l, 32);
@@ -1017,7 +1039,8 @@ int verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t
         ns[i] = blob_poly_len(lens[i]);
     }
     std::vector<Fr> zs(m), ys(m);  // per-blob challenges and evaluations: the stage the per-blob verification shares
-    int rc = blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys, [](size_t, size_t, const Fr*) { return (int)KZGB_OK; });
+    int rc = blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys,
+                              [](size_t, size_t, const Fr*, const Fr*) { return (int)KZGB_OK; });
     if (rc) return rc;
     rc = rlc_combine(c, L, Cs, Ps, ns, zs, ys, d_bases, &lhs, &rhs);
     if (rc) return rc;
@@ -1071,6 +1094,39 @@ int verify_openings_rlc(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, c
     return KZGB_OK;
 }
 
+// verify_proof (verify.rs:10-75) on lane 0 for m openings: the 2m points as verify_openings_rlc checks them, then every
+// z_i and y_i below r, then the pairing checks (no blob, no hashing, no SRS).
+int verify_proofs(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                  const uint64_t* proofs_xy, const uint8_t* proofs_inf, const uint64_t* zs_mont, const uint64_t* ys_mont,
+                  uint8_t* ok) {
+    if (m == 0) return KZGB_OK;
+    Lane& L = c->lanes[0];
+    std::vector<Affine> Cs, Ps;
+    Affine* d_bases = nullptr;
+    if (int rc = upload_rlc_points(c, L, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, Cs, Ps, &d_bases)) return rc;
+    for (size_t i = 0; i < m; i++)
+        if (!fr_words_reduced(zs_mont + 4 * i) || !fr_words_reduced(ys_mont + 4 * i))
+            return fail(c, KZGB_ERR_INVALID_FIELD_ELEMENT,
+                        "z or y of opening " + std::to_string(i) + " is not a reduced field element");
+    if (int rc = ensure_gen_table(c)) return rc;
+    if (int rc = ensure_pairing_tables(c)) return rc;
+    std::vector<uint8_t> flags(m);
+    for (size_t i0 = 0; i0 < m; i0 += 65536) {  // bounded workspace
+        const size_t b = std::min<size_t>(m - i0, 65536);
+        CK(c, L.work.reserve(2 * b * sizeof(Fr)));
+        CK(c, L.pairing.reserve(pairing_workspace_bytes((uint32_t)b)));
+        Fr* d_zy = (Fr*)L.work.p;  // z then y
+        CK(c, cudaMemcpyAsync(d_zy, zs_mont + 4 * i0, b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+        CK(c, cudaMemcpyAsync(d_zy + b, ys_mont + 4 * i0, b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+        const uint8_t* d_flags = pairing_check_launch(d_bases + i0, d_bases + m + i0, d_zy, d_zy + b, c->gen_table,
+                                                      c->pair_tab, L.pairing.p, (uint32_t)b, L.st);
+        CK(c, cudaMemcpyAsync(&flags[i0], d_flags, b, cudaMemcpyDeviceToHost, L.st));
+        CK(c, cudaStreamSynchronize(L.st));
+        CK(c, cudaGetLastError());
+    }
+    return pairing_finish(c, flags, ok);
+}
+
 }  // namespace
 
 // =====================================================================================
@@ -1122,6 +1178,28 @@ int kzgb_verify_blob_proofs_g1_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev,
     Guard g(c);
     return verify_blob_proofs(c, blobs_dev, blobs_host, lens, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf,
                               out_xy, out_inf, z_out, y_out);
+}
+// ------------------------------------------------------------------------------- per-blob verification, the bools
+int kzgb_verify_proofs(kzgb_ctx* c, size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                       const uint64_t* proofs_xy, const uint8_t* proofs_inf, const uint64_t* zs_mont, const uint64_t* ys_mont,
+                       uint8_t* ok) {
+    Guard g(c);
+    return verify_proofs(c, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, zs_mont, ys_mont, ok);
+}
+int kzgb_verify_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                            const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
+                            const uint8_t* proofs_inf, uint8_t* ok) {
+    Guard g(c);
+    return verify_blob_proofs(c, nullptr, blobs, lens, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, nullptr,
+                              nullptr, nullptr, nullptr, ok);
+}
+int kzgb_verify_blob_proofs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
+                                const size_t* lens, size_t count, const uint64_t* commitments_xy,
+                                const uint8_t* commitments_inf, const uint64_t* proofs_xy, const uint8_t* proofs_inf,
+                                uint8_t* ok) {
+    Guard g(c);
+    return verify_blob_proofs(c, blobs_dev, blobs_host, lens, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf,
+                              nullptr, nullptr, nullptr, nullptr, ok);
 }
 // ------------------------------------------------------------------------------- batch verification (RLC)
 int kzgb_verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,

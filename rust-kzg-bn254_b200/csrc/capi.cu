@@ -177,6 +177,7 @@ int lane_init(kzgb_ctx* c, Lane& L, cudaStream_t st) {
 void lane_destroy(Lane& L) {
     L.bytes.release(); L.evals.release(); L.work.release(); L.ntt_scratch.release();
     L.eval_scratch.release(); L.msm_ws.release(); L.small.release(); L.bases.release(); L.bucket_total.release();
+    L.pairing.release();
     if (L.h_sets) cudaFreeHost(L.h_sets);
     if (L.h_fr) cudaFreeHost(L.h_fr);
     if (L.h_entries) cudaFreeHost(L.h_entries);
@@ -822,6 +823,7 @@ void kzgb_ctx_destroy(kzgb_ctx* c) {
     if (c->tw) cudaFree(c->tw);
     c->batch_bytes.release();
     if (c->gen_table) cudaFree(c->gen_table);
+    if (c->pair_tab) cudaFree(c->pair_tab);
     if (c->t0) cudaEventDestroy(c->t0);
     if (c->t1) cudaEventDestroy(c->t1);
     if (c->copy_st) cudaStreamDestroy(c->copy_st);

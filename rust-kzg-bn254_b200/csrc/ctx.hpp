@@ -37,7 +37,7 @@ struct Lane {
                                     // slip in between its blocks instead of queueing behind the whole grid
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     bool own_stream = false;
-    DevBuf bytes, evals, work, ntt_scratch, eval_scratch, msm_ws, small, bases, bucket_total;
+    DevBuf bytes, evals, work, ntt_scratch, eval_scratch, msm_ws, small, bases, bucket_total, pairing;
     XYZZ* h_sets = nullptr;   // pinned
     uint32_t* h_entries = nullptr;  // pinned: length of the sorted list of the MSM in flight (= its point additions)
     Fr* h_fr = nullptr;       // pinned, 16 elements
@@ -74,6 +74,11 @@ struct kzgb_ctx {
     kzgb::Affine* allroots[kzgb::ALLROOTS_MAX_LOG + 1] = {};
     kzgb::DevBuf batch_bytes;  // blob bytes of the batch in flight (commit_and_prove_blobs)
     kzgb::Affine* gen_table = nullptr;  // generator_window_table() on this device, uploaded by the first per-blob verification
+    // [tau]G2 of the pairing checks (kzgb_set_g2_tau; no SRS is involved, so reloading the SRS leaves it alone) and its
+    // PairingTables on the device, rebuilt by the first pairing check after a change
+    kzgb::G2Affine g2_tau = kzgb::default_g2_tau();
+    kzgb::PairingTables* pair_tab = nullptr;
+    bool pair_stale = true;
     // twiddles
     kzgb::Fr* tw = nullptr;
     int logN = 0;
@@ -188,5 +193,11 @@ int proof_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z
 int blob_upload(kzgb_ctx* c, Lane& L, const uint8_t* blob_host, size_t len);
 int blob_to_evals(kzgb_ctx* c, Lane& L, const uint8_t* blob_host, const uint8_t* blob_dev, size_t len, size_t n);
 int validate_points_dev(kzgb_ctx* c, Lane& L, const Affine* d_pts, size_t n);
+// ---- pairing checks (pairing.cu)
+// c->pair_tab up to date with c->g2_tau
+int ensure_pairing_tables(kzgb_ctx* c);
+// the flags of pairing_check_launch -> ok[0 .. flags.size()), or GenericError "Evaluation point equals trusted setup
+// secret" if any flag is 2, ok untouched
+int pairing_finish(kzgb_ctx* c, const std::vector<uint8_t>& flags, uint8_t* ok);
 
 }  // namespace kzgb

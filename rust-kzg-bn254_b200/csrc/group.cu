@@ -242,6 +242,31 @@ int kzgb_group_verify_blob_proofs_g1(kzgb_group* g, const uint8_t* const* blobs,
     });
 }
 
+// verify_blob_kzg_proof (verifier/src/verify.rs:77-115) through the pairing for `count` blobs, cut as
+// kzgb_group_commit_and_prove_blobs cuts them.
+int kzgb_group_verify_blob_proofs(kzgb_group* g, const uint8_t* const* blobs, const size_t* lens, size_t count,
+                                  const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
+                                  const uint8_t* proofs_inf, uint8_t* ok) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    if (count == 0) return KZGB_OK;
+    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
+    return for_members(g, [&](int i) {
+        const size_t a = cut[i], b = cut[i + 1];
+        if (a >= b) return (int)KZGB_OK;
+        return kzgb_verify_blob_proofs(g->ctx[i], blobs + a, lens + a, b - a, commitments_xy + 8 * a,
+                                       commitments_inf ? commitments_inf + a : nullptr, proofs_xy + 8 * a,
+                                       proofs_inf ? proofs_inf + a : nullptr, ok + a);
+    });
+}
+
+// [tau]G2 of every member: checked on member 0 first, so an invalid point changes no member
+int kzgb_group_set_g2_tau(kzgb_group* g, const uint64_t xy[16]) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    const int rc = kzgb_set_g2_tau(g->ctx[0], xy);
+    if (rc) return gfail(g, rc, kzgb_last_error(g->ctx[0]));
+    return for_members(g, [&](int i) { return i == 0 ? (int)KZGB_OK : kzgb_set_g2_tau(g->ctx[i], xy); });
+}
+
 // verify_blob_kzg_proof_batch (verifier/src/batch.rs:16-249) up to the pairing.  The per-blob challenges and evaluations,
 // nearly all of the work, are cut by bytes across the members; the combination (two MSMs of m and 2m + 1 points) runs
 // on member 0 over all m openings, so the result is the one-context call's.

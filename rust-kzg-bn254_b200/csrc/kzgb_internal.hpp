@@ -5,7 +5,7 @@
 #include <stddef.h>
 #include <stdint.h>
 #include <atomic>
-#include "ec.cuh"
+#include "pairing.cuh"
 
 namespace kzgb {
 
@@ -200,6 +200,24 @@ const Affine* generator_window_table();
 // points of generator_window_table() on the device
 void commit_minus_value_launch(const Affine* C, const Fr* y_mont, const Affine* gen_table, Affine* out, uint32_t count,
                                cudaStream_t st);
+// ---- per-opening pairing checks (pairing.cu) ----------------------------------------------
+// One context's pairing constants on the device: the Miller-loop lines of the G2 generator ([0]) and of [tau]G2 ([1]),
+// [tau]G2 itself and the G2 generator's signed 4-bit window multiples j 16^w G2 at [8 w + j - 1] (the shape of
+// generator_window_table).
+struct PairingTables {
+    Line lines[2][PAIRING_LINES];
+    G2Affine tau;
+    G2Affine g2tab[GEN_TABLE_POINTS];
+};
+// Device workspace of pairing_check_launch for `count` openings.
+size_t pairing_workspace_bytes(uint32_t count);
+// For openings i < count (C_i, pi_i affine, z_i, y_i Montgomery, all on the device): three kernels on st, one thread per
+// opening.  Returns the device flags inside ws: 1 if e(C_i - [y_i]G1, G2) == e(pi_i, [tau - z_i]G2), 0 if not, 2 if
+// [z_i]G2 == [tau]G2 (the reference raises an error there).  gen_table: generator_window_table() on the device.
+uint8_t* pairing_check_launch(const Affine* C, const Affine* Pi, const Fr* z_mont, const Fr* y_mont, const Affine* gen_table,
+                              const PairingTables* tab, void* ws, uint32_t count, cudaStream_t st);
+// the reference's G2_TAU (primitives/src/consts.rs:55-64), the default [tau]G2 of a context
+G2Affine default_g2_tau();
 // out[i] = base^(first + i) (Montgomery), i < n
 void fr_powers_launch(Fr* out, uint32_t n, const Fr* base_mont_host, cudaStream_t st, uint32_t first = 0);
 // out[i] = a[i] * b[i]

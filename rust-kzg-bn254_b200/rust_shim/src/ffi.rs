@@ -82,6 +82,21 @@ extern "C" {
                                             commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,
                                             proofs_inf: *const u8, out_xy: *mut u64, out_inf: *mut u8, z_out: *mut u64,
                                             y_out: *mut u64) -> c_int;
+    pub fn kzgb_set_g2_tau(ctx: *mut kzgb_ctx, xy: *const u64) -> c_int;
+    pub fn kzgb_group_set_g2_tau(group: *mut kzgb_group, xy: *const u64) -> c_int;
+    pub fn kzgb_verify_proofs(ctx: *mut kzgb_ctx, count: usize, commitments_xy: *const u64, commitments_inf: *const u8,
+                              proofs_xy: *const u64, proofs_inf: *const u8, zs_mont: *const u64, ys_mont: *const u64,
+                              ok: *mut u8) -> c_int;
+    pub fn kzgb_verify_blob_proofs(ctx: *mut kzgb_ctx, blobs: *const *const u8, lens: *const usize, count: usize,
+                                   commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,
+                                   proofs_inf: *const u8, ok: *mut u8) -> c_int;
+    pub fn kzgb_verify_blob_proofs_dev(ctx: *mut kzgb_ctx, blobs_dev: *const *const u8, blobs_host: *const *const u8,
+                                       lens: *const usize, count: usize, commitments_xy: *const u64,
+                                       commitments_inf: *const u8, proofs_xy: *const u64, proofs_inf: *const u8,
+                                       ok: *mut u8) -> c_int;
+    pub fn kzgb_group_verify_blob_proofs(group: *mut kzgb_group, blobs: *const *const u8, lens: *const usize, count: usize,
+                                         commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,
+                                         proofs_inf: *const u8, ok: *mut u8) -> c_int;
     pub fn kzgb_group_msm_srs(group: *mut kzgb_group, scalars: *const u64, n: usize, out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_verify_batch_rlc(ctx: *mut kzgb_ctx, blobs: *const *const u8, lens: *const usize, count: usize,
                                  commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,
