@@ -118,21 +118,28 @@ HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible, bool 
 }
 
 // ---------------------------------------------------------------- planning
-// One kzgb_commit_and_prove_blobs{,_dev}, kzgb_commit_blobs{,_dev} or kzgb_compute_blob_proofs{,_dev} call: its arguments
-// and the plan made for them.
+// What a batch computes: kzgb_commit_and_prove_blobs{,_dev}, kzgb_commit_blobs{,_dev} (commitments, no transcripts) or
+// kzgb_compute_blob_proofs{,_dev} (proofs against the caller's commitments, no commit phase).
+enum class Job { CommitAndProve, Commit, Prove };
+
+// One batch call: its arguments and the plan made for them.  The entry points set their job's outputs by name.
 struct Batch {
+    Batch(kzgb_ctx* c, Job job, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
+          size_t count)
+        : c(c), job(job), blobs_dev(blobs_dev), blobs_host(blobs_host), lens(lens), count(count) {}
     kzgb_ctx* c;
+    Job job;
     const uint8_t* const* blobs_dev;   // nullptr: the blobs are only on the host
-    const uint8_t* const* blobs_host;  // the transcripts are hashed from these (commit-only with blobs_dev: nullptr)
+    const uint8_t* const* blobs_host;  // the transcripts are hashed from these (Commit with blobs_dev: nullptr)
     const size_t* lens;
     size_t count;
-    uint8_t* commitments32;
-    uint8_t* proofs32;
-    bool commit_only = false;  // kzgb_commit_blobs: commitments into out_xy / out_inf, no proofs
-    uint64_t* out_xy = nullptr;
+    uint8_t* commitments32 = nullptr;  // CommitAndProve: compressed points
+    uint8_t* proofs32 = nullptr;
+    uint64_t* out_xy = nullptr;        // Commit, Prove: the affine ABI, out_inf optional
     uint8_t* out_inf = nullptr;
-    bool prove_only = false;      // kzgb_compute_blob_proofs: proofs against `commits` into out_xy / out_inf, no commit phase
-    std::vector<Affine> commits;  // prove_only: the caller's commitments
+    const uint64_t* commitments_xy = nullptr;  // Prove: the caller's commitments in the ABI ...
+    const uint8_t* commitments_inf = nullptr;
+    std::vector<Affine> commits;               // ... read and checked by plan_batch
     size_t max_n = 0;
     std::vector<std::pair<size_t, size_t>> groups;  // small blobs: (first blob, blobs); empty: one blob per task
     int n_lanes = 0;
@@ -149,10 +156,13 @@ int plan_batch(Batch& b) {
     const size_t* lens = b.lens;
     const size_t count = b.count;
     for (size_t i = 0; i < count; i++) {
-        if (b.commit_only) {
+        if (b.job == Job::Commit) {
             if (int rc = check_commit_blob_len(c, blob_poly_len(lens[i]))) return rc;
         } else {
-            if (b.prove_only && !aff_on_curve(b.commits[i])) return fail(c, KZGB_ERR_NOT_ON_CURVE, "G1 point not on curve");
+            if (b.job == Job::Prove) {
+                b.commits.push_back(affine_from_abi(b.commitments_xy + 8 * i, b.commitments_inf ? b.commitments_inf[i] : 0));
+                if (!aff_on_curve(b.commits[i])) return fail(c, KZGB_ERR_NOT_ON_CURVE, "G1 point not on curve");
+            }
             if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
             if (int rc = check_srs_capacity(c, blob_poly_len(lens[i]))) return rc;
         }
@@ -217,33 +227,38 @@ void stage_blob_bytes(Batch& b) {
 }
 
 // ---------------------------------------------------------------- hashing stage
-// Transcript midstates (everything but the commitment): a pool of host threads from the front of the batch and, when
-// the host cannot keep up with the GPU, one warp per transcript on the device for the blobs at its end
-// (device_hash_share).  Whoever delivers a midstate first installs it; the lanes take proofs as they become ready.
-// The lane schedulers keep their own shared state under the stage's lock as well.
-class HashStage {
-public:
+// What the lanes of one batch share: a lane that fails stops the others.  The hashing stage and the large-blob task
+// queue keep their state under the same lock and signal on the same condition.
+struct LaneSync {
     std::mutex mu;
     std::condition_variable cv;
-    std::vector<Sha256> mid;   // midstate of blob i, once ready[i]
-    std::vector<uint8_t> ready;
-    bool failed = false;       // a lane failed: everyone stops
-    const size_t dev_first;    // blobs [dev_first, count) are the device's share
-
-    HashStage(const Batch& batch, const HashPlan& hp);
-    // The one teardown, on every exit path: stop the device hashing and wait for it (it reads the blob bytes), then
-    // for the pool.
-    ~HashStage();
+    std::atomic<bool> failed{false};  // set under mu, so that a wait on cv sees it
     void fail() {
         std::lock_guard<std::mutex> lk(mu);
         failed = true;
         cv.notify_all();
     }
+};
+
+// Transcript midstates (everything but the commitment): a pool of host threads from the front of the batch and, when
+// the host cannot keep up with the GPU, one warp per transcript on the device for the blobs at its end
+// (device_hash_share).  Whoever delivers a midstate first installs it; the lanes take proofs as they become ready.
+class HashStage {
+public:
+    LaneSync& sync;
+    std::vector<Sha256> mid;   // midstate of blob i, once ready[i]
+    std::vector<uint8_t> ready;
+    const size_t dev_first;    // blobs [dev_first, count) are the device's share
+
+    HashStage(const Batch& batch, const HashPlan& hp, LaneSync& sync);
+    // The one teardown, on every exit path: stop the device hashing and wait for it (it reads the blob bytes), then
+    // for the pool.
+    ~HashStage();
     // Waits for the midstates of blobs [first, first + n); false: a lane failed.
     bool wait_ready(size_t first, size_t n) {
-        std::unique_lock<std::mutex> lk(mu);
-        for (size_t k = 0; k < n; k++) cv.wait(lk, [&] { return ready[first + k] != 0 || failed; });
-        return !failed;
+        std::unique_lock<std::mutex> lk(sync.mu);
+        for (size_t k = 0; k < n; k++) sync.cv.wait(lk, [&] { return ready[first + k] != 0 || sync.failed.load(); });
+        return !sync.failed.load();
     }
     // blob i went up to c->batch_bytes on the hashing stream (ev_hash_uploaded)
     bool uploaded_here(size_t i) const { return i >= dev_first && !dev_failed.load(); }
@@ -267,13 +282,13 @@ private:
     void poll_device();
     void hash_tasks();
     void install(size_t i, const Sha256& sh) {
-        std::lock_guard<std::mutex> lk(mu);
+        std::lock_guard<std::mutex> lk(sync.mu);
         if (!ready[i]) { mid[i] = sh; ready[i] = 1; }
     }
 };
 
-HashStage::HashStage(const Batch& batch, const HashPlan& hp)
-    : mid(batch.count), ready(batch.count, 0), dev_first(batch.count - hp.dev_k), b(batch), c(batch.c), dev_k(hp.dev_k) {
+HashStage::HashStage(const Batch& batch, const HashPlan& hp, LaneSync& sync)
+    : sync(sync), mid(batch.count), ready(batch.count, 0), dev_first(batch.count - hp.dev_k), b(batch), c(batch.c), dev_k(hp.dev_k) {
     if (dev_k && start_device(hp.dev_lanes) != cudaSuccess) { cudaGetLastError(); dev_failed.store(true); }  // the host pool takes the whole batch
     if (dev_k && !dev_failed.load()) poller = std::thread(&HashStage::poll_device, this);
     for (size_t i = 0; i < b.count;) {
@@ -290,10 +305,10 @@ HashStage::HashStage(const Batch& batch, const HashPlan& hp)
 }
 
 HashStage::~HashStage() {
-    { std::lock_guard<std::mutex> lk(mu); dev_stop.store(true); }
+    { std::lock_guard<std::mutex> lk(sync.mu); dev_stop.store(true); }
     if (fsl_cancel) *fsl_cancel = 1;
     next_task.store(tasks.size());
-    cv.notify_all();
+    sync.cv.notify_all();
     if (poller.joinable()) poller.join();
     for (auto& t : pool) t.join();
     if (dev_k && c->hash_st) cudaStreamSynchronize(c->hash_st);
@@ -354,7 +369,7 @@ void HashStage::poll_device() {
             install(i, challenge_midstate_resume(st, b.blobs_host[i], b.lens[i] / 32));
             seen[j] = 1; remaining--; any = true;
         }
-        if (any) cv.notify_all();
+        if (any) sync.cv.notify_all();
         else { struct timespec ts = {0, 100000}; nanosleep(&ts, nullptr); }
     }
 }
@@ -381,18 +396,18 @@ void HashStage::hash_tasks() {
                         (w1.tv_sec - w0.tv_sec) * 1e3 + (w1.tv_nsec - w0.tv_nsec) * 1e-6, (c1.tv_sec - c0.tv_sec) * 1e3 + (c1.tv_nsec - c0.tv_nsec) * 1e-6);
             }
             for (size_t m = 0; m < members; m++) install(i + m, challenge_midstate_resume(st[m], b.blobs_host[i + m], b.lens[i + m] / 32));
-            cv.notify_all();
+            sync.cv.notify_all();
             continue;
         }
         if (i >= dev_first) {  // the device's share: only if the device path failed
-            std::unique_lock<std::mutex> lk(mu);
-            cv.wait(lk, [&] { return ready[i] != 0 || failed || dev_failed.load() || dev_stop.load(); });
-            if (ready[i] || failed || dev_stop.load()) continue;
+            std::unique_lock<std::mutex> lk(sync.mu);
+            sync.cv.wait(lk, [&] { return ready[i] != 0 || sync.failed.load() || dev_failed.load() || dev_stop.load(); });
+            if (ready[i] || sync.failed.load() || dev_stop.load()) continue;
         }
         Sha256 sh;
         challenge_midstate(sh, b.blobs_host[i], b.lens[i], blob_poly_len(b.lens[i]));
         install(i, sh);
-        cv.notify_all();
+        sync.cv.notify_all();
     }
 }
 
@@ -417,10 +432,14 @@ int run_lanes(const Batch& b, F lane_main) {
     return KZGB_OK;
 }
 
-// Where proof i goes: arkworks-compressed bytes (commit_and_prove), or the affine ABI (compute_blob_proofs).
+// Where commitment i and proof i go: arkworks-compressed bytes (CommitAndProve), or the affine ABI (Commit, Prove).
+void put_commitment(const Batch& b, size_t i, const Affine& p) {
+    if (b.job == Job::CommitAndProve) serialize_compressed(p, b.commitments32 + 32 * i);
+    else affine_to_abi(p, b.out_xy + 8 * i, b.out_inf ? b.out_inf + i : nullptr);
+}
 void put_proof(const Batch& b, size_t i, const Affine& p) {
-    if (b.prove_only) affine_to_abi(p, b.out_xy + 8 * i, b.out_inf ? b.out_inf + i : nullptr);
-    else serialize_compressed(p, b.proofs32 + 32 * i);
+    if (b.job == Job::CommitAndProve) serialize_compressed(p, b.proofs32 + 32 * i);
+    else affine_to_abi(p, b.out_xy + 8 * i, b.out_inf ? b.out_inf + i : nullptr);
 }
 
 // The bytes of the bn blobs from blob i0 (all of n elements) at a stride of 32 n with zero-filled tails, so that one launch
@@ -457,7 +476,7 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
     const int logn = log2_exact(n);
     const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
     MsmJob job;
-    if (b.commit_only && lag) {
+    if (b.job == Job::Commit && lag) {
         const uint8_t* src = nullptr;
         int r = group_bytes(b, L, i0, bn, &src);
         if (!r) r = msm_enqueue(c, L, {nullptr, src, (uint64_t)bn * n * 32}, n, bn, lag, nullptr, 0, &job);
@@ -531,22 +550,21 @@ int group_prove(const Batch& b, const HashStage& hs, Lane& L, size_t i0, size_t 
     return r;
 }
 
-// Small blobs: groups of equal-size blobs, each phase of a group is ONE batched launch set.  A proof-only group has no
-// commitment phase: its blob bytes (group_bytes) become Montgomery evaluations in one conversion launch and the
-// commitments are the caller's.
-int group_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next_group, int li) {
+// Small blobs: groups of equal-size blobs, each phase of a group is ONE batched launch set.  A commit-only group ends
+// with its commitment phase (no hashing stage: hs is null).  A proof-only group has no commitment phase: its blob bytes
+// (group_bytes) become Montgomery evaluations in one conversion launch and the commitments are the caller's.
+int group_lane(const Batch& b, LaneSync& sync, HashStage* hs, std::atomic<size_t>& next_group, int li) {
     kzgb_ctx* c = b.c;
     Lane& L = c->lanes[li];
     std::vector<Affine> commits, pts;
     for (;;) {
         size_t gi = next_group.fetch_add(1);
-        if (gi >= b.groups.size()) return KZGB_OK;
-        { std::lock_guard<std::mutex> lk(hs.mu); if (hs.failed) return KZGB_OK; }
+        if (gi >= b.groups.size() || sync.failed.load()) return KZGB_OK;
         const size_t i0 = b.groups[gi].first, bn = b.groups[gi].second;
         const size_t n = blob_poly_len(b.lens[i0]);
         int r = KZGB_OK;
         const Affine* cs = nullptr;
-        if (b.prove_only) {
+        if (b.job == Job::Prove) {
             const uint8_t* src = nullptr;
             r = group_bytes(b, L, i0, bn, &src);
             if (!r && L.evals.reserve(bn * n * sizeof(Fr)) != cudaSuccess) r = fail(c, KZGB_ERR_DEVICE, "CUDA error: evals");
@@ -555,52 +573,63 @@ int group_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next_group, i
         } else {
             commits.resize(bn);
             r = group_commit(b, L, i0, bn, commits.data());
-            if (!r) for (size_t k = 0; k < bn; k++) serialize_compressed(commits[k], b.commitments32 + 32 * (i0 + k));
+            if (!r) for (size_t k = 0; k < bn; k++) put_commitment(b, i0 + k, commits[k]);
             cs = commits.data();
         }
-        pts.resize(bn);
-        if (!r) {
-            if (!hs.wait_ready(i0, bn)) return KZGB_OK;  // the transcript midstates come from the hashing stage
-            r = group_prove(b, hs, L, i0, bn, cs, pts.data());
+        if (!r && b.job != Job::Commit) {
+            if (!hs->wait_ready(i0, bn)) return KZGB_OK;  // the transcript midstates come from the hashing stage
+            pts.resize(bn);
+            r = group_prove(b, *hs, L, i0, bn, cs, pts.data());
+            if (!r) for (size_t k = 0; k < bn; k++) put_proof(b, i0 + k, pts[k]);
         }
-        if (r) { hs.fail(); return r; }
-        for (size_t k = 0; k < bn; k++) put_proof(b, i0 + k, pts[k]);
+        if (r) { sync.fail(); return r; }
     }
-}
-
-int run_groups(const Batch& b, HashStage& hs) {
-    std::atomic<size_t> next_group{0};
-    return run_lanes(b, [&](int li) { return group_lane(b, hs, next_group, li); });
 }
 
 // Task scheduler.  commit(i) needs nothing; proof(i) needs commit(i) and the transcript midstate of
 // blob i (host SHA-256, ~9 ms for 16 MiB).  A lane takes the lowest ready proof, else the next
-// commit, so the GPU never idles behind the hashing pool.  The queue lives under the hashing stage's lock.
+// commit, so the GPU never idles behind the hashing pool.  The queue lives under the lanes' lock.
 struct TaskQueue {
+    explicit TaskQueue(size_t count) : commit_done(count, 0), proof_taken(count, 0), commits(count) {}
     std::vector<uint8_t> commit_done, proof_taken;
     std::vector<Affine> commits;
     size_t next_commit = 0, proofs_taken = 0, proof_scan = 0;
 };
 
 // false: nothing left for this lane (every proof taken, or a lane failed)
-bool take_task(const Batch& b, HashStage& hs, TaskQueue& q, size_t* task, bool* is_proof) {
-    std::unique_lock<std::mutex> lk(hs.mu);
+bool take_task(const Batch& b, const HashStage& hs, TaskQueue& q, size_t* task, bool* is_proof) {
+    LaneSync& s = hs.sync;
+    std::unique_lock<std::mutex> lk(s.mu);
     for (;;) {
-        if (hs.failed) return false;
+        if (s.failed.load()) return false;
         while (q.proof_scan < b.count && q.proof_taken[q.proof_scan]) q.proof_scan++;
         for (size_t k = q.proof_scan; k < b.count && k < q.next_commit; k++) {
             if (q.proof_taken[k] || !q.commit_done[k] || !hs.ready[k]) continue;
             q.proof_taken[k] = 1; q.proofs_taken++;
             *task = k; *is_proof = true;
-            if (q.proofs_taken == b.count) hs.cv.notify_all();  // lanes with nothing left to take can leave
+            if (q.proofs_taken == b.count) s.cv.notify_all();  // lanes with nothing left to take can leave
             return true;
         }
         if (q.next_commit < b.count) { *task = q.next_commit++; *is_proof = false; return true; }
         if (q.proofs_taken == b.count) return false;
-        hs.cv.wait(lk);
+        s.cv.wait(lk);
     }
 }
 
+// Where blob i's bytes are on the device for a task of lane L: the caller's device blob, the slot of c->batch_bytes the
+// hashing stream uploaded it to (with `wait`, L.st first waits for that upload), or nullptr: not on the device yet.
+int device_blob(const Batch& b, const HashStage& hs, Lane& L, size_t i, bool wait, const uint8_t** bytes) {
+    kzgb_ctx* c = b.c;
+    *bytes = b.blobs_dev ? b.blobs_dev[i] : nullptr;
+    if (*bytes || !hs.uploaded_here(i)) return KZGB_OK;
+    *bytes = (const uint8_t*)c->batch_bytes.p + b.byte_off[i];
+    if (wait && cudaStreamWaitEvent(L.st, c->ev_hash_uploaded, 0) != cudaSuccess)
+        return fail(c, KZGB_ERR_DEVICE, "CUDA error: cudaStreamWaitEvent failed");
+    return KZGB_OK;
+}
+
+// Large blobs, commit and prove: the tasks of the queue.  A staged blob goes up into its slot with its commit task (unless
+// the hashing stream has put it there) and stays for its proof.
 int task_lane(const Batch& b, HashStage& hs, TaskQueue& q, int li) {
     kzgb_ctx* c = b.c;
     Lane& L = c->lanes[li];
@@ -608,17 +637,12 @@ int task_lane(const Batch& b, HashStage& hs, TaskQueue& q, int li) {
     bool is_proof = false;
     while (take_task(b, hs, q, &i, &is_proof)) {
         size_t len = b.lens[i], n = blob_poly_len(len);
-        const uint8_t* dev_bytes = b.blobs_dev ? b.blobs_dev[i] : nullptr;
-        int r = KZGB_OK;
-        if (!dev_bytes && b.resident) {
+        const uint8_t* dev_bytes = nullptr;
+        int r = device_blob(b, hs, L, i, !is_proof, &dev_bytes);
+        if (!r && !dev_bytes && b.resident) {
             uint8_t* slot = (uint8_t*)c->batch_bytes.p + b.byte_off[i];
-            if (hs.uploaded_here(i)) {
-                if (!is_proof && cudaStreamWaitEvent(L.st, c->ev_hash_uploaded, 0) != cudaSuccess)
-                    r = fail(c, KZGB_ERR_DEVICE, "CUDA error: cudaStreamWaitEvent failed");
-            } else if (!is_proof && len) {
-                if (cudaMemcpyAsync(slot, b.blobs_host[i], len, cudaMemcpyHostToDevice, L.st) != cudaSuccess)
-                    r = fail(c, KZGB_ERR_DEVICE, "CUDA error: H2D copy of a blob failed");
-            }
+            if (!is_proof && len && cudaMemcpyAsync(slot, b.blobs_host[i], len, cudaMemcpyHostToDevice, L.st) != cudaSuccess)
+                r = fail(c, KZGB_ERR_DEVICE, "CUDA error: H2D copy of a blob failed");
             dev_bytes = slot;
         }
         MsmJob job;
@@ -630,63 +654,27 @@ int task_lane(const Batch& b, HashStage& hs, TaskQueue& q, int li) {
             r = proof_enqueue(c, L, (Fr*)L.evals.p, n, z, &job);
         }
         if (!r) r = msm_finish(c, L, job, &out);
-        if (r) { hs.fail(); return r; }
+        if (r) { hs.sync.fail(); return r; }
         if (is_proof) {
-            serialize_compressed(out, b.proofs32 + 32 * i);
+            put_proof(b, i, out);
         } else {
-            serialize_compressed(out, b.commitments32 + 32 * i);
-            { std::lock_guard<std::mutex> lk(hs.mu); q.commits[i] = out; q.commit_done[i] = 1; }
-            hs.cv.notify_all();
+            put_commitment(b, i, out);
+            { std::lock_guard<std::mutex> lk(hs.sync.mu); q.commits[i] = out; q.commit_done[i] = 1; }
+            hs.sync.cv.notify_all();
         }
     }
     return KZGB_OK;
 }
 
-int run_tasks(const Batch& b, HashStage& hs) {
-    TaskQueue q{std::vector<uint8_t>(b.count, 0), std::vector<uint8_t>(b.count, 0), std::vector<Affine>(b.count)};
-    return run_lanes(b, [&](int li) { return task_lane(b, hs, q, li); });
-}
-
-int commit_and_prove(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
-                     size_t count, uint8_t* commitments32, uint8_t* proofs32) {
-    if (count == 0) return KZGB_OK;
-    Batch b{c, blobs_dev, blobs_host, lens, count, commitments32, proofs32};
-    int rc = plan_batch(b);
-    if (rc) return rc;
-    stage_blob_bytes(b);
-    const HashPlan hplan = b.groups.empty() ? hash_plan(lens, count, blobs_dev || b.resident, false) : HashPlan();
-    {
-        HashStage hs(b, hplan);
-        rc = b.groups.empty() ? run_tasks(b, hs) : run_groups(b, hs);
-    }
-    if (b.groups.empty() && c->batch_bytes.cap > ((size_t)g_batch_keep_mib.load() << 20)) c->batch_bytes.release();  // bounded residency between calls
-    return rc;
-}
-
-// ---------------------------------------------------------------- commitments only
-// Small blobs: the groups' commitment phase and nothing else.
-int commit_group_lane(const Batch& b, std::atomic<size_t>& next_group, std::atomic<bool>& failed, int li) {
-    Lane& L = b.c->lanes[li];
-    std::vector<Affine> pts;
-    for (;;) {
-        const size_t gi = next_group.fetch_add(1);
-        if (gi >= b.groups.size() || failed.load()) return KZGB_OK;
-        const size_t i0 = b.groups[gi].first, bn = b.groups[gi].second;
-        pts.resize(bn);
-        if (int r = group_commit(b, L, i0, bn, pts.data())) { failed.store(true); return r; }
-        for (size_t k = 0; k < bn; k++) affine_to_abi(pts[k], b.out_xy + 8 * (i0 + k), b.out_inf ? b.out_inf + i0 + k : nullptr);
-    }
-}
-
-// Large blobs: every task is "commit blob i", taken in blob order.  A blob is read once, so it goes up into the lane's
-// own buffer; over a Lagrange table the MSM reads its bytes, otherwise they are converted, inverse-transformed and
-// committed over the monomial table (commit_evals_enqueue).
-int commit_task_lane(const Batch& b, std::atomic<size_t>& next, std::atomic<bool>& failed, int li) {
+// Large blobs, commitments only: every task is "commit blob i", taken in blob order.  A blob is read once, so it goes up
+// into the lane's own buffer; over a Lagrange table the MSM reads its bytes, otherwise they are converted,
+// inverse-transformed and committed over the monomial table (commit_evals_enqueue).
+int commit_task_lane(const Batch& b, LaneSync& sync, std::atomic<size_t>& next, int li) {
     kzgb_ctx* c = b.c;
     Lane& L = c->lanes[li];
     for (;;) {
         const size_t i = next.fetch_add(1);
-        if (i >= b.count || failed.load()) return KZGB_OK;
+        if (i >= b.count || sync.failed.load()) return KZGB_OK;
         const size_t len = b.lens[i], n = blob_poly_len(len);
         const kzgb_ctx::LagTable* lag = lagrange_table(c, log2_exact(n));
         const uint8_t* blob_host = b.blobs_dev ? nullptr : b.blobs_host[i];
@@ -705,28 +693,14 @@ int commit_task_lane(const Batch& b, std::atomic<size_t>& next, std::atomic<bool
             if (!r) r = commit_evals_enqueue(c, L, (Fr*)L.evals.p, n, &job);
         }
         if (!r) r = msm_finish(c, L, job, &out);
-        if (r) { failed.store(true); return r; }
-        affine_to_abi(out, b.out_xy + 8 * i, b.out_inf ? b.out_inf + i : nullptr);
+        if (r) { sync.fail(); return r; }
+        put_commitment(b, i, out);
     }
 }
 
-int commit_blobs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
-                 size_t count, uint64_t* out_xy, uint8_t* out_inf) {
-    if (count == 0) return KZGB_OK;
-    Batch b{c, blobs_dev, blobs_host, lens, count, nullptr, nullptr, true, out_xy, out_inf};
-    int rc = plan_batch(b);
-    if (rc) return rc;
-    std::atomic<size_t> next{0};
-    std::atomic<bool> failed{false};
-    return run_lanes(b, [&](int li) {
-        return b.groups.empty() ? commit_task_lane(b, next, failed, li) : commit_group_lane(b, next, failed, li);
-    });
-}
-
-// ---------------------------------------------------------------- proofs only
-// Large blobs: every task is "prove blob i", taken in blob order.  A blob is read once, so it goes up into the lane's own
-// buffer (unless the device's share of the hashing has staged it already) and is converted while its transcript is
-// hashed.  Then the challenge with the caller's commitment, the quotient and its MSM.
+// Large blobs, proofs only: every task is "prove blob i", taken in blob order.  A blob is read once, so it goes up into
+// the lane's own buffer (unless the device's share of the hashing has staged it already) and is converted while its
+// transcript is hashed.  Then the challenge with the caller's commitment, the quotient and its MSM.
 int prove_task_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next, int li) {
     kzgb_ctx* c = b.c;
     Lane& L = c->lanes[li];
@@ -734,45 +708,54 @@ int prove_task_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next, in
         const size_t i = next.fetch_add(1);
         if (i >= b.count) return KZGB_OK;
         const size_t len = b.lens[i], n = blob_poly_len(len);
-        const uint8_t* dev_bytes = b.blobs_dev ? b.blobs_dev[i] : nullptr;
-        int r = KZGB_OK;
-        if (!dev_bytes && hs.uploaded_here(i)) {
-            if (cudaStreamWaitEvent(L.st, c->ev_hash_uploaded, 0) != cudaSuccess)
-                r = fail(c, KZGB_ERR_DEVICE, "CUDA error: cudaStreamWaitEvent failed");
-            dev_bytes = (const uint8_t*)c->batch_bytes.p + b.byte_off[i];
-        }
+        const uint8_t* dev_bytes = nullptr;
+        int r = device_blob(b, hs, L, i, true, &dev_bytes);
         if (!r) r = blob_to_evals(c, L, b.blobs_host[i], dev_bytes, len, n);
         if (!r && !hs.wait_ready(i, 1)) return KZGB_OK;
         MsmJob job;
         Affine out;
         if (!r) r = proof_enqueue(c, L, (Fr*)L.evals.p, n, challenge_finish(hs.mid[i], b.commits[i]), &job);
         if (!r) r = msm_finish(c, L, job, &out);
-        if (r) { hs.fail(); return r; }
+        if (r) { hs.sync.fail(); return r; }
         put_proof(b, i, out);
     }
 }
 
-int compute_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
-                        size_t count, const uint64_t* commitments_xy, const uint8_t* commitments_inf, uint64_t* out_xy,
-                        uint8_t* out_inf) {
-    if (count == 0) return KZGB_OK;
-    Batch b{c, blobs_dev, blobs_host, lens, count, nullptr, nullptr, false, out_xy, out_inf};
-    b.prove_only = true;
-    b.commits.resize(count);
-    for (size_t i = 0; i < count; i++) b.commits[i] = affine_from_abi(commitments_xy + 8 * i, commitments_inf ? commitments_inf[i] : 0);
+// ---------------------------------------------------------------- driver
+// The plan, then the lanes.  Commit has no transcripts: no staging, no hashing stage.  CommitAndProve stages host blobs
+// (stage_blob_bytes) and may hash on the device what is staged or the caller's; Prove stages host blobs only for the
+// device's share of the hashing.  Groups hash on the host pool alone.
+int run_batch(Batch& b) {
+    if (b.count == 0) return KZGB_OK;
     int rc = plan_batch(b);
     if (rc) return rc;
-    HashPlan hplan = b.groups.empty() ? hash_plan(lens, count, true, true) : HashPlan();
-    if (hplan.dev_k && !blobs_dev) {  // the device hashes blobs it holds: stage the host blobs
+    LaneSync sync;
+    std::atomic<size_t> next{0};  // the next group, or the next blob of a commit-only or proof-only task lane
+    if (b.job == Job::Commit)
+        return run_lanes(b, [&](int li) {
+            return b.groups.empty() ? commit_task_lane(b, sync, next, li) : group_lane(b, sync, nullptr, next, li);
+        });
+    HashPlan hplan;
+    if (b.job == Job::CommitAndProve) {
         stage_blob_bytes(b);
-        if (!b.resident) hplan.dev_k = 0;
+        if (b.groups.empty()) hplan = hash_plan(b.lens, b.count, b.blobs_dev || b.resident, false);
+    } else if (b.groups.empty()) {
+        hplan = hash_plan(b.lens, b.count, true, true);
+        if (hplan.dev_k && !b.blobs_dev) {  // the device hashes blobs it holds: stage the host blobs
+            stage_blob_bytes(b);
+            if (!b.resident) hplan.dev_k = 0;
+        }
     }
     {
-        HashStage hs(b, hplan);
-        std::atomic<size_t> next{0};
-        rc = run_lanes(b, [&](int li) { return b.groups.empty() ? prove_task_lane(b, hs, next, li) : group_lane(b, hs, next, li); });
+        HashStage hs(b, hplan, sync);
+        TaskQueue q(b.job == Job::CommitAndProve && b.groups.empty() ? b.count : 0);  // task_lane's
+        rc = run_lanes(b, [&](int li) {
+            if (!b.groups.empty()) return group_lane(b, sync, &hs, next, li);
+            return b.job == Job::Prove ? prove_task_lane(b, hs, next, li) : task_lane(b, hs, q, li);
+        });
     }
-    if (b.resident && c->batch_bytes.cap > ((size_t)g_batch_keep_mib.load() << 20)) c->batch_bytes.release();
+    // bounded residency between calls: only stage_blob_bytes grows the buffer
+    if (b.c->batch_bytes.cap > ((size_t)g_batch_keep_mib.load() << 20)) b.c->batch_bytes.release();
     return rc;
 }
 
@@ -1017,36 +1000,46 @@ int upload_rlc_points(kzgb_ctx* c, Lane& L, size_t m, const uint64_t* commitment
     return validate_points_dev(c, L, *d_bases, 2 * m);
 }
 
+// The random linear combination on lane 0 of m openings into lhs / rhs in the ABI; m == 0: the identity twice.  The 2m
+// points are read and checked first, then openings(L, Cs, ns, zs, ys) checks the rest of the input and fills in the
+// polynomial lengths, challenges and evaluations.
+template <class F>
+int rlc_to_abi(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
+               const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8], uint8_t* rhs_inf, F openings) {
+    Affine lhs, rhs;
+    if (m == 0) {
+        aff_set_inf(lhs);
+        rhs = lhs;
+    } else {
+        Lane& L = c->lanes[0];
+        std::vector<Affine> Cs, Ps;
+        Affine* d_bases = nullptr;
+        if (int rc = upload_rlc_points(c, L, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, Cs, Ps, &d_bases)) return rc;
+        std::vector<size_t> ns(m);
+        std::vector<Fr> zs(m), ys(m);
+        if (int rc = openings(L, Cs, ns, zs, ys)) return rc;
+        if (int rc = rlc_combine(c, L, Cs, Ps, ns, zs, ys, d_bases, &lhs, &rhs)) return rc;
+    }
+    affine_to_abi(lhs, lhs_xy, lhs_inf);
+    affine_to_abi(rhs, rhs_xy, rhs_inf);
+    return KZGB_OK;
+}
+
 // verify_blob_kzg_proof_batch (batch.rs:16-249) up to the pairing on lane 0: the 2m points, then the lengths, then the
 // per-blob stage (blobs_dev as blob_evals_stage reads it) and the combination.
 int verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host, const size_t* lens,
                      size_t m, const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
                      const uint8_t* proofs_inf, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8], uint8_t* rhs_inf) {
-    Lane& L = c->lanes[0];
-    Affine lhs, rhs;
-    if (m == 0) {
-        aff_set_inf(lhs);
-        affine_to_abi(lhs, lhs_xy, lhs_inf);
-        affine_to_abi(lhs, rhs_xy, rhs_inf);
-        return KZGB_OK;
-    }
-    std::vector<Affine> Cs, Ps;
-    Affine* d_bases = nullptr;
-    if (int rc = upload_rlc_points(c, L, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, Cs, Ps, &d_bases)) return rc;
-    std::vector<size_t> ns(m);
-    for (size_t i = 0; i < m; i++) {
-        if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
-        ns[i] = blob_poly_len(lens[i]);
-    }
-    std::vector<Fr> zs(m), ys(m);  // per-blob challenges and evaluations: the stage the per-blob verification shares
-    int rc = blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys,
-                              [](size_t, size_t, const Fr*, const Fr*) { return (int)KZGB_OK; });
-    if (rc) return rc;
-    rc = rlc_combine(c, L, Cs, Ps, ns, zs, ys, d_bases, &lhs, &rhs);
-    if (rc) return rc;
-    affine_to_abi(lhs, lhs_xy, lhs_inf);
-    affine_to_abi(rhs, rhs_xy, rhs_inf);
-    return KZGB_OK;
+    return rlc_to_abi(c, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, lhs_xy, lhs_inf, rhs_xy, rhs_inf,
+                      [&](Lane& L, const std::vector<Affine>& Cs, std::vector<size_t>& ns, std::vector<Fr>& zs, std::vector<Fr>& ys) {
+        for (size_t i = 0; i < m; i++) {
+            if (lens[i] == 0) return fail(c, KZGB_ERR_GENERIC, "Length of data after padding is 0");
+            ns[i] = blob_poly_len(lens[i]);
+        }
+        // per-blob challenges and evaluations: the stage the per-blob verification shares
+        return blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys,
+                                [](size_t, size_t, const Fr*, const Fr*) { return (int)KZGB_OK; });
+    });
 }
 
 // the 4 little-endian words at w hold a value below r
@@ -1060,38 +1053,31 @@ bool fr_words_reduced(const uint64_t* w) {
     return false;
 }
 
-// verify_kzg_proof_batch (batch.rs:185-249) on lane 0 over m openings that are already evaluated: the 2m points, then
-// every z_i and y_i a reduced Montgomery value (< r, as an arkworks Fr always is: a larger word would be hashed as other
-// bytes than the reference hashes), then the combination with the caller's n_i.
-int verify_openings_rlc(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
-                        const uint64_t* proofs_xy, const uint8_t* proofs_inf, const uint64_t* zs_mont, const uint64_t* ys_mont,
-                        const uint64_t* poly_lens, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8], uint8_t* rhs_inf) {
-    Lane& L = c->lanes[0];
-    Affine lhs, rhs;
-    if (m == 0) {
-        aff_set_inf(lhs);
-        affine_to_abi(lhs, lhs_xy, lhs_inf);
-        affine_to_abi(lhs, rhs_xy, rhs_inf);
-        return KZGB_OK;
-    }
-    std::vector<Affine> Cs, Ps;
-    Affine* d_bases = nullptr;
-    if (int rc = upload_rlc_points(c, L, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, Cs, Ps, &d_bases)) return rc;
-    std::vector<Fr> zs(m), ys(m);
-    std::vector<size_t> ns(m);
-    for (size_t i = 0; i < m; i++) {
+// Every z_i and y_i of m openings is a reduced Montgomery value (< r, as an arkworks Fr always is: a larger word would be
+// hashed as other bytes than the reference hashes); else KZGB_ERR_INVALID_FIELD_ELEMENT for the first opening that is not.
+int check_openings_reduced(kzgb_ctx* c, size_t m, const uint64_t* zs_mont, const uint64_t* ys_mont) {
+    for (size_t i = 0; i < m; i++)
         if (!fr_words_reduced(zs_mont + 4 * i) || !fr_words_reduced(ys_mont + 4 * i))
             return fail(c, KZGB_ERR_INVALID_FIELD_ELEMENT,
                         "z or y of opening " + std::to_string(i) + " is not a reduced field element");
-        memcpy(zs[i].l, zs_mont + 4 * i, 32);
-        memcpy(ys[i].l, ys_mont + 4 * i, 32);
-        ns[i] = (size_t)poly_lens[i];
-    }
-    int rc = rlc_combine(c, L, Cs, Ps, ns, zs, ys, d_bases, &lhs, &rhs);
-    if (rc) return rc;
-    affine_to_abi(lhs, lhs_xy, lhs_inf);
-    affine_to_abi(rhs, rhs_xy, rhs_inf);
     return KZGB_OK;
+}
+
+// verify_kzg_proof_batch (batch.rs:185-249) on lane 0 over m openings that are already evaluated: the 2m points, then
+// every z_i and y_i reduced, then the combination with the caller's n_i.
+int verify_openings_rlc(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, const uint8_t* commitments_inf,
+                        const uint64_t* proofs_xy, const uint8_t* proofs_inf, const uint64_t* zs_mont, const uint64_t* ys_mont,
+                        const uint64_t* poly_lens, uint64_t lhs_xy[8], uint8_t* lhs_inf, uint64_t rhs_xy[8], uint8_t* rhs_inf) {
+    return rlc_to_abi(c, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, lhs_xy, lhs_inf, rhs_xy, rhs_inf,
+                      [&](Lane&, const std::vector<Affine>&, std::vector<size_t>& ns, std::vector<Fr>& zs, std::vector<Fr>& ys) {
+        if (int rc = check_openings_reduced(c, m, zs_mont, ys_mont)) return rc;
+        for (size_t i = 0; i < m; i++) {
+            memcpy(zs[i].l, zs_mont + 4 * i, 32);
+            memcpy(ys[i].l, ys_mont + 4 * i, 32);
+            ns[i] = (size_t)poly_lens[i];
+        }
+        return (int)KZGB_OK;
+    });
 }
 
 // verify_proof (verify.rs:10-75) on lane 0 for m openings: the 2m points as verify_openings_rlc checks them, then every
@@ -1104,10 +1090,7 @@ int verify_proofs(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, const u
     std::vector<Affine> Cs, Ps;
     Affine* d_bases = nullptr;
     if (int rc = upload_rlc_points(c, L, m, commitments_xy, commitments_inf, proofs_xy, proofs_inf, Cs, Ps, &d_bases)) return rc;
-    for (size_t i = 0; i < m; i++)
-        if (!fr_words_reduced(zs_mont + 4 * i) || !fr_words_reduced(ys_mont + 4 * i))
-            return fail(c, KZGB_ERR_INVALID_FIELD_ELEMENT,
-                        "z or y of opening " + std::to_string(i) + " is not a reduced field element");
+    if (int rc = check_openings_reduced(c, m, zs_mont, ys_mont)) return rc;
     if (int rc = ensure_gen_table(c)) return rc;
     if (int rc = ensure_pairing_tables(c)) return rc;
     std::vector<uint8_t> flags(m);
@@ -1132,36 +1115,49 @@ int verify_proofs(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, const u
 // =====================================================================================
 extern "C" {
 
+// kzgb_commit_and_prove_blobs and kzgb_compute_blob_proofs are their _dev forms without device blobs.
 int kzgb_commit_and_prove_blobs(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,
                                 uint8_t* commitments32, uint8_t* proofs32) {
-    Guard g(c);
-    return commit_and_prove(c, nullptr, blobs, lens, count, commitments32, proofs32);
+    return kzgb_commit_and_prove_blobs_dev(c, nullptr, blobs, lens, count, commitments32, proofs32);
 }
 int kzgb_commit_and_prove_blobs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
                                     const size_t* lens, size_t count, uint8_t* commitments32, uint8_t* proofs32) {
     Guard g(c);
-    return commit_and_prove(c, blobs_dev, blobs_host, lens, count, commitments32, proofs32);
+    Batch b(c, Job::CommitAndProve, blobs_dev, blobs_host, lens, count);
+    b.commitments32 = commitments32;
+    b.proofs32 = proofs32;
+    return run_batch(b);
 }
 int kzgb_commit_blobs(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count, uint64_t* out_xy,
                       uint8_t* out_inf) {
     Guard g(c);
-    return commit_blobs(c, nullptr, blobs, lens, count, out_xy, out_inf);
+    Batch b(c, Job::Commit, nullptr, blobs, lens, count);
+    b.out_xy = out_xy;
+    b.out_inf = out_inf;
+    return run_batch(b);
 }
 int kzgb_commit_blobs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const size_t* lens, size_t count,
                           uint64_t* out_xy, uint8_t* out_inf) {
     Guard g(c);
-    return commit_blobs(c, blobs_dev, nullptr, lens, count, out_xy, out_inf);
+    Batch b(c, Job::Commit, blobs_dev, nullptr, lens, count);
+    b.out_xy = out_xy;
+    b.out_inf = out_inf;
+    return run_batch(b);
 }
 int kzgb_compute_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,
                              const uint64_t* commitments_xy, const uint8_t* commitments_inf, uint64_t* out_xy, uint8_t* out_inf) {
-    Guard g(c);
-    return compute_blob_proofs(c, nullptr, blobs, lens, count, commitments_xy, commitments_inf, out_xy, out_inf);
+    return kzgb_compute_blob_proofs_dev(c, nullptr, blobs, lens, count, commitments_xy, commitments_inf, out_xy, out_inf);
 }
 int kzgb_compute_blob_proofs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t* const* blobs_host,
                                  const size_t* lens, size_t count, const uint64_t* commitments_xy,
                                  const uint8_t* commitments_inf, uint64_t* out_xy, uint8_t* out_inf) {
     Guard g(c);
-    return compute_blob_proofs(c, blobs_dev, blobs_host, lens, count, commitments_xy, commitments_inf, out_xy, out_inf);
+    Batch b(c, Job::Prove, blobs_dev, blobs_host, lens, count);
+    b.commitments_xy = commitments_xy;
+    b.commitments_inf = commitments_inf;
+    b.out_xy = out_xy;
+    b.out_inf = out_inf;
+    return run_batch(b);
 }
 // ------------------------------------------------------------------------------- per-blob verification, G1 side
 int kzgb_verify_blob_proofs_g1(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,

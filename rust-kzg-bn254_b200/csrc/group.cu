@@ -73,6 +73,22 @@ std::vector<size_t> byte_balanced_cut(const size_t* lens, size_t count, int G) {
     return cut;
 }
 
+// fn(ctx, first, n) on every member whose byte-balanced share [first, first + n) of a blob batch is not empty.  The
+// caller holds g->mu.
+template <class F>
+int for_blob_shares(kzgb_group* g, const size_t* lens, size_t count, F fn) {
+    if (count == 0) return KZGB_OK;
+    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
+    return for_members(g, [&](int i) {
+        const size_t a = cut[i], b = cut[i + 1];
+        return a < b ? fn(g->ctx[i], a, b - a) : (int)KZGB_OK;
+    });
+}
+
+// p + off, or nullptr for an optional array the caller left out
+template <class T>
+T* at_or_null(T* p, size_t off) { return p ? p + off : nullptr; }
+
 int replicate_from_member0(kzgb_group* g) {
     return for_members(g, [&](int i) { return i == 0 ? KZGB_OK : kzgb_srs_clone(g->ctx[i], g->ctx[0]); });
 }
@@ -184,12 +200,8 @@ int kzgb_group_srs_precompute_ranges(kzgb_group* g, size_t n, int window_bits) {
 int kzgb_group_commit_and_prove_blobs(kzgb_group* g, const uint8_t* const* blobs, const size_t* lens, size_t count,
                                       uint8_t* commitments32, uint8_t* proofs32) {
     std::lock_guard<std::mutex> lk(g->mu);
-    if (count == 0) return KZGB_OK;
-    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
-    return for_members(g, [&](int i) {
-        const size_t a = cut[i], b = cut[i + 1];
-        if (a >= b) return (int)KZGB_OK;
-        return kzgb_commit_and_prove_blobs(g->ctx[i], blobs + a, lens + a, b - a, commitments32 + 32 * a, proofs32 + 32 * a);
+    return for_blob_shares(g, lens, count, [&](kzgb_ctx* c, size_t a, size_t n) {
+        return kzgb_commit_and_prove_blobs(c, blobs + a, lens + a, n, commitments32 + 32 * a, proofs32 + 32 * a);
     });
 }
 
@@ -197,12 +209,8 @@ int kzgb_group_commit_and_prove_blobs(kzgb_group* g, const uint8_t* const* blobs
 int kzgb_group_commit_blobs(kzgb_group* g, const uint8_t* const* blobs, const size_t* lens, size_t count,
                             uint64_t* out_xy, uint8_t* out_inf) {
     std::lock_guard<std::mutex> lk(g->mu);
-    if (count == 0) return KZGB_OK;
-    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
-    return for_members(g, [&](int i) {
-        const size_t a = cut[i], b = cut[i + 1];
-        if (a >= b) return (int)KZGB_OK;
-        return kzgb_commit_blobs(g->ctx[i], blobs + a, lens + a, b - a, out_xy + 8 * a, out_inf ? out_inf + a : nullptr);
+    return for_blob_shares(g, lens, count, [&](kzgb_ctx* c, size_t a, size_t n) {
+        return kzgb_commit_blobs(c, blobs + a, lens + a, n, out_xy + 8 * a, at_or_null(out_inf, a));
     });
 }
 
@@ -212,14 +220,9 @@ int kzgb_group_compute_blob_proofs(kzgb_group* g, const uint8_t* const* blobs, c
                                    const uint64_t* commitments_xy, const uint8_t* commitments_inf, uint64_t* out_xy,
                                    uint8_t* out_inf) {
     std::lock_guard<std::mutex> lk(g->mu);
-    if (count == 0) return KZGB_OK;
-    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
-    return for_members(g, [&](int i) {
-        const size_t a = cut[i], b = cut[i + 1];
-        if (a >= b) return (int)KZGB_OK;
-        return kzgb_compute_blob_proofs(g->ctx[i], blobs + a, lens + a, b - a, commitments_xy + 8 * a,
-                                        commitments_inf ? commitments_inf + a : nullptr, out_xy + 8 * a,
-                                        out_inf ? out_inf + a : nullptr);
+    return for_blob_shares(g, lens, count, [&](kzgb_ctx* c, size_t a, size_t n) {
+        return kzgb_compute_blob_proofs(c, blobs + a, lens + a, n, commitments_xy + 8 * a, at_or_null(commitments_inf, a),
+                                        out_xy + 8 * a, at_or_null(out_inf, a));
     });
 }
 
@@ -230,15 +233,10 @@ int kzgb_group_verify_blob_proofs_g1(kzgb_group* g, const uint8_t* const* blobs,
                                      const uint64_t* proofs_xy, const uint8_t* proofs_inf, uint64_t* out_xy,
                                      uint8_t* out_inf, uint64_t* z_out, uint64_t* y_out) {
     std::lock_guard<std::mutex> lk(g->mu);
-    if (count == 0) return KZGB_OK;
-    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
-    return for_members(g, [&](int i) {
-        const size_t a = cut[i], b = cut[i + 1];
-        if (a >= b) return (int)KZGB_OK;
-        return kzgb_verify_blob_proofs_g1(g->ctx[i], blobs + a, lens + a, b - a, commitments_xy + 8 * a,
-                                          commitments_inf ? commitments_inf + a : nullptr, proofs_xy + 8 * a,
-                                          proofs_inf ? proofs_inf + a : nullptr, out_xy + 8 * a, out_inf ? out_inf + a : nullptr,
-                                          z_out ? z_out + 4 * a : nullptr, y_out ? y_out + 4 * a : nullptr);
+    return for_blob_shares(g, lens, count, [&](kzgb_ctx* c, size_t a, size_t n) {
+        return kzgb_verify_blob_proofs_g1(c, blobs + a, lens + a, n, commitments_xy + 8 * a, at_or_null(commitments_inf, a),
+                                          proofs_xy + 8 * a, at_or_null(proofs_inf, a), at_or_null(out_xy, 8 * a),
+                                          at_or_null(out_inf, a), at_or_null(z_out, 4 * a), at_or_null(y_out, 4 * a));
     });
 }
 
@@ -248,14 +246,9 @@ int kzgb_group_verify_blob_proofs(kzgb_group* g, const uint8_t* const* blobs, co
                                   const uint64_t* commitments_xy, const uint8_t* commitments_inf, const uint64_t* proofs_xy,
                                   const uint8_t* proofs_inf, uint8_t* ok) {
     std::lock_guard<std::mutex> lk(g->mu);
-    if (count == 0) return KZGB_OK;
-    const std::vector<size_t> cut = byte_balanced_cut(lens, count, (int)g->ctx.size());
-    return for_members(g, [&](int i) {
-        const size_t a = cut[i], b = cut[i + 1];
-        if (a >= b) return (int)KZGB_OK;
-        return kzgb_verify_blob_proofs(g->ctx[i], blobs + a, lens + a, b - a, commitments_xy + 8 * a,
-                                       commitments_inf ? commitments_inf + a : nullptr, proofs_xy + 8 * a,
-                                       proofs_inf ? proofs_inf + a : nullptr, ok + a);
+    return for_blob_shares(g, lens, count, [&](kzgb_ctx* c, size_t a, size_t n) {
+        return kzgb_verify_blob_proofs(c, blobs + a, lens + a, n, commitments_xy + 8 * a, at_or_null(commitments_inf, a),
+                                       proofs_xy + 8 * a, at_or_null(proofs_inf, a), ok + a);
     });
 }
 
@@ -294,13 +287,9 @@ int kzgb_group_verify_batch_rlc(kzgb_group* g, const uint8_t* const* blobs, cons
             while (n < (lens[i] + 31) / 32) n <<= 1;
             ns[i] = n;
         }
-        const std::vector<size_t> cut = byte_balanced_cut(lens, m, (int)g->ctx.size());
-        rc = for_members(g, [&](int i) {
-            const size_t a = cut[i], b = cut[i + 1];
-            if (a >= b) return (int)KZGB_OK;
-            return kzgb_verify_blob_proofs_g1(g->ctx[i], blobs + a, lens + a, b - a, commitments_xy + 8 * a,
-                                              commitments_inf ? commitments_inf + a : nullptr, proofs_xy + 8 * a,
-                                              proofs_inf ? proofs_inf + a : nullptr, nullptr, nullptr, &zs[4 * a], &ys[4 * a]);
+        rc = for_blob_shares(g, lens, m, [&](kzgb_ctx* c, size_t a, size_t n) {
+            return kzgb_verify_blob_proofs_g1(c, blobs + a, lens + a, n, commitments_xy + 8 * a, at_or_null(commitments_inf, a),
+                                              proofs_xy + 8 * a, at_or_null(proofs_inf, a), nullptr, nullptr, &zs[4 * a], &ys[4 * a]);
         });
         if (rc) return rc;
     }

@@ -315,4 +315,12 @@ def test_group_verify_blobs_equal_single_context(pkg, devices):
     assert grp.verify_blob_kzg_proofs_g1(_blobs(pkg, datas), cs, ps) == want
     assert grp.verify_blob_kzg_proofs_g1(_blobs(pkg, datas[:1]), cs[:1], ps[:1]) == want[:1]
     assert grp.verify_blob_kzg_proofs_g1([], [], []) == []
+    # out_xy == NULL, as the one-context call allows it: z and y only, every member writing its own share
+    _keep, ptrs, lens = pkg._blobs_to_abi(_blobs(pkg, datas))
+    cxy, cinf = pkg.g1_to_abi(cs)
+    pxy, pinf = pkg.g1_to_abi(ps)
+    z, y = C.create_string_buffer(32 * len(datas)), C.create_string_buffer(32 * len(datas))
+    grp.check(pkg.lib.kzgb_group_verify_blob_proofs_g1(grp.h, ptrs, lens, len(datas), cxy, cinf, pxy, pinf, None, None, z, y))
+    assert pkg.fr_from_mont_bytes(z.raw) == [w[1] for w in want]
+    assert pkg.fr_from_mont_bytes(y.raw) == [w[2] for w in want]
     grp.close()
