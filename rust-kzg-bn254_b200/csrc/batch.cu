@@ -311,24 +311,29 @@ HashStage::~HashStage() {
     sync.cv.notify_all();
     if (poller.joinable()) poller.join();
     for (auto& t : pool) t.join();
-    if (dev_k && c->hash_st) cudaStreamSynchronize(c->hash_st);
+    if (dev_k && c->hash_st) cudaStreamSynchronize(c->hash_st.get());
 }
 
 // The device's share: host blobs go up on the hashing stream, then one kernel hashes all of it.
 cudaError_t HashStage::start_device(bool lanes) {
     cudaError_t e = cudaSuccess;
-    if (!c->hash_st) {
+    if (!c->hash_st) {  // the stream, its event and the mapped block go into the context together or not at all
         int lo = 0, hi = 0;
         cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        e = cudaStreamCreateWithPriority(&c->hash_st, cudaStreamNonBlocking, hi);  // its few blocks must become resident at once
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&c->ev_hash_uploaded, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaHostAlloc((void**)&c->fsl_host, (9 * FSL_CAP + 16) * 4, cudaHostAllocMapped);
+        StreamPtr st;
+        EventPtr uploaded;
+        HostPtr<uint32_t[]> host;
+        e = stream_create(st, hi);  // its few blocks must become resident at once
+        if (e == cudaSuccess) e = event_create(uploaded, cudaEventDisableTiming);
+        if (e == cudaSuccess) e = host_alloc(host, (9 * FSL_CAP + 16) * 4, cudaHostAllocMapped);
+        if (e != cudaSuccess) return e;
+        c->hash_st = std::move(st); c->ev_hash_uploaded = std::move(uploaded); c->fsl_host = std::move(host);
     }
-    if (e == cudaSuccess) e = c->fsl_args.reserve(FSL_CAP * 16);
+    e = c->fsl_args.reserve(FSL_CAP * 16);
     if (e != cudaSuccess) return e;
-    fsl_state = c->fsl_host;
-    fsl_done = c->fsl_host + 8 * FSL_CAP;
-    fsl_cancel = c->fsl_host + 9 * FSL_CAP;
+    fsl_state = c->fsl_host.get();
+    fsl_done = fsl_state + 8 * FSL_CAP;
+    fsl_cancel = fsl_state + 9 * FSL_CAP;
     for (size_t j = 0; j < dev_k; j++) fsl_done[j] = 0;
     *fsl_cancel = 0;
     std::vector<const uint8_t*> ptrs(dev_k);
@@ -339,18 +344,18 @@ cudaError_t HashStage::start_device(bool lanes) {
         if (b.blobs_dev) ptrs[j] = b.blobs_dev[i];
         else {
             uint8_t* slot = (uint8_t*)c->batch_bytes.p + b.byte_off[i];
-            e = cudaMemcpyAsync(slot, b.blobs_host[i], b.lens[i], cudaMemcpyHostToDevice, c->hash_st);
+            e = cudaMemcpyAsync(slot, b.blobs_host[i], b.lens[i], cudaMemcpyHostToDevice, c->hash_st.get());
             ptrs[j] = slot;
         }
     }
     const uint8_t** d_ptrs = (const uint8_t**)c->fsl_args.p;
     uint32_t* d_ns = (uint32_t*)((char*)c->fsl_args.p + FSL_CAP * 8);
-    if (e == cudaSuccess) e = cudaEventRecord(c->ev_hash_uploaded, c->hash_st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_ptrs, ptrs.data(), dev_k * 8, cudaMemcpyHostToDevice, c->hash_st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_ns, ns.data(), dev_k * 4, cudaMemcpyHostToDevice, c->hash_st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->hash_st);  // the argument vectors die with this scope
+    if (e == cudaSuccess) e = cudaEventRecord(c->ev_hash_uploaded.get(), c->hash_st.get());
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_ptrs, ptrs.data(), dev_k * 8, cudaMemcpyHostToDevice, c->hash_st.get());
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_ns, ns.data(), dev_k * 4, cudaMemcpyHostToDevice, c->hash_st.get());
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->hash_st.get());  // the argument vectors die with this scope
     if (e != cudaSuccess) return e;
-    fs_midstate_long_launch(d_ptrs, d_ns, (uint32_t)dev_k, fsl_state, (uint32_t*)fsl_done, (const uint32_t*)fsl_cancel, lanes, c->hash_st);
+    fs_midstate_long_launch(d_ptrs, d_ns, (uint32_t)dev_k, fsl_state, (uint32_t*)fsl_done, (const uint32_t*)fsl_cancel, lanes, c->hash_st.get());
     return cudaGetLastError();
 }
 
@@ -511,7 +516,7 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
         const Fr* sc = (const Fr*)L.evals.p;
         if (!lag) {
             ck(cudaMemcpyAsync(L.work.p, L.evals.p, bn * n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st), "copy");
-            ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+            ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
             sc = (const Fr*)L.work.p;
         }
         if (!r) r = msm_enqueue(c, L, {sc}, n, bn, lag, nullptr, 0, &job);
@@ -541,9 +546,9 @@ int group_prove(const Batch& b, const HashStage& hs, Lane& L, size_t i0, size_t 
     }
     Fr* d_z = (Fr*)L.small.p;  // [z x bn | tinv x bn | y x bn]
     CK(c, cudaMemcpyAsync(d_z, zt.data(), 2 * bn * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-    eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)bn, d_z, d_z + bn, c->tw, c->logN, &ninv,
+    eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)bn, d_z, d_z + bn, c->tw.get(), c->logN, &ninv,
                          (Fr*)L.eval_scratch.p, (Fr*)L.work.p, d_z + 2 * bn, L.st, !any_in_domain);
-    if (!lag) ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+    if (!lag) ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
     MsmJob job;
     int r = msm_enqueue(c, L, {(const Fr*)L.work.p}, n, bn, lag, nullptr, 0, &job);
     if (!r) r = msm_finish(c, L, job, pts);
@@ -623,7 +628,7 @@ int device_blob(const Batch& b, const HashStage& hs, Lane& L, size_t i, bool wai
     *bytes = b.blobs_dev ? b.blobs_dev[i] : nullptr;
     if (*bytes || !hs.uploaded_here(i)) return KZGB_OK;
     *bytes = (const uint8_t*)c->batch_bytes.p + b.byte_off[i];
-    if (wait && cudaStreamWaitEvent(L.st, c->ev_hash_uploaded, 0) != cudaSuccess)
+    if (wait && cudaStreamWaitEvent(L.st, c->ev_hash_uploaded.get(), 0) != cudaSuccess)
         return fail(c, KZGB_ERR_DEVICE, "CUDA error: cudaStreamWaitEvent failed");
     return KZGB_OK;
 }
@@ -854,7 +859,7 @@ int blob_evals_stage(kzgb_ctx* c, Lane& L, const uint8_t* const* blobs_dev, cons
             CK(c, cudaMemcpyAsync(d_z, &zs[i0], b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
             CK(c, cudaMemcpyAsync(d_t, tinvs.data(), b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
         }
-        eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_z, d_t, c->tw, c->logN, &ninv,
+        eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)b, d_z, d_t, c->tw.get(), c->logN, &ninv,
                              (Fr*)L.eval_scratch.p, nullptr, d_y, L.st, !fs_device && !any_in_domain, d_in_domain);
         CK(c, cudaMemcpyAsync(&ys[i0], d_y, b * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
         rc = after_round(i0, b, (const Fr*)d_z, (const Fr*)d_y);
@@ -869,12 +874,10 @@ int blob_evals_stage(kzgb_ctx* c, Lane& L, const uint8_t* const* blobs_dev, cons
 // generator_window_table() on c's device, uploaded once
 int ensure_gen_table(kzgb_ctx* c) {
     if (c->gen_table) return KZGB_OK;
-    Affine* t = nullptr;
-    CK(c, cudaMalloc(&t, GEN_TABLE_POINTS * sizeof(Affine)));
-    const cudaError_t e = cudaMemcpy(t, generator_window_table(), GEN_TABLE_POINTS * sizeof(Affine), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) cudaFree(t);
-    CK(c, e);
-    c->gen_table = t;
+    DevPtr<Affine[]> t;
+    CK(c, dev_alloc(t, GEN_TABLE_POINTS * sizeof(Affine)));
+    CK(c, cudaMemcpy(t.get(), generator_window_table(), GEN_TABLE_POINTS * sizeof(Affine), cudaMemcpyHostToDevice));
+    c->gen_table = std::move(t);
     return KZGB_OK;
 }
 
@@ -917,12 +920,12 @@ int verify_blob_proofs(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8
     int rc = blob_evals_stage(c, L, blobs_dev, blobs_host, lens, ns, Cs, zs, ys,
                               [&](size_t i0, size_t b, const Fr* d_z, const Fr* d_y) {
         if (ok) {  // a round holds at most 65 535 blobs
-            const uint8_t* d_flags = pairing_check_launch(d_c + i0, d_c + count + i0, d_z, d_y, c->gen_table, c->pair_tab,
-                                                          L.pairing.p, (uint32_t)b, L.st);
+            const uint8_t* d_flags = pairing_check_launch(d_c + i0, d_c + count + i0, d_z, d_y, c->gen_table.get(),
+                                                          c->pair_tab.get(), L.pairing.p, (uint32_t)b, L.st);
             CK(c, cudaMemcpyAsync(&flags[i0], d_flags, b, cudaMemcpyDeviceToHost, L.st));
         }
         if (!out_xy) return (int)KZGB_OK;
-        commit_minus_value_launch(d_c + i0, d_y, c->gen_table, d_out + i0, (uint32_t)b, L.st);
+        commit_minus_value_launch(d_c + i0, d_y, c->gen_table.get(), d_out + i0, (uint32_t)b, L.st);
         CK(c, cudaMemcpyAsync(&outs[i0], d_out + i0, b * sizeof(Affine), cudaMemcpyDeviceToHost, L.st));
         return (int)KZGB_OK;
     });
@@ -1101,8 +1104,8 @@ int verify_proofs(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, const u
         Fr* d_zy = (Fr*)L.work.p;  // z then y
         CK(c, cudaMemcpyAsync(d_zy, zs_mont + 4 * i0, b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
         CK(c, cudaMemcpyAsync(d_zy + b, ys_mont + 4 * i0, b * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-        const uint8_t* d_flags = pairing_check_launch(d_bases + i0, d_bases + m + i0, d_zy, d_zy + b, c->gen_table,
-                                                      c->pair_tab, L.pairing.p, (uint32_t)b, L.st);
+        const uint8_t* d_flags = pairing_check_launch(d_bases + i0, d_bases + m + i0, d_zy, d_zy + b, c->gen_table.get(),
+                                                      c->pair_tab.get(), L.pairing.p, (uint32_t)b, L.st);
         CK(c, cudaMemcpyAsync(&flags[i0], d_flags, b, cudaMemcpyDeviceToHost, L.st));
         CK(c, cudaStreamSynchronize(L.st));
         CK(c, cudaGetLastError());

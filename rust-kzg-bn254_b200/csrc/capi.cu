@@ -13,6 +13,7 @@
 #include <cstring>
 #include <ctime>
 #include <mutex>
+#include <new>
 #include <string>
 #include <thread>
 #include <vector>
@@ -152,52 +153,36 @@ int choose_c_fixed(size_t n) {
 }
 
 // ---------------------------------------------------------------- lanes
-int lane_init(kzgb_ctx* c, Lane& L, cudaStream_t st) {
-    if (st) { L.st = st; L.own_stream = false; }
-    else {
+// Appends a lane on the caller's stream st, or on streams of its own when st is null.  The lane is built aside and
+// installed only once every part of it exists; on failure what was built is freed and the context is unchanged.
+int lane_init(kzgb_ctx* c, cudaStream_t st) {
+    Lane L;
+    L.st = st;
+    if (!st) {
         int lo = 0, hi = 0;
         CK(c, cudaDeviceGetStreamPriorityRange(&lo, &hi));  // numerically lower = higher priority
-        CK(c, cudaStreamCreateWithPriority(&L.st, cudaStreamNonBlocking, hi));
-        L.own_stream = true;
+        CK(c, stream_create(L.own_st, hi));
+        L.st = L.own_st.get();
         if (g_stream_priority.load() && lo != hi) {
-            CK(c, cudaStreamCreateWithPriority(&L.st_acc, cudaStreamNonBlocking, lo));
-            CK(c, cudaEventCreateWithFlags(&L.ev_fork, cudaEventDisableTiming));
-            CK(c, cudaEventCreateWithFlags(&L.ev_join, cudaEventDisableTiming));
+            CK(c, stream_create(L.st_acc, lo));
+            CK(c, event_create(L.ev_fork, cudaEventDisableTiming));
+            CK(c, event_create(L.ev_join, cudaEventDisableTiming));
         }
     }
-    CK(c, cudaMallocHost((void**)&L.h_sets, sizeof(XYZZ) * MAX_SETS));
-    CK(c, cudaMallocHost((void**)&L.h_fr, sizeof(Fr) * 16));
-    CK(c, cudaMallocHost((void**)&L.h_entries, 16));
-    CK(c, cudaEventCreate(&L.ev0));
-    CK(c, cudaEventCreate(&L.ev1));
-    CK(c, cudaEventCreateWithFlags(&L.ev_done, cudaEventDisableTiming));
-    CK(c, cudaEventCreateWithFlags(&L.ev_block, cudaEventDisableTiming | cudaEventBlockingSync));
+    CK(c, host_alloc(L.h_sets, sizeof(XYZZ) * MAX_SETS));
+    CK(c, host_alloc(L.h_fr, sizeof(Fr) * 16));
+    CK(c, host_alloc(L.h_entries, 16));
+    CK(c, event_create(L.ev0));
+    CK(c, event_create(L.ev1));
+    CK(c, event_create(L.ev_done, cudaEventDisableTiming));
+    CK(c, event_create(L.ev_block, cudaEventDisableTiming | cudaEventBlockingSync));
+    c->lanes[c->n_lanes++] = std::move(L);
     return KZGB_OK;
-}
-void lane_destroy(Lane& L) {
-    L.bytes.release(); L.evals.release(); L.work.release(); L.ntt_scratch.release();
-    L.eval_scratch.release(); L.msm_ws.release(); L.small.release(); L.bases.release(); L.bucket_total.release();
-    L.pairing.release();
-    if (L.h_sets) cudaFreeHost(L.h_sets);
-    if (L.h_fr) cudaFreeHost(L.h_fr);
-    if (L.h_entries) cudaFreeHost(L.h_entries);
-    if (L.ev0) cudaEventDestroy(L.ev0);
-    if (L.ev1) cudaEventDestroy(L.ev1);
-    if (L.ev_done) cudaEventDestroy(L.ev_done);
-    if (L.ev_block) cudaEventDestroy(L.ev_block);
-    if (L.ev_fork) cudaEventDestroy(L.ev_fork);
-    if (L.ev_join) cudaEventDestroy(L.ev_join);
-    if (L.st_acc) cudaStreamDestroy(L.st_acc);
-    if (L.own_stream && L.st) cudaStreamDestroy(L.st);
-    L = Lane();
 }
 int ensure_lanes(kzgb_ctx* c, int want) {
     if (want > MAX_LANES) want = MAX_LANES;
-    while (c->n_lanes < want) {
-        int rc = lane_init(c, c->lanes[c->n_lanes], nullptr);
-        if (rc) return rc;
-        c->n_lanes++;
-    }
+    while (c->n_lanes < want)
+        if (int rc = lane_init(c, nullptr)) return rc;
     return KZGB_OK;
 }
 cudaError_t drain_lanes(kzgb_ctx* c) {  // waits for every lane's stream, up to the first error
@@ -209,7 +194,7 @@ cudaError_t drain_lanes(kzgb_ctx* c) {  // waits for every lane's stream, up to 
 void lane_collect_acc(Lane& L) {
     if (L.ev_pending) {
         float ms = 0;
-        if (cudaEventElapsedTime(&ms, L.ev0, L.ev1) == cudaSuccess) { L.acc_ms += ms; L.acc_launches++; L.acc_adds += *L.h_entries; }
+        if (cudaEventElapsedTime(&ms, L.ev0.get(), L.ev1.get()) == cudaSuccess) { L.acc_ms += ms; L.acc_launches++; L.acc_adds += *L.h_entries; }
         L.ev_pending = false;
     }
 }
@@ -220,21 +205,21 @@ void lane_collect_acc(Lane& L) {
 int lane_index(kzgb_ctx* c, const Lane& L) { return (int)(&L - &c->lanes[0]); }
 cudaEvent_t trace_mark(kzgb_ctx* c, const Lane& L, int kind, cudaStream_t st) {
     if (!c->trace_on.load()) return nullptr;
-    cudaEvent_t ev = nullptr;
-    if (st) { if (cudaEventCreate(&ev) != cudaSuccess) return nullptr; cudaEventRecord(ev, st); }
+    EventPtr ev;
+    if (st) { if (event_create(ev) != cudaSuccess) return nullptr; cudaEventRecord(ev.get(), st); }
     double host = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - c->trace_host0).count();
     std::lock_guard<std::mutex> lk(c->trace_mu);
-    c->trace.push_back({lane_index(c, L), kind, ev, host});
-    return ev;
+    c->trace.push_back({lane_index(c, L), kind, std::move(ev), host});
+    return c->trace.back().ev.get();
 }
 // an event the caller records itself (accumulate begin / end inside msm_launch_buckets)
 cudaEvent_t trace_event(kzgb_ctx* c, const Lane& L, int kind) {
     if (!c->trace_on.load()) return nullptr;
-    cudaEvent_t ev = nullptr;
-    if (cudaEventCreate(&ev) != cudaSuccess) return nullptr;
+    EventPtr ev;
+    if (event_create(ev) != cudaSuccess) return nullptr;
     std::lock_guard<std::mutex> lk(c->trace_mu);
-    c->trace.push_back({lane_index(c, L), kind, ev, -1.0});
-    return ev;
+    c->trace.push_back({lane_index(c, L), kind, std::move(ev), -1.0});
+    return c->trace.back().ev.get();
 }
 
 // ---------------------------------------------------------------- twiddles
@@ -244,10 +229,10 @@ int ensure_twiddles(kzgb_ctx* c, int logn) {
     if (c->srs_n) want = std::max(want, log2_exact(next_pow2(c->srs_n)) > 28 ? 28 : log2_exact(next_pow2(c->srs_n)));
     if (want > 28) return fail(c, KZGB_ERR_GENERIC, "power must be <= 28");
     CK(c, drain_lanes(c));
-    if (c->tw) { cudaFree(c->tw); c->tw = nullptr; }
-    CK(c, cudaMalloc((void**)&c->tw, sizeof(Fr) * ((size_t)1 << (want - 1))));
+    c->tw.reset();
+    CK(c, dev_alloc(c->tw, sizeof(Fr) * ((size_t)1 << (want - 1))));
     Fr w = root_of_unity_mont(want);
-    ntt_twiddles_launch(c->tw, want, &w, c->lanes[0].st);
+    ntt_twiddles_launch(c->tw.get(), want, &w, c->lanes[0].st);
     CK(c, cudaStreamSynchronize(c->lanes[0].st));
     c->logN = want;
     return KZGB_OK;
@@ -262,8 +247,9 @@ int check_table_fits(kzgb_ctx* c, size_t bytes, size_t reusable) {
         return fail(c, KZGB_ERR_DEVICE, "not enough device memory for the fixed-base window tables");
     return KZGB_OK;
 }
-// Window table over `points` (n affine points on the device): table[w*n + i] = 2^(c*w) * points[i].
-int build_window_table(kzgb_ctx* c, const Affine* points, size_t n, int cb, Affine** out, int* W_out) {
+// Window table over `points` (n affine points on the device): table[w*n + i] = 2^(c*w) * points[i].  *out (empty) gets the
+// table only on success.
+int build_window_table(kzgb_ctx* c, const Affine* points, size_t n, int cb, DevPtr<Affine[]>* out, int* W_out) {
     if (cb < 2 || cb > 24) return fail(c, KZGB_ERR_GENERIC, "window_bits out of range");
     int W = window_count(cb);
     if ((uint64_t)W * n >= ((uint64_t)1 << 31))  // sorted refs are 31 bits + sign (msm.cu k_scatter)
@@ -271,20 +257,19 @@ int build_window_table(kzgb_ctx* c, const Affine* points, size_t n, int cb, Affi
     size_t bytes = (size_t)W * n * sizeof(Affine);
     if (int rc = check_table_fits(c, bytes, 0)) return rc;
     Lane& L = c->lanes[0];
-    Affine* table = nullptr;
-    CK(c, cudaMalloc((void**)&table, bytes));
-    cudaError_t e = cudaMemcpyAsync(table, points, n * sizeof(Affine), cudaMemcpyDeviceToDevice, L.st);
+    DevPtr<Affine[]> table;
+    CK(c, dev_alloc(table, bytes));
+    cudaError_t e = cudaMemcpyAsync(table.get(), points, n * sizeof(Affine), cudaMemcpyDeviceToDevice, L.st);
     uint32_t batch = (uint32_t)std::min<size_t>(n, (size_t)1 << 18);
     DevBuf scratch;
     if (e == cudaSuccess) e = scratch.reserve(srs_precompute_scratch_bytes(batch, W));
     if (e == cudaSuccess) {
-        srs_precompute_launch(table, (uint32_t)n, (uint32_t)n, cb, W, (XYZZ*)scratch.p, batch, L.st);
+        srs_precompute_launch(table.get(), (uint32_t)n, (uint32_t)n, cb, W, (XYZZ*)scratch.p, batch, L.st);
         e = cudaStreamSynchronize(L.st);
     }
-    scratch.release();
     if (e == cudaSuccess) e = cudaGetLastError();
-    if (e != cudaSuccess) { cudaFree(table); CK(c, e); }
-    *out = table; *W_out = W;
+    CK(c, e);
+    *out = std::move(table); *W_out = W;
     return KZGB_OK;
 }
 
@@ -300,16 +285,15 @@ int do_precompute(kzgb_ctx* c, size_t first, size_t count, int window_bits) {
     size_t reusable = c->wtable ? (size_t)c->wt_W * c->wt_n * sizeof(Affine) : 0;
     if (int rc = check_table_fits(c, (size_t)window_count(cb) * count * sizeof(Affine), reusable)) return rc;
     drop_window_table(c);
-    Affine* table = nullptr;
     int W = 0;
-    int rc = build_window_table(c, c->srs + first, count, cb, &table, &W);
+    int rc = build_window_table(c, c->srs.get() + first, count, cb, &c->wtable, &W);
     if (rc) return rc;
-    c->wtable = table; c->wt_first = first; c->wt_n = count; c->wt_c = cb; c->wt_W = W;
+    c->wt_first = first; c->wt_n = count; c->wt_c = cb; c->wt_W = W;
     return KZGB_OK;
 }
 
 void drop_window_table(kzgb_ctx* c) {
-    if (c->wtable) { cudaFree(c->wtable); c->wtable = nullptr; c->wt_n = 0; c->wt_first = 0; }
+    c->wtable.reset(); c->wt_n = 0; c->wt_first = 0;
 }
 bool wtable_covers(const kzgb_ctx* c, size_t first, size_t n) { return c->wtable && first >= c->wt_first && first + n <= c->wt_first + c->wt_n; }
 // Lazy build of the monomial window table over [0, next_pow2(first + n)) when none covers [first, first + n); SRS above
@@ -318,10 +302,6 @@ int ensure_window_table(kzgb_ctx* c, size_t first, size_t n) {
     if (!c->auto_precompute || wtable_covers(c, first, n) || c->srs_n > ((size_t)1 << 22)) return KZGB_OK;
     int rc = do_precompute(c, 0, std::min(c->srs_n, next_pow2(first + n)), 0);
     return rc == KZGB_ERR_DEVICE ? KZGB_OK : rc;
-}
-
-void lagrange_release(kzgb_ctx* c) {
-    for (auto& t : c->lag) { if (t.table) cudaFree(t.table); t = kzgb_ctx::LagTable(); }
 }
 
 // Lagrange-basis window table for the domain of size n = 2^logn: L = IFFT_G1(SRS[..n]) (the points
@@ -364,8 +344,7 @@ int ensure_lagrange(kzgb_ctx* c, int logn, uint32_t weight, bool force) {
             }
             if (held + need <= budget || !lru) break;
             CK(c, drain_lanes(c));
-            cudaFree(lru->table);
-            lru->table = nullptr; lru->n = 0; lru->calls = 0;
+            lru->table.reset(); lru->n = 0; lru->calls = 0;
         }
     }
     int rc = ensure_twiddles(c, logn);
@@ -374,22 +353,20 @@ int ensure_lagrange(kzgb_ctx* c, int logn, uint32_t weight, bool force) {
     Lane& L = c->lanes[0];
     DevBuf work, pts;
     if (work.reserve(n * sizeof(XYZZ)) != cudaSuccess || pts.reserve(n * sizeof(Affine)) != cudaSuccess) {
-        cudaGetLastError(); work.release(); pts.release();
+        cudaGetLastError();
         return KZGB_OK;
     }
     Fr ninv = ninv_mont(logn), ninv_canon;
     fe_from_mont(ninv_canon, ninv);
-    g1_intt_launch(c->srs, logn, (XYZZ*)work.p, (Affine*)pts.p, c->tw, c->logN, &ninv_canon, L.st);
+    g1_intt_launch(c->srs.get(), logn, (XYZZ*)work.p, (Affine*)pts.p, c->tw.get(), c->logN, &ninv_canon, L.st);
     cudaError_t e = cudaStreamSynchronize(L.st);
-    work.release();
-    if (e != cudaSuccess) { pts.release(); CK(c, e); }
-    Affine* table = nullptr;
+    work.release();  // before the table is sized against the free memory
+    CK(c, e);
     int W = 0, cb = cb_plan;  // an explicit window override of the monomial table carries over
-    rc = build_window_table(c, (const Affine*)pts.p, n, cb, &table, &W);
-    pts.release();
+    rc = build_window_table(c, (const Affine*)pts.p, n, cb, &t.table, &W);
     if (rc == KZGB_ERR_DEVICE) { cudaGetLastError(); return KZGB_OK; }  // short of memory: stay on the monomial path
     if (rc) return rc;
-    t.table = table; t.n = n; t.c = cb; t.W = W;
+    t.n = n; t.c = cb; t.W = W;
     return KZGB_OK;
 }
 
@@ -399,10 +376,6 @@ const kzgb_ctx::LagTable* lagrange_table(const kzgb_ctx* c, int logn) {
 }
 
 // ---------------------------------------------------------------- proofs at every root: the s_hat tables (allroots.cu)
-void allroots_release(kzgb_ctx* c) {
-    for (auto& t : c->allroots) { if (t) cudaFree(t); t = nullptr; }
-}
-
 // Canonical 1: g1_ntt_finish_launch converts to affine without scaling.
 Fr fr_one_canon() { Fr one; fe_zero(one); one.l[0] = 1; return one; }
 
@@ -410,8 +383,8 @@ Fr fr_one_canon() { Fr one; fe_zero(one); one.l[0] = 1; return one; }
 // The twiddles of size 2n must be resident.
 void allroots_shat_launch(kzgb_ctx* c, int logn, XYZZ* work, Affine* out, cudaStream_t st) {
     const Fr one = fr_one_canon();
-    allroots_embed_launch(c->srs, logn, work, st);
-    g1_ntt_stages_launch(work, logn + 1, false, c->tw, c->logN, st);
+    allroots_embed_launch(c->srs.get(), logn, work, st);
+    g1_ntt_stages_launch(work, logn + 1, false, c->tw.get(), c->logN, st);
     g1_ntt_finish_launch(work, out, logn + 1, &one, st);
 }
 
@@ -426,25 +399,24 @@ int ensure_allroots(kzgb_ctx* c, int logn, const Affine** out) {
         Lane& L = c->lanes[0];
         const size_t m = (size_t)2 << logn;
         CK(c, L.work.reserve(m * sizeof(XYZZ)));
-        Affine* table = nullptr;
-        CK(c, cudaMalloc((void**)&table, m * sizeof(Affine)));
-        allroots_shat_launch(c, logn, (XYZZ*)L.work.p, table, L.st);
+        DevPtr<Affine[]> table;
+        CK(c, dev_alloc(table, m * sizeof(Affine)));
+        allroots_shat_launch(c, logn, (XYZZ*)L.work.p, table.get(), L.st);
         cudaError_t e = cudaStreamSynchronize(L.st);
         if (e == cudaSuccess) e = cudaGetLastError();
-        if (e != cudaSuccess) { cudaFree(table); CK(c, e); }
-        c->allroots[logn] = table;
+        CK(c, e);
+        c->allroots[logn] = std::move(table);
     }
-    *out = c->allroots[logn];
+    *out = c->allroots[logn].get();
     return KZGB_OK;
 }
 
-int srs_install(kzgb_ctx* c, Affine* dev_points, size_t n) {
+int srs_install(kzgb_ctx* c, DevPtr<Affine[]> dev_points, size_t n) {
     drain_lanes(c);
-    if (c->srs) cudaFree(c->srs);
     drop_window_table(c);
-    lagrange_release(c);
-    allroots_release(c);
-    c->srs = dev_points;
+    for (auto& t : c->lag) t = {};
+    for (auto& t : c->allroots) t.reset();
+    c->srs = std::move(dev_points);
     c->srs_n = n;
     return KZGB_OK;
 }
@@ -463,12 +435,12 @@ int msm_enqueue(kzgb_ctx* c, Lane& L, const MsmScalars& scalars, size_t n, size_
     int cb = 0;
     size_t stride = 0, offset = 0;
     if (lag) {
-        table = lag->table; cb = lag->c; stride = lag->n;
+        table = lag->table.get(); cb = lag->c; stride = lag->n;
     } else if (!var_bases) {
         if (first > c->srs_n || n > c->srs_n - first) return fail(c, KZGB_ERR_GENERIC, "MSM range exceeds the SRS");
         if (batch == 1 && !c->lanes_running.load())
             if (int rc = ensure_window_table(c, first, n)) return rc;
-        if (wtable_covers(c, first, n)) { table = c->wtable; cb = c->wt_c; stride = c->wt_n; offset = first - c->wt_first; }
+        if (wtable_covers(c, first, n)) { table = c->wtable.get(); cb = c->wt_c; stride = c->wt_n; offset = first - c->wt_first; }
     }
     MsmPlan p;
     if (table) {
@@ -476,7 +448,7 @@ int msm_enqueue(kzgb_ctx* c, Lane& L, const MsmScalars& scalars, size_t n, size_
     } else {
         if (batch > 1) return fail(c, KZGB_ERR_GENERIC, "batched MSM needs a fixed-base table");
         p = msm_make_plan((uint32_t)n, choose_c_var(n), false, 0, 0);
-        table = var_bases ? var_bases : c->srs + first;
+        table = var_bases ? var_bases : c->srs.get() + first;
     }
     if ((uint64_t)n * batch * p.W >= 0xfff00000ull) return fail(c, KZGB_ERR_GENERIC, "MSM too large for one launch");
     CK(c, L.msm_ws.reserve(msm_workspace_bytes(p)));
@@ -485,13 +457,14 @@ int msm_enqueue(kzgb_ctx* c, Lane& L, const MsmScalars& scalars, size_t n, size_
     lane_collect_acc(L);
     trace_mark(c, L, 0, L.st);
     cudaEvent_t tr1 = trace_event(c, L, 1), tr2 = trace_event(c, L, 2);
-    msm_launch_buckets(p, ws, scalars, table, {L.st, L.st_acc, L.ev_fork, L.ev_join, tr1 ? tr1 : L.ev0, tr2 ? tr2 : L.ev1});
+    msm_launch_buckets(p, ws, scalars, table,
+                       {L.st, L.st_acc.get(), L.ev_fork.get(), L.ev_join.get(), tr1 ? tr1 : L.ev0.get(), tr2 ? tr2 : L.ev1.get()});
     msm_launch_reduce(p, ws, ws.buckets, L.st);
     trace_mark(c, L, 3, L.st);
     trace_mark(c, L, 10, nullptr);
     L.ev_pending = !tr1;
-    CK(c, cudaMemcpyAsync(L.h_entries, ws.hist + p.nbuckets, 4, cudaMemcpyDeviceToHost, L.st));
-    CK(c, cudaMemcpyAsync(L.h_sets, ws.set_sums, sizeof(XYZZ) * p.sets, cudaMemcpyDeviceToHost, L.st));
+    CK(c, cudaMemcpyAsync(L.h_entries.get(), ws.hist + p.nbuckets, 4, cudaMemcpyDeviceToHost, L.st));
+    CK(c, cudaMemcpyAsync(L.h_sets.get(), ws.set_sums, sizeof(XYZZ) * p.sets, cudaMemcpyDeviceToHost, L.st));
     job->plan = p;
     job->active = true;
     return KZGB_OK;
@@ -519,12 +492,12 @@ bool lane_wait_polls() { return lane_wait_mode() != 0; }
 int lane_wait(kzgb_ctx* c, Lane& L) {
     const int mode = (g_lane_wait.load() < 0 && c->lanes_block.load()) ? 2 : lane_wait_mode();
     if (mode == 2) {  // sleep in the driver until the GPU's interrupt: no CPU at all while waiting
-        CK(c, cudaEventRecord(L.ev_block, L.st));
-        CK(c, cudaEventSynchronize(L.ev_block));
+        CK(c, cudaEventRecord(L.ev_block.get(), L.st));
+        CK(c, cudaEventSynchronize(L.ev_block.get()));
     } else if (mode == 1) {
-        CK(c, cudaEventRecord(L.ev_done, L.st));
+        CK(c, cudaEventRecord(L.ev_done.get(), L.st));
         for (;;) {
-            cudaError_t q = cudaEventQuery(L.ev_done);
+            cudaError_t q = cudaEventQuery(L.ev_done.get());
             if (q == cudaSuccess) break;
             if (q != cudaErrorNotReady) CK(c, q);
             struct timespec ts = {0, 30000};
@@ -578,12 +551,16 @@ int msm_srs_host_pipelined(kzgb_ctx* c, Lane& L, const uint64_t* scalars, size_t
     const size_t S = n >= ((size_t)1 << 24) ? 8 : 4;
     const size_t per = ((n + S - 1) / S + 31) & ~(size_t)31;
     if ((uint64_t)per * window_count(c->wt_c) >= 0xfff00000ull) return KZGB_OK;
-    if (!c->copy_st) {
-        CK(c, cudaStreamCreateWithFlags(&c->copy_st, cudaStreamNonBlocking));
+    if (!c->copy_st) {  // the stream and its four events go into the context together or not at all
+        StreamPtr st;
+        EventPtr copied[2], consumed[2];
+        CK(c, stream_create(st, 0));
         for (int k = 0; k < 2; k++) {
-            CK(c, cudaEventCreateWithFlags(&c->ev_copied[k], cudaEventDisableTiming));
-            CK(c, cudaEventCreateWithFlags(&c->ev_consumed[k], cudaEventDisableTiming));
+            CK(c, event_create(copied[k], cudaEventDisableTiming));
+            CK(c, event_create(consumed[k], cudaEventDisableTiming));
         }
+        c->copy_st = std::move(st);
+        for (int k = 0; k < 2; k++) { c->ev_copied[k] = std::move(copied[k]); c->ev_consumed[k] = std::move(consumed[k]); }
     }
     const MsmPlan p0 = msm_make_plan((uint32_t)per, c->wt_c, true, (uint32_t)c->wt_n, (uint32_t)(first - c->wt_first));
     CK(c, L.msm_ws.reserve(msm_workspace_bytes(p0)));
@@ -593,24 +570,24 @@ int msm_srs_host_pipelined(kzgb_ctx* c, Lane& L, const uint64_t* scalars, size_t
     msm_workspace_carve(p0, L.msm_ws.p, &ws);
     Fr* stage[2] = {(Fr*)L.work.p, (Fr*)L.work.p + per};
     XYZZ* total = (XYZZ*)L.bucket_total.p;
-    CK(c, cudaEventRecord(c->ev_consumed[0], L.st));  // the staging buffers are free once earlier work on the lane is done
-    CK(c, cudaEventRecord(c->ev_consumed[1], L.st));
+    CK(c, cudaEventRecord(c->ev_consumed[0].get(), L.st));  // the staging buffers are free once earlier work on the lane is done
+    CK(c, cudaEventRecord(c->ev_consumed[1].get(), L.st));
     size_t k = 0;
     for (size_t off = 0; off < n; off += per, k++) {
         const size_t cnt = std::min(per, n - off);
         const int b = (int)(k & 1);
-        CK(c, cudaStreamWaitEvent(c->copy_st, c->ev_consumed[b], 0));
-        CK(c, cudaMemcpyAsync(stage[b], scalars + 4 * off, cnt * sizeof(Fr), cudaMemcpyHostToDevice, c->copy_st));
-        CK(c, cudaEventRecord(c->ev_copied[b], c->copy_st));
-        CK(c, cudaStreamWaitEvent(L.st, c->ev_copied[b], 0));
+        CK(c, cudaStreamWaitEvent(c->copy_st.get(), c->ev_consumed[b].get(), 0));
+        CK(c, cudaMemcpyAsync(stage[b], scalars + 4 * off, cnt * sizeof(Fr), cudaMemcpyHostToDevice, c->copy_st.get()));
+        CK(c, cudaEventRecord(c->ev_copied[b].get(), c->copy_st.get()));
+        CK(c, cudaStreamWaitEvent(L.st, c->ev_copied[b].get(), 0));
         const MsmPlan p = msm_make_plan((uint32_t)cnt, c->wt_c, true, (uint32_t)c->wt_n, (uint32_t)(first + off - c->wt_first));
-        msm_launch_buckets(p, ws, {stage[b]}, c->wtable, {L.st, L.st_acc, L.ev_fork, L.ev_join});
-        CK(c, cudaEventRecord(c->ev_consumed[b], L.st));
+        msm_launch_buckets(p, ws, {stage[b]}, c->wtable.get(), {L.st, L.st_acc.get(), L.ev_fork.get(), L.ev_join.get()});
+        CK(c, cudaEventRecord(c->ev_consumed[b].get(), L.st));
         if (k == 0) CK(c, cudaMemcpyAsync(total, ws.buckets, (size_t)p0.nbuckets * sizeof(XYZZ), cudaMemcpyDeviceToDevice, L.st));
         else msm_merge_buckets(total, ws.buckets, p0.nbuckets, L.st);
     }
     msm_launch_reduce(p0, ws, total, L.st);
-    CK(c, cudaMemcpyAsync(L.h_sets, ws.set_sums, sizeof(XYZZ), cudaMemcpyDeviceToHost, L.st));
+    CK(c, cudaMemcpyAsync(L.h_sets.get(), ws.set_sums, sizeof(XYZZ), cudaMemcpyDeviceToHost, L.st));
     { int rc = lane_wait(c, L); if (rc) return rc; }
     xyzz_to_affine(*out, L.h_sets[0]);
     *done = true;
@@ -630,7 +607,7 @@ int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJ
     if ((const void*)d_evals != L.work.p)
         CK(c, cudaMemcpyAsync(L.work.p, d_evals, n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st));
     Fr ninv = ninv_mont(logn);
-    ntt_launch((Fr*)L.work.p, logn, 1, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+    ntt_launch((Fr*)L.work.p, logn, 1, true, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
     return msm_enqueue(c, L, {(Fr*)L.work.p}, n, 1, nullptr, nullptr, 0, job);
 }
 
@@ -645,7 +622,7 @@ int eval_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z,
     L.h_fr[1] = eval_tinv(z, logn, &in_domain);
     CK(c, cudaMemcpyAsync(d_z, &L.h_fr[0], 2 * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
     Fr ninv = ninv_mont(logn);
-    eval_quotient_launch(d_evals, (uint32_t)n, logn, 1, d_z, d_z + 1, c->tw, c->logN, &ninv, (Fr*)L.eval_scratch.p,
+    eval_quotient_launch(d_evals, (uint32_t)n, logn, 1, d_z, d_z + 1, c->tw.get(), c->logN, &ninv, (Fr*)L.eval_scratch.p,
                          d_quotient, d_z + 2, L.st, !in_domain);
     return KZGB_OK;
 }
@@ -716,31 +693,23 @@ int srs_ingest_stream(kzgb_ctx* c, size_t n, bool raw, Reader read) {
     size_t chunk = (size_t)g_srs_chunk.load();
     if (chunk == 0) chunk = (size_t)1 << 22;
     chunk = std::min(chunk, n);
-    uint8_t* pin[2] = {nullptr, nullptr};
-    cudaEvent_t ev[2] = {nullptr, nullptr};
+    const size_t n_chunks = (n + chunk - 1) / chunk;
+    const bool pinned = n_chunks > 1;  // a single chunk has nothing to overlap with: skip the (slow) pinned allocation
+    HostPtr<uint8_t[]> pin[2];
+    std::unique_ptr<uint8_t[]> unpinned(pinned ? nullptr : new (std::nothrow) uint8_t[chunk * unit]);
+    EventPtr ev[2];
     DevBuf stage[2], errb;
-    Affine* pts = nullptr;
+    DevPtr<Affine[]> pts;
     int rc = KZGB_OK;
-    bool pinned = true;
-    auto cleanup = [&]() {
-        for (int k = 0; k < 2; k++) {
-            if (pin[k]) { if (pinned) cudaFreeHost(pin[k]); else free(pin[k]); }
-            if (ev[k]) cudaEventDestroy(ev[k]);
-            stage[k].release();
-        }
-        errb.release();
-    };
     auto ck = [&](cudaError_t e, const char* what) {
         if (!rc && e != cudaSuccess) rc = fail(c, KZGB_ERR_DEVICE, std::string("CUDA error: ") + cudaGetErrorString(e) + " at " + what);
     };
-    const size_t n_chunks = (n + chunk - 1) / chunk;
-    pinned = n_chunks > 1;  // a single chunk has nothing to overlap with: skip the (slow) pinned allocation
-    ck(cudaMalloc((void**)&pts, n * sizeof(Affine)), "cudaMalloc(SRS points)");
+    ck(dev_alloc(pts, n * sizeof(Affine)), "cudaMalloc(SRS points)");
     ck(errb.reserve(4 * n_chunks), "cudaMalloc");
     for (int k = 0; k < (pinned ? 2 : 1) && !rc; k++) {
-        if (pinned) ck(cudaMallocHost((void**)&pin[k], chunk * unit), "cudaMallocHost(staging)");
-        else if (!(pin[k] = (uint8_t*)malloc(chunk * unit))) rc = fail(c, KZGB_ERR_GENERIC, "out of host memory");
-        ck(cudaEventCreateWithFlags(&ev[k], cudaEventDisableTiming), "cudaEventCreate");
+        if (pinned) ck(host_alloc(pin[k], chunk * unit), "cudaMallocHost(staging)");
+        else if (!unpinned) rc = fail(c, KZGB_ERR_GENERIC, "out of host memory");
+        ck(event_create(ev[k], cudaEventDisableTiming), "cudaEventCreate");
         if (!raw) ck(stage[k].reserve(chunk * unit), "cudaMalloc(staging)");
     }
     std::vector<uint32_t> herr(n_chunks, 0xffffffffu);
@@ -749,17 +718,18 @@ int srs_ingest_stream(kzgb_ctx* c, size_t n, bool raw, Reader read) {
     for (size_t k = 0; k < n_chunks && !rc; k++) {
         const size_t first = k * chunk, count = std::min(chunk, n - first);
         const int b = (int)(k & 1);
-        if (k >= 2) ck(cudaEventSynchronize(ev[b]), "cudaEventSynchronize");  // staging buffer free again
+        if (k >= 2) ck(cudaEventSynchronize(ev[b].get()), "cudaEventSynchronize");  // staging buffer free again
         if (rc) break;
-        if (!read(pin[b], first, count)) { rc = fail(c, KZGB_ERR_GENERIC, "Failed to read G1 points: file shorter than points_to_load"); break; }
+        uint8_t* const buf = pinned ? pin[b].get() : unpinned.get();
+        if (!read(buf, first, count)) { rc = fail(c, KZGB_ERR_GENERIC, "Failed to read G1 points: file shorter than points_to_load"); break; }
         if (raw) {
-            ck(cudaMemcpyAsync(pts + first, pin[b], count * unit, cudaMemcpyHostToDevice, L.st), "H2D copy of SRS points");
-            g1_validate_launch(pts + first, (uint32_t)count, d_err + k, L.st);
+            ck(cudaMemcpyAsync(pts.get() + first, buf, count * unit, cudaMemcpyHostToDevice, L.st), "H2D copy of SRS points");
+            g1_validate_launch(pts.get() + first, (uint32_t)count, d_err + k, L.st);
         } else {
-            ck(cudaMemcpyAsync(stage[b].p, pin[b], count * unit, cudaMemcpyHostToDevice, L.st), "H2D copy of SRS points");
-            srs_decompress_launch((const uint8_t*)stage[b].p, (uint32_t)count, pts + first, d_err + k, L.st);
+            ck(cudaMemcpyAsync(stage[b].p, buf, count * unit, cudaMemcpyHostToDevice, L.st), "H2D copy of SRS points");
+            srs_decompress_launch((const uint8_t*)stage[b].p, (uint32_t)count, pts.get() + first, d_err + k, L.st);
         }
-        ck(cudaEventRecord(ev[b], L.st), "cudaEventRecord");
+        ck(cudaEventRecord(ev[b].get(), L.st), "cudaEventRecord");
     }
     if (!rc) ck(cudaMemcpyAsync(herr.data(), d_err, 4 * n_chunks, cudaMemcpyDeviceToHost, L.st), "D2H");
     ck(cudaStreamSynchronize(L.st), "sync");
@@ -778,9 +748,8 @@ int srs_ingest_stream(kzgb_ctx* c, size_t n, bool raw, Reader read) {
             rc = fail(c, KZGB_ERR_NOT_ON_CURVE, msg);
         }
     }
-    cleanup();
-    if (rc) { if (pts) cudaFree(pts); return rc; }
-    return srs_install(c, pts, n);
+    if (rc) return rc;
+    return srs_install(c, std::move(pts), n);
 }
 
 }  // namespace
@@ -798,45 +767,26 @@ int kzgb_ctx_create(kzgb_ctx** out, int device, void* stream) {
     int prev = 0;
     cudaGetDevice(&prev);
     if (cudaSetDevice(device) != cudaSuccess) { delete c; return KZGB_ERR_DEVICE; }
-    int rc = lane_init(c, c->lanes[0], (cudaStream_t)stream);
+    int rc = lane_init(c, (cudaStream_t)stream);
+    if (rc == KZGB_OK && (event_create(c->t0) != cudaSuccess || event_create(c->t1) != cudaSuccess)) rc = KZGB_ERR_DEVICE;
     if (rc == KZGB_OK && !stream && g_l2_fetch_64.load()) { l2_limit_acquire(device); c->set_l2_limit = true; }
-    if (rc == KZGB_OK) {
-        c->n_lanes = 1;
-        if (cudaEventCreate(&c->t0) != cudaSuccess || cudaEventCreate(&c->t1) != cudaSuccess) rc = KZGB_ERR_DEVICE;
-    }
+    if (rc) delete c;  // with the device still current: frees whatever was built
     cudaSetDevice(prev);
-    if (rc) { delete c; return rc; }
+    if (rc) return rc;
     *out = c;
     return KZGB_OK;
 }
 
+// Members free themselves in `delete c`; the lanes' streams are drained first, and the device is current throughout.
 void kzgb_ctx_destroy(kzgb_ctx* c) {
     if (!c) return;
     int prev = 0;
     cudaGetDevice(&prev);
     cudaSetDevice(c->device);
-    for (int i = 0; i < c->n_lanes; i++) { cudaStreamSynchronize(c->lanes[i].st); lane_destroy(c->lanes[i]); }
-    if (c->srs) cudaFree(c->srs);
-    drop_window_table(c);
-    lagrange_release(c);
-    allroots_release(c);
-    if (c->tw) cudaFree(c->tw);
-    c->batch_bytes.release();
-    if (c->gen_table) cudaFree(c->gen_table);
-    if (c->pair_tab) cudaFree(c->pair_tab);
-    if (c->t0) cudaEventDestroy(c->t0);
-    if (c->t1) cudaEventDestroy(c->t1);
-    if (c->copy_st) cudaStreamDestroy(c->copy_st);
-    if (c->hash_st) cudaStreamDestroy(c->hash_st);
-    if (c->ev_hash_uploaded) cudaEventDestroy(c->ev_hash_uploaded);
-    if (c->fsl_host) cudaFreeHost(c->fsl_host);
-    c->fsl_args.release();
-    for (int k = 0; k < 2; k++) { if (c->ev_copied[k]) cudaEventDestroy(c->ev_copied[k]); if (c->ev_consumed[k]) cudaEventDestroy(c->ev_consumed[k]); }
-    if (c->trace_base) cudaEventDestroy(c->trace_base);
-    for (auto& r : c->trace) if (r.ev) cudaEventDestroy(r.ev);
+    for (int i = 0; i < c->n_lanes; i++) cudaStreamSynchronize(c->lanes[i].st);
     if (c->set_l2_limit) l2_limit_release(c->device);
-    cudaSetDevice(prev);
     delete c;
+    cudaSetDevice(prev);
 }
 
 const char* kzgb_last_error(const kzgb_ctx* c) { return c ? c->err.c_str() : "null context"; }
@@ -891,7 +841,7 @@ int kzgb_srs_save_cache(kzgb_ctx* c, const char* path) {
     std::vector<Affine> buf(std::min(chunk, c->srs_n));
     for (size_t first = 0; first < c->srs_n && ok; first += chunk) {
         size_t count = std::min(chunk, c->srs_n - first);
-        cudaError_t e = cudaMemcpy(buf.data(), c->srs + first, count * sizeof(Affine), cudaMemcpyDeviceToHost);
+        cudaError_t e = cudaMemcpy(buf.data(), c->srs.get() + first, count * sizeof(Affine), cudaMemcpyDeviceToHost);
         if (e != cudaSuccess) { fclose(f); remove(path); CK(c, e); }
         ok = fwrite(buf.data(), sizeof(Affine), count, f) == count;
     }
@@ -929,11 +879,10 @@ int kzgb_srs_load_affine_mont(kzgb_ctx* c, const uint64_t* xy, const uint8_t* in
     std::vector<Affine> host(n);
     memcpy(host.data(), xy, n * sizeof(Affine));
     if (inf) for (size_t i = 0; i < n; i++) if (inf[i]) aff_set_inf(host[i]);
-    Affine* pts = nullptr;
-    CK(c, cudaMalloc((void**)&pts, n * sizeof(Affine)));
-    cudaError_t e = cudaMemcpy(pts, host.data(), n * sizeof(Affine), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) { cudaFree(pts); CK(c, e); }
-    return srs_install(c, pts, n);
+    DevPtr<Affine[]> pts;
+    CK(c, dev_alloc(pts, n * sizeof(Affine)));
+    CK(c, cudaMemcpy(pts.get(), host.data(), n * sizeof(Affine), cudaMemcpyHostToDevice));
+    return srs_install(c, std::move(pts), n);
 }
 
 // dst gets a copy of src's SRS points, device to device (peer copy over NVLink when the contexts sit on different
@@ -946,16 +895,15 @@ int kzgb_srs_clone(kzgb_ctx* dst, kzgb_ctx* src) {
     {
         Guard gs(src);
         CK(src, drain_lanes(src));
-        n = src->srs_n; from = src->srs; src_dev = src->device;
+        n = src->srs_n; from = src->srs.get(); src_dev = src->device;
     }
     Guard g(dst);
     if (n == 0) return fail(dst, KZGB_ERR_GENERIC, "no SRS loaded in the source context");
-    Affine* pts = nullptr;
-    CK(dst, cudaMalloc((void**)&pts, n * sizeof(Affine)));
-    cudaError_t e = (src_dev == dst->device) ? cudaMemcpy(pts, from, n * sizeof(Affine), cudaMemcpyDeviceToDevice)
-                                              : cudaMemcpyPeer(pts, dst->device, from, src_dev, n * sizeof(Affine));
-    if (e != cudaSuccess) { cudaFree(pts); CK(dst, e); }
-    return srs_install(dst, pts, n);
+    DevPtr<Affine[]> pts;
+    CK(dst, dev_alloc(pts, n * sizeof(Affine)));
+    CK(dst, (src_dev == dst->device) ? cudaMemcpy(pts.get(), from, n * sizeof(Affine), cudaMemcpyDeviceToDevice)
+                                     : cudaMemcpyPeer(pts.get(), dst->device, from, src_dev, n * sizeof(Affine)));
+    return srs_install(dst, std::move(pts), n);
 }
 
 int kzgb_srs_load_synthetic_range(kzgb_ctx* c, const uint64_t tau_mont[4], size_t first, size_t n);
@@ -965,14 +913,13 @@ int kzgb_srs_load_synthetic(kzgb_ctx* c, const uint64_t tau_mont[4], size_t n) {
 int kzgb_srs_load_synthetic_range(kzgb_ctx* c, const uint64_t tau_mont[4], size_t first, size_t n) {
     Guard g(c);
     if (n == 0 || n > ((size_t)1 << 28)) return fail(c, KZGB_ERR_GENERIC, "invalid number of SRS points");
-    Affine* pts = nullptr;
-    CK(c, cudaMalloc((void**)&pts, n * sizeof(Affine)));
+    DevPtr<Affine[]> pts;
+    CK(c, dev_alloc(pts, n * sizeof(Affine)));
     Fr tau;
     memcpy(tau.l, tau_mont, 32);
-    srs_synthetic_launch(pts, (uint32_t)n, &tau, (uint32_t)first, c->lanes[0].st);
-    cudaError_t e = cudaStreamSynchronize(c->lanes[0].st);
-    if (e != cudaSuccess) { cudaFree(pts); CK(c, e); }
-    return srs_install(c, pts, n);
+    srs_synthetic_launch(pts.get(), (uint32_t)n, &tau, (uint32_t)first, c->lanes[0].st);
+    CK(c, cudaStreamSynchronize(c->lanes[0].st));
+    return srs_install(c, std::move(pts), n);
 }
 
 size_t kzgb_srs_len(const kzgb_ctx* c) { return c ? c->srs_n : 0; }
@@ -980,7 +927,7 @@ size_t kzgb_srs_len(const kzgb_ctx* c) { return c ? c->srs_n : 0; }
 int kzgb_srs_get_affine_mont(kzgb_ctx* c, size_t start, size_t count, uint64_t* out_xy, uint8_t* out_inf) {
     Guard g(c);
     if (start > c->srs_n || count > c->srs_n - start) return fail(c, KZGB_ERR_GENERIC, "SRS range out of bounds");
-    CK(c, cudaMemcpy(out_xy, c->srs + start, count * sizeof(Affine), cudaMemcpyDeviceToHost));
+    CK(c, cudaMemcpy(out_xy, c->srs.get() + start, count * sizeof(Affine), cudaMemcpyDeviceToHost));
     if (out_inf) {
         const Affine* a = (const Affine*)out_xy;
         for (size_t i = 0; i < count; i++) out_inf[i] = aff_is_inf(a[i]) ? 1 : 0;
@@ -994,7 +941,7 @@ int kzgb_srs_precompute(kzgb_ctx* c, size_t max_n, int window_bits) {
         c->auto_precompute = false;
         drain_lanes(c);
         drop_window_table(c);
-        lagrange_release(c);
+        for (auto& t : c->lag) t = {};
         return KZGB_OK;
     }
     if (!c->srs_n) return fail(c, KZGB_ERR_GENERIC, "no SRS loaded");
@@ -1133,7 +1080,7 @@ int kzgb_ntt_fr(kzgb_ctx* c, uint64_t* inout, size_t n, int inverse) {
     CK(c, L.ntt_scratch.reserve(n * sizeof(Fr)));
     CK(c, cudaMemcpyAsync(L.work.p, inout, n * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
     Fr ninv = ninv_mont(logn);
-    ntt_launch((Fr*)L.work.p, logn, 1, inverse != 0, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+    ntt_launch((Fr*)L.work.p, logn, 1, inverse != 0, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
     CK(c, cudaMemcpyAsync(inout, L.work.p, n * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
     CK(c, cudaStreamSynchronize(L.st));
     CK(c, cudaGetLastError());
@@ -1231,7 +1178,7 @@ int kzgb_g1_ifft(kzgb_ctx* c, size_t n, uint64_t* out_xy, uint8_t* out_inf) {
     CK(c, L.bases.reserve(n * sizeof(Affine)));
     Fr ninv = ninv_mont(logn), ninv_canon;
     fe_from_mont(ninv_canon, ninv);
-    g1_intt_launch(c->srs, logn, (XYZZ*)L.work.p, (Affine*)L.bases.p, c->tw, c->logN, &ninv_canon, L.st);
+    g1_intt_launch(c->srs.get(), logn, (XYZZ*)L.work.p, (Affine*)L.bases.p, c->tw.get(), c->logN, &ninv_canon, L.st);
     std::vector<Affine> host(n);
     CK(c, cudaMemcpyAsync(host.data(), L.bases.p, n * sizeof(Affine), cudaMemcpyDeviceToHost, L.st));
     CK(c, cudaStreamSynchronize(L.st));
@@ -1287,12 +1234,12 @@ static int proofs_all_roots(kzgb_ctx* c, const uint64_t* evals, int logn, const 
     CK(c, cudaMemcpyAsync(f, evals, n * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
     CK(c, cudaMemsetAsync(f + n, 0, n * sizeof(Fr), L.st));
     const Fr ninv = ninv_mont(logn), inv2n = ninv_mont(logn + 1), one = fr_one_canon();
-    ntt_launch(f, logn, 1, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-    ntt_launch(f, logn + 1, 1, false, c->tw, c->logN, &inv2n, (Fr*)L.ntt_scratch.p, L.st);
+    ntt_launch(f, logn, 1, true, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+    ntt_launch(f, logn + 1, 1, false, c->tw.get(), c->logN, &inv2n, (Fr*)L.ntt_scratch.p, L.st);
     allroots_hadamard_launch(f, &inv2n, shat, u, logn + 1, L.st);  // the 1/2n of the inverse transform, on the scalars
-    g1_ntt_stages_launch(u, logn + 1, true, c->tw, c->logN, L.st);
+    g1_ntt_stages_launch(u, logn + 1, true, c->tw.get(), c->logN, L.st);
     allroots_extract_launch(u, H, logn, L.st);
-    g1_ntt_stages_launch(H, logn, false, c->tw, c->logN, L.st);
+    g1_ntt_stages_launch(H, logn, false, c->tw.get(), c->logN, L.st);
     g1_ntt_finish_launch(H, (Affine*)L.work.p, logn, &one, L.st);  // u is consumed: its buffer takes the proofs
     std::vector<Affine> host(n);
     CK(c, cudaMemcpyAsync(host.data(), L.work.p, n * sizeof(Affine), cudaMemcpyDeviceToHost, L.st));
@@ -1311,9 +1258,7 @@ int kzgb_compute_proofs_all_roots(kzgb_ctx* c, const uint64_t* evals, size_t n, 
     const Affine* shat = nullptr;
     if (int rc = ensure_allroots(c, logn, &shat)) return rc;
     DevBuf own;  // s_hat of a domain above 2^22, for this call only
-    int rc = proofs_all_roots(c, evals, logn, shat, &own, out_xy, out_inf);
-    own.release();
-    return rc;
+    return proofs_all_roots(c, evals, logn, shat, &own, out_xy, out_inf);
 }
 
 int kzgb_srs_prepare_all_roots(kzgb_ctx* c, size_t n) {
@@ -1473,13 +1418,13 @@ int kzgb_microbench(kzgb_ctx* c, int kind, double* ops_per_second) {
     double per_thread = (kind == 3) ? iters * 4.0 : (kind == 2 ? iters * 64.0 : iters * 128.0);
     float best = 1e30f;
     for (int rep = 0; rep < 4; rep++) {
-        CK(c, cudaEventRecord(c->t0, L.st));
+        CK(c, cudaEventRecord(c->t0.get(), L.st));
         if (kind == 3) fqmul_peak_launch((uint32_t*)L.work.p, iters, blocks, threads, L.st);
         else imad_peak_launch((uint32_t*)L.work.p, iters, kind, blocks, threads, L.st);
-        CK(c, cudaEventRecord(c->t1, L.st));
-        CK(c, cudaEventSynchronize(c->t1));
+        CK(c, cudaEventRecord(c->t1.get(), L.st));
+        CK(c, cudaEventSynchronize(c->t1.get()));
         float ms = 0;
-        CK(c, cudaEventElapsedTime(&ms, c->t0, c->t1));
+        CK(c, cudaEventElapsedTime(&ms, c->t0.get(), c->t1.get()));
         if (rep > 0 && ms < best) best = ms;
     }
     CK(c, cudaGetLastError());
@@ -1500,15 +1445,15 @@ int kzgb_bench_msm(kzgb_ctx* c, size_t n, int reps, double* ms_total, double* ms
     if (rc) return rc;
     double acc0 = L.acc_ms;
     uint64_t l0 = L.acc_launches;
-    CK(c, cudaEventRecord(c->t0, L.st));
+    CK(c, cudaEventRecord(c->t0.get(), L.st));
     for (int i = 0; i < reps; i++) {
         rc = msm_blocking(c, L, (Fr*)L.evals.p, 0, n, nullptr, &r);
         if (rc) return rc;
     }
-    CK(c, cudaEventRecord(c->t1, L.st));
-    CK(c, cudaEventSynchronize(c->t1));
+    CK(c, cudaEventRecord(c->t1.get(), L.st));
+    CK(c, cudaEventSynchronize(c->t1.get()));
     float ms = 0;
-    CK(c, cudaEventElapsedTime(&ms, c->t0, c->t1));
+    CK(c, cudaEventElapsedTime(&ms, c->t0.get(), c->t1.get()));
     *ms_total = ms / reps;
     uint64_t nl = L.acc_launches - l0;
     *ms_accumulate = nl ? (L.acc_ms - acc0) / nl : 0.0;
@@ -1527,15 +1472,15 @@ int kzgb_bench_ntt(kzgb_ctx* c, int logn, size_t batch, int reps, double* ms_per
     Fr base = fr_from_u64(0x9e3779b97f4a7c15ull);
     fr_powers_launch((Fr*)L.work.p, (uint32_t)std::min<size_t>(total, 0xffffffffu), &base, L.st);
     Fr ninv = ninv_mont(logn);
-    ntt_launch((Fr*)L.work.p, logn, (uint32_t)batch, true, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);  // warm-up
-    CK(c, cudaEventRecord(c->t0, L.st));
+    ntt_launch((Fr*)L.work.p, logn, (uint32_t)batch, true, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);  // warm-up
+    CK(c, cudaEventRecord(c->t0.get(), L.st));
     for (int i = 0; i < reps; i++)
-        ntt_launch((Fr*)L.work.p, logn, (uint32_t)batch, (i & 1) == 0, c->tw, c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-    CK(c, cudaEventRecord(c->t1, L.st));
-    CK(c, cudaEventSynchronize(c->t1));
+        ntt_launch((Fr*)L.work.p, logn, (uint32_t)batch, (i & 1) == 0, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+    CK(c, cudaEventRecord(c->t1.get(), L.st));
+    CK(c, cudaEventSynchronize(c->t1.get()));
     CK(c, cudaGetLastError());
     float ms = 0;
-    CK(c, cudaEventElapsedTime(&ms, c->t0, c->t1));
+    CK(c, cudaEventElapsedTime(&ms, c->t0.get(), c->t1.get()));
     *ms_per_call = ms / reps;
     return KZGB_OK;
 }
@@ -1543,31 +1488,30 @@ int kzgb_bench_ntt(kzgb_ctx* c, int logn, size_t batch, int reps, double* ms_per
 // Device-side stopwatch over ALL lanes: everything queued between begin and end is inside [t0, t1].
 int kzgb_timer_begin(kzgb_ctx* c) {
     Guard g(c);
-    CK(c, cudaEventRecord(c->t0, c->lanes[0].st));
-    for (int i = 1; i < c->n_lanes; i++) CK(c, cudaStreamWaitEvent(c->lanes[i].st, c->t0, 0));
+    CK(c, cudaEventRecord(c->t0.get(), c->lanes[0].st));
+    for (int i = 1; i < c->n_lanes; i++) CK(c, cudaStreamWaitEvent(c->lanes[i].st, c->t0.get(), 0));
     return KZGB_OK;
 }
 int kzgb_timer_end(kzgb_ctx* c, double* ms_out) {
     Guard g(c);
     for (int i = 1; i < c->n_lanes; i++) {
-        CK(c, cudaEventRecord(c->lanes[i].ev_done, c->lanes[i].st));
-        CK(c, cudaStreamWaitEvent(c->lanes[0].st, c->lanes[i].ev_done, 0));
+        CK(c, cudaEventRecord(c->lanes[i].ev_done.get(), c->lanes[i].st));
+        CK(c, cudaStreamWaitEvent(c->lanes[0].st, c->lanes[i].ev_done.get(), 0));
     }
-    CK(c, cudaEventRecord(c->t1, c->lanes[0].st));
-    CK(c, cudaEventSynchronize(c->t1));
+    CK(c, cudaEventRecord(c->t1.get(), c->lanes[0].st));
+    CK(c, cudaEventSynchronize(c->t1.get()));
     float ms = 0;
-    CK(c, cudaEventElapsedTime(&ms, c->t0, c->t1));
+    CK(c, cudaEventElapsedTime(&ms, c->t0.get(), c->t1.get()));
     *ms_out = ms;
     return KZGB_OK;
 }
 int kzgb_trace_begin(kzgb_ctx* c) {
     Guard g(c);
     CK(c, drain_lanes(c));
-    for (auto& r : c->trace) if (r.ev) cudaEventDestroy(r.ev);
     c->trace.clear();
-    if (!c->trace_base) CK(c, cudaEventCreate(&c->trace_base));
-    CK(c, cudaEventRecord(c->trace_base, c->lanes[0].st));
-    CK(c, cudaEventSynchronize(c->trace_base));
+    if (!c->trace_base) CK(c, event_create(c->trace_base));
+    CK(c, cudaEventRecord(c->trace_base.get(), c->lanes[0].st));
+    CK(c, cudaEventSynchronize(c->trace_base.get()));
     c->trace_host0 = std::chrono::steady_clock::now();
     c->trace_on.store(true);
     return KZGB_OK;
@@ -1578,15 +1522,14 @@ int kzgb_trace_end(kzgb_ctx* c, double* out, size_t capacity_records, size_t* n_
     c->trace_on.store(false);
     for (int i = 0; i < c->n_lanes; i++) {
         CK(c, cudaStreamSynchronize(c->lanes[i].st));
-        if (c->lanes[i].st_acc) CK(c, cudaStreamSynchronize(c->lanes[i].st_acc));
+        if (c->lanes[i].st_acc) CK(c, cudaStreamSynchronize(c->lanes[i].st_acc.get()));
     }
     size_t n = 0;
     for (auto& r : c->trace) {
         float ms = -1.f;
-        if (r.ev && cudaEventElapsedTime(&ms, c->trace_base, r.ev) != cudaSuccess) { ms = -1.f; cudaGetLastError(); }
+        if (r.ev && cudaEventElapsedTime(&ms, c->trace_base.get(), r.ev.get()) != cudaSuccess) { ms = -1.f; cudaGetLastError(); }
         if (out && n < capacity_records) { out[4 * n] = r.lane; out[4 * n + 1] = r.kind; out[4 * n + 2] = ms; out[4 * n + 3] = r.host_ms; }
         n++;
-        if (r.ev) cudaEventDestroy(r.ev);
     }
     c->trace.clear();
     if (n_records) *n_records = n;

@@ -3,8 +3,11 @@
 #pragma once
 #include <atomic>
 #include <chrono>
+#include <memory>
 #include <mutex>
 #include <string>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "../../include/kzg_bn254_b200.h"
@@ -16,13 +19,55 @@ constexpr int MAX_LANES = 8;
 constexpr int MAX_SETS = 96;
 constexpr int ALLROOTS_MAX_LOG = 22;  // largest domain 2^k whose kzgb_compute_proofs_all_roots table is kept
 
+// ---- owners of CUDA resources: each frees its resource when it is destroyed or reset, so a partly built object
+// releases what it holds and no teardown list has to name it.  An owner must be destroyed while its device is current:
+// locals are declared after the entry point's Guard, context members die inside kzgb_ctx_destroy.
+struct CudaFree { void operator()(void* p) const { cudaFree(p); } };
+struct CudaFreeHost { void operator()(void* p) const { cudaFreeHost(p); } };
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+template <class T> using DevPtr = std::unique_ptr<T, CudaFree>;       // device memory
+template <class T> using HostPtr = std::unique_ptr<T, CudaFreeHost>;  // pinned or mapped host memory
+using StreamPtr = std::unique_ptr<CUstream_st, StreamDestroy>;
+using EventPtr = std::unique_ptr<CUevent_st, EventDestroy>;
+
+// Each creates into an empty owner, which holds the resource only if the call succeeded.
+template <class T> cudaError_t dev_alloc(DevPtr<T>& o, size_t bytes) {
+    void* p = nullptr;
+    cudaError_t e = cudaMalloc(&p, bytes);
+    o.reset(e == cudaSuccess ? static_cast<std::remove_extent_t<T>*>(p) : nullptr);
+    return e;
+}
+template <class T> cudaError_t host_alloc(HostPtr<T>& o, size_t bytes, unsigned flags = cudaHostAllocDefault) {
+    void* p = nullptr;
+    cudaError_t e = cudaHostAlloc(&p, bytes, flags);
+    o.reset(e == cudaSuccess ? static_cast<std::remove_extent_t<T>*>(p) : nullptr);
+    return e;
+}
+inline cudaError_t stream_create(StreamPtr& o, int priority) {  // non-blocking; priority 0 is the default
+    cudaStream_t s = nullptr;
+    cudaError_t e = cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, priority);
+    o.reset(e == cudaSuccess ? s : nullptr);
+    return e;
+}
+inline cudaError_t event_create(EventPtr& o, unsigned flags = cudaEventDefault) {
+    cudaEvent_t ev = nullptr;
+    cudaError_t e = cudaEventCreateWithFlags(&ev, flags);
+    o.reset(e == cudaSuccess ? ev : nullptr);
+    return e;
+}
+
+// Device memory that only grows (reserve rounds up to 1 MiB and frees the old block before allocating the new one).
 struct DevBuf {
     void* p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(DevBuf&& o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); }
+    DevBuf& operator=(DevBuf&& o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }  // o frees our old block
+    ~DevBuf() { release(); }
     cudaError_t reserve(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
+        release();
         size_t want = (bytes + (1u << 20) - 1) & ~(size_t)((1u << 20) - 1);
         cudaError_t e = cudaMalloc(&p, want);
         if (e == cudaSuccess) cap = want;
@@ -33,15 +78,15 @@ struct DevBuf {
 
 struct Lane {
     cudaStream_t st = nullptr;      // everything but the bucket accumulation (high priority when owned)
-    cudaStream_t st_acc = nullptr;  // bucket accumulation: low priority, so other lanes' short kernels
+    StreamPtr own_st;               // st when the lane created it; empty on a caller's stream, which is never destroyed
+    StreamPtr st_acc;               // bucket accumulation: low priority, so other lanes' short kernels
                                     // slip in between its blocks instead of queueing behind the whole grid
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    bool own_stream = false;
+    EventPtr ev_fork, ev_join;
     DevBuf bytes, evals, work, ntt_scratch, eval_scratch, msm_ws, small, bases, bucket_total, pairing;
-    XYZZ* h_sets = nullptr;   // pinned
-    uint32_t* h_entries = nullptr;  // pinned: length of the sorted list of the MSM in flight (= its point additions)
-    Fr* h_fr = nullptr;       // pinned, 16 elements
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_done = nullptr, ev_block = nullptr;
+    HostPtr<XYZZ[]> h_sets;
+    HostPtr<uint32_t> h_entries;  // length of the sorted list of the MSM in flight (= its point additions)
+    HostPtr<Fr[]> h_fr;           // 16 elements
+    EventPtr ev0, ev1, ev_done, ev_block;
     bool ev_pending = false;
     double acc_ms = 0;        // summed duration of bucket-accumulation kernels
     uint64_t acc_launches = 0;
@@ -57,9 +102,9 @@ struct kzgb_ctx {
     kzgb::Lane lanes[kzgb::MAX_LANES];
     int n_lanes = 0;
     // SRS
-    kzgb::Affine* srs = nullptr;
+    kzgb::DevPtr<kzgb::Affine[]> srs;
     size_t srs_n = 0;
-    kzgb::Affine* wtable = nullptr;   // fixed-base window table over SRS points [wt_first, wt_first + wt_n)
+    kzgb::DevPtr<kzgb::Affine[]> wtable;  // fixed-base window table over SRS points [wt_first, wt_first + wt_n)
     size_t wt_first = 0, wt_n = 0;
     int wt_c = 0, wt_W = 0;
     bool auto_precompute = true;
@@ -67,40 +112,40 @@ struct kzgb_ctx {
     bool set_l2_limit = false;
     // Lagrange-basis tables, one per domain size 2^k: window table over L = IFFT_G1(SRS[..2^k]) so that
     // evaluation-form commitments are ONE MSM on the evaluations themselves (no Fr NTT on the path)
-    struct LagTable { kzgb::Affine* table = nullptr; size_t n = 0; int c = 0, W = 0; uint64_t last_use = 0; uint32_t calls = 0; } lag[29];
+    struct LagTable { kzgb::DevPtr<kzgb::Affine[]> table; size_t n = 0; int c = 0, W = 0; uint64_t last_use = 0; uint32_t calls = 0; } lag[29];
     uint64_t lag_clock = 0;
     // kzgb_compute_proofs_all_roots: s_hat = DFT_2n of the reversed SRS prefix, 2n affine points per domain 2^k, built by
     // the first call of that size (or kzgb_srs_prepare_all_roots) and dropped with the SRS
-    kzgb::Affine* allroots[kzgb::ALLROOTS_MAX_LOG + 1] = {};
+    kzgb::DevPtr<kzgb::Affine[]> allroots[kzgb::ALLROOTS_MAX_LOG + 1];
     kzgb::DevBuf batch_bytes;  // blob bytes of the batch in flight (commit_and_prove_blobs)
-    kzgb::Affine* gen_table = nullptr;  // generator_window_table() on this device, uploaded by the first per-blob verification
+    kzgb::DevPtr<kzgb::Affine[]> gen_table;  // generator_window_table() on this device, uploaded by the first per-blob verification
     // [tau]G2 of the pairing checks (kzgb_set_g2_tau; no SRS is involved, so reloading the SRS leaves it alone) and its
     // PairingTables on the device, rebuilt by the first pairing check after a change
     kzgb::G2Affine g2_tau = kzgb::default_g2_tau();
-    kzgb::PairingTables* pair_tab = nullptr;
+    kzgb::DevPtr<kzgb::PairingTables> pair_tab;
     bool pair_stale = true;
     // twiddles
-    kzgb::Fr* tw = nullptr;
+    kzgb::DevPtr<kzgb::Fr[]> tw;
     int logN = 0;
     // timer
-    cudaEvent_t t0 = nullptr, t1 = nullptr;
+    kzgb::EventPtr t0, t1;
     // device-side hashing of long Fiat-Shamir transcripts (fs.cu k_fs_midstate_long): its stream, the mapped host block the
     // kernel reports through ([state 8 x cap | done cap | cancel 1] words) and the device-side argument arrays
-    cudaStream_t hash_st = nullptr;
-    cudaEvent_t ev_hash_uploaded = nullptr;
-    uint32_t* fsl_host = nullptr;
+    kzgb::StreamPtr hash_st;
+    kzgb::EventPtr ev_hash_uploaded;
+    kzgb::HostPtr<uint32_t[]> fsl_host;
     std::atomic<bool> lanes_block{false};  // lanes of the running large-blob batch sleep on a blocking event (lane_wait)
     kzgb::DevBuf fsl_args;
     // upload stream + double-buffer fences of msm_srs_host_pipelined
-    cudaStream_t copy_st = nullptr;
-    cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr};
+    kzgb::StreamPtr copy_st;
+    kzgb::EventPtr ev_copied[2], ev_consumed[2];
     // timeline trace (kzgb_trace_begin / kzgb_trace_end, include/kzg_bn254_b200_bench.h): device events and host time
     // stamps of every MSM of every lane, for reading pipeline stalls without a system profiler
-    struct TraceRec { int lane, kind; cudaEvent_t ev; double host_ms; };
+    struct TraceRec { int lane, kind; kzgb::EventPtr ev; double host_ms; };
     std::atomic<bool> trace_on{false};
     std::mutex trace_mu;
     std::vector<TraceRec> trace;
-    cudaEvent_t trace_base = nullptr;
+    kzgb::EventPtr trace_base;
     std::chrono::steady_clock::time_point trace_host0;
 };
 

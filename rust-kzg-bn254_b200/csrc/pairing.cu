@@ -165,8 +165,8 @@ int ensure_pairing_tables(kzgb_ctx* c) {
     std::unique_ptr<PairingTables> h(new PairingTables(*pairing_fixed_tables()));
     h->tau = c->g2_tau;
     g2_lines(h->lines[1], c->g2_tau);
-    if (!c->pair_tab) CK(c, cudaMalloc(&c->pair_tab, sizeof(PairingTables)));
-    CK(c, cudaMemcpy(c->pair_tab, h.get(), sizeof(PairingTables), cudaMemcpyHostToDevice));
+    if (!c->pair_tab) CK(c, dev_alloc(c->pair_tab, sizeof(PairingTables)));
+    CK(c, cudaMemcpy(c->pair_tab.get(), h.get(), sizeof(PairingTables), cudaMemcpyHostToDevice));
     c->pair_stale = false;
     return KZGB_OK;
 }
