@@ -160,6 +160,24 @@ int kzgb_g1_ifft(kzgb_ctx* ctx, size_t n, uint64_t* out_xy, uint8_t* out_inf);
  * caller-supplied z (Montgomery).  Optionally returns y = p(z) (Montgomery) if y_out != NULL. */
 int kzgb_compute_proof(kzgb_ctx* ctx, const uint64_t* evals_mont, size_t n, const uint64_t z_mont[4],
                        uint64_t out_xy[8], uint8_t* out_inf, uint64_t y_out[4]);
+/* KZG::compute_proof / compute_proof_impl / compute_proof_with_known_z_fr_index (kzg.rs:128-178, 187-234) for `count`
+ * polynomials, each at a point the caller chooses, in one pipelined call.  Polynomial i is ns[i] evaluations (Montgomery)
+ * at evals_mont[i], HOST memory; z_i is the 4 words at zs_mont + 4 i (Montgomery, host memory).  out_xy: count x 8 words
+ * (x||y Montgomery); out_inf: count flags, may be NULL; ys_mont: count x 4 words, y_i = p_i(z_i) (Montgomery), may be
+ * NULL.  Entry i is exactly what kzgb_compute_proof(evals_mont[i], ns[i], z_i, ..., y_out) returns, for z_i inside the
+ * domain (the quotient of compute_quotient_eval_on_domain, kzg.rs:237-260) and outside it.  Checks, entry by entry in
+ * index order: ns[i] a power of two (KZGB_ERR_FFT "length provided is not a power of 2"), ns[i] <= srs_len
+ * (KZGB_ERR_SRS_CAPACITY), z_i a reduced Montgomery word, below r (KZGB_ERR_INVALID_FIELD_ELEMENT, the message names i; the
+ * single call does not check this, kzgb_verify_proofs demands it of the same z).  The error of the lowest failing entry is
+ * returned before any work starts and the outputs are left untouched.  The evaluation words are not validated, as in
+ * kzgb_compute_proof.  count == 0 writes nothing.  The batch has no per-instance roots of unity, so the reference's
+ * roots-length check (kzg.rs:135-139) is not made. */
+int kzgb_compute_proofs(kzgb_ctx* ctx, const uint64_t* const* evals_mont, const size_t* ns, size_t count,
+                        const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont);
+/* Same with the evaluations in device memory (evals_dev[i]: ns[i] x 4 words), read in place; z, the outputs and the checks
+ * as kzgb_compute_proofs. */
+int kzgb_compute_proofs_dev(kzgb_ctx* ctx, const uint64_t* const* evals_dev, const size_t* ns, size_t count,
+                            const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont);
 /* KZG::compute_proof_with_known_z_fr_index (kzg.rs:187-207) at EVERY index: out proof i (x||y Montgomery, n x 8 words;
  * out_inf n flags, may be NULL) is the point kzgb_compute_proof(evals, n, w^i) returns.  FK20: one Toeplitz product in G1
  * (two G1 FFTs + 2n scalar multiplications) instead of n MSMs.  Errors and their order as kzgb_compute_proof: KZGB_ERR_FFT
@@ -406,6 +424,11 @@ int kzgb_group_commit_blobs(kzgb_group* group, const uint8_t* const* blobs, cons
 int kzgb_group_compute_blob_proofs(kzgb_group* group, const uint8_t* const* blobs, const size_t* lens, size_t count,
                                    const uint64_t* commitments_xy, const uint8_t* commitments_inf,
                                    uint64_t* out_xy, uint8_t* out_inf);
+/* kzgb_compute_proofs (KZG::compute_proof, kzg.rs:128-178, 187-234) cut into contiguous shares of about equal evaluation
+ * bytes (32 ns[i] per polynomial), one per member; identical to the one-context call.  Each member checks its own share
+ * before it starts (so on an error, members with valid shares may have written their outputs). */
+int kzgb_group_compute_proofs(kzgb_group* group, const uint64_t* const* evals_mont, const size_t* ns, size_t count,
+                              const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont);
 /* kzgb_verify_blob_proofs_g1 cut into contiguous shares of about equal bytes, one per member; identical to the one-context
  * call.  Each member checks its own share before it starts (so on an error, members with valid shares may have written
  * their outputs). */

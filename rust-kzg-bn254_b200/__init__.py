@@ -107,6 +107,22 @@ def _compute_blob_proofs(call, blobs: Sequence["Blob"], commitments: Sequence[Af
     return g1_from_abi(xy.raw[: 64 * count], inf.raw[:count])
 
 
+def _compute_proofs(call, polynomials: Sequence["PolynomialEvalForm"], zs: Sequence[int]) -> Tuple[List[Affine], List[int]]:
+    """Runs call(evaluation pointers, lengths, count, zs_mont, out_xy, out_inf, ys_mont) of a kzgb_*compute_proofs entry
+    point; returns the proofs and the values y_i = p_i(z_i)."""
+    if len(polynomials) != len(zs):
+        raise KzgError("GenericError", "length's of the input are not the same")
+    count = len(polynomials)
+    keep = [C.create_string_buffer(fr_to_mont_bytes(p.evaluations), max(32, 32 * len(p))) for p in polynomials]
+    ptrs = (C.c_void_p * count)(*[C.cast(k, C.c_void_p).value for k in keep])
+    ns = (C.c_size_t * count)(*[len(p) for p in polynomials])
+    xy = C.create_string_buffer(64 * count if count else 1)
+    inf = C.create_string_buffer(count if count else 1)
+    ys = C.create_string_buffer(32 * count if count else 1)
+    call(ptrs, ns, count, fr_to_mont_bytes(zs), xy, inf, ys)
+    return g1_from_abi(xy.raw[: 64 * count], inf.raw[:count]), fr_from_mont_bytes(ys.raw[: 32 * count])
+
+
 def _verify_blob_proofs(call, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]):
     """Runs call(blob pointers, lengths, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, out_xy, out_inf,
     z_out, y_out) of a kzgb_*verify_blob_proofs_g1 entry point; returns (C_i - [y_i] G1, z_i, y_i) for every blob."""
@@ -294,6 +310,10 @@ class Group:
         """KZG::compute_blob_proof for every (blob, commitment) pair (prover/src/kzg.rs:288-309), the batch cut by blob
         across the members."""
         return _compute_blob_proofs(lambda *a: self.check(lib.kzgb_group_compute_blob_proofs(self.h, *a)), blobs, commitments)
+
+    def compute_proofs(self, polynomials: Sequence["PolynomialEvalForm"], zs: Sequence[int]) -> Tuple[List[Affine], List[int]]:
+        """KZG.compute_proofs with the batch cut by evaluation bytes across the members."""
+        return _compute_proofs(lambda *a: self.check(lib.kzgb_group_compute_proofs(self.h, *a)), polynomials, zs)
 
     def verify_blob_kzg_proofs_g1(
         self, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]
@@ -698,6 +718,14 @@ class KZG:
         inf = C.create_string_buffer(n)
         e.check(lib.kzgb_compute_proofs_all_roots(e.h, fr_to_mont_bytes(polynomial.evaluations), n, xy, inf))
         return g1_from_abi(xy.raw, inf.raw)
+
+    @staticmethod
+    def compute_proofs(polynomials: Sequence[PolynomialEvalForm], zs: Sequence[int], srs: SRS) -> Tuple[List[Affine], List[int]]:
+        """compute_proof / compute_proof_with_known_z_fr_index (kzg.rs:128-178, 187-234) of polynomial i at zs[i] for every i in one call, pipelined inside the
+        library: returns the proofs and the values y_i = p_i(zs[i]).  Entry i is what compute_proof returns for polynomial
+        i alone, without the per-instance roots-length check; the lowest failing entry's error is raised."""
+        e = srs.engine
+        return _compute_proofs(lambda *a: e.check(lib.kzgb_compute_proofs(e.h, *a)), polynomials, zs)
 
     def g1_ifft(self, length: int, srs: SRS) -> List[Affine]:
         """kzg.rs:263-285."""

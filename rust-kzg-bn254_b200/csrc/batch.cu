@@ -1,6 +1,7 @@
 // The blob-batch pipelines: kzgb_commit_and_prove_blobs{,_dev} -- commitment and proof of many blobs on several lanes
 // while a hashing stage produces the Fiat-Shamir transcripts --, kzgb_commit_blobs{,_dev} -- the commitments alone, on
-// the same plan and lanes --, kzgb_compute_blob_proofs{,_dev} -- the proofs alone, against the caller's commitments --
+// the same plan and lanes --, kzgb_compute_blob_proofs{,_dev} -- the proofs alone, against the caller's commitments --,
+// kzgb_compute_proofs{,_dev} -- proofs of evaluation-form polynomials at the caller's points, on the same plan and lanes --
 // and the verifier's calls, kzgb_verify_blob_proofs{,_g1}{,_dev} and kzgb_verify_batch_rlc{,_dev}, over one per-blob stage,
 // kzgb_verify_kzg_proof_batch_rlc, the random linear combination alone over openings the caller has evaluated, and
 // kzgb_verify_proofs, the pairing check of each such opening.
@@ -118,9 +119,10 @@ HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible, bool 
 }
 
 // ---------------------------------------------------------------- planning
-// What a batch computes: kzgb_commit_and_prove_blobs{,_dev}, kzgb_commit_blobs{,_dev} (commitments, no transcripts) or
-// kzgb_compute_blob_proofs{,_dev} (proofs against the caller's commitments, no commit phase).
-enum class Job { CommitAndProve, Commit, Prove };
+// What a batch computes: kzgb_commit_and_prove_blobs{,_dev}, kzgb_commit_blobs{,_dev} (commitments, no transcripts),
+// kzgb_compute_blob_proofs{,_dev} (proofs against the caller's commitments, no commit phase) or kzgb_compute_proofs{,_dev}
+// (proofs of the caller's Montgomery evaluations at the caller's points: no blob bytes, no transcripts, no commitments).
+enum class Job { CommitAndProve, Commit, Prove, ProveAt };
 
 // One batch call: its arguments and the plan made for them.  The entry points set their job's outputs by name.
 struct Batch {
@@ -140,6 +142,14 @@ struct Batch {
     const uint64_t* commitments_xy = nullptr;  // Prove: the caller's commitments in the ABI ...
     const uint8_t* commitments_inf = nullptr;
     std::vector<Affine> commits;               // ... read and checked by plan_batch
+    // ProveAt: polynomial i is ns[i] Montgomery evaluations at evals[i] (device memory when evals_on_device), opened at the
+    // 4 words zs_mont + 4 i; its y goes to ys_mont + 4 i (optional).  lens[i] = 32 ns[i], so that the plan groups the
+    // polynomials as it groups blobs of that many bytes.
+    const uint64_t* const* evals = nullptr;
+    bool evals_on_device = false;
+    const size_t* ns = nullptr;
+    const uint64_t* zs_mont = nullptr;
+    uint64_t* ys_mont = nullptr;
     size_t max_n = 0;
     std::vector<std::pair<size_t, size_t>> groups;  // small blobs: (first blob, blobs); empty: one blob per task
     int n_lanes = 0;
@@ -148,15 +158,33 @@ struct Batch {
     bool resident = false;
 };
 
+// the 4 little-endian words at w hold a value below r
+bool fr_words_reduced(const uint64_t* w) {
+    uint32_t r[8];
+    FeConst<FR>::mod(r);
+    for (int k = 7; k >= 0; k--) {
+        const uint32_t x = (uint32_t)(w[k / 2] >> (32 * (k & 1)));
+        if (x != r[k]) return x < r[k];
+    }
+    return false;
+}
+
 // Validation, groups, lanes and the tables every size of the batch needs.  A commit-only batch checks every blob as
 // kzgb_commit_blob does (a blob of length 0 commits the zero polynomial of size 1); with proofs, length 0 is
 // compute_blob_proof's error, and a proof-only batch checks each commitment first, as kzgb_compute_blob_proof does.
+// Proofs at the caller's points check each polynomial as kzgb_compute_proof does, then its z.
 int plan_batch(Batch& b) {
     kzgb_ctx* c = b.c;
     const size_t* lens = b.lens;
     const size_t count = b.count;
     for (size_t i = 0; i < count; i++) {
-        if (b.job == Job::Commit) {
+        if (b.job == Job::ProveAt) {
+            const size_t n = b.ns[i];
+            if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_FFT, "length provided is not a power of 2");
+            if (int rc = check_srs_capacity(c, n)) return rc;
+            if (!fr_words_reduced(b.zs_mont + 4 * i))
+                return fail(c, KZGB_ERR_INVALID_FIELD_ELEMENT, "z of opening " + std::to_string(i) + " is not a reduced field element");
+        } else if (b.job == Job::Commit) {
             if (int rc = check_commit_blob_len(c, blob_poly_len(lens[i]))) return rc;
         } else {
             if (b.job == Job::Prove) {
@@ -525,39 +553,90 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
     return r;
 }
 
-// The proof phase of one group whose transcript midstates are ready and whose Montgomery evaluations are in L.evals: the
-// challenges of blobs i0 .. i0 + bn - 1 against the commitments cs[0 .. bn), ONE batched evaluation / quotient launch set
-// with a challenge per blob and ONE batched MSM of the quotients; pts[k] is the proof of blob i0 + k.
-int group_prove(const Batch& b, const HashStage& hs, Lane& L, size_t i0, size_t bn, const Affine* cs, Affine* pts) {
+// The points of a blob group whose transcript midstates are ready: the challenges of blobs i0 .. i0 + bn - 1 against the
+// commitments cs[0 .. bn) and their tinv (eval_tinv) up to L.small as group_prove reads them.  *outside: no challenge is a
+// root of the domain.
+int group_challenges(const Batch& b, const HashStage& hs, Lane& L, size_t i0, size_t bn, const Affine* cs, bool* outside) {
     kzgb_ctx* c = b.c;
-    const size_t n = blob_poly_len(b.lens[i0]);
-    const int logn = log2_exact(n);
-    const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
-    Fr ninv = ninv_mont(logn);
+    const int logn = log2_exact(blob_poly_len(b.lens[i0]));
     CK(c, L.small.reserve((3 * bn + 8) * sizeof(Fr)));
-    CK(c, L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)bn) * sizeof(Fr)));
-    CK(c, L.work.reserve(bn * n * sizeof(Fr)));
-    if (!lag) CK(c, L.ntt_scratch.reserve(bn * n * sizeof(Fr)));
     std::vector<Fr> zt(2 * bn);
     bool any_in_domain = false;
     for (size_t k = 0; k < bn; k++) {
         zt[k] = challenge_finish(hs.mid[i0 + k], cs[k]);
         zt[bn + k] = eval_tinv(zt[k], logn, &any_in_domain);
     }
-    Fr* d_z = (Fr*)L.small.p;  // [z x bn | tinv x bn | y x bn]
-    CK(c, cudaMemcpyAsync(d_z, zt.data(), 2 * bn * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
-    eval_quotient_launch((Fr*)L.evals.p, (uint32_t)n, logn, (uint32_t)bn, d_z, d_z + bn, c->tw.get(), c->logN, &ninv,
-                         (Fr*)L.eval_scratch.p, (Fr*)L.work.p, d_z + 2 * bn, L.st, !any_in_domain);
+    CK(c, cudaMemcpyAsync(L.small.p, zt.data(), 2 * bn * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+    *outside = !any_in_domain;
+    return KZGB_OK;
+}
+
+// The points of a group of proofs at the caller's points, entries i0 .. i0 + bn - 1: the caller's z up to L.small, then
+// their tinv and in-domain flags on the device (eval_points_launch), laid out as group_prove reads them; the flags follow
+// the y.
+int group_points_at(const Batch& b, Lane& L, size_t i0, size_t bn, const uint32_t** in_domain) {
+    kzgb_ctx* c = b.c;
+    const int logn = log2_exact(b.ns[i0]);
+    CK(c, L.small.reserve((4 * bn + 8) * sizeof(Fr)));
+    Fr* d_z = (Fr*)L.small.p;
+    uint32_t* d_flags = (uint32_t*)(d_z + 3 * bn);
+    CK(c, cudaMemcpyAsync(d_z, b.zs_mont + 4 * i0, bn * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+    const Fr ninv = ninv_mont(logn);
+    eval_points_launch(d_z, logn, (uint32_t)bn, &ninv, d_z + bn, d_flags, L.st);
+    *in_domain = d_flags;
+    return KZGB_OK;
+}
+
+// The evaluations of the polynomials i0 .. i0 + bn - 1 of a ProveAt group (all of n elements) back to back on the device:
+// device polynomials that already are back to back are read in place, the others are gathered into L.evals, one copy per
+// run of polynomials that are adjacent in the caller's memory.
+int group_evals(const Batch& b, Lane& L, size_t i0, size_t bn, const Fr** evals) {
+    kzgb_ctx* c = b.c;
+    const uint64_t* const* src = b.evals + i0;
+    const size_t n = b.ns[i0];
+    size_t run = 1;
+    while (run < bn && src[run] == src[0] + run * 4 * n) run++;
+    if (b.evals_on_device && run == bn) { *evals = (const Fr*)src[0]; return KZGB_OK; }
+    CK(c, L.evals.reserve(bn * n * sizeof(Fr)));
+    const cudaMemcpyKind kind = b.evals_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    for (size_t k = 0; k < bn; k += run) {
+        run = 1;
+        while (k + run < bn && src[k + run] == src[k] + run * 4 * n) run++;
+        CK(c, cudaMemcpyAsync((Fr*)L.evals.p + k * n, src[k], run * n * sizeof(Fr), kind, L.st));
+    }
+    *evals = (const Fr*)L.evals.p;
+    return KZGB_OK;
+}
+
+// The proof phase of one group of bn polynomials of n = blob_poly_len(lens[i0]) evaluations at `evals` (stride n, on the
+// device) whose points are in L.small: [z x bn | tinv x bn | y x bn].  ONE batched evaluation / quotient launch set with a
+// point per polynomial (outside and in_domain as eval_quotient_launch takes them) and ONE batched MSM of the quotients;
+// pts[k] is the proof of polynomial i0 + k.  ys (optional, host) receives the bn y.
+int group_prove(const Batch& b, Lane& L, const Fr* evals, size_t i0, size_t bn, bool outside, const uint32_t* in_domain,
+                uint64_t* ys, Affine* pts) {
+    kzgb_ctx* c = b.c;
+    const size_t n = blob_poly_len(b.lens[i0]);
+    const int logn = log2_exact(n);
+    const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
+    Fr ninv = ninv_mont(logn);
+    CK(c, L.eval_scratch.reserve(eval_quotient_scratch_elems((uint32_t)n, (uint32_t)bn) * sizeof(Fr)));
+    CK(c, L.work.reserve(bn * n * sizeof(Fr)));
+    if (!lag) CK(c, L.ntt_scratch.reserve(bn * n * sizeof(Fr)));
+    Fr* d_z = (Fr*)L.small.p;
+    eval_quotient_launch(evals, (uint32_t)n, logn, (uint32_t)bn, d_z, d_z + bn, c->tw.get(), c->logN, &ninv,
+                         (Fr*)L.eval_scratch.p, (Fr*)L.work.p, d_z + 2 * bn, L.st, outside, in_domain);
     if (!lag) ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
     MsmJob job;
     int r = msm_enqueue(c, L, {(const Fr*)L.work.p}, n, bn, lag, nullptr, 0, &job);
+    if (!r && ys) CK(c, cudaMemcpyAsync(ys, d_z + 2 * bn, bn * sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
     if (!r) r = msm_finish(c, L, job, pts);
     return r;
 }
 
 // Small blobs: groups of equal-size blobs, each phase of a group is ONE batched launch set.  A commit-only group ends
 // with its commitment phase (no hashing stage: hs is null).  A proof-only group has no commitment phase: its blob bytes
-// (group_bytes) become Montgomery evaluations in one conversion launch and the commitments are the caller's.
+// (group_bytes) become Montgomery evaluations in one conversion launch and the commitments are the caller's.  A group of
+// proofs at the caller's points is its evaluations (group_evals) and its points (group_points_at), then the proof phase.
 int group_lane(const Batch& b, LaneSync& sync, HashStage* hs, std::atomic<size_t>& next_group, int li) {
     kzgb_ctx* c = b.c;
     Lane& L = c->lanes[li];
@@ -569,6 +648,17 @@ int group_lane(const Batch& b, LaneSync& sync, HashStage* hs, std::atomic<size_t
         const size_t n = blob_poly_len(b.lens[i0]);
         int r = KZGB_OK;
         const Affine* cs = nullptr;
+        if (b.job == Job::ProveAt) {
+            const Fr* evals = nullptr;
+            const uint32_t* in_domain = nullptr;
+            pts.resize(bn);
+            r = group_evals(b, L, i0, bn, &evals);
+            if (!r) r = group_points_at(b, L, i0, bn, &in_domain);
+            if (!r) r = group_prove(b, L, evals, i0, bn, false, in_domain, b.ys_mont ? b.ys_mont + 4 * i0 : nullptr, pts.data());
+            if (!r) for (size_t k = 0; k < bn; k++) put_proof(b, i0 + k, pts[k]);
+            if (r) { sync.fail(); return r; }
+            continue;
+        }
         if (b.job == Job::Prove) {
             const uint8_t* src = nullptr;
             r = group_bytes(b, L, i0, bn, &src);
@@ -584,7 +674,9 @@ int group_lane(const Batch& b, LaneSync& sync, HashStage* hs, std::atomic<size_t
         if (!r && b.job != Job::Commit) {
             if (!hs->wait_ready(i0, bn)) return KZGB_OK;  // the transcript midstates come from the hashing stage
             pts.resize(bn);
-            r = group_prove(b, *hs, L, i0, bn, cs, pts.data());
+            bool outside = false;
+            r = group_challenges(b, *hs, L, i0, bn, cs, &outside);
+            if (!r) r = group_prove(b, L, (const Fr*)L.evals.p, i0, bn, outside, nullptr, nullptr, pts.data());
             if (!r) for (size_t k = 0; k < bn; k++) put_proof(b, i0 + k, pts[k]);
         }
         if (r) { sync.fail(); return r; }
@@ -726,10 +818,42 @@ int prove_task_lane(const Batch& b, HashStage& hs, std::atomic<size_t>& next, in
     }
 }
 
+// Large polynomials, and batches without groups, of proofs at the caller's points: every task is "prove polynomial i",
+// taken in index order.  The quotient is taken on the caller's device polynomial, or on a copy in the lane's own buffer,
+// and y is read as kzgb_compute_proof reads it.
+int prove_at_task_lane(const Batch& b, LaneSync& sync, std::atomic<size_t>& next, int li) {
+    kzgb_ctx* c = b.c;
+    Lane& L = c->lanes[li];
+    auto prove = [&](size_t i, Affine* out) {
+        const size_t n = b.ns[i];
+        const Fr* evals = (const Fr*)b.evals[i];
+        if (!b.evals_on_device) {
+            CK(c, L.evals.reserve(n * sizeof(Fr)));
+            CK(c, cudaMemcpyAsync(L.evals.p, b.evals[i], n * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+            evals = (const Fr*)L.evals.p;
+        }
+        Fr z;
+        memcpy(z.l, b.zs_mont + 4 * i, 32);
+        MsmJob job;
+        if (int rc = proof_enqueue(c, L, evals, n, z, &job)) return rc;
+        if (b.ys_mont) CK(c, cudaMemcpyAsync(&L.h_fr[3], (Fr*)L.small.p + 2, sizeof(Fr), cudaMemcpyDeviceToHost, L.st));
+        if (int rc = msm_finish(c, L, job, out)) return rc;
+        if (b.ys_mont) memcpy(b.ys_mont + 4 * i, &L.h_fr[3], 32);
+        return (int)KZGB_OK;
+    };
+    for (;;) {
+        const size_t i = next.fetch_add(1);
+        if (i >= b.count || sync.failed.load()) return KZGB_OK;
+        Affine out;
+        if (int r = prove(i, &out)) { sync.fail(); return r; }
+        put_proof(b, i, out);
+    }
+}
+
 // ---------------------------------------------------------------- driver
-// The plan, then the lanes.  Commit has no transcripts: no staging, no hashing stage.  CommitAndProve stages host blobs
-// (stage_blob_bytes) and may hash on the device what is staged or the caller's; Prove stages host blobs only for the
-// device's share of the hashing.  Groups hash on the host pool alone.
+// The plan, then the lanes.  Commit and ProveAt have no transcripts: no staging, no hashing stage.  CommitAndProve stages
+// host blobs (stage_blob_bytes) and may hash on the device what is staged or the caller's; Prove stages host blobs only
+// for the device's share of the hashing.  Groups hash on the host pool alone.
 int run_batch(Batch& b) {
     if (b.count == 0) return KZGB_OK;
     int rc = plan_batch(b);
@@ -739,6 +863,10 @@ int run_batch(Batch& b) {
     if (b.job == Job::Commit)
         return run_lanes(b, [&](int li) {
             return b.groups.empty() ? commit_task_lane(b, sync, next, li) : group_lane(b, sync, nullptr, next, li);
+        });
+    if (b.job == Job::ProveAt)
+        return run_lanes(b, [&](int li) {
+            return b.groups.empty() ? prove_at_task_lane(b, sync, next, li) : group_lane(b, sync, nullptr, next, li);
         });
     HashPlan hplan;
     if (b.job == Job::CommitAndProve) {
@@ -1045,17 +1173,6 @@ int verify_batch_rlc(kzgb_ctx* c, const uint8_t* const* blobs_dev, const uint8_t
     });
 }
 
-// the 4 little-endian words at w hold a value below r
-bool fr_words_reduced(const uint64_t* w) {
-    uint32_t r[8];
-    FeConst<FR>::mod(r);
-    for (int k = 7; k >= 0; k--) {
-        const uint32_t x = (uint32_t)(w[k / 2] >> (32 * (k & 1)));
-        if (x != r[k]) return x < r[k];
-    }
-    return false;
-}
-
 // Every z_i and y_i of m openings is a reduced Montgomery value (< r, as an arkworks Fr always is: a larger word would be
 // hashed as other bytes than the reference hashes); else KZGB_ERR_INVALID_FIELD_ELEMENT for the first opening that is not.
 int check_openings_reduced(kzgb_ctx* c, size_t m, const uint64_t* zs_mont, const uint64_t* ys_mont) {
@@ -1113,6 +1230,23 @@ int verify_proofs(kzgb_ctx* c, size_t m, const uint64_t* commitments_xy, const u
     return pairing_finish(c, flags, ok);
 }
 
+// KZG::compute_proof (kzg.rs:128-178, 187-234) for `count` polynomials at the caller's points: the batch driver, with
+// polynomial i planned as a blob of 32 ns[i] bytes.  plan_batch checks ns[i] before that length is used.
+int compute_proofs(kzgb_ctx* c, const uint64_t* const* evals, bool on_device, const size_t* ns, size_t count,
+                   const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont) {
+    std::vector<size_t> lens(count);
+    for (size_t i = 0; i < count; i++) lens[i] = 32 * ns[i];
+    Batch b(c, Job::ProveAt, nullptr, nullptr, lens.data(), count);
+    b.evals = evals;
+    b.evals_on_device = on_device;
+    b.ns = ns;
+    b.zs_mont = zs_mont;
+    b.ys_mont = ys_mont;
+    b.out_xy = out_xy;
+    b.out_inf = out_inf;
+    return run_batch(b);
+}
+
 }  // namespace
 
 // =====================================================================================
@@ -1161,6 +1295,17 @@ int kzgb_compute_blob_proofs_dev(kzgb_ctx* c, const uint8_t* const* blobs_dev, c
     b.out_xy = out_xy;
     b.out_inf = out_inf;
     return run_batch(b);
+}
+// ------------------------------------------------------------------------------- proofs at the caller's points
+int kzgb_compute_proofs(kzgb_ctx* c, const uint64_t* const* evals_mont, const size_t* ns, size_t count,
+                        const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont) {
+    Guard g(c);
+    return compute_proofs(c, evals_mont, false, ns, count, zs_mont, out_xy, out_inf, ys_mont);
+}
+int kzgb_compute_proofs_dev(kzgb_ctx* c, const uint64_t* const* evals_dev, const size_t* ns, size_t count,
+                            const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont) {
+    Guard g(c);
+    return compute_proofs(c, evals_dev, true, ns, count, zs_mont, out_xy, out_inf, ys_mont);
 }
 // ------------------------------------------------------------------------------- per-blob verification, G1 side
 int kzgb_verify_blob_proofs_g1(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,

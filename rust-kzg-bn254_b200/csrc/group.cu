@@ -226,6 +226,21 @@ int kzgb_group_compute_blob_proofs(kzgb_group* g, const uint8_t* const* blobs, c
     });
 }
 
+// KZG::compute_proof (prover/src/kzg.rs:128-178, 187-234) for `count` polynomials at the caller's points, cut as
+// kzgb_group_commit_and_prove_blobs cuts a batch whose blob i has the 32 ns[i] bytes of polynomial i.
+int kzgb_group_compute_proofs(kzgb_group* g, const uint64_t* const* evals_mont, const size_t* ns, size_t count,
+                              const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    // the weights of the cut, before any member has checked ns[i]: capped at 32 * 2^31, so that a length no SRS holds
+    // (which its member rejects) cannot wrap the product or the cut's sum
+    std::vector<size_t> bytes(count);
+    for (size_t i = 0; i < count; i++) bytes[i] = 32 * std::min<size_t>(ns[i], (size_t)1 << 31);
+    return for_blob_shares(g, bytes.data(), count, [&](kzgb_ctx* c, size_t a, size_t n) {
+        return kzgb_compute_proofs(c, evals_mont + a, ns + a, n, zs_mont + 4 * a, out_xy + 8 * a, at_or_null(out_inf, a),
+                                   at_or_null(ys_mont, 4 * a));
+    });
+}
+
 // verify_blob_kzg_proof (verifier/src/verify.rs:77-115) up to the pairing for `count` blobs, cut as
 // kzgb_group_commit_and_prove_blobs cuts them.
 int kzgb_group_verify_blob_proofs_g1(kzgb_group* g, const uint8_t* const* blobs, const size_t* lens, size_t count,

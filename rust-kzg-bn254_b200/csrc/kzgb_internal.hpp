@@ -176,6 +176,11 @@ void eval_quotient_launch(const Fr* evals, uint32_t n, int logn, uint32_t batch,
 size_t eval_quotient_scratch_elems(uint32_t n, uint32_t batch);
 // 0: always the generic prefix/suffix-product inverses (tests compare the two forms)
 void eval_set_structured(int on);
+// For `batch` caller-given points z_mont_dev[k] (device, Montgomery) of polynomials of 2^logn evaluations: tinv_out[k] =
+// 1/(z^n - 1), or z/n when z^n == 1, and in_domain_out[k] = 1 exactly then -- the tinv and the in_domain_dev flags
+// eval_quotient_launch takes, with no inversion on the host.
+void eval_points_launch(const Fr* z_mont_dev, int logn, uint32_t batch, const Fr* ninv_mont_host, Fr* tinv_out,
+                        uint32_t* in_domain_out, cudaStream_t st);
 // Fiat-Shamir challenges of `batch` blobs of n evaluations each on the device (fs.cu; reference
 // primitives/src/helpers.rs:411-472): z_out[k] (Montgomery) and tinv_out[k] = 1/(z^n - 1) (or z/n in the
 // domain).  commit32_dev: batch x 32 bytes, arkworks-compressed commitments.

@@ -448,6 +448,23 @@ __global__ void __launch_bounds__(EVAL_THREADS) k_quotient_fix(uint32_t n, int l
     }
 }
 
+// The points of a batch of openings at caller-given z (kzgb_compute_proofs), one thread per opening: tinv_k = 1/(z^n - 1),
+// or z/n when z^n == 1 (eval_tinv's formula), and in_domain_k = 1 in that case.
+__global__ void __launch_bounds__(64) k_eval_points(const Fr* __restrict__ z_all, int logn, uint32_t batch, Fr ninv,
+                                                    Fr* __restrict__ tinv_out, uint32_t* __restrict__ in_domain_out) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= batch) return;
+    const Fr z = fe_load(&z_all[k]);
+    Fr zn = z, one, t;
+    for (int s = 0; s < logn; s++) fe_sqr(zn, zn);
+    fe_one(one);
+    const bool in_domain = fe_eq(zn, one);
+    if (in_domain) fe_mul(t, z, ninv);
+    else { fe_sub(zn, zn, one); fe_inv_fast(t, zn); }
+    fe_store(&tinv_out[k], t);
+    in_domain_out[k] = in_domain ? 1u : 0u;
+}
+
 __global__ void __launch_bounds__(256) k_fr_powers(Fr* __restrict__ out, uint32_t n, Fr base, uint32_t first) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -537,6 +554,13 @@ void eval_quotient_launch(const Fr* evals, uint32_t n, int logn, uint32_t batch,
         k_quotient_fix<<<batch, EVAL_THREADS, 0, st>>>(n, logn, tw, logN, partial2, parts2, zidx, q_out);
         g_launch_count += 2;
     }
+}
+
+void eval_points_launch(const Fr* z_mont_dev, int logn, uint32_t batch, const Fr* ninv_mont_host, Fr* tinv_out,
+                        uint32_t* in_domain_out, cudaStream_t st) {
+    if (!batch) return;
+    k_eval_points<<<(batch + 63) / 64, 64, 0, st>>>(z_mont_dev, logn, batch, *ninv_mont_host, tinv_out, in_domain_out);
+    g_launch_count++;
 }
 
 void fr_powers_launch(Fr* out, uint32_t n, const Fr* base_mont_host, cudaStream_t st, uint32_t first) {

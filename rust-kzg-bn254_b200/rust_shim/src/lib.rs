@@ -474,6 +474,49 @@ impl KZG {
         }
         Ok((0..blobs.len()).map(|i| unpack_point(xy[8 * i..8 * i + 8].try_into().unwrap(), inf[i])).collect())
     }
+    /// Addition next to the reference's API: `compute_proof` (prover/src/kzg.rs:128-178, 187-234) of polynomial i at
+    /// zs[i] for every i in ONE call, returning each proof with its value y_i = p_i(zs[i]) -- the openings a caller of
+    /// `compute_proof` or `compute_proof_with_known_z_fr_index` makes in a loop, and that `verify_proof` checks.  The
+    /// batch is cut by evaluation bytes across the GPUs of the box (`kzgb_group_compute_proofs`).  Entry i is
+    /// `compute_proof(polynomial i, zs[i])` without the per-instance roots-length check, which a batch of sizes has no use
+    /// for; an error is the one `compute_proof` reports for the first polynomial the library rejects.  Source only, like
+    /// the rest of this crate: it has not been compiled, because the build image has no Rust toolchain.
+    pub fn compute_proofs(&self, polynomials: &[PolynomialEvalForm], zs: &[Fr], srs: &SRS) -> Result<Vec<(G1Affine, Fr)>, KzgError> {
+        if polynomials.len() != zs.len() {
+            return Err(KzgError::GenericError("length's of the input are not the same".to_string()));
+        }
+        let m = polynomials.len();
+        let ptrs: Vec<*const u64> = polynomials.iter().map(|p| fr_words(p.evaluations())).collect();
+        let ns: Vec<usize> = polynomials.iter().map(|p| p.evaluations().len()).collect();
+        let mut xy = vec![0u64; 8 * m];
+        let mut inf = vec![0u8; m];
+        let mut ys = vec![0u64; 4 * m];
+        let gpu = gpu_for(srs)?;
+        let rc = unsafe {
+            ffi::kzgb_group_compute_proofs(gpu.group, ptrs.as_ptr(), ns.as_ptr(), m, fr_words(zs), xy.as_mut_ptr(),
+                                           inf.as_mut_ptr(), ys.as_mut_ptr())
+        };
+        if rc != 0 {
+            // the library fails on the lowest-index polynomial that does not pass compute_proof's checks (an Fr is always
+            // reduced, so its z passes); the group's message names the member, so the error is rebuilt from that polynomial
+            let srs_len = srs.g1.len();
+            for &polynomial_len in &ns {
+                if !polynomial_len.is_power_of_two() {
+                    return Err(KzgError::FFTError("length provided is not a power of 2".to_string()));
+                }
+                if polynomial_len > srs_len {
+                    return Err(KzgError::SrsCapacityExceeded { polynomial_len, srs_len });
+                }
+            }
+            return Err(group_err(gpu.group, rc));
+        }
+        Ok((0..m)
+            .map(|i| {
+                let y = Fr::new_unchecked(ark_ff::BigInt([ys[4 * i], ys[4 * i + 1], ys[4 * i + 2], ys[4 * i + 3]]));
+                (unpack_point(xy[8 * i..8 * i + 8].try_into().unwrap(), inf[i]), y)  // y: Montgomery limbs, as fr_words passes them
+            })
+            .collect())
+    }
 }
 
 impl KZG {
