@@ -150,6 +150,35 @@ int kzgb_to_byte_array(kzgb_ctx* ctx, const uint64_t* fr_mont, size_t n, uint8_t
 int kzgb_commit_eval(kzgb_ctx* ctx, const uint64_t* evals_mont, size_t n, uint64_t out_xy[8], uint8_t* out_inf);
 /* KZG::commit_coeff_form (kzg.rs:107-125).  Err KZGB_ERR_SERIALIZATION if n > srs_len. */
 int kzgb_commit_coeff(kzgb_ctx* ctx, const uint64_t* coeffs_mont, size_t n, uint64_t out_xy[8], uint8_t* out_inf);
+/* KZG::commit_eval_form (kzg.rs:84-104) for `count` polynomials in one pipelined call.  Polynomial i is ns[i] evaluations
+ * (Montgomery) at evals_mont[i], HOST memory.  out_xy: count x 8 words (x||y Montgomery); out_inf: count flags, may be NULL.
+ * Entry i is exactly what kzgb_commit_eval(evals_mont[i], ns[i], ...) returns.  Checks, entry by entry in index order, in
+ * kzgb_commit_eval's order: ns[i] <= srs_len (KZGB_ERR_SRS_CAPACITY), then ns[i] a power of two (KZGB_ERR_FFT "length
+ * provided is not a power of 2").  The error of the lowest failing entry is returned before any work starts and the outputs
+ * are left untouched.  The evaluation words are not validated, as in kzgb_commit_eval.  count == 0 writes nothing.
+ * Polynomials of up to 2^17 values are committed in groups of one size, whatever their order in the batch (one batched
+ * launch set per group); larger ones one per lane, as kzgb_commit_eval commits them. */
+int kzgb_commit_evals(kzgb_ctx* ctx, const uint64_t* const* evals_mont, const size_t* ns, size_t count,
+                      uint64_t* out_xy, uint8_t* out_inf);
+/* Same with the evaluations in device memory (evals_dev[i]: ns[i] x 4 words), read in place; the outputs and the checks as
+ * kzgb_commit_evals. */
+int kzgb_commit_evals_dev(kzgb_ctx* ctx, const uint64_t* const* evals_dev, const size_t* ns, size_t count,
+                          uint64_t* out_xy, uint8_t* out_inf);
+/* KZG::commit_coeff_form (kzg.rs:107-125) for `count` polynomials in one pipelined call.  Polynomial i is ns[i]
+ * coefficients (Montgomery) at coeffs_mont[i], HOST memory, of any length (no power of two needed; ns[i] == 0 commits to
+ * the identity).  out_xy / out_inf as kzgb_commit_evals.  Entry i is exactly what kzgb_commit_coeff(coeffs_mont[i], ns[i],
+ * ...) returns.  Check, entry by entry in index order: ns[i] <= srs_len, else KZGB_ERR_SERIALIZATION "polynomial length is
+ * not correct"; the lowest failing entry's error is returned before any work starts, outputs untouched.  The coefficient
+ * words are not validated, as in kzgb_commit_coeff.  count == 0 writes nothing.  Polynomials whose next power of two N is at
+ * most 2^17 and srs_len are committed in groups of one N (zero-padded to N): one batched MSM over the monomial window
+ * table, or one batched forward Fr NTT and one batched MSM over the Lagrange table of size N when that table is resident
+ * and has the narrower window; the others one per lane over SRS[0, ns[i]), as kzgb_commit_coeff commits them. */
+int kzgb_commit_coeffs(kzgb_ctx* ctx, const uint64_t* const* coeffs_mont, const size_t* ns, size_t count,
+                       uint64_t* out_xy, uint8_t* out_inf);
+/* Same with the coefficients in device memory (coeffs_dev[i]: ns[i] x 4 words), read in place; the outputs and the checks
+ * as kzgb_commit_coeffs. */
+int kzgb_commit_coeffs_dev(kzgb_ctx* ctx, const uint64_t* const* coeffs_dev, const size_t* ns, size_t count,
+                           uint64_t* out_xy, uint8_t* out_inf);
 /* KZG::commit_blob (kzg.rs:182-185): blob.data() bytes (32 B big-endian elements). */
 int kzgb_commit_blob(kzgb_ctx* ctx, const uint8_t* blob, size_t len, uint64_t out_xy[8], uint8_t* out_inf);
 /* KZG::g1_ifft (kzg.rs:263-285): Lagrange-basis SRS of size n (natural order).  Err KZGB_ERR_FFT if n is not 2^k. */
@@ -429,6 +458,14 @@ int kzgb_group_compute_blob_proofs(kzgb_group* group, const uint8_t* const* blob
  * before it starts (so on an error, members with valid shares may have written their outputs). */
 int kzgb_group_compute_proofs(kzgb_group* group, const uint64_t* const* evals_mont, const size_t* ns, size_t count,
                               const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont);
+/* kzgb_commit_evals (KZG::commit_eval_form, kzg.rs:84-104) and kzgb_commit_coeffs (KZG::commit_coeff_form, kzg.rs:107-125)
+ * cut into contiguous shares of about equal bytes (32 ns[i] per polynomial), one per member; identical to the one-context
+ * call.  Each member checks its own share before it starts (so on an error, members with valid shares may have written
+ * their outputs). */
+int kzgb_group_commit_evals(kzgb_group* group, const uint64_t* const* evals_mont, const size_t* ns, size_t count,
+                            uint64_t* out_xy, uint8_t* out_inf);
+int kzgb_group_commit_coeffs(kzgb_group* group, const uint64_t* const* coeffs_mont, const size_t* ns, size_t count,
+                             uint64_t* out_xy, uint8_t* out_inf);
 /* kzgb_verify_blob_proofs_g1 cut into contiguous shares of about equal bytes, one per member; identical to the one-context
  * call.  Each member checks its own share before it starts (so on an error, members with valid shares may have written
  * their outputs). */

@@ -123,6 +123,19 @@ def _compute_proofs(call, polynomials: Sequence["PolynomialEvalForm"], zs: Seque
     return g1_from_abi(xy.raw[: 64 * count], inf.raw[:count]), fr_from_mont_bytes(ys.raw[: 32 * count])
 
 
+def _commit_polys(call, values: Sequence[Sequence[int]]) -> List[Affine]:
+    """Runs call(value pointers, lengths, count, out_xy, out_inf) of a kzgb_*commit_evals / kzgb_*commit_coeffs entry
+    point on polynomials given by their values; returns the commitments."""
+    count = len(values)
+    keep = [C.create_string_buffer(fr_to_mont_bytes(v), max(32, 32 * len(v))) for v in values]
+    ptrs = (C.c_void_p * count)(*[C.cast(k, C.c_void_p).value for k in keep])
+    ns = (C.c_size_t * count)(*[len(v) for v in values])
+    xy = C.create_string_buffer(64 * count if count else 1)
+    inf = C.create_string_buffer(count if count else 1)
+    call(ptrs, ns, count, xy, inf)
+    return g1_from_abi(xy.raw[: 64 * count], inf.raw[:count])
+
+
 def _verify_blob_proofs(call, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]):
     """Runs call(blob pointers, lengths, count, commitments_xy, commitments_inf, proofs_xy, proofs_inf, out_xy, out_inf,
     z_out, y_out) of a kzgb_*verify_blob_proofs_g1 entry point; returns (C_i - [y_i] G1, z_i, y_i) for every blob."""
@@ -314,6 +327,14 @@ class Group:
     def compute_proofs(self, polynomials: Sequence["PolynomialEvalForm"], zs: Sequence[int]) -> Tuple[List[Affine], List[int]]:
         """KZG.compute_proofs with the batch cut by evaluation bytes across the members."""
         return _compute_proofs(lambda *a: self.check(lib.kzgb_group_compute_proofs(self.h, *a)), polynomials, zs)
+
+    def commit_eval_forms(self, polynomials: Sequence["PolynomialEvalForm"]) -> List[Affine]:
+        """KZG.commit_eval_forms with the batch cut by evaluation bytes across the members."""
+        return _commit_polys(lambda *a: self.check(lib.kzgb_group_commit_evals(self.h, *a)), [p.evaluations for p in polynomials])
+
+    def commit_coeff_forms(self, polynomials: Sequence["PolynomialCoeffForm"]) -> List[Affine]:
+        """KZG.commit_coeff_forms with the batch cut by coefficient bytes across the members."""
+        return _commit_polys(lambda *a: self.check(lib.kzgb_group_commit_coeffs(self.h, *a)), [p.coeffs for p in polynomials])
 
     def verify_blob_kzg_proofs_g1(
         self, blobs: Sequence["Blob"], commitments: Sequence[Affine], proofs: Sequence[Affine]
@@ -679,6 +700,20 @@ class KZG:
         e = srs.engine
         m = fr_to_mont_bytes(polynomial.coeffs)
         return e._point_call(lambda h, *a: lib.kzgb_commit_coeff(h, m, len(polynomial), *a))
+
+    @staticmethod
+    def commit_eval_forms(polynomials: Sequence[PolynomialEvalForm], srs: SRS) -> List[Affine]:
+        """commit_eval_form (kzg.rs:84-104) of every polynomial in one call, pipelined inside the library: entry i is what
+        commit_eval_form returns for polynomial i alone; the lowest failing entry's error is raised."""
+        e = srs.engine
+        return _commit_polys(lambda *a: e.check(lib.kzgb_commit_evals(e.h, *a)), [p.evaluations for p in polynomials])
+
+    @staticmethod
+    def commit_coeff_forms(polynomials: Sequence[PolynomialCoeffForm], srs: SRS) -> List[Affine]:
+        """commit_coeff_form (kzg.rs:107-125) of every polynomial in one call, pipelined inside the library: entry i is what
+        commit_coeff_form returns for polynomial i alone; the lowest failing entry's error is raised."""
+        e = srs.engine
+        return _commit_polys(lambda *a: e.check(lib.kzgb_commit_coeffs(e.h, *a)), [p.coeffs for p in polynomials])
 
     def commit_blob(self, blob: Blob, srs: SRS) -> Affine:
         """kzg.rs:182-185."""

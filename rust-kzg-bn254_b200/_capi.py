@@ -61,6 +61,10 @@ SIGNATURES = {
     "kzgb_compute_proofs_all_roots": (C.c_int, [ctx_p, buf, C.c_size_t, buf, buf]),
     "kzgb_compute_proofs": (C.c_int, [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf, buf]),
     "kzgb_compute_proofs_dev": (C.c_int, [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf, buf, buf]),
+    "kzgb_commit_evals": (C.c_int, [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf]),
+    "kzgb_commit_evals_dev": (C.c_int, [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf]),
+    "kzgb_commit_coeffs": (C.c_int, [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf]),
+    "kzgb_commit_coeffs_dev": (C.c_int, [ctx_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_size_t, buf, buf]),
     "kzgb_evaluate_polynomial": (C.c_int, [ctx_p, buf, C.c_size_t, buf, buf]),
     "kzgb_compute_challenge": (C.c_int, [ctx_p, buf, C.c_size_t, buf, C.c_uint8, buf]),
     "kzgb_compute_blob_proof": (C.c_int, [ctx_p, buf, C.c_size_t, buf, C.c_uint8, buf, u8p]),
@@ -147,6 +151,8 @@ SIGNATURES = {
     "kzgb_group_commit_blobs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf]),
     "kzgb_group_compute_blob_proofs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf]),
     "kzgb_group_compute_proofs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf]),
+    "kzgb_group_commit_evals": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf]),
+    "kzgb_group_commit_coeffs": (C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf]),
     "kzgb_group_verify_blob_proofs_g1": (
         C.c_int, [grp_p, C.c_void_p, C.c_void_p, C.c_size_t, buf, buf, buf, buf, buf, buf, buf, buf]
     ),

@@ -121,8 +121,10 @@ HashPlan hash_plan(const size_t* lens, size_t count, bool device_possible, bool 
 // ---------------------------------------------------------------- planning
 // What a batch computes: kzgb_commit_and_prove_blobs{,_dev}, kzgb_commit_blobs{,_dev} (commitments, no transcripts),
 // kzgb_compute_blob_proofs{,_dev} (proofs against the caller's commitments, no commit phase) or kzgb_compute_proofs{,_dev}
-// (proofs of the caller's Montgomery evaluations at the caller's points: no blob bytes, no transcripts, no commitments).
-enum class Job { CommitAndProve, Commit, Prove, ProveAt };
+// (proofs of the caller's Montgomery evaluations at the caller's points: no blob bytes, no transcripts, no commitments) or
+// kzgb_commit_evals{,_dev} / kzgb_commit_coeffs{,_dev} (commitments of the caller's polynomials, in evaluation or
+// coefficient form: no blob bytes, no transcripts, no proofs).
+enum class Job { CommitAndProve, Commit, Prove, ProveAt, CommitPolys };
 
 // One batch call: its arguments and the plan made for them.  The entry points set their job's outputs by name.
 struct Batch {
@@ -150,6 +152,13 @@ struct Batch {
     const size_t* ns = nullptr;
     const uint64_t* zs_mont = nullptr;
     uint64_t* ys_mont = nullptr;
+    // CommitPolys: polynomial i is ns[i] Montgomery values at evals[i] (as ProveAt), coefficients when `coeff`, and
+    // lens[i] = 32 N_i for its domain N_i (ns[i], or next_pow2(ns[i]) for coefficients).  plan_batch sorts the entries
+    // stably by N_i: from then on evals, ns and lens are in that order, and entry k of the batch is the caller's order[k].
+    bool coeff = false;
+    std::vector<size_t> order;
+    std::vector<const uint64_t*> sorted_evals;
+    std::vector<size_t> sorted_ns, sorted_lens;
     size_t max_n = 0;
     std::vector<std::pair<size_t, size_t>> groups;  // small blobs: (first blob, blobs); empty: one blob per task
     int n_lanes = 0;
@@ -172,13 +181,22 @@ bool fr_words_reduced(const uint64_t* w) {
 // Validation, groups, lanes and the tables every size of the batch needs.  A commit-only batch checks every blob as
 // kzgb_commit_blob does (a blob of length 0 commits the zero polynomial of size 1); with proofs, length 0 is
 // compute_blob_proof's error, and a proof-only batch checks each commitment first, as kzgb_compute_blob_proof does.
-// Proofs at the caller's points check each polynomial as kzgb_compute_proof does, then its z.
+// Proofs at the caller's points check each polynomial as kzgb_compute_proof does, then its z.  Commitments of the
+// caller's polynomials check each one as kzgb_commit_eval or kzgb_commit_coeff does.
 int plan_batch(Batch& b) {
     kzgb_ctx* c = b.c;
     const size_t* lens = b.lens;
     const size_t count = b.count;
     for (size_t i = 0; i < count; i++) {
-        if (b.job == Job::ProveAt) {
+        if (b.job == Job::CommitPolys) {
+            const size_t n = b.ns[i];
+            if (b.coeff) {
+                if (n > c->srs_n) return fail(c, KZGB_ERR_SERIALIZATION, "polynomial length is not correct");
+            } else {
+                if (int rc = check_srs_capacity(c, n)) return rc;
+                if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_FFT, "length provided is not a power of 2");
+            }
+        } else if (b.job == Job::ProveAt) {
             const size_t n = b.ns[i];
             if (n == 0 || (n & (n - 1))) return fail(c, KZGB_ERR_FFT, "length provided is not a power of 2");
             if (int rc = check_srs_capacity(c, n)) return rc;
@@ -195,6 +213,22 @@ int plan_batch(Batch& b) {
             if (int rc = check_srs_capacity(c, blob_poly_len(lens[i]))) return rc;
         }
         b.max_n = std::max(b.max_n, blob_poly_len(lens[i]));
+    }
+    // A commitment batch gathers every polynomial of a group anyway (group_evals), so its groups are cut from the entries
+    // sorted by size rather than from adjacent runs: polynomials of mixed sizes in any order still form full groups, and
+    // device polynomials of one size that are back to back stay so.
+    if (b.job == Job::CommitPolys) {
+        b.order.resize(count);
+        for (size_t i = 0; i < count; i++) b.order[i] = i;
+        std::stable_sort(b.order.begin(), b.order.end(), [&](size_t x, size_t y) { return b.lens[x] < b.lens[y]; });
+        for (size_t k = 0; k < count; k++) {
+            b.sorted_evals.push_back(b.evals[b.order[k]]);
+            b.sorted_ns.push_back(b.ns[b.order[k]]);
+            b.sorted_lens.push_back(b.lens[b.order[k]]);
+        }
+        b.evals = b.sorted_evals.data();
+        b.ns = b.sorted_ns.data();
+        b.lens = lens = b.sorted_lens.data();
     }
     // Small blobs (<= 2^17 Fr): runs of equal-size blobs are processed as groups, every kernel of a phase
     // launched ONCE for the whole group (batched conversion, evaluation/quotient and MSM with one bucket set
@@ -235,7 +269,8 @@ int plan_batch(Batch& b) {
         if (rc) return rc;
         if (!lagrange_table(c, logn)) all_lagrange = false;
     }
-    rc = all_lagrange ? KZGB_OK : ensure_window_table(c, 0, b.max_n);  // built here: the lanes only read the tables
+    // built here: the lanes only read the tables (coefficient tasks always run over the monomial one)
+    rc = all_lagrange && !b.coeff ? KZGB_OK : ensure_window_table(c, 0, std::min(b.max_n, c->srs_n));
     if (rc) return rc;
     for (size_t gi = 0; gi < b.groups.size(); gi++) {  // the batched MSM needs a window table for every size
         size_t n = blob_poly_len(lens[b.groups[gi].first]);
@@ -465,8 +500,10 @@ int run_lanes(const Batch& b, F lane_main) {
     return KZGB_OK;
 }
 
-// Where commitment i and proof i go: arkworks-compressed bytes (CommitAndProve), or the affine ABI (Commit, Prove).
+// Where commitment i and proof i go: arkworks-compressed bytes (CommitAndProve), or the affine ABI (the other jobs); the
+// commitment of a CommitPolys entry goes to the caller's index of it.
 void put_commitment(const Batch& b, size_t i, const Affine& p) {
+    if (!b.order.empty()) i = b.order[i];
     if (b.job == Job::CommitAndProve) serialize_compressed(p, b.commitments32 + 32 * i);
     else affine_to_abi(p, b.out_xy + 8 * i, b.out_inf ? b.out_inf + i : nullptr);
 }
@@ -516,7 +553,6 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
         if (!r) r = msm_finish(c, L, job, pts);
         return r;
     }
-    Fr ninv = ninv_mont(logn);
     int r = KZGB_OK;
     auto ck = [&](cudaError_t e, const char* what) {
         if (!r && e != cudaSuccess) r = fail(c, KZGB_ERR_DEVICE, std::string("CUDA error: ") + cudaGetErrorString(e) + " at " + what);
@@ -526,8 +562,6 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
     bool dev_run = blobs_dev && full;  // device blobs back to back: one conversion launch too
     for (size_t k = 0; k < bn && dev_run; k++) dev_run = blobs_dev[i0 + k] == blobs_dev[i0] + k * n * 32;
     ck(L.evals.reserve(bn * n * sizeof(Fr)), "evals");
-    ck(L.work.reserve(bn * n * sizeof(Fr)), "work");
-    if (!lag) ck(L.ntt_scratch.reserve(bn * n * sizeof(Fr)), "ntt scratch");
     if (!blobs_dev) ck(L.bytes.reserve(bn * n * 32), "bytes");
     if (dev_run) bytes_to_fr_launch(blobs_dev[i0], (uint64_t)bn * n * 32, (Fr*)L.evals.p, (uint32_t)(bn * n), L.st);
     for (size_t k = 0; k < bn && !r && !dev_run; k++) {
@@ -540,15 +574,7 @@ int group_commit(const Batch& b, Lane& L, size_t i0, size_t bn, Affine* pts) {
         if (!full || blobs_dev) bytes_to_fr_launch(src, lens[i0 + k], (Fr*)L.evals.p + k * n, (uint32_t)n, L.st);
     }
     if (!r && full && !blobs_dev) bytes_to_fr_launch((const uint8_t*)L.bytes.p, (uint64_t)bn * n * 32, (Fr*)L.evals.p, (uint32_t)(bn * n), L.st);
-    if (!r) {
-        const Fr* sc = (const Fr*)L.evals.p;
-        if (!lag) {
-            ck(cudaMemcpyAsync(L.work.p, L.evals.p, bn * n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st), "copy");
-            ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, true, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-            sc = (const Fr*)L.work.p;
-        }
-        if (!r) r = msm_enqueue(c, L, {sc}, n, bn, lag, nullptr, 0, &job);
-    }
+    if (!r) r = commit_evals_enqueue(c, L, (const Fr*)L.evals.p, n, &job, bn);
     if (!r) r = msm_finish(c, L, job, pts);
     return r;
 }
@@ -587,25 +613,63 @@ int group_points_at(const Batch& b, Lane& L, size_t i0, size_t bn, const uint32_
     return KZGB_OK;
 }
 
-// The evaluations of the polynomials i0 .. i0 + bn - 1 of a ProveAt group (all of n elements) back to back on the device:
-// device polynomials that already are back to back are read in place, the others are gathered into L.evals, one copy per
-// run of polynomials that are adjacent in the caller's memory.
+// The values of the polynomials i0 .. i0 + bn - 1 of a ProveAt or CommitPolys group (domain n = blob_poly_len(lens[i0]))
+// back to back on the device at a stride of n, zero-filled past ns[i]: device polynomials of n values that already are
+// back to back are read in place, the others are gathered into L.evals, one copy per run of polynomials of n values that
+// are adjacent in the caller's memory.
 int group_evals(const Batch& b, Lane& L, size_t i0, size_t bn, const Fr** evals) {
     kzgb_ctx* c = b.c;
     const uint64_t* const* src = b.evals + i0;
-    const size_t n = b.ns[i0];
+    const size_t* ns = b.ns + i0;
+    const size_t n = blob_poly_len(b.lens[i0]);
+    auto adjacent = [&](size_t k, size_t run) { return ns[k] == n && ns[k + run] == n && src[k + run] == src[k] + run * 4 * n; };
     size_t run = 1;
-    while (run < bn && src[run] == src[0] + run * 4 * n) run++;
-    if (b.evals_on_device && run == bn) { *evals = (const Fr*)src[0]; return KZGB_OK; }
+    while (run < bn && adjacent(0, run)) run++;
+    if (b.evals_on_device && run == bn && ns[0] == n) { *evals = (const Fr*)src[0]; return KZGB_OK; }
     CK(c, L.evals.reserve(bn * n * sizeof(Fr)));
     const cudaMemcpyKind kind = b.evals_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     for (size_t k = 0; k < bn; k += run) {
         run = 1;
-        while (k + run < bn && src[k + run] == src[k] + run * 4 * n) run++;
-        CK(c, cudaMemcpyAsync((Fr*)L.evals.p + k * n, src[k], run * n * sizeof(Fr), kind, L.st));
+        while (k + run < bn && adjacent(k, run)) run++;
+        Fr* dst = (Fr*)L.evals.p + k * n;
+        const size_t len = run > 1 ? run * n : ns[k];
+        if (len) CK(c, cudaMemcpyAsync(dst, src[k], len * sizeof(Fr), kind, L.st));
+        if (len < n) CK(c, cudaMemsetAsync(dst + len, 0, (n - len) * sizeof(Fr), L.st));  // zero coefficients add nothing
     }
     *evals = (const Fr*)L.evals.p;
     return KZGB_OK;
+}
+
+// The commitments of a CommitPolys group of bn polynomials of domain n at `values` (stride n, on the device), ONE batched
+// launch set.  Evaluations: commit_evals_enqueue.  Coefficients: the scalars of one batched MSM over the monomial window
+// table when its window is no wider than that of the Lagrange table of size n, or there is no such table (plan_batch made
+// sure a monomial table covers n); else one batched forward Fr NTT into L.work and one batched MSM over the Lagrange table
+// (sum c_i [tau^i]G = sum p(w^j) L_j).  A batched plan carries one bucket set of 2^(c-1) buckets per polynomial: a Lagrange
+// table has the window of its own size (choose_c_fixed(n)), the monomial table that of the largest polynomial it was built
+// for.  Measured on 2048 polynomials of 2^9 .. 2^12 coefficients (DESIGN.md section 4): at equal windows the monomial MSM
+// is 0-5 % faster (no transform); with a 2^19 table resident (c = 17) it is 4-10x slower.
+int group_commit_polys(const Batch& b, Lane& L, const Fr* values, size_t n, size_t bn, Affine* pts) {
+    kzgb_ctx* c = b.c;
+    const int logn = log2_exact(n);
+    const kzgb_ctx::LagTable* lag = lagrange_table(c, logn);
+    MsmJob job;
+    int r = KZGB_OK;
+    if (b.coeff && (!lag || (wtable_covers(c, 0, n) && c->wt_c <= lag->c))) {
+        r = msm_enqueue(c, L, {values}, n, bn, nullptr, nullptr, 0, &job);
+    } else {
+        if (b.coeff) {
+            CK(c, L.work.reserve(bn * n * sizeof(Fr)));
+            CK(c, L.ntt_scratch.reserve(bn * n * sizeof(Fr)));
+            if ((const void*)values != L.work.p)
+                CK(c, cudaMemcpyAsync(L.work.p, values, bn * n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st));
+            const Fr ninv = ninv_mont(logn);  // read by the inverse transform only
+            ntt_launch((Fr*)L.work.p, logn, (uint32_t)bn, false, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+            values = (const Fr*)L.work.p;
+        }
+        r = commit_evals_enqueue(c, L, values, n, &job, bn);
+    }
+    if (!r) r = msm_finish(c, L, job, pts);
+    return r;
 }
 
 // The proof phase of one group of bn polynomials of n = blob_poly_len(lens[i0]) evaluations at `evals` (stride n, on the
@@ -648,6 +712,15 @@ int group_lane(const Batch& b, LaneSync& sync, HashStage* hs, std::atomic<size_t
         const size_t n = blob_poly_len(b.lens[i0]);
         int r = KZGB_OK;
         const Affine* cs = nullptr;
+        if (b.job == Job::CommitPolys) {
+            const Fr* values = nullptr;
+            commits.resize(bn);
+            r = group_evals(b, L, i0, bn, &values);
+            if (!r) r = group_commit_polys(b, L, values, n, bn, commits.data());
+            if (!r) for (size_t k = 0; k < bn; k++) put_commitment(b, i0 + k, commits[k]);
+            if (r) { sync.fail(); return r; }
+            continue;
+        }
         if (b.job == Job::ProveAt) {
             const Fr* evals = nullptr;
             const uint32_t* in_domain = nullptr;
@@ -850,8 +923,36 @@ int prove_at_task_lane(const Batch& b, LaneSync& sync, std::atomic<size_t>& next
     }
 }
 
+// Large polynomials, and batches without groups, of commitments to the caller's polynomials: every task is "commit entry
+// k", taken in the batch's order.  Host values go up on the lane's stream into its own buffer; device values are read in
+// place.  Evaluations are committed as kzgb_commit_eval commits them (commit_evals_enqueue), coefficients by one MSM over
+// SRS[0, ns), as kzgb_commit_coeff does (no pipelined upload: its copy stream belongs to the context, not to a lane).
+int commit_polys_task_lane(const Batch& b, LaneSync& sync, std::atomic<size_t>& next, int li) {
+    kzgb_ctx* c = b.c;
+    Lane& L = c->lanes[li];
+    auto commit = [&](size_t k, Affine* out) {
+        const size_t n = b.ns[k];
+        const Fr* values = (const Fr*)b.evals[k];
+        if (!b.evals_on_device && n) {  // into L.work, where commit_evals_enqueue transforms without a copy
+            CK(c, L.work.reserve(n * sizeof(Fr)));
+            CK(c, cudaMemcpyAsync(L.work.p, b.evals[k], n * sizeof(Fr), cudaMemcpyHostToDevice, L.st));
+            values = (const Fr*)L.work.p;
+        }
+        MsmJob job;
+        int rc = b.coeff ? msm_enqueue(c, L, {values}, n, 1, nullptr, nullptr, 0, &job) : commit_evals_enqueue(c, L, values, n, &job);
+        return rc ? rc : msm_finish(c, L, job, out);
+    };
+    for (;;) {
+        const size_t k = next.fetch_add(1);
+        if (k >= b.count || sync.failed.load()) return KZGB_OK;
+        Affine out;
+        if (int r = commit(k, &out)) { sync.fail(); return r; }
+        put_commitment(b, k, out);
+    }
+}
+
 // ---------------------------------------------------------------- driver
-// The plan, then the lanes.  Commit and ProveAt have no transcripts: no staging, no hashing stage.  CommitAndProve stages
+// The plan, then the lanes.  Commit, ProveAt and CommitPolys have no transcripts: no staging, no hashing stage.  CommitAndProve stages
 // host blobs (stage_blob_bytes) and may hash on the device what is staged or the caller's; Prove stages host blobs only
 // for the device's share of the hashing.  Groups hash on the host pool alone.
 int run_batch(Batch& b) {
@@ -867,6 +968,10 @@ int run_batch(Batch& b) {
     if (b.job == Job::ProveAt)
         return run_lanes(b, [&](int li) {
             return b.groups.empty() ? prove_at_task_lane(b, sync, next, li) : group_lane(b, sync, nullptr, next, li);
+        });
+    if (b.job == Job::CommitPolys)
+        return run_lanes(b, [&](int li) {
+            return b.groups.empty() ? commit_polys_task_lane(b, sync, next, li) : group_lane(b, sync, nullptr, next, li);
         });
     HashPlan hplan;
     if (b.job == Job::CommitAndProve) {
@@ -1247,6 +1352,23 @@ int compute_proofs(kzgb_ctx* c, const uint64_t* const* evals, bool on_device, co
     return run_batch(b);
 }
 
+// KZG::commit_eval_form / commit_coeff_form (kzg.rs:84-104, 107-125) for `count` polynomials: the batch driver, with
+// polynomial i planned as a blob of 32 N_i bytes.  A length no SRS holds is planned as 0 bytes; plan_batch rejects it
+// before that length is used.
+int commit_polys(kzgb_ctx* c, bool coeff, const uint64_t* const* values, bool on_device, const size_t* ns, size_t count,
+                 uint64_t* out_xy, uint8_t* out_inf) {
+    std::vector<size_t> lens(count);
+    for (size_t i = 0; i < count; i++) lens[i] = ns[i] <= c->srs_n ? 32 * next_pow2(ns[i]) : 0;
+    Batch b(c, Job::CommitPolys, nullptr, nullptr, lens.data(), count);
+    b.coeff = coeff;
+    b.evals = values;
+    b.evals_on_device = on_device;
+    b.ns = ns;
+    b.out_xy = out_xy;
+    b.out_inf = out_inf;
+    return run_batch(b);
+}
+
 }  // namespace
 
 // =====================================================================================
@@ -1306,6 +1428,27 @@ int kzgb_compute_proofs_dev(kzgb_ctx* c, const uint64_t* const* evals_dev, const
                             const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont) {
     Guard g(c);
     return compute_proofs(c, evals_dev, true, ns, count, zs_mont, out_xy, out_inf, ys_mont);
+}
+// ------------------------------------------------------------------------------- commitments of the caller's polynomials
+int kzgb_commit_evals(kzgb_ctx* c, const uint64_t* const* evals_mont, const size_t* ns, size_t count, uint64_t* out_xy,
+                      uint8_t* out_inf) {
+    Guard g(c);
+    return commit_polys(c, false, evals_mont, false, ns, count, out_xy, out_inf);
+}
+int kzgb_commit_evals_dev(kzgb_ctx* c, const uint64_t* const* evals_dev, const size_t* ns, size_t count, uint64_t* out_xy,
+                          uint8_t* out_inf) {
+    Guard g(c);
+    return commit_polys(c, false, evals_dev, true, ns, count, out_xy, out_inf);
+}
+int kzgb_commit_coeffs(kzgb_ctx* c, const uint64_t* const* coeffs_mont, const size_t* ns, size_t count, uint64_t* out_xy,
+                       uint8_t* out_inf) {
+    Guard g(c);
+    return commit_polys(c, true, coeffs_mont, false, ns, count, out_xy, out_inf);
+}
+int kzgb_commit_coeffs_dev(kzgb_ctx* c, const uint64_t* const* coeffs_dev, const size_t* ns, size_t count, uint64_t* out_xy,
+                           uint8_t* out_inf) {
+    Guard g(c);
+    return commit_polys(c, true, coeffs_dev, true, ns, count, out_xy, out_inf);
 }
 // ------------------------------------------------------------------------------- per-blob verification, G1 side
 int kzgb_verify_blob_proofs_g1(kzgb_ctx* c, const uint8_t* const* blobs, const size_t* lens, size_t count,

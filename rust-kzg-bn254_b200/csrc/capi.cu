@@ -595,20 +595,20 @@ int msm_srs_host_pipelined(kzgb_ctx* c, Lane& L, const uint64_t* scalars, size_t
 }
 
 // ---------------------------------------------------------------- polynomial pipeline pieces
-// d_evals (n Fr, Montgomery) -> commitment.  Uses L.work / L.ntt_scratch.
-int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJob* job) {
+// d_evals (batch x n Fr, Montgomery) -> batch commitments.  Uses L.work / L.ntt_scratch.
+int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJob* job, size_t batch) {
     int logn = log2_exact(n);
     if (const kzgb_ctx::LagTable* lag = lagrange_table(c, logn))  // the evaluations ARE the scalars
-        return msm_enqueue(c, L, {d_evals}, n, 1, lag, nullptr, 0, job);
+        return msm_enqueue(c, L, {d_evals}, n, batch, lag, nullptr, 0, job);
     int rc = ensure_twiddles(c, logn);
     if (rc) return rc;
-    CK(c, L.work.reserve(n * sizeof(Fr)));
-    CK(c, L.ntt_scratch.reserve(n * sizeof(Fr)));
+    CK(c, L.work.reserve(batch * n * sizeof(Fr)));
+    CK(c, L.ntt_scratch.reserve(batch * n * sizeof(Fr)));
     if ((const void*)d_evals != L.work.p)
-        CK(c, cudaMemcpyAsync(L.work.p, d_evals, n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st));
+        CK(c, cudaMemcpyAsync(L.work.p, d_evals, batch * n * sizeof(Fr), cudaMemcpyDeviceToDevice, L.st));
     Fr ninv = ninv_mont(logn);
-    ntt_launch((Fr*)L.work.p, logn, 1, true, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
-    return msm_enqueue(c, L, {(Fr*)L.work.p}, n, 1, nullptr, nullptr, 0, job);
+    ntt_launch((Fr*)L.work.p, logn, (uint32_t)batch, true, c->tw.get(), c->logN, &ninv, (Fr*)L.ntt_scratch.p, L.st);
+    return msm_enqueue(c, L, {(Fr*)L.work.p}, n, batch, nullptr, nullptr, 0, job);
 }
 
 // y = p(z) into L.small[2] and, unless d_quotient is nullptr, the quotient; the twiddles of size n must be resident.

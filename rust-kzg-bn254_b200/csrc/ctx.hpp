@@ -231,7 +231,10 @@ int msm_enqueue(kzgb_ctx* c, Lane& L, const MsmScalars& scalars, size_t n, size_
                 const Affine* var_bases, size_t first, MsmJob* job);
 int msm_finish(kzgb_ctx* c, Lane& L, const MsmJob& job, Affine* outs);
 int msm_blocking(kzgb_ctx* c, Lane& L, const Fr* d_scalars, size_t first, size_t n, const Affine* var_bases, Affine* out);
-int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJob* job);
+// The commitments of `batch` evaluation-form polynomials of n values each at d_evals (stride n): one batched MSM over the
+// Lagrange table of size n when it is resident, else one batched Fr IFFT (in L.work) and one batched MSM over the
+// monomial window table.  d_evals is never written.
+int commit_evals_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, MsmJob* job, size_t batch = 1);
 int eval_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z, Fr* d_quotient);
 int eval_read_y(kzgb_ctx* c, Lane& L, Fr* y);
 int proof_enqueue(kzgb_ctx* c, Lane& L, const Fr* d_evals, size_t n, const Fr& z_mont, MsmJob* job);

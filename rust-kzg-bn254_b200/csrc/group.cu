@@ -85,6 +85,14 @@ int for_blob_shares(kzgb_group* g, const size_t* lens, size_t count, F fn) {
     });
 }
 
+// The weights of the cut of a batch of polynomials, 32 ns[i] bytes each, before any member has checked ns[i]: capped at
+// 32 * 2^31, so that a length no SRS holds (which its member rejects) cannot wrap the product or the cut's sum.
+std::vector<size_t> poly_bytes(const size_t* ns, size_t count) {
+    std::vector<size_t> bytes(count);
+    for (size_t i = 0; i < count; i++) bytes[i] = 32 * std::min<size_t>(ns[i], (size_t)1 << 31);
+    return bytes;
+}
+
 // p + off, or nullptr for an optional array the caller left out
 template <class T>
 T* at_or_null(T* p, size_t off) { return p ? p + off : nullptr; }
@@ -231,13 +239,30 @@ int kzgb_group_compute_blob_proofs(kzgb_group* g, const uint8_t* const* blobs, c
 int kzgb_group_compute_proofs(kzgb_group* g, const uint64_t* const* evals_mont, const size_t* ns, size_t count,
                               const uint64_t* zs_mont, uint64_t* out_xy, uint8_t* out_inf, uint64_t* ys_mont) {
     std::lock_guard<std::mutex> lk(g->mu);
-    // the weights of the cut, before any member has checked ns[i]: capped at 32 * 2^31, so that a length no SRS holds
-    // (which its member rejects) cannot wrap the product or the cut's sum
-    std::vector<size_t> bytes(count);
-    for (size_t i = 0; i < count; i++) bytes[i] = 32 * std::min<size_t>(ns[i], (size_t)1 << 31);
+    const std::vector<size_t> bytes = poly_bytes(ns, count);
     return for_blob_shares(g, bytes.data(), count, [&](kzgb_ctx* c, size_t a, size_t n) {
         return kzgb_compute_proofs(c, evals_mont + a, ns + a, n, zs_mont + 4 * a, out_xy + 8 * a, at_or_null(out_inf, a),
                                    at_or_null(ys_mont, 4 * a));
+    });
+}
+
+// KZG::commit_eval_form (prover/src/kzg.rs:84-104) for `count` polynomials, cut as kzgb_group_compute_proofs cuts them.
+int kzgb_group_commit_evals(kzgb_group* g, const uint64_t* const* evals_mont, const size_t* ns, size_t count,
+                            uint64_t* out_xy, uint8_t* out_inf) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    const std::vector<size_t> bytes = poly_bytes(ns, count);
+    return for_blob_shares(g, bytes.data(), count, [&](kzgb_ctx* c, size_t a, size_t n) {
+        return kzgb_commit_evals(c, evals_mont + a, ns + a, n, out_xy + 8 * a, at_or_null(out_inf, a));
+    });
+}
+
+// KZG::commit_coeff_form (prover/src/kzg.rs:107-125) for `count` polynomials, cut as kzgb_group_compute_proofs cuts them.
+int kzgb_group_commit_coeffs(kzgb_group* g, const uint64_t* const* coeffs_mont, const size_t* ns, size_t count,
+                             uint64_t* out_xy, uint8_t* out_inf) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    const std::vector<size_t> bytes = poly_bytes(ns, count);
+    return for_blob_shares(g, bytes.data(), count, [&](kzgb_ctx* c, size_t a, size_t n) {
+        return kzgb_commit_coeffs(c, coeffs_mont + a, ns + a, n, out_xy + 8 * a, at_or_null(out_inf, a));
     });
 }
 

@@ -80,6 +80,10 @@ extern "C" {
                                           out_inf: *mut u8) -> c_int;
     pub fn kzgb_group_compute_proofs(group: *mut kzgb_group, evals: *const *const u64, ns: *const usize, count: usize,
                                      zs_mont: *const u64, out_xy: *mut u64, out_inf: *mut u8, ys_mont: *mut u64) -> c_int;
+    pub fn kzgb_group_commit_evals(group: *mut kzgb_group, evals: *const *const u64, ns: *const usize, count: usize,
+                                   out_xy: *mut u64, out_inf: *mut u8) -> c_int;
+    pub fn kzgb_group_commit_coeffs(group: *mut kzgb_group, coeffs: *const *const u64, ns: *const usize, count: usize,
+                                    out_xy: *mut u64, out_inf: *mut u8) -> c_int;
     pub fn kzgb_group_verify_blob_proofs_g1(group: *mut kzgb_group, blobs: *const *const u8, lens: *const usize, count: usize,
                                             commitments_xy: *const u64, commitments_inf: *const u8, proofs_xy: *const u64,
                                             proofs_inf: *const u8, out_xy: *mut u64, out_inf: *mut u8, z_out: *mut u64,

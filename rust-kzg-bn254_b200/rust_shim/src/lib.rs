@@ -287,6 +287,25 @@ fn gpu_for(srs: &SRS) -> Result<Arc<Gpu>, KzgError> {
     Ok(gpu)
 }
 
+type GroupCommitFn = unsafe extern "C" fn(*mut ffi::kzgb_group, *const *const u64, *const usize, usize, *mut u64, *mut u8) -> std::os::raw::c_int;
+
+// One kzgb_group_commit_{evals,coeffs} call over the polynomials at ptrs (lengths ns).  The group's message names the member,
+// so on an error the reference's error is rebuilt from the lowest polynomial that `check(len, srs_len)` rejects.
+fn commit_polys(
+    call: GroupCommitFn, ptrs: &[*const u64], ns: &[usize], srs: &SRS, check: impl Fn(usize, usize) -> Option<KzgError>,
+) -> Result<Vec<G1Affine>, KzgError> {
+    let m = ptrs.len();
+    let mut xy = vec![0u64; 8 * m];
+    let mut inf = vec![0u8; m];
+    let gpu = gpu_for(srs)?;
+    let rc = unsafe { call(gpu.group, ptrs.as_ptr(), ns.as_ptr(), m, xy.as_mut_ptr(), inf.as_mut_ptr()) };
+    if rc != 0 {
+        let srs_len = srs.g1.len();
+        return Err(ns.iter().find_map(|&n| check(n, srs_len)).unwrap_or_else(|| group_err(gpu.group, rc)));
+    }
+    Ok((0..m).map(|i| unpack_point(xy[8 * i..8 * i + 8].try_into().unwrap(), inf[i])).collect())
+}
+
 /// Runs `f` on member 0's context of the SRS's group (single-polynomial entry points).
 fn with_ctx<T>(srs: &SRS, f: impl FnOnce(*mut ffi::kzgb_ctx) -> Result<T, KzgError>) -> Result<T, KzgError> {
     let gpu = gpu_for(srs)?;
@@ -516,6 +535,38 @@ impl KZG {
                 (unpack_point(xy[8 * i..8 * i + 8].try_into().unwrap(), inf[i]), y)  // y: Montgomery limbs, as fr_words passes them
             })
             .collect())
+    }
+    /// Addition next to the reference's API: `commit_eval_form` (prover/src/kzg.rs:84-104) of every polynomial in ONE
+    /// call.  The batch is cut by evaluation bytes across the GPUs of the box (`kzgb_group_commit_evals`) and pipelined on
+    /// each.  Point i is `commit_eval_form(polynomial i)`; an error is the one `commit_eval_form` reports for the first
+    /// polynomial the library rejects.  Source only, like the rest of this crate: it has not been compiled, because the
+    /// build image has no Rust toolchain.
+    pub fn commit_eval_forms(&self, polynomials: &[PolynomialEvalForm], srs: &SRS) -> Result<Vec<G1Affine>, KzgError> {
+        let ptrs: Vec<*const u64> = polynomials.iter().map(|p| fr_words(p.evaluations())).collect();
+        let ns: Vec<usize> = polynomials.iter().map(|p| p.evaluations().len()).collect();
+        commit_polys(ffi::kzgb_group_commit_evals, &ptrs, &ns, srs, |polynomial_len, srs_len| {
+            // commit_eval_form's order: SRS capacity (kzg.rs:89-94), then the power of two of its G1 IFFT (kzg.rs:265-269)
+            if polynomial_len > srs_len {
+                Some(KzgError::SrsCapacityExceeded { polynomial_len, srs_len })
+            } else if !polynomial_len.is_power_of_two() {
+                Some(KzgError::FFTError("length provided is not a power of 2".to_string()))
+            } else {
+                None
+            }
+        })
+    }
+    /// Addition next to the reference's API: `commit_coeff_form` (prover/src/kzg.rs:107-125) of every polynomial in ONE
+    /// call, for callers with many polynomials (the reference's own commit benchmark commits blobs of 10 000 to 50 000
+    /// bytes in coefficient form).  The batch is cut by coefficient bytes across the GPUs of the box
+    /// (`kzgb_group_commit_coeffs`).  Point i is `commit_coeff_form(polynomial i)`; an error is the one `commit_coeff_form`
+    /// reports for the first polynomial the library rejects.  Source only, not compiled (no Rust toolchain in the build
+    /// image).
+    pub fn commit_coeff_forms(&self, polynomials: &[PolynomialCoeffForm], srs: &SRS) -> Result<Vec<G1Affine>, KzgError> {
+        let ptrs: Vec<*const u64> = polynomials.iter().map(|p| fr_words(p.coeffs())).collect();
+        let ns: Vec<usize> = polynomials.iter().map(|p| p.coeffs().len()).collect();
+        commit_polys(ffi::kzgb_group_commit_coeffs, &ptrs, &ns, srs, |polynomial_len, srs_len| {
+            (polynomial_len > srs_len).then(|| KzgError::SerializationError("polynomial length is not correct".to_string()))
+        })
     }
 }
 
